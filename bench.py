@@ -2,7 +2,7 @@
 """bench.py -- headline benchmark of the DMesh tile rasterizer hot path on B200.
 
     python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload C4|C2|C1|C5]
-                    [--views-per-call V] [--no-per-config]
+                    [--views-per-call V] [--no-per-config] [--dump-outputs DIR]
 
 Metric (BASELINE.json): fwd+bwd throughput in views/s (and ms per 1024x1024 view) of the tri renderer, at
 1/2/4/8 B200, next to the reference CUDA extension on the same box.
@@ -25,6 +25,14 @@ of the reference arm when oracle/_ref cannot be loaded.
 
 At N = 1 both arms also time the other BASELINE configs at the `_C` level (`per_config`: C1, C2, C5 tri; C3 tet),
 so that every ours-vs-reference ratio quoted in README.md is a driver-run number.
+
+--dump-outputs DIR (our arm): after the timed steps, write what the last timed step computed for rank 0 -- the
+gradients the step leaves in the scene leaves (all-reduced) and in the per-call verts_depth / faces_intense leaves,
+and the colour and depth images of every call -- as DIR/<name>.npy (float32).  An array of more than DUMP_SAMPLE
+elements is stored as a fixed sample of it: the flattened array at sorted indices drawn by
+torch.randint(0, numel, (DUMP_SAMPLE,)) from a CPU generator seeded with 0.  The inputs are seeded, so two builds
+run with the same arguments can be compared output for output.  The last timed step keeps its images alive (about
+1 GB at C4 on one GPU) until they are written, so the timings of a dumping run are not the headline numbers.
 """
 import argparse
 import ctypes
@@ -44,6 +52,7 @@ import torch.distributed as dist  # noqa: E402
 METRIC = "tri_fwd_bwd_views_per_sec_1024x1024"
 UNIT = "views/s"
 TOTAL_VIEWS_C4 = 64
+DUMP_SAMPLE = 1 << 21     # elements kept per dumped array: 7 arrays x 8 MB stay under 64 MB
 
 
 # --------------------------------------------------------------------------- helpers
@@ -144,6 +153,19 @@ def bit_length(n):
     return max(int(n).bit_length(), 1)
 
 
+def dump_outputs(out_dir, arrays):
+    """Write each device tensor as out_dir/<name>.npy (float32): whole, or a flat seeded sample if it is large
+    (module doc)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_SAMPLE:
+            idx = torch.randint(0, t.numel(), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0))
+            t = t.reshape(-1)[idx.sort().values.to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
 # --------------------------------------------------------------------------- workload
 class Workload:
     """Scene replicated on every rank (device) + this rank's views split into calls + pinned host copies of the
@@ -220,14 +242,17 @@ def run_ours(args, ws, rank, local):
     tgt_c = [wl.host["target_color"][a:b].to(dev) for a, b in wl.calls]
     tgt_d = [wl.host["target_depth"][a:b].to(dev) for a, b in wl.calls]
     flush = L2Flush(dev)
+    images = [None] * len(wl.calls)     # --dump-outputs: the images of the last timed step, per call
 
-    def step_device():
+    def step_device(keep_images=False):
         leaves.zero_()
         with leaves.direct():   # backward kernels accumulate straight into the packed gradient buffer
             for i in range(len(wl.calls)):
                 vdep[i].grad = None
                 fint[i].grad = None
                 color, depth = renderer(verts, s.faces, vcol, fopa, mvs[i], pjs[i], vdep[i], fint[i])
+                if keep_images:
+                    images[i] = (color.detach(), depth.detach())
                 # gradient of the image loss 0.5 * ||render - target||^2 as cotangent (device resident targets)
                 torch.autograd.backward([color, depth], [color.detach() - tgt_c[i], depth.detach() - tgt_d[i]])
         leaves.all_reduce()
@@ -330,12 +355,12 @@ def run_ours(args, ws, rank, local):
         sampler.start()
     launches0 = lib.dmr_launch_count()
     total_ms = 0.0
-    for _ in range(args.steps):
+    for k in range(args.steps):
         flush()
         barrier(ws)
         a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         a.record()
-        step_device()
+        step_device(keep_images=bool(args.dump_outputs) and k == args.steps - 1)
         b.record()
         barrier(ws)
         total_ms += a.elapsed_time(b)
@@ -344,6 +369,11 @@ def run_ours(args, ws, rank, local):
     clocks = sampler.stop() if rank == 0 else None
     ms_per_step = total_ms / args.steps
     value = wl.total_views / (ms_per_step / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {
+            "grad_verts": verts.grad, "grad_verts_color": vcol.grad, "grad_faces_opacity": fopa.grad,
+            "grad_verts_depth": torch.cat([t.grad for t in vdep]), "grad_faces_intense": torch.cat([t.grad for t in fint]),
+            "color": torch.cat([c for c, _ in images]), "depth": torch.cat([d for _, d in images])})
 
     # ---- timed region 2: per-kernel durations (stage events inside the library, on the launching stream) for the
     #      roofline: one step, read after every call (a stage's events are overwritten by the next call)
@@ -726,7 +756,13 @@ def main():
     ap.add_argument("--views-per-call", type=int, default=8,
                     help="views rendered per renderer call (both arms; C4 only -- the other workloads have one view per rank)")
     ap.add_argument("--no-per-config", action="store_true", help="skip the C1/C2/C3/C5 `_C`-level timings (N = 1 only)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (our arm; see the module doc)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of our arm only")
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device (B200); there is no CPU fallback")
     ws, rank, local = dist_setup(args.gpus)

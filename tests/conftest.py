@@ -13,6 +13,14 @@ def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
 
 
+def pytest_report_header(config):
+    import ref_harness
+    if ref_harness.ref_module() is not None:
+        return "parity reference: the reference CUDA extension (oracle/_ref)"
+    return ("parity reference: the CPU oracle, checked against the recorded reference outputs "
+            "(tests/golden/parity_record.npz); the reference CUDA extension oracle/_ref is not built")
+
+
 def pytest_collection_modifyitems(config, items):
     try:
         import torch

@@ -41,6 +41,8 @@ def input_checksum(s):
 
 
 def main(out_dir):
+    if ref_harness.ref_module() is None:   # the harness would answer with the CPU oracle, which these fixtures pin
+        raise SystemExit("the reference extension oracle/_ref is not built (oracle/build_ref.py)")
     os.makedirs(out_dir, exist_ok=True)
     for name in TRI:
         cpu = scenes.config(name)
