@@ -386,12 +386,15 @@ def grad_sink_for(verts, verts_color, faces_opacity):
 
 def render_tris_backward(background, verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, inv_mv_mats,
                          inv_proj_mats, verts_depth, faces_intense, dL_dout_color, dL_dout_depth, R, pointBuffer,
-                         faceBuffer, binningBuffer, imageBuffer, accumulate_into=None, deterministic=False):
+                         faceBuffer, binningBuffer, imageBuffer, accumulate_into=None, deterministic=False,
+                         camera_grads=False):
     """RasterizeTrianglesBackwardCUDA (render.cu:134-208).
     Returns (dL_dverts[P,3], dL_dvcolor[P,3], dL_dfopacity[F], dL_dvdepth[B,P], dL_dfintense[B,F]).
     `accumulate_into` (beyond the reference's 18 arguments): existing contiguous fp32 (dL_dverts, dL_dvcolor,
     dL_dfopacity) tensors that the gradients are ADDED to (and that are returned) instead of fresh zero tensors.
-    `deterministic`: run-to-run reproducible gradients (64-bit fixed-point accumulation, dmr_tri_backward_deterministic)."""
+    `deterministic`: run-to-run reproducible gradients (64-bit fixed-point accumulation, dmr_tri_backward_deterministic).
+    `camera_grads`: also return dL_dmv_mats, dL_dproj_mats [B,4,4] (gradients with respect to the mv_mats / proj_mats
+    tensors passed here, through the rays; dmr_tri_backward_camera) as two more elements."""
     lib = _lib.load()
     B, P, F = mv_mats.size(0), verts.size(0), faces.size(0)
     H, W = dL_dout_color.size(2), dL_dout_color.size(3)
@@ -399,7 +402,7 @@ def render_tris_backward(background, verts, faces, verts_color, faces_opacity, m
     with _on_device(dev):
         # the five zero-initialised gradient tensors of render.cu:166-171, carved out of ONE allocation
         # (one memset instead of five); each starts on a 16-byte boundary
-        sizes = [3 * P, NUM_CHANNELS * P, F, B * P, B * F]
+        sizes = [3 * P, NUM_CHANNELS * P, F, B * P, B * F] + ([16 * B, 16 * B] if camera_grads else [])
         if accumulate_into is not None:
             sizes[0] = sizes[1] = sizes[2] = 0
         offs, o = [], 0
@@ -420,7 +423,12 @@ def render_tris_backward(background, verts, faces, verts_color, faces_opacity, m
                  _ptr(binningBuffer), _ptr(imageBuffer), _ptr(gc), _ptr(gd), gp[0], gp[1], gp[2], gp[3], gp[4])
             # scratch of the call (statistics per (view, face), per-vertex accumulators): the state buffers saved for
             # backward are only read.  The caching allocator reuses the block for later work on the same stream.
-            if deterministic:
+            if camera_grads:
+                ws = torch.empty(lib.dmr_tri_backward_camera_bytes(B, P, F, W, H, int(bool(deterministic))),
+                                 dtype=torch.uint8, device=dev)
+                _lib.check(lib.dmr_tri_backward_camera(*a, int(bool(deterministic)), gp[5], gp[6], _ptr(ws), ws.numel(),
+                                                       _stream()))
+            elif deterministic:
                 ws = torch.empty(lib.dmr_tri_backward_deterministic_bytes(B, P, F), dtype=torch.uint8, device=dev)
                 _lib.check(lib.dmr_tri_backward_deterministic(*a, _ptr(ws), ws.numel(), _stream()))
             else:
@@ -434,18 +442,35 @@ def render_tris_backward(background, verts, faces, verts_color, faces_opacity, m
             dL_dfopacity = flat[offs[2]:offs[2] + sizes[2]]
         dL_dvdepth = flat[offs[3]:offs[3] + sizes[3]].view(B, P)
         dL_dfintense = flat[offs[4]:offs[4] + sizes[4]].view(B, F)
+        if camera_grads:
+            # [B,16] column-major = [B,4,4] gradients of the (column-major, i.e. transposed) matrix tensors given here
+            return (dL_dverts, dL_dvcolor, dL_dfopacity, dL_dvdepth, dL_dfintense,
+                    flat[offs[5]:offs[5] + sizes[5]].view(B, 4, 4), flat[offs[6]:offs[6] + sizes[6]].view(B, 4, 4))
     return dL_dverts, dL_dvcolor, dL_dfopacity, dL_dvdepth, dL_dfintense
 
 
-def tri_depth_chain(verts, mv_mats, proj_mats, dL_dvdepth, dL_dverts):
-    """Fused vertex depth (verts_depth=None): dL_dverts += sum_b dL_dvdepth[b] * d ndc_z / d verts, in place."""
+def tri_depth_chain(verts, mv_mats, proj_mats, dL_dvdepth, dL_dverts, dL_dmv=None, dL_dproj=None):
+    """Fused vertex depth (verts_depth=None): dL_dverts += sum_b dL_dvdepth[b] * d ndc_z / d verts, in place.
+    With `dL_dmv` and `dL_dproj` (contiguous fp32 [B,4,4], e.g. from render_tris_backward(camera_grads=True)) the
+    depth's chain into the matrices is added to them as well (dmr_tri_depth_chain_camera)."""
     lib = _lib.load()
     B, P = mv_mats.size(0), verts.size(0)
+    if (dL_dmv is None) != (dL_dproj is None):
+        _err("tri_depth_chain: pass both dL_dmv and dL_dproj, or neither")
     with _on_device(verts.device):
         # keep the contiguous copies alive in locals until the launch is enqueued (a temporary would be freed, and
         # its memory handed to the next .contiguous(), before the call)
         v, mv, pj = _f32(verts, "verts"), _f32(mv_mats, "mv_mats"), _f32(proj_mats, "proj_mats")
-        _lib.check(lib.dmr_tri_depth_chain(B, P, _ptr(v), _ptr(mv), _ptr(pj), _ptr(dL_dvdepth), _ptr(dL_dverts), _stream()))
+        if dL_dmv is None:
+            _lib.check(lib.dmr_tri_depth_chain(B, P, _ptr(v), _ptr(mv), _ptr(pj), _ptr(dL_dvdepth), _ptr(dL_dverts),
+                                               _stream()))
+        else:
+            for t, n in ((dL_dmv, "dL_dmv"), (dL_dproj, "dL_dproj")):
+                if t.dtype != torch.float32 or not t.is_contiguous() or t.numel() != 16 * B:
+                    _err("%s must be a contiguous float32 (B, 4, 4) tensor" % n)
+            ws = torch.empty(lib.dmr_tri_depth_chain_camera_bytes(B, P), dtype=torch.uint8, device=verts.device)
+            _lib.check(lib.dmr_tri_depth_chain_camera(B, P, _ptr(v), _ptr(mv), _ptr(pj), _ptr(dL_dvdepth), _ptr(dL_dverts),
+                                                      _ptr(dL_dmv), _ptr(dL_dproj), _ptr(ws), ws.numel(), _stream()))
     return dL_dverts
 
 

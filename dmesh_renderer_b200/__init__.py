@@ -102,22 +102,31 @@ class _RenderTri(th.autograd.Function):
             into = tuple(leaf.grad for leaf in sink.leaves)
         # (bind() != 0: a leaf's .grad was dropped or replaced between forward and backward -- e.g. zero_grad with
         # set_to_none=True; the sink has re-attached it and this call hands its gradients to autograd the ordinary way)
+        # camera gradients (extension): requested by setting requires_grad on mv_mats or proj_mats; they are per view and
+        # always go through autograd (never into a gradient sink)
+        camera = ctx.needs_input_grad[4] or ctx.needs_input_grad[5]
+        grad_mv = grad_proj = None
         try:
-            grad_verts, grad_verts_color, grad_faces_opacity, grad_verts_depth, grad_faces_intense = \
-                _C.render_tris_backward(*args, accumulate_into=into, deterministic=ctx.deterministic)
+            grads = _C.render_tris_backward(*args, accumulate_into=into, deterministic=ctx.deterministic,
+                                            camera_grads=camera)
         except Exception as ex:
             print("\nAn error occured in backward.\n")
             raise ex
+        grad_verts, grad_verts_color, grad_faces_opacity, grad_verts_depth, grad_faces_intense = grads[:5]
+        if camera:
+            grad_mv, grad_proj = grads[5], grads[6]
         if ctx.fused_depth:
             # verts_depth=None: the depth was the vertex's own NDC z -> chain its gradient into the vertex positions
-            _C.tri_depth_chain(verts, mv_mats, proj_mats, grad_verts_depth, grad_verts)
+            # (and, for camera gradients, into the matrices)
+            _C.tri_depth_chain(verts, mv_mats, proj_mats, grad_verts_depth, grad_verts, grad_mv, grad_proj)
             grad_verts_depth = None
         if into is not None:
             # already added to the leaves' .grad by the kernels
             grad_verts = grad_verts_color = grad_faces_opacity = None
-        # gradient positions: reference __init__.py:156-168
-        return (grad_verts, None, grad_verts_color, grad_faces_opacity, None, None, grad_verts_depth,
-                grad_faces_intense, None, None)
+        # gradient positions: reference __init__.py:156-168; positions 4 and 5 (the matrices) are an extension
+        return (grad_verts, None, grad_verts_color, grad_faces_opacity,
+                grad_mv if ctx.needs_input_grad[4] else None, grad_proj if ctx.needs_input_grad[5] else None,
+                grad_verts_depth, grad_faces_intense, None, None)
 
 
 class TriRenderer(th.nn.Module):

@@ -40,7 +40,8 @@ static const char* const g_stage_names[ST_COUNT] = {
     "preprocess_points", "preprocess_faces", "face_depth_sort", "scan", "duplicate_with_keys", "sort_histogram", "sort_plan",
     "sort_pass0", "sort_pass1", "sort_pass2", "sort_pass3", "sort_pass4", "sort_pass5", "sort_pass6", "sort_pass7",
     "tile_ranges", "tri_render_forward", "tri_render_backward", "tri_grad_finish", "tet_build_records", "tet_jitter",
-    "tet_first_intersect", "tet_march_forward", "tet_march_backward", "tet_grad_vertex" };
+    "tet_first_intersect", "tet_march_forward", "tet_march_backward", "tet_grad_vertex", "tri_render_backward_camera",
+    "tri_camera_finish", "depth_chain_camera", "depth_chain_camera_finish" };
 struct Prof {
     bool on = false, created = false;
     cudaEvent_t ev[ST_COUNT][2];
@@ -91,6 +92,15 @@ static bool sizes_ok(long long B, long long P, long long F, long long W, long lo
         return false;
     }
     return true;
+}
+
+// workspace of the camera-gradient backward: the mode's own scratch, then 24 floats per (view, tile)
+static size_t tri_cam_bytes(int B, int P, int F, int W, int H, bool deterministic)
+{
+    const size_t base = deterministic ? TriDetLayout::make((size_t)B, (size_t)P, (size_t)F).total
+                                      : TriBwdLayout::make((size_t)B * F, (size_t)P).total;
+    const size_t tiles = (size_t)B * ((W + DMR_TILE - 1) / DMR_TILE) * ((H + DMR_TILE - 1) / DMR_TILE);
+    return align_up(base, 256) + align_up(96 * tiles, 256) + 256;
 }
 
 template <typename T>
@@ -253,8 +263,9 @@ static int tri_backward_impl(int B, int P, int F, int W, int H, int R, const flo
                              const void* binning_buffer, const void* image_buffer, const float* dL_dcolor,
                              const float* dL_ddepth, float* dL_dverts, float* dL_dvcolor, float* dL_dfopacity,
                              float* dL_dvdepth, float* dL_dfintense, void* workspace, size_t workspace_bytes,
-                             bool deterministic, dmr_stream_t stream_)
+                             bool deterministic, dmr_stream_t stream_, float* dL_dmv = nullptr, float* dL_dproj = nullptr)
 {
+    const bool cam = dL_dmv != nullptr;
     cudaStream_t stream = (cudaStream_t)stream_;
     if (!sizes_ok(B, P, F, W, H) || R < 0) return DMR_ETOOLARGE;
     if (B == 0 || F == 0 || R == 0) return DMR_OK;   // nothing was composited: all gradients stay zero
@@ -279,6 +290,19 @@ static int tri_backward_impl(int B, int P, int F, int W, int H, int R, const flo
     p.dL_dcolor = dL_dcolor; p.dL_ddepth = dL_ddepth;
     p.dL_dverts = dL_dverts; p.dL_dvcolor = dL_dvcolor; p.dL_dfopacity = dL_dfopacity;
     p.dL_dvdepth = dL_dvdepth; p.dL_dfintense = dL_dfintense;
+    // camera gradients: one 96-byte record per (view, tile) behind the mode's own scratch, written by every CTA
+    // (empty tiles store zeros), so it is not cleared
+    const size_t base_bytes = deterministic ? TriDetLayout::make((size_t)B, (size_t)P, (size_t)F).total
+                                            : TriBwdLayout::make((size_t)B * F, (size_t)P).total;
+    float* cam_tiles = nullptr;
+    if (cam) {
+        const size_t need = tri_cam_bytes(B, P, F, W, H, deterministic);
+        if (!workspace || workspace_bytes < need) {
+            set_error("camera-gradient backward needs a workspace of %zu bytes (dmr_tri_backward_camera_bytes)", need);
+            return DMR_EINVAL;
+        }
+        cam_tiles = at<float>(workspace, align_up(base_bytes, 256));
+    }
     if (deterministic) {
         TriDetLayout DL = TriDetLayout::make((size_t)B, (size_t)P, (size_t)F);
         void* det_workspace = workspace;
@@ -292,7 +316,9 @@ static int tri_backward_impl(int B, int P, int F, int W, int H, int R, const flo
         p.det_vdepth = at<long long>(det_workspace, DL.vdepth);
         p.det_fopa = at<long long>(det_workspace, DL.fopa);
         DMR_CUDA(cudaMemsetAsync(det_workspace, 0, DL.total, stream));
-        return tri_render_backward_deterministic(p, stream);
+        int rc = tri_render_backward_deterministic(p, stream, cam_tiles);
+        if (rc || !cam) return rc;
+        return tri_camera_finish(B, W, H, cam_tiles, inv_mv_mats, inv_proj_mats, dL_dmv, dL_dproj, stream);
     }
     // backward scratch: the caller's workspace (the forward's state buffers stay read-only)
     TriBwdLayout WL = TriBwdLayout::make((size_t)B * F, (size_t)P);
@@ -307,7 +333,9 @@ static int tri_backward_impl(int B, int P, int F, int W, int H, int R, const flo
     const bool use_vacc = 3 * (size_t)F >= 4 * (size_t)P;
     p.grad_vacc = use_vacc ? at<float4>(workspace, WL.grad_vacc) : nullptr;
     DMR_CUDA(cudaMemsetAsync(workspace, 0, use_vacc ? WL.total - 256 : WL.stats_end, stream));
-    return tri_render_backward(p, stream);
+    int rc = tri_render_backward(p, stream, cam_tiles);
+    if (rc || !cam) return rc;
+    return tri_camera_finish(B, W, H, cam_tiles, inv_mv_mats, inv_proj_mats, dL_dmv, dL_dproj, stream);
 }
 
 int dmr_tri_backward(int B, int P, int F, int W, int H, int R, const float* background, const float* inv_mv_mats,
@@ -343,6 +371,52 @@ int dmr_tri_backward_deterministic(int B, int P, int F, int W, int H, int R, con
     return tri_backward_impl(B, P, F, W, H, R, background, inv_mv_mats, inv_proj_mats, point_buffer, face_buffer,
                              binning_buffer, image_buffer, dL_dcolor, dL_ddepth, dL_dverts, dL_dvcolor, dL_dfopacity,
                              dL_dvdepth, dL_dfintense, workspace, workspace_bytes, true, stream);
+}
+
+size_t dmr_tri_backward_camera_bytes(int B, int P, int F, int W, int H, int deterministic)
+{
+    if (B < 0 || P < 0 || F < 0 || W < 0 || H < 0) return 0;
+    return tri_cam_bytes(B, P, F, W, H, deterministic != 0);
+}
+
+int dmr_tri_backward_camera(int B, int P, int F, int W, int H, int R, const float* background, const float* inv_mv_mats,
+                            const float* inv_proj_mats, const void* point_buffer, const void* face_buffer,
+                            const void* binning_buffer, const void* image_buffer, const float* dL_dcolor,
+                            const float* dL_ddepth, float* dL_dverts, float* dL_dvcolor, float* dL_dfopacity,
+                            float* dL_dvdepth, float* dL_dfintense, int deterministic, float* dL_dmv, float* dL_dproj,
+                            void* workspace, size_t workspace_bytes, dmr_stream_t stream)
+{
+    if (B > 0 && (!dL_dmv || !dL_dproj)) { set_error("null pointer"); return DMR_EINVAL; }
+    return tri_backward_impl(B, P, F, W, H, R, background, inv_mv_mats, inv_proj_mats, point_buffer, face_buffer,
+                             binning_buffer, image_buffer, dL_dcolor, dL_ddepth, dL_dverts, dL_dvcolor, dL_dfopacity,
+                             dL_dvdepth, dL_dfintense, workspace, workspace_bytes, deterministic != 0, stream, dL_dmv,
+                             dL_dproj);
+}
+
+size_t dmr_tri_depth_chain_camera_bytes(int B, int P)
+{
+    if (B < 0 || P < 0) return 0;
+    return depth_chain_camera_bytes(B, P);
+}
+
+int dmr_tri_depth_chain_camera(int B, int P, const float* verts, const float* mv_mats, const float* proj_mats,
+                               const float* dL_dvdepth, float* dL_dverts, float* dL_dmv, float* dL_dproj, void* workspace,
+                               size_t workspace_bytes, dmr_stream_t stream)
+{
+    if (B < 0 || P < 0) { set_error("negative size"); return DMR_EINVAL; }
+    if (B == 0 || P == 0) return DMR_OK;
+    if (!verts || !mv_mats || !proj_mats || !dL_dvdepth || !dL_dverts || !dL_dmv || !dL_dproj) {
+        set_error("null pointer");
+        return DMR_EINVAL;
+    }
+    const size_t need = depth_chain_camera_bytes(B, P);
+    if (!workspace || workspace_bytes < need) {
+        set_error("camera depth chain needs a workspace of %zu bytes (dmr_tri_depth_chain_camera_bytes)", need);
+        return DMR_EINVAL;
+    }
+    int rc = depth_chain(B, P, verts, mv_mats, proj_mats, dL_dvdepth, dL_dverts, (cudaStream_t)stream);
+    if (rc) return rc;
+    return depth_chain_camera(B, P, verts, mv_mats, proj_mats, dL_dvdepth, dL_dmv, dL_dproj, workspace, (cudaStream_t)stream);
 }
 
 int dmr_debug_view(int renderer, int kind, int B, int P, int F, int T, int W, int H, size_t R, const void* buffer,

@@ -15,6 +15,7 @@
 #include "tri.cuh"
 #include "tet.cuh"
 #include "radix_sort.cuh"
+#include <algorithm>
 
 namespace dmr {
 
@@ -131,6 +132,104 @@ int depth_chain(int B, int P, const float* verts, const float* mv, const float* 
     count_launch(1);
     DMR_CUDA(dmr_launch(depth_chain_kernel, dim3((P + 255) / 256), dim3(256), 0, stream, B, P, verts, mv, proj, dL_dvdepth, dL_dverts));
     DMR_LAUNCH_CHECK("depth_chain_kernel");
+    return 0;
+}
+
+// Camera variant (dmr_tri_depth_chain_camera): the same per-(view, vertex) terms -- pv = MV p, clip = Proj (pv, 1),
+// ndc_z = z_clip / clamp_w(w_clip), no derivative through a clamped w -- reduced over the vertices into the 20 nonzero
+// partials of dL/dmv[b] and dL/dproj[b]:
+//   gz = g / w, gw = -g ndc_z / w  (0 if clamped),  gpv = gz Proj[2, 0:3] + gw Proj[3, 0:3]
+//   [0..3]   dL/dproj[2, 0..3] = gz (pv, 1)       [4..7]   dL/dproj[3, 0..3] = gw (pv, 1)
+//   [8 + 3c + i]  dL/dmv[i, c] = gpv[i] (p, 1)[c]    (i < 3, c < 4)
+// Fixed grid (DMR_DEPTH_CAM_BLOCKS blocks per view at most, a function of P only), per-block partials in a fixed
+// order, and one CTA per view that adds the partials in block order: reproducible, no float atomics.
+#define DMR_DEPTH_CAM_TERMS 20
+#define DMR_DEPTH_CAM_BLOCKS 256
+static int depth_cam_blocks(int P) { return (int)std::min<long long>(DMR_DEPTH_CAM_BLOCKS, ((long long)P + 1023) / 1024); }
+size_t depth_chain_camera_bytes(int B, int P)
+{
+    return align_up(sizeof(float) * DMR_DEPTH_CAM_TERMS * (size_t)B * depth_cam_blocks(P), 256) + 256;
+}
+
+__global__ void __launch_bounds__(256) depth_chain_camera_kernel(int P, const float* __restrict__ verts,
+                                                                 const float* __restrict__ mv_mats, const float* __restrict__ proj_mats,
+                                                                 const float* __restrict__ dL_dvdepth, float* __restrict__ partials)
+{
+    griddep_wait();   // programmatic dependent launch: see dmr_launch (common.cuh)
+    __shared__ float s_w[8][DMR_DEPTH_CAM_TERMS];
+    const int b = blockIdx.y;
+    const float* mv = mv_mats + 16 * b;
+    const float* pj = proj_mats + 16 * b;
+    float acc[DMR_DEPTH_CAM_TERMS];
+#pragma unroll
+    for (int k = 0; k < DMR_DEPTH_CAM_TERMS; k++) acc[k] = 0.0f;
+    for (size_t idx = (size_t)blockIdx.x * 256 + threadIdx.x; idx < (size_t)P; idx += (size_t)gridDim.x * 256) {
+        const float g = dL_dvdepth[(size_t)b * P + idx];
+        if (g == 0.0f) continue;
+        const float3 p = f3(verts[3 * idx + 0], verts[3 * idx + 1], verts[3 * idx + 2]);
+        const float3 pv = xform43(p, mv);
+        const float4 pp = xform44(pv, pj);
+        const float wc = clamp_w(pp.w);
+        const float pw = 1.0f / wc;
+        const float ndc_z = pp.z * pw;
+        const bool clamped = wc != pp.w;
+        const float gz = g * pw, gw = clamped ? 0.0f : -gz * ndc_z;
+        acc[0] += gz * pv.x; acc[1] += gz * pv.y; acc[2] += gz * pv.z; acc[3] += gz;
+        acc[4] += gw * pv.x; acc[5] += gw * pv.y; acc[6] += gw * pv.z; acc[7] += gw;
+        const float gpv[3] = { gz * pj[2] + gw * pj[3], gz * pj[6] + gw * pj[7], gz * pj[10] + gw * pj[11] };
+#pragma unroll
+        for (int i = 0; i < 3; i++) {
+            acc[8 + i] += gpv[i] * p.x; acc[11 + i] += gpv[i] * p.y; acc[14 + i] += gpv[i] * p.z; acc[17 + i] += gpv[i];
+        }
+    }
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int k = 0; k < DMR_DEPTH_CAM_TERMS; k++) {
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) acc[k] += __shfl_xor_sync(0xffffffffu, acc[k], o);
+    }
+    if (lane == 0) {
+#pragma unroll
+        for (int k = 0; k < DMR_DEPTH_CAM_TERMS; k++) s_w[warp][k] = acc[k];
+    }
+    __syncthreads();
+    if (threadIdx.x < DMR_DEPTH_CAM_TERMS) {
+        float sum = 0.0f;
+#pragma unroll
+        for (int w = 0; w < 8; w++) sum += s_w[w][threadIdx.x];
+        partials[((size_t)b * gridDim.x + blockIdx.x) * DMR_DEPTH_CAM_TERMS + threadIdx.x] = sum;
+    }
+}
+
+// One warp per view: the view's block partials in block order, ADDED to dL_dmv[b] / dL_dproj[b] (column-major).
+__global__ void __launch_bounds__(32) depth_chain_camera_finish_kernel(int nblk, const float* __restrict__ partials,
+                                                                       float* __restrict__ dL_dmv, float* __restrict__ dL_dproj)
+{
+    griddep_wait();   // programmatic dependent launch: see dmr_launch (common.cuh)
+    const int b = blockIdx.x, k = threadIdx.x;
+    if (k >= DMR_DEPTH_CAM_TERMS) return;
+    float sum = 0.0f;
+    for (int j = 0; j < nblk; j++) sum += partials[((size_t)b * nblk + j) * DMR_DEPTH_CAM_TERMS + k];
+    if (k < 8) dL_dproj[16 * b + 4 * (k & 3) + 2 + (k >> 2)] += sum;    // row 2 (k < 4) / row 3, column k & 3
+    else dL_dmv[16 * b + 4 * ((k - 8) / 3) + (k - 8) % 3] += sum;        // row (k - 8) % 3, column (k - 8) / 3
+}
+
+int depth_chain_camera(int B, int P, const float* verts, const float* mv, const float* proj, const float* dL_dvdepth,
+                       float* dL_dmv, float* dL_dproj, void* workspace, cudaStream_t stream)
+{
+    if (B <= 0 || P <= 0) return 0;
+    const int nblk = depth_cam_blocks(P);
+    float* partials = static_cast<float*>(workspace);
+    {
+        ProfScope prof(ST_DEPTH_CAM, stream);
+        DMR_CUDA(dmr_launch(depth_chain_camera_kernel, dim3(nblk, B), dim3(256), 0, stream, P, verts, mv, proj, dL_dvdepth, partials));
+        DMR_LAUNCH_CHECK("depth_chain_camera_kernel");
+    }
+    {
+        ProfScope prof(ST_DEPTH_CAM_FINISH, stream);
+        DMR_CUDA(dmr_launch(depth_chain_camera_finish_kernel, dim3(B), dim3(32), 0, stream, nblk, (const float*)partials, dL_dmv, dL_dproj));
+        DMR_LAUNCH_CHECK("depth_chain_camera_finish_kernel");
+    }
     return 0;
 }
 

@@ -168,6 +168,10 @@ int preprocess_points(int B, int P, int W, int H, const float* verts, const floa
                       const float* verts_depth, int depth_mode, float4* vimg, cudaStream_t stream);
 int depth_chain(int B, int P, const float* verts, const float* mv, const float* proj, const float* dL_dvdepth,
                 float* dL_dverts, cudaStream_t stream);
+// camera variant of the fused-depth chain: += dL_dmv[B,16], dL_dproj[B,16]; workspace of depth_chain_camera_bytes
+size_t depth_chain_camera_bytes(int B, int P);
+int depth_chain_camera(int B, int P, const float* verts, const float* mv, const float* proj, const float* dL_dvdepth,
+                       float* dL_dmv, float* dL_dproj, void* workspace, cudaStream_t stream);
 int tet_preprocess_faces(int B, int P, int F, int W, int H, const int* faces, const float4* vimg, const float* verts,
                          uint32_t* tiles_touched, uint32_t* depth_key, uint2* rect, TetFaceRec* rec,
                          const SortPre& face_sort, cudaStream_t stream);

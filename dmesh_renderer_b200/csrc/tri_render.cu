@@ -427,8 +427,19 @@ static_assert(stat_slot_is_permutation(), "stat_slot must map the 24 statistics 
 #ifndef DMR_TRI_BWD_RCP_ALPHA
 #define DMR_TRI_BWD_RCP_ALPHA 1
 #endif
-template <bool DET>
-__device__ __forceinline__ void tri_render_bwd_body(const TriRenderParams& p)
+// Camera gradients (CAM = true; DESIGN.md 3.3).  The rays are the only place the camera enters a pixel's colour and
+// depth: ro = inv_mv[12..14], rd = d / (|d| + 1e-7), d = L pv, pv = (inv_proj (nx, ny, -1, 1)).xyz, L = the linear
+// part of inv_mv.  Per covered hit, with T = ro - p0, E1, E2, P = rd x E2, Q = T x E1, D = P.E1, u = P.T / D and
+// v = Q.rd / D, each lane (one pixel) accumulates
+//     g_ro += (dL_du P + dL_dv (E1 x rd)) / D
+//     g_rd += (dL_du (E2 x T) + dL_dv Q - (dL_du u + dL_dv v) (E2 x E1)) / D
+// -- the exact derivative of v, not the reference's t-derivative the vertex-position statistics keep.  After the walk
+// the lane chains its pixel into the 24 nonzero partials of dL/dinv_mv and dL/dinv_proj (cam_record_slot), the CTA
+// sums them in a fixed order and stores ONE 96-byte record per (view, tile): no float atomics, so the camera
+// gradients are reproducible in both modes.  tri_camera_finish_kernel sums a view's records and applies the inverse.
+#define DMR_CAM_REC 24
+template <bool DET, bool CAM>
+__device__ __forceinline__ void tri_render_bwd_body(const TriRenderParams& p, float* __restrict__ cam_tiles)
 {
     __shared__ uint4 s_rec[RB * 9];      // staged records; two vertex-id slots (unused here: tri_grad_finish_kernel reads the
                                          // global record) carry the face id and 1 / (1 - opacity) of the instance
@@ -476,6 +487,7 @@ __device__ __forceinline__ void tri_render_bwd_body(const TriRenderParams& p)
 
     float acc0 = 0, acc1 = 0, acc2 = 0, accd = 0;
     float last_alpha = 0, lc0 = 0, lc1 = 0, lc2 = 0, ld = 0;
+    float3 g_ro = f3(0, 0, 0), g_rd = f3(0, 0, 0);   // CAM only: dL/dro, dL/drd of this pixel
 
     // The tile walks only the prefix some pixel of it composited; a warp only its own.
     int warp_last = last_contributor;
@@ -662,6 +674,14 @@ __device__ __forceinline__ void tri_render_bwd_body(const TriRenderParams& p)
                         v[0] = k1 * rd.x; v[1] = k1 * rd.y; v[2] = k1 * rd.z;
                         v[3] = k24 * rd.x; v[4] = k24 * rd.y; v[5] = k24 * rd.z;
                         v[6] = dL_dv * inv_denom;
+                        if constexpr (CAM) {
+                            const float3 p0 = f3(a0.x, a0.y, a0.z);
+                            const float3 Tv = ro - p0, E1 = f3(a1.x, a1.y, a1.z) - p0, E2 = f3(a2.x, a2.y, a2.z) - p0;
+                            const float kv = dL_dv * inv_denom;
+                            const float kn = (dL_du * tuv.y + dL_dv * tuv.z) * inv_denom;
+                            g_ro = g_ro + k1 * cross3(rd, E2) + kv * cross3(E1, rd);
+                            g_rd = g_rd + k1 * cross3(E2, Tv) + kv * cross3(Tv, E1) - kn * cross3(E2, E1);
+                        }
                     }
                 }
 
@@ -691,18 +711,136 @@ __device__ __forceinline__ void tri_render_bwd_body(const TriRenderParams& p)
             __syncwarp();   // the next pass overwrites the index list and the masks
         }
     }
+    if constexpr (CAM) {
+        // chain this pixel into the 24 partials: g_d = dL/dd, then d = L pv, pv = (inv_proj n).xyz, n = (nx, ny, -1, 1)
+        //   [3j + i]       dL/dinv_mv[4j + i]  = g_d[i] pv[j]     (i, j < 3)
+        //   [9 + i]        dL/dinv_mv[12 + i]  = g_ro[i]
+        //   [12 + 3k + j]  dL/dinv_proj[4k + j] = (L^T g_d)[j] n[k]  (j < 3, k < 4)
+        float g[DMR_CAM_REC];
+#pragma unroll
+        for (int k = 0; k < DMR_CAM_REC; k++) g[k] = 0.0f;
+        if (inside) {
+            const float* imv = p.inv_mv + 16 * b;
+            const float* ipj = p.inv_proj + 16 * b;
+            const float n[4] = { pix2ndc(px + 0.5f, p.W), pix2ndc(py + 0.5f, p.H), -1.0f, 1.0f };
+            float pv[3], d[3];
+#pragma unroll
+            for (int j = 0; j < 3; j++) pv[j] = ipj[j] * n[0] + ipj[4 + j] * n[1] + ipj[8 + j] * n[2] + ipj[12 + j];
+#pragma unroll
+            for (int i = 0; i < 3; i++) d[i] = imv[i] * pv[0] + imv[4 + i] * pv[1] + imv[8 + i] * pv[2];
+            const float dn = sqrtf(d[0] * d[0] + d[1] * d[1] + d[2] * d[2]);
+            const float sl = dn + 0.0000001f;
+            const float dg = (d[0] * g_rd.x + d[1] * g_rd.y + d[2] * g_rd.z) / (sl * sl * fmaxf(dn, 1e-30f));
+            const float gd[3] = { g_rd.x / sl - d[0] * dg, g_rd.y / sl - d[1] * dg, g_rd.z / sl - d[2] * dg };
+#pragma unroll
+            for (int j = 0; j < 3; j++) {
+#pragma unroll
+                for (int i = 0; i < 3; i++) g[3 * j + i] = gd[i] * pv[j];
+                const float lg = imv[4 * j] * gd[0] + imv[4 * j + 1] * gd[1] + imv[4 * j + 2] * gd[2];
+#pragma unroll
+                for (int k = 0; k < 4; k++) g[12 + 3 * k + j] = lg * n[k];
+            }
+            g[9] = g_ro.x; g[10] = g_ro.y; g[11] = g_ro.z;
+        }
+        // fixed-order reduction: warp butterfly, then the eight warp sums in warp order
+#pragma unroll
+        for (int k = 0; k < DMR_CAM_REC; k++) {
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) g[k] += __shfl_xor_sync(0xffffffffu, g[k], o);
+        }
+        __syncthreads();                                   // s_rec is free again
+        float* const s_cam = reinterpret_cast<float*>(s_rec);
+        if (lane < DMR_CAM_REC) {
+            float x = g[0];
+#pragma unroll
+            for (int k = 1; k < DMR_CAM_REC; k++) x = lane == k ? g[k] : x;
+            s_cam[warp * DMR_CAM_REC + lane] = x;
+        }
+        __syncthreads();
+        if (tid < DMR_CAM_REC) {
+            float sum = 0.0f;
+#pragma unroll
+            for (int w = 0; w < 8; w++) sum += s_cam[w * DMR_CAM_REC + tid];
+            cam_tiles[((size_t)b * tiles_x * tiles_y + blockIdx.y * tiles_x + blockIdx.x) * DMR_CAM_REC + tid] = sum;
+        }
+    }
 }
 
 __global__ void __launch_bounds__(256, DMR_TRI_BWD_MINB) tri_render_bwd_kernel(TriRenderParams p)
 {
     griddep_wait();   // programmatic dependent launch: see dmr_launch (common.cuh)
-    tri_render_bwd_body<false>(p);
+    tri_render_bwd_body<false, false>(p, nullptr);
 }
 
 __global__ void __launch_bounds__(256, DMR_TRI_BWD_MINB) tri_render_bwd_det_kernel(TriRenderParams p)
 {
     griddep_wait();   // programmatic dependent launch: see dmr_launch (common.cuh)
-    tri_render_bwd_body<true>(p);
+    tri_render_bwd_body<true, false>(p, nullptr);
+}
+
+// Camera-gradient instantiations: the same walk plus g_ro / g_rd per lane (six more live floats) and the per-tile
+// record.  Resident CTAs per SM: see DESIGN.md 3.3 for the -Xptxas -v figures of both choices.
+#ifndef DMR_TRI_BWD_CAM_MINB
+#define DMR_TRI_BWD_CAM_MINB 3
+#endif
+__global__ void __launch_bounds__(256, DMR_TRI_BWD_CAM_MINB) tri_render_bwd_cam_kernel(TriRenderParams p, float* cam_tiles)
+{
+    griddep_wait();   // programmatic dependent launch: see dmr_launch (common.cuh)
+    tri_render_bwd_body<false, true>(p, cam_tiles);
+}
+
+__global__ void __launch_bounds__(256, DMR_TRI_BWD_CAM_MINB) tri_render_bwd_cam_det_kernel(TriRenderParams p, float* cam_tiles)
+{
+    griddep_wait();   // programmatic dependent launch: see dmr_launch (common.cuh)
+    tri_render_bwd_body<true, true>(p, cam_tiles);
+}
+
+// One CTA per view: the view's per-tile camera records (tri_render_bwd_cam_kernel) are summed in a fixed order -- a
+// thread owns one component (240 = 10 x 24 threads, coalesced reads of the flat record array), then the ten partial
+// sums of a component are added in thread order -- and chained through the inverses: with N = A^-1,
+// dL/dA = -N^T (dL/dN) N^T.  The result is ADDED to dL_dmv[b] / dL_dproj[b]; this CTA is the only writer of view b.
+__global__ void __launch_bounds__(240) tri_camera_finish_kernel(int ntiles, const float* __restrict__ cam_tiles,
+                                                                const float* __restrict__ inv_mv, const float* __restrict__ inv_proj,
+                                                                float* __restrict__ dL_dmv, float* __restrict__ dL_dproj)
+{
+    griddep_wait();   // programmatic dependent launch: see dmr_launch (common.cuh)
+    __shared__ float s_part[240];
+    __shared__ float s_g[2][16];      // dL/dinv_mv, dL/dinv_proj (column-major, zeros where the forward reads nothing)
+    const int b = blockIdx.x, t = threadIdx.x;
+    const float* rec = cam_tiles + (size_t)b * ntiles * DMR_CAM_REC;
+    const size_t n = (size_t)ntiles * DMR_CAM_REC;
+    float acc = 0.0f;
+    for (size_t i = t; i < n; i += 240) acc += rec[i];   // component t % 24
+    s_part[t] = acc;
+    __syncthreads();
+    if (t < 32) {
+        s_g[t >> 4][t & 15] = 0.0f;
+        __syncwarp();
+        if (t < DMR_CAM_REC) {
+            float sum = 0.0f;
+#pragma unroll
+            for (int k = 0; k < 10; k++) sum += s_part[t + DMR_CAM_REC * k];
+            // record slot -> column-major matrix entry (cam record layout: tri_render_bwd_body)
+            if (t < 9) s_g[0][4 * (t / 3) + t % 3] = sum;
+            else if (t < 12) s_g[0][12 + t - 9] = sum;
+            else s_g[1][4 * ((t - 12) / 3) + (t - 12) % 3] = sum;
+        }
+        __syncwarp();
+        // thread e: entry (i, j) = (e & 3, (e >> 2) & 3) of matrix e >> 4; M(r, c) = m[4c + r]
+        const int m = t >> 4, e = t & 15, i = e & 3, j = e >> 2;
+        const float* N = (m == 0 ? inv_mv : inv_proj) + 16 * b;
+        const float* G = s_g[m];
+        float out = 0.0f;
+#pragma unroll
+        for (int a = 0; a < 4; a++) {
+            float h = 0.0f;                                // (G N^T)(a, j) = sum_c G(a, c) N(j, c)
+#pragma unroll
+            for (int c = 0; c < 4; c++) h += G[4 * c + a] * N[4 * c + j];
+            out += N[4 * i + a] * h;                       // N^T(i, a) = N(a, i)
+        }
+        float* dst = (m == 0 ? dL_dmv : dL_dproj) + 16 * b + e;
+        *dst += -out;
+    }
 }
 
 // Deterministic mode: g = max |dL_dout| over both cotangent images, as float bits (non-negative floats order like
@@ -905,11 +1043,15 @@ int tri_render_forward(const TriRenderParams& p, cudaStream_t stream)
     return 0;
 }
 
-int tri_render_backward(const TriRenderParams& p, cudaStream_t stream)
+int tri_render_backward(const TriRenderParams& p, cudaStream_t stream, float* cam_tiles)
 {
     if (p.B <= 0 || p.W <= 0 || p.H <= 0) return 0;
     dim3 grid((p.W + DMR_TILE - 1) / DMR_TILE, (p.H + DMR_TILE - 1) / DMR_TILE, p.B);
-    {
+    if (cam_tiles) {
+        ProfScope prof(ST_TRI_BWD_CAM, stream);
+        DMR_CUDA(dmr_launch(tri_render_bwd_cam_kernel, dim3(grid), dim3(256), 0, stream, p, cam_tiles));
+        DMR_LAUNCH_CHECK("tri_render_bwd_cam_kernel");
+    } else {
         ProfScope prof(ST_TRI_BWD, stream);
         DMR_CUDA(dmr_launch(tri_render_bwd_kernel, dim3(grid), dim3(256), 0, stream, p));
         DMR_LAUNCH_CHECK("tri_render_bwd_kernel");
@@ -935,18 +1077,23 @@ int det_gmax(const float* a, size_t na, const float* b, size_t nb, uint32_t* gma
     return 0;
 }
 
-int tri_render_backward_deterministic(const TriRenderParams& p, cudaStream_t stream)
+int tri_render_backward_deterministic(const TriRenderParams& p, cudaStream_t stream, float* cam_tiles)
 {
     if (p.B <= 0 || p.W <= 0 || p.H <= 0) return 0;
     dim3 grid((p.W + DMR_TILE - 1) / DMR_TILE, (p.H + DMR_TILE - 1) / DMR_TILE, p.B);
     const size_t HW = (size_t)p.W * p.H;
     {
-        ProfScope prof(ST_TRI_BWD, stream);
+        ProfScope prof(cam_tiles ? ST_TRI_BWD_CAM : ST_TRI_BWD, stream);
         count_launch(1);   // two kernels under one scope
         int rc = det_gmax(p.dL_dcolor, 3 * p.B * HW, p.dL_ddepth, p.B * HW, const_cast<uint32_t*>(p.det_gmax), stream);
         if (rc) return rc;
-        DMR_CUDA(dmr_launch(tri_render_bwd_det_kernel, dim3(grid), dim3(256), 0, stream, p));
-        DMR_LAUNCH_CHECK("tri_render_bwd_det_kernel");
+        if (cam_tiles) {
+            DMR_CUDA(dmr_launch(tri_render_bwd_cam_det_kernel, dim3(grid), dim3(256), 0, stream, p, cam_tiles));
+            DMR_LAUNCH_CHECK("tri_render_bwd_cam_det_kernel");
+        } else {
+            DMR_CUDA(dmr_launch(tri_render_bwd_det_kernel, dim3(grid), dim3(256), 0, stream, p));
+            DMR_LAUNCH_CHECK("tri_render_bwd_det_kernel");
+        }
     }
     {
         ProfScope prof(ST_TRI_BWD_FINISH, stream);
@@ -957,6 +1104,17 @@ int tri_render_backward_deterministic(const TriRenderParams& p, cudaStream_t str
         DMR_CUDA(dmr_launch(tri_det_convert_kernel, dim3((unsigned)((n + 255) / 256)), dim3(256), 0, stream, p));
         DMR_LAUNCH_CHECK("tri_det_convert_kernel");
     }
+    return 0;
+}
+
+int tri_camera_finish(int B, int W, int H, const float* cam_tiles, const float* inv_mv, const float* inv_proj, float* dL_dmv,
+                      float* dL_dproj, cudaStream_t stream)
+{
+    if (B <= 0 || W <= 0 || H <= 0) return 0;
+    const int ntiles = ((W + DMR_TILE - 1) / DMR_TILE) * ((H + DMR_TILE - 1) / DMR_TILE);
+    ProfScope prof(ST_TRI_CAM_FINISH, stream);
+    DMR_CUDA(dmr_launch(tri_camera_finish_kernel, dim3(B), dim3(240), 0, stream, ntiles, cam_tiles, inv_mv, inv_proj, dL_dmv, dL_dproj));
+    DMR_LAUNCH_CHECK("tri_camera_finish_kernel");
     return 0;
 }
 

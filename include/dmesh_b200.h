@@ -197,6 +197,38 @@ int dmr_tri_backward_deterministic(
     void* workspace, size_t workspace_bytes,
     dmr_stream_t stream);
 
+/* Camera gradients of the tri renderer (no reference counterpart: the reference returns no gradient for the      */
+/* matrices).  The same backward pass as dmr_tri_backward (deterministic == 0) or dmr_tri_backward_deterministic  */
+/* (deterministic != 0), with the same arguments and the same five gradients, plus dL/dmv_mats and                */
+/* dL/dproj_mats [B,16] (column-major, like the matrices), ADDED to the caller's zeroed buffers.  The derivative   */
+/* is that of the rays (ray origin and direction formed from inv_mv_mats / inv_proj_mats) with coverage, depth    */
+/* order and n_contrib held fixed, chained through the inverses (dL/dA = -A^-T dL/dA^-1 A^-T); with the fused     */
+/* vertex depth add dmr_tri_depth_chain_camera.  Accumulated without float atomics: reproducible in both modes.  */
+/* `workspace`: dmr_tri_backward_camera_bytes(B, P, F, W, H, deterministic) bytes of device scratch.              */
+size_t dmr_tri_backward_camera_bytes(int B, int P, int F, int W, int H, int deterministic);
+int dmr_tri_backward_camera(
+    int B, int P, int F, int W, int H, int R,
+    const float* background,
+    const float* inv_mv_mats, const float* inv_proj_mats,
+    const void* point_buffer, const void* face_buffer,
+    const void* binning_buffer, const void* image_buffer,
+    const float* dL_dcolor, const float* dL_ddepth,
+    float* dL_dverts, float* dL_dvcolor, float* dL_dfopacity, float* dL_dvdepth, float* dL_dfintense,
+    int deterministic,
+    float* dL_dmv,               /* [B,16] */
+    float* dL_dproj,             /* [B,16] */
+    void* workspace, size_t workspace_bytes,
+    dmr_stream_t stream);
+
+/* dmr_tri_depth_chain plus the camera part of the fused vertex depth (no reference counterpart):                 */
+/* dL_dmv[b] / dL_dproj[b] += sum_p dL_dvdepth[b,p] * d ndc_z[b,p] / d(mv_mats[b], proj_mats[b]) (no derivative   */
+/* through a clamped clip w).  Reduced in a fixed order without float atomics.  `workspace`:                      */
+/* dmr_tri_depth_chain_camera_bytes(B, P) bytes of device scratch.                                                */
+size_t dmr_tri_depth_chain_camera_bytes(int B, int P);
+int dmr_tri_depth_chain_camera(int B, int P, const float* verts, const float* mv_mats, const float* proj_mats,
+                               const float* dL_dvdepth, float* dL_dverts, float* dL_dmv, float* dL_dproj,
+                               void* workspace, size_t workspace_bytes, dmr_stream_t stream);
+
 /* ------------------------------------------------------------------------ */
 /* Tet renderer, forward, phase 1.  Replaces E1, E4, E5 of                   */
 /* CudaRenderer::Renderer::forward (cuda_renderer/renderer_impl.cu:241-310): */
