@@ -189,9 +189,6 @@ class _Inverses:
         else:
             self.check(info)
 
-    def join(self):
-        """The inverses are computed on the current stream: nothing to wait for."""
-
     def check(self, *infos):
         """Call after the current stream has been synchronised."""
         if infos:
@@ -306,7 +303,6 @@ def tri_forward_finish(st, inv_mv_mats, inv_proj_mats, inverses=None, speculativ
             # render.cu:88-89,105: zero images (not background), empty state
             z = torch.zeros
             if inverses is not None:
-                inverses.join()
                 torch.cuda.current_stream().synchronize()
                 inverses.check()
             return (0, z((B, NUM_CHANNELS, H, W), dtype=torch.float32, device=dev),
@@ -321,8 +317,6 @@ def tri_forward_finish(st, inv_mv_mats, inv_proj_mats, inverses=None, speculativ
         # everything that does not depend on R is prepared before the wait
         a = (_ptr(st.bg), _ptr(imv), _ptr(ipj), _ptr(point_buf), _ptr(face_buf))
         b2 = (_ptr(img_buf), _ptr(out_color), _ptr(out_depth), _stream())
-        if inverses is not None:
-            inverses.join()
         try:
             if speculative and spec is not None:
                 # phase 2 goes out first; the wait below overlaps with it
@@ -567,8 +561,6 @@ def render_tets(background, verts, faces, verts_color, faces_opacity, mv_mats, p
                                                _ptr(face_buf), _ptr(tet_rec), rec_valid, pinned[2], stream))
             key = ("tet", B, P, F, T, W, H)
             spec, _cap = _speculative_binning(lib, key, u8)
-            if inverses is not None:
-                inverses.join()
             R, bin_buf = _wait_R(lib, pinned, key, spec, u8)
         finally:
             _Pinned.release(pinned)

@@ -30,10 +30,6 @@ class TriRenderSettings(NamedTuple):      # reference __init__.py:13-16
 
 
 _deterministic_default = False
-# TriRenderer launches phase 2 of a forward call before num_rendered has reached the host (see
-# _C.tri_forward_finish); DMESH_B200_NO_SPECULATIVE=1 restores wait-then-launch (debugging / A-B timing)
-import os as _os
-_speculative_phase2 = _os.environ.get("DMESH_B200_NO_SPECULATIVE") != "1"
 
 
 def set_deterministic(flag: bool) -> bool:
@@ -74,7 +70,7 @@ class _RenderTri(th.autograd.Function):
             # speculative: phase 2 is enqueued before num_rendered reaches the host; `num_rendered` is then the count
             # the binning buffer was laid out for (>= the real one), which is what backward needs
             num_rendered, color, depth, pointBuffer, faceBuffer, binningBuffer, imgBuffer = \
-                _C.tri_forward_finish(pending, inv_mv_mats, inv_proj_mats, inv, speculative=_speculative_phase2)
+                _C.tri_forward_finish(pending, inv_mv_mats, inv_proj_mats, inv, speculative=True)
         except Exception as ex:
             print("\nAn error occured in forward.")
             print(ex)

@@ -7,8 +7,8 @@ import ctypes
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# DMESH_B200_LIB: development override -- load another build of the SAME library (e.g. an experiment variant made by
-# tools/build_variant.sh) instead of the in-tree one.  It is not a fallback: a missing file still raises.
+# DMESH_B200_LIB: development override -- load another build of the SAME library (e.g. an experiment variant built
+# from a modified tree) instead of the in-tree one.  It is not a fallback: a missing file still raises.
 LIB_PATH = os.environ.get("DMESH_B200_LIB") or os.path.join(_HERE, "libdmesh_b200.so")
 
 c_int = ctypes.c_int
@@ -46,7 +46,6 @@ SIGNATURES = {
     "dmr_tet_backward_deterministic_bytes": (c_size_t, [c_int] * 2),
     "dmr_tet_backward_deterministic": (c_int, [c_int] * 7 + [c_void_p] * 14 + [c_void_p, c_size_t] + [c_void_p]),
     "dmr_debug_view": (c_int, [c_int] * 8 + [c_size_t, c_void_p, ctypes.POINTER(c_void_p), ctypes.POINTER(c_size_t)]),
-    "dmr_nvls_allreduce_sum_f32": (c_int, [c_void_p, c_size_t, c_int, c_int, c_void_p]),
     "dmr_nvls_allreduce_sum_f32_fused": (c_int, [c_void_p, c_size_t, c_int, c_int, c_void_p, c_void_p, ctypes.c_uint, c_void_p]),
     "dmr_camera_inverses": (c_int, [c_int, c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_int64, c_void_p, ctypes.c_int64,
                                    ctypes.c_int64, ctypes.c_int64, c_void_p, c_void_p, c_void_p]),

@@ -28,13 +28,6 @@ int cuda_fail(cudaError_t e, const char* what)
     return DMR_ECUDA;
 }
 
-bool pdl_enabled()
-{
-    static int on = -1;
-    if (on < 0) { const char* e = getenv("DMESH_B200_NO_PDL"); on = (e && e[0] == '1') ? 0 : 1; }
-    return on == 1;
-}
-
 // ---- stage timing ------------------------------------------------------------
 static const char* const g_stage_names[ST_COUNT] = {
     "preprocess_points", "preprocess_faces", "face_depth_sort", "scan", "duplicate_with_keys", "sort_histogram", "sort_plan",

@@ -8,9 +8,9 @@
 //     multimem.ld_reduce.add.v4.f32  [mc + i]   -> the switch returns the sum of the 16 bytes over all ranks
 //     multimem.st.v4.f32             [mc + i]   -> the switch writes the sum into every rank's copy
 // so every float crosses each GPU's NVLink port once in each direction (2 x n/W x (W-1)/W ... ~n bytes per
-// port in total) and no GPU ever reads W copies.  Cross-GPU barriers before (all ranks' gradients complete)
-// and after (all slices broadcast) are the symmetric-memory signal-pad barriers issued by the caller on the
-// same stream (dmesh_renderer_b200/multiview.py).  Measured on 8 x B200: 15 MB in [see profiles/README.md].
+// port in total) and no GPU ever reads W copies.  The cross-GPU barriers before (all ranks' gradients complete)
+// and after (all slices broadcast) run inside the same kernel, on flags in symmetric memory (see
+// nvls_allreduce_sum_fused_kernel).  Measured on 8 x B200: 15 MB in [see profiles/README.md].
 #include "common.cuh"
 #include "../../include/dmesh_b200.h"
 
@@ -34,9 +34,7 @@ __device__ __forceinline__ void multimem_st(float* mc, float4 v)
 // The depth does not matter beyond 8: 76 MB on 8 x B200 take 228 / 234 / 241 us with 8 / 16 / 32 vectors in flight per
 // thread (NCCL: 309 us), 15 MB 60 / 60 / 61 us -- the transfer is bound by the switch path (each GPU's port moves
 // ~85 MB in each direction: ~375 GB/s), not by latency.
-#ifndef DMR_NVLS_UNROLL
-#define DMR_NVLS_UNROLL 8
-#endif
+constexpr int DMR_NVLS_UNROLL = 8;
 __device__ __forceinline__ void nvls_reduce_slice(float* __restrict__ mc, size_t i, size_t end, size_t stride)
 {
     for (; i < end; i += DMR_NVLS_UNROLL * stride) {
@@ -50,21 +48,11 @@ __device__ __forceinline__ void nvls_reduce_slice(float* __restrict__ mc, size_t
     }
 }
 
-// n4 = number of float4 of the whole buffer (the caller pads to a multiple of world); DMR_NVLS_UNROLL vectors in flight
-// per thread; persistent grid (one wave).
-__global__ void __launch_bounds__(512) nvls_allreduce_sum_kernel(float* __restrict__ mc, size_t n4, int rank, int world)
-{
-    const size_t per = n4 / (size_t)world;
-    const size_t begin = per * (size_t)rank, end = begin + per;
-    const size_t stride = (size_t)gridDim.x * blockDim.x;
-    size_t i = begin + (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    nvls_reduce_slice(mc, i, end, stride);
-}
-
 // ---------------------------------------------------------------------------
-// Same reduction with the two cross-GPU barriers INSIDE the kernel (no extra launches): the separate
+// The reduction with the two cross-GPU barriers INSIDE the kernel (no extra launches): separate
 // signal-pad barriers cost more than the transfer itself (15 MB on 8 GPUs: 63 us with two barrier kernels
 // around a ~10 us reduction).
+//   n4 = number of float4 of the whole buffer (the caller pads to a multiple of world); persistent grid (one wave).
 //   peer_flags[r] -> rank r's flag array in symmetric memory (W + 2 words used: word s = last epoch value
 //                    signalled by rank s); local_ctl: [0] = "go" flag, [1] = finished-CTA counter (this GPU only).
 //   epoch e = 1, 2, 3, ... (host counter, identical on all ranks); flag values only grow, nothing is reset.
@@ -127,31 +115,6 @@ __global__ void __launch_bounds__(512) nvls_allreduce_sum_fused_kernel(float* __
 }  // namespace dmr
 
 using namespace dmr;
-
-extern "C" int dmr_nvls_allreduce_sum_f32(void* multicast_ptr, size_t n_floats, int rank, int world, dmr_stream_t stream_)
-{
-    cudaStream_t stream = (cudaStream_t)stream_;
-    if (!multicast_ptr) { set_error("multicast_ptr is null"); return DMR_EINVAL; }
-    if (world <= 0 || rank < 0 || rank >= world) { set_error("bad rank/world"); return DMR_EINVAL; }
-    if (n_floats % (4 * (size_t)world) != 0) { set_error("n_floats must be a multiple of 4*world"); return DMR_EINVAL; }
-    if (((uintptr_t)multicast_ptr & 15) != 0) { set_error("multicast_ptr must be 16-byte aligned"); return DMR_EINVAL; }
-    const size_t n4 = n_floats / 4, per = n4 / (size_t)world;
-    if (per == 0) return DMR_OK;
-    static int sm_count = 0;
-    if (sm_count == 0) {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev);
-        if (sm_count <= 0) sm_count = 148;
-    }
-    size_t blocks = (per + 4 * 512 - 1) / (4 * 512);
-    if (blocks > (size_t)sm_count) blocks = (size_t)sm_count;   // one CTA per SM at most: the switch, not the SMs, is the limit
-    if (blocks == 0) blocks = 1;
-    count_launch(1);
-    nvls_allreduce_sum_kernel<<<(unsigned)blocks, 512, 0, stream>>>(static_cast<float*>(multicast_ptr), n4, rank, world);
-    DMR_LAUNCH_CHECK("nvls_allreduce_sum_kernel");
-    return DMR_OK;
-}
 
 // grid size of the fused kernel for a buffer of n_floats: fixed per buffer (the finished-CTA counter relies on it)
 static unsigned nvls_fused_blocks(size_t per)

@@ -60,13 +60,11 @@ struct ProfScope {
 // chain is set up and its CTAs become resident while the previous one is still draining.  EVERY kernel launched
 // this way begins with griddep_wait() -- it blocks until the preceding kernel has completed and its writes are
 // visible -- so the data flow is exactly that of ordinary stream order; only the launch latency overlaps.
-// DMESH_B200_NO_PDL=1 in the environment restores ordinary launches (A/B timing).
 // ---------------------------------------------------------------------------
 __device__ __forceinline__ void griddep_wait()
 {
     asm volatile("griddepcontrol.wait;" ::: "memory");
 }
-bool pdl_enabled();
 template <typename... KArgs, typename... Args>
 inline cudaError_t dmr_launch(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args&&... args)
 {
@@ -76,7 +74,7 @@ inline cudaError_t dmr_launch(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = pdl_enabled() ? 1 : 0;
+    cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 

@@ -24,9 +24,7 @@ namespace dmr {
 // algorithmic bytes per (b,p): 4 (depth) read, 16 written; + 12 (xyz) per vertex and call.
 // The reference also stores ndc.xy (never read downstream, SURVEY 8a1).
 // ---------------------------------------------------------------------------
-#ifndef DMR_POINTS_PER_THREAD
-#define DMR_POINTS_PER_THREAD 4
-#endif
+constexpr int DMR_POINTS_PER_THREAD = 4;
 __global__ void __launch_bounds__(256) preprocess_points_kernel(
     int B, int P, int W, int H,
     const float* __restrict__ verts, const float* __restrict__ mv_mats, const float* __restrict__ proj_mats,
@@ -330,9 +328,7 @@ __device__ __forceinline__ void edge_setup(float2 p1, float2 p2, float2 p3, int 
 // algorithmic bytes per (b,f): read 3*16 (vimg) + 4 (intensity), write 4 + 4 + 8 + 144; per face and call: read
 // 12 (idx) + 3*12 (pos) + 3*12 (colour) + 4 (opacity).
 // ---------------------------------------------------------------------------
-#ifndef DMR_FACES_MINB
-#define DMR_FACES_MINB 4
-#endif
+constexpr int DMR_FACES_MINB = 4;
 template <bool HIST, bool MULTI>   // HIST: accumulate the face sort's histograms as a by-product (small inputs only);
                                    // MULTI = false: B == 1 (no view loop: 58 instead of 64 registers + spills)
 __global__ void __launch_bounds__(256, DMR_FACES_MINB) tri_preprocess_faces_kernel(

@@ -29,38 +29,23 @@ namespace dmr {
 //     512 x 16, 1 CTA (124 regs)     246 us        256 x 24 / 32, 2 CTAs        205 / 207 us (spills)
 // More keys per thread amortise the per-tile work (256-digit scan, look-back, three barriers); the 4096-key tile is
 // kept because the 5120 / 8192-key shapes cost 20 % on the small face sorts (C1: 30 -> 36 us).
-#ifndef DMR_RS_THREADS
-#define DMR_RS_THREADS 256
-#endif
-#ifndef DMR_RS_KPT
-#define DMR_RS_KPT 16
-#endif
-#ifndef DMR_RS_MINB
-#define DMR_RS_MINB 4
-#endif
-#ifndef DMR_RS_SPLIT_RANK
-#define DMR_RS_SPLIT_RANK 0   // 1: form the peer masks of all rounds before the serial running-offset updates (more ILP, KPT more registers)
-#endif
-#define RS_TILE_KEYS (DMR_RS_THREADS * DMR_RS_KPT)
-#define RS_MIN_TILE 2048   // smallest tile of any configuration of the large shape (sizes the descriptor array)
+constexpr int DMR_RS_THREADS = 256;
+constexpr int DMR_RS_KPT = 16;
+constexpr int DMR_RS_MINB = 4;
+constexpr int RS_TILE_KEYS = DMR_RS_THREADS * DMR_RS_KPT;
+#define RS_MIN_TILE 2048   // the descriptor array is sized for tiles of at least this many keys
 // Small sorts (the face / tile sorts of C1, C2) are a handful of tiles on an otherwise idle GPU: a pass lasts as long as
 // ONE tile takes (16 serial ranking rounds, ~6 us), not as long as the data takes to move.  Up to RS_SMALL_N keys the
 // tiles are 256 x RS_SMALL_KPT keys: four times as many CTAs, a quarter of the serial rounds each.
 // (Measured and rejected for these sizes: 32 instead of 8 descriptors per look-back step -- the walk over the
 // predecessors is not what a small pass waits for.  And for the large shape: key and value through shared memory as
 // one 64-bit word, one STS.64 / LDS.64 per pair: C5 pass 182.7 -> 186.8 us.)
-#ifndef RS_SMALL_N
-#define RS_SMALL_N (1u << 20)
-#endif
-#ifndef RS_SMALL_KPT
-#define RS_SMALL_KPT 8
-#endif
-#define RS_SMALL_TILE (256 * RS_SMALL_KPT)
+constexpr unsigned RS_SMALL_N = 1u << 20;
+constexpr int RS_SMALL_KPT = 8;
+constexpr int RS_SMALL_TILE = 256 * RS_SMALL_KPT;
 __host__ __device__ constexpr size_t rs_tile_keys(size_t n) { return n <= RS_SMALL_N ? (size_t)RS_SMALL_TILE : (size_t)RS_TILE_KEYS; }
 static_assert(DMR_RS_THREADS >= 256 && DMR_RS_THREADS % 32 == 0 && RS_TILE_KEYS >= RS_MIN_TILE, "onesweep tile shape");
-#ifndef RS_LB
-#define RS_LB 8          // look-back descriptors fetched per step (C5 pass: 8 -> 180 us, 16 -> 185 us, 32 -> 186 us)
-#endif
+constexpr int RS_LB = 8;         // look-back descriptors fetched per step (C5 pass: 8 -> 180 us, 16 -> 185 us, 32 -> 186 us)
 
 #define RS_FLAG_AGG  (1u << 30)
 #define RS_FLAG_INCL (2u << 30)
@@ -287,8 +272,9 @@ __device__ __forceinline__ void rs_onesweep_tile(const RsBuffers<KeyT>& buf, siz
     __syncthreads();
 
     // ---- stable rank inside the warp (running per-warp offsets), scatter into shared memory.
-    //      The peer masks of all RS_KPT rounds are formed first (independent ballots, no memory traffic in between);
-    //      only the running-offset update is serial.
+    //      One round per key of the thread: digit_peers gives the lanes holding the same digit (padding lanes of a
+    //      partial tile form a class of their own), the lowest of them advances the warp's running offset for that
+    //      digit, and each lane scatters to digit base + offset + its rank among the peers.
     //      (Measured and rejected: packed per-round counters -- 8 x 8-bit counts per (warp, digit) filled by the
     //      leader of every digit run, ranks from byte prefixes -- which make the 8 rounds independent of each
     //      other: 306 vs 282 us per pass at C5; the extra shared-memory traffic costs more than the chain.
@@ -298,31 +284,13 @@ __device__ __forceinline__ void rs_onesweep_tile(const RsBuffers<KeyT>& buf, siz
     //      182.7 -> 182.7 us, C4 105 / 99 -> 107 / 103 us, face sorts +2..6 % -- the aggregate is published a ranking
     //      phase later and the successors' look-back waits for it; the atomics were not what the pass waits for.)
     const uint32_t lt_mask = (1u << lane) - 1u;
-#if DMR_RS_SPLIT_RANK
-    unsigned peers[RS_KPT];
-#pragma unroll
-    for (int i = 0; i < RS_KPT; i++) {
-        if (FULL) {
-            peers[i] = digit_peers<NBITS>(dig[i], 0xffffffffu);
-        } else {
-            const bool ok = wbase + i * 32 + lane < nvalid;
-            unsigned pm = __ballot_sync(0xffffffffu, ok);
-            if (!ok) pm = ~pm;                               // padding: own class
-            peers[i] = digit_peers<NBITS>(dig[i], pm);
-        }
-    }
-#endif
 #pragma unroll
     for (int i = 0; i < RS_KPT; i++) {
         const bool ok = FULL || wbase + i * 32 + lane < nvalid;
         const uint32_t d = dig[i];
-#if DMR_RS_SPLIT_RANK
-        const unsigned pr = peers[i];
-#else
         unsigned pr = 0xffffffffu;
         if (!FULL) { pr = __ballot_sync(0xffffffffu, ok); if (!ok) pr = ~pr; }
         pr = digit_peers<NBITS>(d, pr);
-#endif
         const int leader = __ffs(pr) - 1;
         const uint32_t before = __popc(pr & lt_mask);
         uint32_t old = 0;

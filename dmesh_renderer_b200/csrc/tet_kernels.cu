@@ -467,15 +467,11 @@ int tet_first_intersect(const TetParams& p, cudaStream_t stream)
 // The march is independent per pixel (no shared memory, no tile lists) and its cost per ray has a
 // long tail (rays along the cube diagonal cross several times more faces than the mean), so it is
 // launched as many small CTAs: 64 threads = 8x8 pixels = two 8x4 warps.
-#ifndef MARCH_THREADS
-#define MARCH_THREADS 64
-#endif
-#define MARCH_ROWS (MARCH_THREADS / 8)   // pixel rows of a CTA: 8 columns x 4 rows per warp
+constexpr int MARCH_THREADS = 64;
+constexpr int MARCH_ROWS = MARCH_THREADS / 8;   // pixel rows of a CTA: 8 columns x 4 rows per warp
 // 10 CTAs/SM = 96 registers (forward march at C3 after the depth computation left the loop: 8 CTAs / 112 registers
 // 820 us, 10 / 96 (2 spill slots) 772 us, 12 / 80 (14 spill accesses per step) 783 us; round 1: 64 registers 947 us)
-#ifndef MARCH_MIN_BLOCKS
-#define MARCH_MIN_BLOCKS 10
-#endif
+constexpr int MARCH_MIN_BLOCKS = 10;
 
 struct TetStep {   // result of looking for the exit (or entry) face of a tet
     int face, tet;

@@ -166,10 +166,8 @@ __device__ __forceinline__ void stage_records_warp(uint4* __restrict__ dstw, con
     __syncwarp();
 }
 
-#ifndef HB
-#define HB 256           // staged instances a warp compacts / rasterises / shades in one go (measured: 128 -> 256 = -5 % at C4, -3 % at C2, +-0 at C5)
-#endif
-#define HS (HB / 32)     // 32-entry slices of the compacted list of such a pass
+constexpr int HB = 256;          // staged instances a warp compacts / rasterises / shades in one go (measured: 128 -> 256 = -5 % at C4, -3 % at C2, +-0 at C5)
+constexpr int HS = HB / 32;      // 32-entry slices of the compacted list of such a pass
 
 // (Measured and rejected, round 2: L2 prefetch -- prefetch.global.L2, SASS CCTL.E.PF2, one per 32-byte sector -- of the
 // record each thread stages in the NEXT round and of the first round of the tile two waves of CTAs later in the grid.
@@ -210,9 +208,7 @@ __device__ __forceinline__ void stage_records_warp(uint4* __restrict__ dstw, con
 //       whole pass are known up front, so a lane with few hits in one 32-instance slice moves straight on to the
 //       next one: the number of SIMD passes is the largest per-pixel hit count over HB instances, not the sum of
 //       the per-slice maxima (the shading path ran at 15 of 32 lanes before).
-#ifndef DMR_TRI_FWD_MINB
-#define DMR_TRI_FWD_MINB 4
-#endif
+constexpr int DMR_TRI_FWD_MINB = 4;
 __global__ void __launch_bounds__(256, DMR_TRI_FWD_MINB) tri_render_fwd_kernel(TriRenderParams p)
 {
     griddep_wait();   // programmatic dependent launch: see dmr_launch (common.cuh)
@@ -419,14 +415,7 @@ static_assert(stat_slot_is_permutation(), "stat_slot must map the 24 statistics 
 // Resident CTAs per SM.  3 (80 registers, no spills) against 4 (64 registers, 80 bytes of spill): the kernel issues
 // on only ~64 % of the cycles with 5.6 warps per scheduler and its stalls spread evenly over memory, barrier and
 // dependency waits, so two more warps per scheduler win slightly -- C4 3677 -> 3640 us, C5 788 -> 766 us, C2 291 -> 289 us.
-#ifndef DMR_TRI_BWD_MINB
-#define DMR_TRI_BWD_MINB 4
-#endif
-// 1 = form 1/(1-alpha) once per staged instance and multiply, instead of the reference's two divisions per covered
-// pixel (backward.cu:244-252, 299-308).  Changes T and the background term by an ulp per step.
-#ifndef DMR_TRI_BWD_RCP_ALPHA
-#define DMR_TRI_BWD_RCP_ALPHA 1
-#endif
+constexpr int DMR_TRI_BWD_MINB = 4;
 // Camera gradients (CAM = true; DESIGN.md 3.3).  The rays are the only place the camera enters a pixel's colour and
 // depth: ro = inv_mv[12..14], rd = d / (|d| + 1e-7), d = L pv, pv = (inv_proj (nx, ny, -1, 1)).xyz, L = the linear
 // part of inv_mv.  Per covered hit, with T = ro - p0, E1, E2, P = rd x E2, Q = T x E1, D = P.E1, u = P.T / D and
@@ -613,13 +602,11 @@ __device__ __forceinline__ void tri_render_bwd_body(const TriRenderParams& p, fl
                         const float iC0 = raw0 * intense, iC1 = raw1 * intense, iC2 = raw2 * intense;
                         const float iD = i0 * q6.w + i1 * q7.w + i2 * q8.w;
 
-                        // backward.cu:244-252
-#if DMR_TRI_BWD_RCP_ALPHA
+                        // backward.cu:244-252.  1/(1-alpha) is formed once per staged instance and multiplied, instead
+                        // of the reference's two divisions per covered pixel (here and in the background term,
+                        // backward.cu:299-308); T and the background term change by an ulp per step.
                         const float rcpa = lds_f32(&sh[2].w);
                         if (!T_first) T = T * rcpa;
-#else
-                        if (!T_first) T = T / (1.f - alpha);
-#endif
                         T_first = false;
 
                         float dL_dalpha = 0.0f;
@@ -640,11 +627,7 @@ __device__ __forceinline__ void tri_render_bwd_body(const TriRenderParams& p, fl
                         // times dL_dD.  The pixel constants -T_final * (bg . dL_dC + dL_dD) and its alpha == 1 counterpart
                         // are formed once (two live registers instead of four; one rounding apart from the reference's
                         // two separate products, far inside the gradient tolerance)
-#if DMR_TRI_BWD_RCP_ALPHA
                         dL_dalpha += (alpha == 1.0f) ? bgk1 : bgk * rcpa;
-#else
-                        dL_dalpha += (alpha == 1.0f) ? bgk1 : bgk / (1.f - alpha);
-#endif
 
                         // backward.cu:327-349.  The per-term products are the reference's; the common factor
                         // dic*intense is formed once (the reference multiplies (x*dic)*intense per term: one
@@ -780,9 +763,7 @@ __global__ void __launch_bounds__(256, DMR_TRI_BWD_MINB) tri_render_bwd_det_kern
 
 // Camera-gradient instantiations: the same walk plus g_ro / g_rd per lane (six more live floats) and the per-tile
 // record.  Resident CTAs per SM: see DESIGN.md 3.3 for the -Xptxas -v figures of both choices.
-#ifndef DMR_TRI_BWD_CAM_MINB
-#define DMR_TRI_BWD_CAM_MINB 3
-#endif
+constexpr int DMR_TRI_BWD_CAM_MINB = 3;
 __global__ void __launch_bounds__(256, DMR_TRI_BWD_CAM_MINB) tri_render_bwd_cam_kernel(TriRenderParams p, float* cam_tiles)
 {
     griddep_wait();   // programmatic dependent launch: see dmr_launch (common.cuh)

@@ -68,7 +68,6 @@ class PackedSceneGrads:
                  use_nvls: Optional[bool] = None):
         self.leaves = [verts, verts_color, faces_opacity]
         self.group = group
-        self._fused = True             # barriers inside the all-reduce kernel (False: separate signal-pad barriers)
         n = sum(t.numel() for t in self.leaves)
         self._nvls = None
         # which collective all_reduce() runs and, for the fallback, why: "nvls" | "nccl: <reason>" | "none: <reason>"
@@ -171,20 +170,15 @@ class PackedSceneGrads:
         if self._nvls is not None:
             import ctypes
             from . import _lib
-            hdl, mc, n_pad, rank, ws = self._nvls
+            _, mc, n_pad, rank, ws = self._nvls
             stream = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
-            if self._fused and self._epoch < (1 << 30) - 2:
-                # one launch: barrier ("every rank's gradients are complete") -> in-switch reduce + broadcast of this
-                # rank's slice -> barrier ("every slice has been broadcast"), all inside the kernel
-                self._epoch += 1
-                flags, fh, peer_ptrs, ctl = self._flags
-                _lib.check(_lib.load().dmr_nvls_allreduce_sum_f32_fused(ctypes.c_void_p(mc), n_pad, rank, ws,
-                                                                        ctypes.c_void_p(peer_ptrs), ctypes.c_void_p(ctl.data_ptr()),
-                                                                        self._epoch, stream))
-                return None
-            hdl.barrier(channel=0)        # signal-pad barriers as separate launches
-            _lib.check(_lib.load().dmr_nvls_allreduce_sum_f32(ctypes.c_void_p(mc), n_pad, rank, ws, stream))
-            hdl.barrier(channel=0)
+            # one launch: barrier ("every rank's gradients are complete") -> in-switch reduce + broadcast of this
+            # rank's slice -> barrier ("every slice has been broadcast"), all inside the kernel
+            self._epoch += 1
+            flags, fh, peer_ptrs, ctl = self._flags
+            _lib.check(_lib.load().dmr_nvls_allreduce_sum_f32_fused(ctypes.c_void_p(mc), n_pad, rank, ws,
+                                                                    ctypes.c_void_p(peer_ptrs), ctypes.c_void_p(ctl.data_ptr()),
+                                                                    self._epoch, stream))
             return None
         group = group if group is not None else self.group
         if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:

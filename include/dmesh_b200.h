@@ -376,14 +376,12 @@ int    dmr_sort_pairs_u32(const uint32_t* keys_in, const uint32_t* vals_in,
 /* (SURVEY.md 8e); this is the single collective of the camera-sharded step.  */
 /* `multicast_ptr` = multicast address of the buffer (every rank passes ITS   */
 /* view of the same multicast object), n_floats a multiple of 4*world.  Rank r */
-/* reduces and broadcasts slice r; the caller issues a cross-GPU barrier on   */
-/* `stream` before and after the call.                                        */
+/* reduces and broadcasts slice r, between two cross-GPU barriers inside the  */
+/* kernel.  `peer_flag_ptrs_dev`: DEVICE array of `world` pointers, entry r = */
+/* rank r's flag words (>= world uint32, zero-initialised symmetric memory);  */
+/* `local_ctl`: 2 zero-initialised uint32 on this GPU; `epoch` = 1, 2, 3, ... */
+/* (< 2^30) identical on all ranks, one per call on a given flag buffer.      */
 /* ------------------------------------------------------------------------ */
-int dmr_nvls_allreduce_sum_f32(void* multicast_ptr, size_t n_floats, int rank, int world, dmr_stream_t stream);
-/* The same with both cross-GPU barriers inside the kernel.  `peer_flag_ptrs_dev`: DEVICE array of `world`    */
-/* pointers, entry r = rank r's flag words (>= world uint32, zero-initialised symmetric memory);              */
-/* `local_ctl`: 2 zero-initialised uint32 on this GPU; `epoch` = 1, 2, 3, ... identical on all ranks, one per  */
-/* call on a given flag buffer.                                                                                */
 int dmr_nvls_allreduce_sum_f32_fused(void* multicast_ptr, size_t n_floats, int rank, int world,
                                      void* const* peer_flag_ptrs_dev, void* local_ctl, unsigned epoch,
                                      dmr_stream_t stream);

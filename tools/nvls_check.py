@@ -54,11 +54,8 @@ def timeit(fn, n=50):
 
 
 t_fused = timeit(g.all_reduce)
-g._fused = False
-t_sep = timeit(g.all_reduce)
-g._fused = True
 t_nccl = timeit(lambda: dist.all_reduce(g.flat))
 if rank == 0:
-    print("all-reduce of %.1f MB on %d GPUs: NVLS kernel with in-kernel barriers %.1f us, with separate barrier launches %.1f us, "
-          "NCCL %.1f us" % (g.flat.numel() * 4 / 1e6, ws, t_fused, t_sep, t_nccl), flush=True)
+    print("all-reduce of %.1f MB on %d GPUs: NVLS kernel with in-kernel barriers %.1f us, NCCL %.1f us"
+          % (g.flat.numel() * 4 / 1e6, ws, t_fused, t_nccl), flush=True)
 dist.destroy_process_group()
