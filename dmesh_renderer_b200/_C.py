@@ -577,14 +577,16 @@ def render_tets(background, verts, faces, verts_color, faces_opacity, mv_mats, p
 def render_tets_backward(background, verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, inv_mv_mats,
                          inv_proj_mats, verts_depth, faces_intense, tets, face_tets, tet_faces, grad_color, grad_depth,
                          pointBuffer, faceBuffer, binningBuffer, imageBuffer, ray_random_seed=None, deterministic=False,
-                         tet_records=None):
+                         tet_records=None, camera_grads=False):
     """RenderFTetsBackwardCUDA (render.cu:338-412).
     Returns (dL_dverts_color[P,3], dL_dfaces_opacity[F]).  `ray_random_seed` is an
     optional trailing argument beyond the reference's 20: the autograd wrapper passes
     the forward's seed so that jittered rays (seed > 0) are re-read from the image
     buffer; with the reference's 20 arguments pixel-centre rays are used.  `deterministic`: run-to-run reproducible
     gradients (dmr_tet_backward_deterministic).  `tet_records`: the adjacency records of the forward call (the
-    autograd wrapper passes them; otherwise they are taken from the face buffer's attribute or rebuilt)."""
+    autograd wrapper passes them; otherwise they are taken from the face buffer's attribute or rebuilt).
+    `camera_grads`: also return dL_dmv_mats, dL_dproj_mats [B,4,4] (gradients with respect to the mv_mats / proj_mats
+    tensors passed here, through the rays and the hit-point depth; dmr_tet_backward_camera) as two more elements."""
     lib = _lib.load()
     B, P, F, T = mv_mats.size(0), verts.size(0), faces.size(0), tets.size(0)
     H, W = grad_color.size(2), grad_color.size(3)
@@ -595,6 +597,8 @@ def render_tets_backward(background, verts, faces, verts_color, faces_opacity, m
         z = dict(dtype=torch.float32, device=dev)
         dL_dverts_color = torch.zeros((P, 3), **z)
         dL_dfaces_opacity = torch.zeros((F,), **z)
+        # [B,16] column-major = [B,4,4] gradients of the (column-major, i.e. transposed) matrix tensors given here
+        cam = torch.zeros((2, B, 4, 4), **z) if camera_grads else None
         if B * H * W > 0 and F > 0 and T > 0:
             bg = _f32(background, "background")
             mv, pj = _f32(mv_mats, "mv_mats"), _f32(proj_mats, "proj_mats")
@@ -612,10 +616,17 @@ def render_tets_backward(background, verts, faces, verts_color, faces_opacity, m
             a = (B, P, F, T, W, H, int(ray_random_seed), _ptr(bg), _ptr(mv), _ptr(pj), _ptr(imv), _ptr(ipj), _ptr(fint),
                  _ptr(pointBuffer), _ptr(faceBuffer), _ptr(tet_rec), _ptr(imageBuffer), _ptr(gc), _ptr(gd),
                  _ptr(dL_dverts_color), _ptr(dL_dfaces_opacity))
-            if deterministic:
+            if camera_grads:
+                ws = torch.empty(lib.dmr_tet_backward_camera_bytes(B, P, F, W, H, int(bool(deterministic))),
+                                 dtype=torch.uint8, device=dev)
+                _lib.check(lib.dmr_tet_backward_camera(*a, int(bool(deterministic)), _ptr(cam[0]), _ptr(cam[1]), _ptr(ws),
+                                                       ws.numel(), _stream()))
+            elif deterministic:
                 ws = torch.empty(lib.dmr_tet_backward_deterministic_bytes(P, F), dtype=torch.uint8, device=dev)
                 _lib.check(lib.dmr_tet_backward_deterministic(*a, _ptr(ws), ws.numel(), _stream()))
             else:
                 ws = torch.empty(lib.dmr_tet_backward_workspace_bytes(P), dtype=torch.uint8, device=dev)
                 _lib.check(lib.dmr_tet_backward(*a, _ptr(ws), ws.numel(), _stream()))
+    if camera_grads:
+        return dL_dverts_color, dL_dfaces_opacity, cam[0], cam[1]
     return dL_dverts_color, dL_dfaces_opacity

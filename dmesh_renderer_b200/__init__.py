@@ -149,7 +149,7 @@ class TriRenderer(th.nn.Module):
 
 # =============================================================================
 # TetRenderer: faces of a tetrahedral complex, exact depth order by ray marching
-# through tet adjacency; gradients to vertex colours and face opacities only.
+# through tet adjacency; gradients to vertex colours, face opacities and (opt-in) the camera matrices.
 # =============================================================================
 class TetRenderSettings(NamedTuple):      # reference __init__.py:237-241
     image_height: int
@@ -201,14 +201,23 @@ class _RenderTet(th.autograd.Function):
         args = (render_settings.bg, verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, inv_mv_mats,
                 inv_proj_mats, verts_depth, faces_intense, tets, face_tets, tet_faces, grad_out_color, grad_out_depth,
                 pointBuffer, faceBuffer, binningBuffer, imgBuffer, render_settings.ray_random_seed)
+        # camera gradients (extension): requested by setting requires_grad on mv_mats or proj_mats; per view, through
+        # autograd only
+        camera = ctx.needs_input_grad[4] or ctx.needs_input_grad[5]
+        grad_mv = grad_proj = None
         try:
-            grad_verts_color, grad_faces_opacity = _C.render_tets_backward(*args, deterministic=ctx.deterministic,
-                                                                           tet_records=ctx.tet_records)
+            grads = _C.render_tets_backward(*args, deterministic=ctx.deterministic, tet_records=ctx.tet_records,
+                                            camera_grads=camera)
         except Exception as ex:
             print("\nAn error occured in backward.\n")
             raise ex
-        # gradient positions: reference __init__.py:407-422
-        return (None, None, grad_verts_color, grad_faces_opacity, None, None, None, None, None, None, None, None, None)
+        grad_verts_color, grad_faces_opacity = grads[:2]
+        if camera:
+            grad_mv, grad_proj = grads[2], grads[3]
+        # gradient positions: reference __init__.py:407-422; positions 4 and 5 (the matrices) are an extension
+        return (None, None, grad_verts_color, grad_faces_opacity,
+                grad_mv if ctx.needs_input_grad[4] else None, grad_proj if ctx.needs_input_grad[5] else None,
+                None, None, None, None, None, None, None)
 
 
 class TetRenderer(th.nn.Module):
@@ -222,8 +231,8 @@ class TetRenderer(th.nn.Module):
     def forward(self, verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, verts_depth, faces_intense, tets,
                 face_tets, tet_faces):
         """
-        Gradients only for verts_color and faces_opacity.  verts_depth is accepted
-        but unused (depth comes from the re-projected hit point).
+        Gradients for verts_color and faces_opacity, and (extension) for mv_mats / proj_mats when they require
+        grad.  verts_depth is accepted but unused (depth comes from the re-projected hit point).
         tets [T,4], face_tets [F,2] (-1 = boundary), tet_faces [T,4]
         returns color [B,3,H,W], depth [B,1,H,W], active [B,H,W] bool
         """

@@ -34,7 +34,7 @@ static const char* const g_stage_names[ST_COUNT] = {
     "sort_pass0", "sort_pass1", "sort_pass2", "sort_pass3", "sort_pass4", "sort_pass5", "sort_pass6", "sort_pass7",
     "tile_ranges", "tri_render_forward", "tri_render_backward", "tri_grad_finish", "tet_build_records", "tet_jitter",
     "tet_first_intersect", "tet_march_forward", "tet_march_backward", "tet_grad_vertex", "tri_render_backward_camera",
-    "tri_camera_finish", "depth_chain_camera", "depth_chain_camera_finish" };
+    "tri_camera_finish", "depth_chain_camera", "depth_chain_camera_finish", "tet_march_backward_camera", "tet_camera_finish" };
 struct Prof {
     bool on = false, created = false;
     cudaEvent_t ev[ST_COUNT][2];
@@ -452,6 +452,7 @@ int dmr_debug_view(int renderer, int kind, int B, int P, int F, int T, int W, in
         case DMR_VIEW_FINAL_T:       off = IL.final_log_T; n = BI; break;
         case DMR_VIEW_FIRST_FACE:    off = IL.first_face; n = BI; break;
         case DMR_VIEW_FIRST_TET:     off = IL.first_tet; n = BI; break;
+        case DMR_VIEW_TET_JITTER:    off = IL.jitter; n = BI; break;
         default: set_error("unknown view kind %d", kind); return DMR_EINVAL;
         }
     }

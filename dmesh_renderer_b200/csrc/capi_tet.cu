@@ -31,6 +31,20 @@ bool tet_sizes_ok(long long B, long long P, long long F, long long T, long long 
     return true;
 }
 
+// scratch of the backward pass of either mode (dmr_tet_backward_workspace_bytes without its slack,
+// dmr_tet_backward_deterministic_bytes)
+size_t tet_bwd_scratch_bytes(int P, int F, bool deterministic)
+{
+    return deterministic ? TetDetLayout::make((size_t)P, (size_t)F).total : sizeof(float4) * (size_t)P;
+}
+
+// workspace of the camera-gradient backward: the mode's own scratch, then DMR_TET_CAM_REC floats per (view, march CTA)
+size_t tet_cam_bytes(int B, int P, int F, int W, int H, bool deterministic)
+{
+    return align_up(tet_bwd_scratch_bytes(P, F, deterministic), 256) +
+           align_up(sizeof(float) * DMR_TET_CAM_REC * tet_cam_records((size_t)B, W, H), 256) + 256;
+}
+
 }  // namespace
 
 extern "C" {
@@ -158,8 +172,9 @@ static int tet_backward_impl(int B, int P, int F, int T, int W, int H, int ray_r
                              const void* face_buffer, const void* tet_records, const void* image_buffer,
                              const float* dL_dcolor, const float* dL_ddepth, float* dL_dverts_color,
                              float* dL_dfaces_opacity, void* workspace, size_t workspace_bytes, bool deterministic,
-                             dmr_stream_t stream_)
+                             dmr_stream_t stream_, float* dL_dmv = nullptr, float* dL_dproj = nullptr)
 {
+    const bool cam = dL_dmv != nullptr;
     cudaStream_t stream = (cudaStream_t)stream_;
     if (!tet_sizes_ok(B, P, F, T, W, H)) return DMR_ETOOLARGE;
     if (B == 0 || F == 0 || T == 0) return DMR_OK;
@@ -169,6 +184,17 @@ static int tet_backward_impl(int B, int P, int F, int T, int W, int H, int ray_r
         return DMR_EINVAL;
     }
     (void)point_buffer;
+    // camera gradients: one record per (view, march CTA) behind the mode's own scratch, written by every CTA, so it is
+    // not cleared
+    float* cam_rec = nullptr;
+    if (cam) {
+        const size_t need = tet_cam_bytes(B, P, F, W, H, deterministic);
+        if (!workspace || workspace_bytes < need) {
+            set_error("camera-gradient backward needs a workspace of %zu bytes (dmr_tet_backward_camera_bytes)", need);
+            return DMR_EINVAL;
+        }
+        cam_rec = at<float>(workspace, align_up(tet_bwd_scratch_bytes(P, F, deterministic), 256));
+    }
     void* det_workspace = workspace;
     const size_t det_workspace_bytes = workspace_bytes;
     TetParams p;
@@ -188,7 +214,9 @@ static int tet_backward_impl(int B, int P, int F, int T, int W, int H, int ray_r
         p.det_fopa = at<long long>(det_workspace, DL.fopa);
         p.grad_vacc = nullptr;
         DMR_CUDA(cudaMemsetAsync(det_workspace, 0, DL.total, stream));
-        return tet_march_backward_deterministic(p, stream);
+        int rc = tet_march_backward_deterministic(p, stream, cam_rec);
+        if (rc || !cam) return rc;
+        return tet_camera_finish(p, cam_rec, dL_dmv, dL_dproj, stream);
     }
     // backward scratch: float4 per vertex (colour gradient, 16-byte aligned for red.v4) in the caller's workspace
     if (!workspace || workspace_bytes < sizeof(float4) * (size_t)P) {
@@ -197,7 +225,9 @@ static int tet_backward_impl(int B, int P, int F, int T, int W, int H, int ray_r
     }
     p.grad_vacc = static_cast<float4*>(workspace);
     DMR_CUDA(cudaMemsetAsync(p.grad_vacc, 0, sizeof(float4) * (size_t)P, stream));
-    return tet_march_backward(p, stream);
+    int rc = tet_march_backward(p, stream, cam_rec);
+    if (rc || !cam) return rc;
+    return tet_camera_finish(p, cam_rec, dL_dmv, dL_dproj, stream);
 }
 
 int dmr_tet_backward(int B, int P, int F, int T, int W, int H, int ray_random_seed, const float* background,
@@ -243,6 +273,27 @@ int dmr_tet_backward_deterministic(int B, int P, int F, int T, int W, int H, int
     return tet_backward_impl(B, P, F, T, W, H, ray_random_seed, background, mv_mats, proj_mats, inv_mv_mats,
                              inv_proj_mats, faces_intense, point_buffer, face_buffer, tet_records, image_buffer, dL_dcolor,
                              dL_ddepth, dL_dverts_color, dL_dfaces_opacity, workspace, workspace_bytes, true, stream);
+}
+
+size_t dmr_tet_backward_camera_bytes(int B, int P, int F, int W, int H, int deterministic)
+{
+    if (B < 0 || P < 0 || F < 0 || W < 0 || H < 0) return 0;
+    return tet_cam_bytes(B, P, F, W, H, deterministic != 0);
+}
+
+int dmr_tet_backward_camera(int B, int P, int F, int T, int W, int H, int ray_random_seed, const float* background,
+                            const float* mv_mats, const float* proj_mats, const float* inv_mv_mats,
+                            const float* inv_proj_mats, const float* faces_intense, const void* point_buffer,
+                            const void* face_buffer, const void* tet_records, const void* image_buffer,
+                            const float* dL_dcolor, const float* dL_ddepth, float* dL_dverts_color,
+                            float* dL_dfaces_opacity, int deterministic, float* dL_dmv, float* dL_dproj, void* workspace,
+                            size_t workspace_bytes, dmr_stream_t stream)
+{
+    if (B > 0 && (!dL_dmv || !dL_dproj)) { set_error("null pointer"); return DMR_EINVAL; }
+    return tet_backward_impl(B, P, F, T, W, H, ray_random_seed, background, mv_mats, proj_mats, inv_mv_mats,
+                             inv_proj_mats, faces_intense, point_buffer, face_buffer, tet_records, image_buffer, dL_dcolor,
+                             dL_ddepth, dL_dverts_color, dL_dfaces_opacity, workspace, workspace_bytes, deterministic != 0,
+                             stream, dL_dmv, dL_dproj);
 }
 
 int dmr_debug_set_tet_first_split(int split)

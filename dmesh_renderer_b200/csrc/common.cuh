@@ -41,7 +41,7 @@ enum Stage {
     ST_POINTS = 0, ST_FACES, ST_FACE_SORT, ST_SCAN, ST_DUPLICATE, ST_SORT_HIST, ST_SORT_PLAN,
     ST_SORT_PASS0, ST_SORT_PASS1, ST_SORT_PASS2, ST_SORT_PASS3, ST_SORT_PASS4, ST_SORT_PASS5, ST_SORT_PASS6, ST_SORT_PASS7,
     ST_RANGES, ST_TRI_FWD, ST_TRI_BWD, ST_TRI_BWD_FINISH, ST_TET_RECORDS, ST_TET_JITTER, ST_TET_FIRST, ST_TET_FWD, ST_TET_BWD, ST_TET_BWD_FINISH,
-    ST_TRI_BWD_CAM, ST_TRI_CAM_FINISH, ST_DEPTH_CAM, ST_DEPTH_CAM_FINISH, ST_COUNT
+    ST_TRI_BWD_CAM, ST_TRI_CAM_FINISH, ST_DEPTH_CAM, ST_DEPTH_CAM_FINISH, ST_TET_BWD_CAM, ST_TET_CAM_FINISH, ST_COUNT
 };
 void count_launch(int n);
 void prof_begin(int stage, cudaStream_t s, bool count = true);   // count: also counts one kernel launch
@@ -124,6 +124,21 @@ __device__ __forceinline__ float4 xform44(float3 p, const float* m)
                        m[1] * p.x + m[5] * p.y + m[9] * p.z + m[13],
                        m[2] * p.x + m[6] * p.y + m[10] * p.z + m[14],
                        m[3] * p.x + m[7] * p.y + m[11] * p.z + m[15]);
+}
+
+// Entry (i, j) of N^T G N^T for column-major 4x4 N, G (M(r, c) = m[4c + r]).  With N = A^-1 and G = dL/dN, the
+// camera-gradient finish kernels of both renderers form dL/dA = -N^T G N^T from it.
+__device__ __forceinline__ float inverse_chain(const float* N, const float* G, int i, int j)
+{
+    float out = 0.0f;
+#pragma unroll
+    for (int a = 0; a < 4; a++) {
+        float h = 0.0f;                                // (G N^T)(a, j) = sum_c G(a, c) N(j, c)
+#pragma unroll
+        for (int c = 0; c < 4; c++) h += G[4 * c + a] * N[4 * c + j];
+        out += N[4 * i + a] * h;                       // N^T(i, a) = N(a, i)
+    }
+    return out;
 }
 
 // auxiliary.h:245-253

@@ -150,6 +150,11 @@ struct TetParams {
     long long* det_fopa;          // [F]
 };
 
+// Camera gradients of the backward march: one record of DMR_TET_CAM_REC floats per (view, march CTA of 8 x 8 pixels),
+// written by every CTA (layout: tet_march_bwd_cam, tet_kernels.cu).
+#define DMR_TET_CAM_REC 32
+__host__ __device__ inline size_t tet_cam_records(size_t B, int W, int H) { return B * (size_t)((W + 7) / 8) * ((H + 7) / 8); }
+
 struct TetDetLayout {             // workspace of the deterministic backward pass
     size_t gmax, vert, fopa, total;
     static TetDetLayout make(size_t P, size_t F)
@@ -183,7 +188,11 @@ int tet_build_records(int P, int F, int T, const float* verts, const int* faces,
 int tet_jitter(int B, int W, int H, int seed, float2* jitter, cudaStream_t stream);
 int tet_first_intersect(const TetParams& p, cudaStream_t stream);
 int tet_march_forward(const TetParams& p, cudaStream_t stream);
-int tet_march_backward(const TetParams& p, cudaStream_t stream);
-int tet_march_backward_deterministic(const TetParams& p, cudaStream_t stream);
+// cam_rec != nullptr: the camera-gradient kernels, which also store one DMR_TET_CAM_REC-float record per (view, march
+// CTA) there
+int tet_march_backward(const TetParams& p, cudaStream_t stream, float* cam_rec = nullptr);
+int tet_march_backward_deterministic(const TetParams& p, cudaStream_t stream, float* cam_rec = nullptr);
+// records of a view -> += dL_dmv[B,16], dL_dproj[B,16]
+int tet_camera_finish(const TetParams& p, const float* cam_rec, float* dL_dmv, float* dL_dproj, cudaStream_t stream);
 
 }  // namespace dmr

@@ -7,6 +7,8 @@
 //   tet_first_intersect_kernel  replaces firstIntersectCUDA (forward.cu:298-445)
 //   tet_march_fwd_kernel        replaces TET_FORWARD::renderCUDA (forward.cu:485-815)
 //   tet_march_bwd_kernel        replaces TET_BACKWARD::renderCUDA (backward.cu:86-487)
+//   tet_march_bwd_cam_kernel,   the same plus gradients with respect to the camera matrices (no reference counterpart)
+//   tet_camera_finish_kernel
 //
 // Forward images must match the reference to 1e-5, which requires IDENTICAL
 // branch decisions along every ray (hit tests, normal signs); all such
@@ -502,15 +504,20 @@ __device__ __forceinline__ float3 sel3(int i, float3 a, float3 b, float3 c)
 // peak at C3).  Same real number as the reference's chain, rounded differently (~1e-7 relative; the depth image
 // is compared at 1e-5).
 struct TetDepth { float az, bz, aw, bw; };
-__device__ __forceinline__ TetDepth tet_depth_setup(const float* __restrict__ mv, const float* __restrict__ pj, float3 ro, float3 rd)
+// z and w rows of proj * mv over the first three rows of mv (the bottom row of mv never enters: xform43)
+__device__ __forceinline__ void tet_depth_rows(const float* __restrict__ mv, const float* __restrict__ pj, float rz[4], float rw[4])
 {
-    float rz[4], rw[4];
 #pragma unroll
     for (int k = 0; k < 4; k++) {
         rz[k] = pj[2] * mv[4 * k] + pj[6] * mv[4 * k + 1] + pj[10] * mv[4 * k + 2];
         rw[k] = pj[3] * mv[4 * k] + pj[7] * mv[4 * k + 1] + pj[11] * mv[4 * k + 2];
     }
     rz[3] += pj[14]; rw[3] += pj[15];
+}
+__device__ __forceinline__ TetDepth tet_depth_setup(const float* __restrict__ mv, const float* __restrict__ pj, float3 ro, float3 rd)
+{
+    float rz[4], rw[4];
+    tet_depth_rows(mv, pj, rz, rw);
     TetDepth d;
     d.az = rz[0] * ro.x + rz[1] * ro.y + rz[2] * ro.z + rz[3];
     d.bz = rz[0] * rd.x + rz[1] * rd.y + rz[2] * rd.z;
@@ -818,6 +825,47 @@ __device__ __forceinline__ void tet_bwd_face(const TetParams& p, TetBwdState& st
     atomicAdd(&p.dL_dfaces_opacity[face], dL_dopa);
 }
 
+// Camera gradients (CAM instantiations; DESIGN.md 3.4).  The camera enters a step through the ray -- (t, u, v) of the
+// Moeller-Trumbore test against the face's triangle p0 p1 p2 in faces[] order -- and through the hit-point depth
+// pd = Z / clamp_w(W), Z = az + t bz, W = aw + t bw, whose coefficients depend on ro, rd and the z / w rows of
+// proj * mv.  A lane accumulates dL/dro and dL/drd through (t, u, v), and dL/d(az, bz, aw, bw); tet_march_bwd_cam
+// chains them into the matrices after the walk.  With T = ro - p0, E1 = p1 - p0, E2 = p2 - p0, N = E2 x E1 and
+// D = rd.N:  dt/dro = -N / D, dt/drd = -t N / D, du/dro = (rd x E2) / D, du/drd = (E2 x T - u N) / D,
+// dv/dro = (E1 x rd) / D, dv/drd = (T x E1 - v N) / D.
+struct TetCamAcc {
+    float3 g_ro, g_rd;
+    float g_az, g_bz, g_aw, g_bw;
+};
+
+__device__ __forceinline__ void tet_cam_step(TetCamAcc& a, const TetBwdState& st, const TetDepth& dep, float3 ro, float3 rd,
+                                             float rt, float iu, float iv, const float4 s0, const float4 s1, const float4 s2,
+                                             float intense, const float dLc[3], float gd, const float4 v0, const float4 v1,
+                                             float v2z)
+{
+    const float3 c0 = f3(s0.x, s0.y, s0.z), c1 = f3(s0.w, s1.x, s1.y), c2 = f3(s1.z, s1.w, s2.x);
+    const float w = s2.y * expf(st.prev_log_T);      // T_k alpha_k of the step (does not depend on the camera)
+    const float3 dc1 = c1 - c0, dc2 = c2 - c0;
+    const float wi = w * intense;
+    const float dL_du = wi * (dLc[0] * dc1.x + dLc[1] * dc1.y + dLc[2] * dc1.z);
+    const float dL_dv = wi * (dLc[0] * dc2.x + dLc[1] * dc2.y + dLc[2] * dc2.z);
+    // depth: no derivative through a clamped w
+    const float Z = dep.az + rt * dep.bz, Wr = dep.aw + rt * dep.bw, Wc = clamp_w(Wr);
+    const float gZ = w * gd / Wc;
+    const float gW = Wc == Wr ? -gZ * (Z / Wc) : 0.0f;
+    a.g_az += gZ; a.g_bz += gZ * rt; a.g_aw += gW; a.g_bw += gW * rt;
+    const float dL_dt = gZ * dep.bz + gW * dep.bw;
+    // (t, u, v): the two rd x / x T terms of u and v share M = (dL_du E2 - dL_dv E1) / D
+    const float3 p0 = f3(v0.x, v0.y, v0.z), p1 = f3(v0.w, v1.x, v1.y), p2 = f3(v1.z, v1.w, v2z);
+    const float3 E1 = p1 - p0, E2 = p2 - p0, Tv = ro - p0;
+    const float3 N = cross3(E2, E1);
+    const float iD = 1.0f / dot3(rd, N);
+    const float ku = dL_du * iD, kv = dL_dv * iD, kt = dL_dt * iD;
+    const float kn = kt * rt + ku * iu + kv * iv;
+    const float3 M = ku * E2 - kv * E1;
+    a.g_ro = a.g_ro + cross3(rd, M) - kt * N;
+    a.g_rd = a.g_rd + cross3(M, Tv) - kn * N;
+}
+
 // Backward march.  Steps recorded in the face trail (all of them unless a ray composited more than
 // trail_cap faces) are replayed in reverse: face id and the forward pass's own (t,u,v) from the trail
 // (one coalesced 16-byte load), all loads independent of the previous step and issued one step ahead.  Steps beyond the cap are re-marched through the adjacency records exactly like
@@ -826,8 +874,10 @@ __device__ __forceinline__ void tet_bwd_face(const TetParams& p, TetBwdState& st
 // it fits 80 / 72 / 64 registers and 12 / 14 / 16 CTAs per SM instead of 10: C3 588.6 / 601 / 652 us against 587.8 us.
 // More resident warps do not help: the kernel is bound by the wavefronts its per-lane gathers and reductions push
 // through the L1 data pipe, not by the latency of a single chain.)
-template <bool DET>
-__device__ __forceinline__ void tet_march_bwd_body(const TetParams& p)
+// CAM: also accumulate the camera terms of every walked step into `cam` (tet_cam_step); the face's vertices are loaded
+// with its shading record.  The early returns end the walk only: tet_march_bwd_cam reduces after it on every lane.
+template <bool DET, bool CAM>
+__device__ __forceinline__ void tet_march_bwd_body(const TetParams& p, TetCamAcc& cam)
 {
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int b = blockIdx.z;
@@ -898,8 +948,16 @@ __device__ __forceinline__ void tet_march_bwd_body(const TetParams& p)
             const float4* sh4 = reinterpret_cast<const float4*>(p.shade + curr_face);
             const float4 s0 = sh4[0], s1 = sh4[1], s2 = sh4[2], s3 = sh4[3];
             const float intense = p.faces_intense[(size_t)b * p.F + curr_face];
+            float4 v0, v1;
+            float v2z;
+            if constexpr (CAM) {
+                const float4* fr = reinterpret_cast<const float4*>(p.face_rec + (size_t)b * p.F + curr_face);
+                v0 = fr[0]; v1 = fr[1]; v2z = reinterpret_cast<const float*>(fr)[8];
+            }
             tet_bwd_face<DET>(p, st, curr_face, rt, iu, iv, s0, s1, s2, s3, intense, dep, dLc, gd, bg_dot, bd_dot,
                          final_T, final_prev_T);
+            // (t, u, v) of the re-march: recomputed, the same bits as the forward march's
+            if constexpr (CAM) tet_cam_step(cam, st, dep, ro, rd, rt, iu, iv, s0, s1, s2, intense, dLc, gd, v0, v1, v2z);
             k--;
             if (curr_face == first_face) return;         // backward.cu:363-366
             if (curr_tet == -1) return;                  // backward.cu:373-376
@@ -924,6 +982,11 @@ __device__ __forceinline__ void tet_march_bwd_body(const TetParams& p)
         s0 = sh4[0]; s1 = sh4[1]; s2 = sh4[2]; s3 = sh4[3];
         intense = fint[face];
     }
+    // CAM: the face's triangle (TetFaceRec p0 p1 p2), loaded together with the shading record
+    const float4* frec = reinterpret_cast<const float4*>(p.face_rec + (size_t)b * p.F);
+    float4 v0, v1;
+    float v2z;
+    if constexpr (CAM) { v0 = frec[4 * face]; v1 = frec[4 * face + 1]; v2z = reinterpret_cast<const float*>(frec + 4 * face)[8]; }
     for (; k >= 0; k--) {
         // issue the loads of step k-1 (face id known since the previous iteration), then work on step k
         const int nf = e_next.x & 0x7fffffff;
@@ -931,6 +994,9 @@ __device__ __forceinline__ void tet_march_bwd_body(const TetParams& p)
         const float4* sh4 = reinterpret_cast<const float4*>(p.shade + nf);
         const float4 ns0 = sh4[0], ns1 = sh4[1], ns2 = sh4[2], ns3 = sh4[3];
         const float nint = fint[nf];
+        float4 nv0, nv1;
+        float nv2z;
+        if constexpr (CAM) { nv0 = frec[4 * nf]; nv1 = frec[4 * nf + 1]; nv2z = reinterpret_cast<const float*>(frec + 4 * nf)[8]; }
         const int4 e_cur = e;
         e = e_next;
         e_next = k > 1 ? __ldcs(trail + (size_t)(k - 2) * BI) : make_int4(0, 0, 0, 0);
@@ -938,17 +1004,172 @@ __device__ __forceinline__ void tet_march_bwd_body(const TetParams& p)
         // (t, u, v) of the step: the forward march's own values
         tet_bwd_face<DET>(p, st, face, __int_as_float(e_cur.y), __int_as_float(e_cur.z), __int_as_float(e_cur.w), s0, s1, s2, s3,
                           intense, dep, dLc, gd, bg_dot, bd_dot, final_T, final_prev_T);
+        if constexpr (CAM)
+            tet_cam_step(cam, st, dep, ro, rd, __int_as_float(e_cur.y), __int_as_float(e_cur.z), __int_as_float(e_cur.w), s0, s1,
+                         s2, intense, dLc, gd, v0, v1, v2z);
 
         if (stop_here) break;
         face = nf;
         s0 = ns0; s1 = ns1; s2 = ns2; s3 = ns3;
         intense = nint;
+        if constexpr (CAM) { v0 = nv0; v1 = nv1; v2z = nv2z; }
     }
 }
 
 // Once per vertex: float4 accumulator -> dL_dverts_color[P,3].
-__global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_kernel(TetParams p) { griddep_wait(); tet_march_bwd_body<false>(p); }
-__global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_det_kernel(TetParams p) { griddep_wait(); tet_march_bwd_body<true>(p); }
+__global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_kernel(TetParams p)
+{
+    griddep_wait();
+    TetCamAcc unused;
+    tet_march_bwd_body<false, false>(p, unused);
+}
+__global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_det_kernel(TetParams p)
+{
+    griddep_wait();
+    TetCamAcc unused;
+    tet_march_bwd_body<true, false>(p, unused);
+}
+
+// Camera-gradient instantiations: the walk of tet_march_bwd_body<DET, true>, then per lane the chain of its pixel into
+// the matrices, and one record of DMR_TET_CAM_REC floats per (view, CTA), summed in a fixed order (no float atomics:
+// reproducible in both modes).  Every CTA stores its record, zeros included, so the record array is not cleared.
+//   [3j + i]       dL/dinv_mv[4j + i]   = g_d[i] pv[j]           (i, j < 3)   d = L pv, L = the linear part of inv_mv
+//   [9 + i]        dL/dinv_mv[12 + i]   = g_ro[i]
+//   [12 + 3k + j]  dL/dinv_proj[4k + j] = (L^T g_d)[j] n[k]      (j < 3, k < 4), n = (nx, ny, -1, 1)
+//   [24 + k]       dL/drz[k],  [28 + k]  dL/drw[k]               z / w rows of proj * mv (tet_depth_rows)
+// tet_camera_finish_kernel applies the inverses and the direct depth-row terms.
+static_assert(MARCH_THREADS == 64 && MARCH_ROWS == 8, "tet_cam_records (tet.cuh) counts 8 x 8-pixel march CTAs");
+static_assert(DMR_TET_CAM_REC == 32, "one record slot per lane");
+template <bool DET>
+__device__ __forceinline__ void tet_march_bwd_cam(const TetParams& p, float* __restrict__ cam_rec)
+{
+    TetCamAcc a;
+    a.g_ro = f3(0, 0, 0); a.g_rd = f3(0, 0, 0);
+    a.g_az = 0.0f; a.g_bz = 0.0f; a.g_aw = 0.0f; a.g_bw = 0.0f;
+    tet_march_bwd_body<DET, true>(p, a);
+
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int b = blockIdx.z;
+    const uint32_t px = blockIdx.x * 8 + (lane & 7);
+    const uint32_t py = blockIdx.y * MARCH_ROWS + warp * 4 + (lane >> 3);
+    float g[DMR_TET_CAM_REC];
+#pragma unroll
+    for (int k = 0; k < DMR_TET_CAM_REC; k++) g[k] = 0.0f;
+    if (px < (uint32_t)p.W && py < (uint32_t)p.H) {   // inactive pixels: the accumulators are zero
+        const size_t bpix = (size_t)b * p.W * p.H + (size_t)py * p.W + px;
+        float fx = px + 0.5f, fy = py + 0.5f;
+        if (p.jitter) { const float2 j = p.jitter[bpix]; fx = j.x; fy = j.y; }   // constants: no gradient through the jitter
+        const float* imv = p.inv_mv + 16 * b;
+        const float* ipj = p.inv_proj + 16 * b;
+        // the ray as pixel_ray<TET> forms it, with the branch of its length clamp
+        const float n[4] = { pix2ndc(fx, p.W), pix2ndc(fy, p.H), -1.0f, 1.0f };
+        const float3 ro = f3(imv[12], imv[13], imv[14]);
+        const float4 pv4 = xform44(f3(n[0], n[1], -1.0f), ipj);
+        const float4 pw = xform44(f3(pv4.x, pv4.y, pv4.z), imv);
+        const float3 dv = f3(pw.x, pw.y, pw.z) - ro;
+        const float len = sqrtf(dot3(dv, dv));
+        const float3 rd = dv / fmaxf(len, 0.0001f);
+        float rz[4], rw[4];
+        tet_depth_rows(p.mv + 16 * b, p.proj + 16 * b, rz, rw);
+        const float3 g_ro = a.g_ro + a.g_az * f3(rz[0], rz[1], rz[2]) + a.g_aw * f3(rw[0], rw[1], rw[2]);
+        const float3 g_rd = a.g_rd + a.g_bz * f3(rz[0], rz[1], rz[2]) + a.g_bw * f3(rw[0], rw[1], rw[2]);
+        // rd = d / max(|d|, 1e-4)
+        const float3 gdv = len >= 0.0001f ? (g_rd - rd * dot3(rd, g_rd)) / len : g_rd / 0.0001f;
+        const float pv[3] = { pv4.x, pv4.y, pv4.z };
+        const float gd[3] = { gdv.x, gdv.y, gdv.z };
+#pragma unroll
+        for (int j = 0; j < 3; j++) {
+#pragma unroll
+            for (int i = 0; i < 3; i++) g[3 * j + i] = gd[i] * pv[j];
+            const float lg = imv[4 * j] * gd[0] + imv[4 * j + 1] * gd[1] + imv[4 * j + 2] * gd[2];
+#pragma unroll
+            for (int k = 0; k < 4; k++) g[12 + 3 * k + j] = lg * n[k];
+        }
+        g[9] = g_ro.x; g[10] = g_ro.y; g[11] = g_ro.z;
+        const float rov[3] = { ro.x, ro.y, ro.z }, rdv[3] = { rd.x, rd.y, rd.z };
+#pragma unroll
+        for (int k = 0; k < 3; k++) {
+            g[24 + k] = a.g_az * rov[k] + a.g_bz * rdv[k];
+            g[28 + k] = a.g_aw * rov[k] + a.g_bw * rdv[k];
+        }
+        g[27] = a.g_az; g[31] = a.g_aw;
+    }
+    // fixed-order reduction: warp butterfly, then the two warp sums in warp order
+#pragma unroll
+    for (int k = 0; k < DMR_TET_CAM_REC; k++) {
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) g[k] += __shfl_xor_sync(0xffffffffu, g[k], o);
+    }
+    __shared__ float s_cam[MARCH_THREADS];
+    float x = g[0];
+#pragma unroll
+    for (int k = 1; k < DMR_TET_CAM_REC; k++) x = lane == k ? g[k] : x;
+    s_cam[tid] = x;
+    __syncthreads();
+    if (tid < DMR_TET_CAM_REC)
+        cam_rec[(((size_t)b * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x) * DMR_TET_CAM_REC + tid] =
+            s_cam[tid] + s_cam[DMR_TET_CAM_REC + tid];
+}
+
+__global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_cam_kernel(TetParams p, float* cam_rec)
+{
+    griddep_wait();
+    tet_march_bwd_cam<false>(p, cam_rec);
+}
+__global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_cam_det_kernel(TetParams p, float* cam_rec)
+{
+    griddep_wait();
+    tet_march_bwd_cam<true>(p, cam_rec);
+}
+
+// One CTA per view: the view's records (tet_march_bwd_cam) are summed in a fixed order -- thread t owns component
+// t % 32 of every eighth record (coalesced reads of the flat record array), then the eight partial sums of a component
+// are added in thread order -- and chained into the matrices: through the inverses, dL/dA = -A^-T (dL/dA^-1) A^-T,
+// plus the direct terms of the depth rows rz[k] = sum_r pj[2 + 4r] mv[4k + r] (+ pj[14] for k = 3), rw likewise with
+// pj[3 + 4r] and pj[15].  The result is ADDED to dL_dmv[b] / dL_dproj[b]; this CTA is the only writer of view b.
+__global__ void __launch_bounds__(256) tet_camera_finish_kernel(int nrec, const float* __restrict__ cam_rec,
+                                                                const float* __restrict__ mv, const float* __restrict__ pj,
+                                                                const float* __restrict__ inv_mv, const float* __restrict__ inv_proj,
+                                                                float* __restrict__ dL_dmv, float* __restrict__ dL_dproj)
+{
+    griddep_wait();   // programmatic dependent launch: see dmr_launch (common.cuh)
+    __shared__ float s_part[256];
+    __shared__ float s_g[2][16];      // dL/dinv_mv, dL/dinv_proj (column-major, zeros where the forward reads nothing)
+    __shared__ float s_r[8];          // dL/drz[0..3], dL/drw[0..3]
+    const int b = blockIdx.x, t = threadIdx.x;
+    const float* rec = cam_rec + (size_t)b * nrec * DMR_TET_CAM_REC;
+    const size_t n = (size_t)nrec * DMR_TET_CAM_REC;
+    float acc = 0.0f;
+    for (size_t i = t; i < n; i += 256) acc += rec[i];
+    s_part[t] = acc;
+    __syncthreads();
+    if (t < 32) {
+        s_g[t >> 4][t & 15] = 0.0f;
+        __syncwarp();
+        float sum = 0.0f;
+#pragma unroll
+        for (int k = 0; k < 8; k++) sum += s_part[t + DMR_TET_CAM_REC * k];
+        if (t < 9) s_g[0][4 * (t / 3) + t % 3] = sum;
+        else if (t < 12) s_g[0][12 + t - 9] = sum;
+        else if (t < 24) s_g[1][4 * ((t - 12) / 3) + (t - 12) % 3] = sum;
+        else s_r[t - 24] = sum;
+        __syncwarp();
+        // thread e: entry (i, j) = (e & 3, e >> 2) of matrix t >> 4; M(r, c) = m[4c + r]
+        const int m = t >> 4, e = t & 15, i = e & 3, j = e >> 2;
+        const float* N = (m == 0 ? inv_mv : inv_proj) + 16 * b;
+        float out = -inverse_chain(N, s_g[m], i, j);
+        const float* mvb = mv + 16 * b;
+        const float* pjb = pj + 16 * b;
+        if (m == 0) {
+            if (i < 3) out += s_r[j] * pjb[2 + 4 * i] + s_r[4 + j] * pjb[3 + 4 * i];
+        } else if (i >= 2) {
+            const float* R = s_r + 4 * (i - 2);
+            out += j < 3 ? R[0] * mvb[j] + R[1] * mvb[4 + j] + R[2] * mvb[8 + j] + R[3] * mvb[12 + j] : R[3];
+        }
+        float* dst = (m == 0 ? dL_dmv : dL_dproj) + 16 * b + e;
+        *dst += out;
+    }
+}
 
 // Deterministic mode, last step: fixed-point accumulators -> += into dL_dverts_color[P,3] and dL_dfaces_opacity[F].
 __global__ void __launch_bounds__(256) tet_det_convert_kernel(TetParams p)
@@ -991,17 +1212,22 @@ __global__ void __launch_bounds__(256) tet_grad_vertex_kernel(TetParams p)
     o[0] += a.x; o[1] += a.y; o[2] += a.z;
 }
 
-int tet_march_backward_deterministic(const TetParams& p, cudaStream_t stream)
+int tet_march_backward_deterministic(const TetParams& p, cudaStream_t stream, float* cam_rec)
 {
     dim3 grid((p.W + 7) / 8, (p.H + MARCH_ROWS - 1) / MARCH_ROWS, p.B);
     const size_t HW = (size_t)p.W * p.H;
     {
-        ProfScope prof(ST_TET_BWD, stream);
+        ProfScope prof(cam_rec ? ST_TET_BWD_CAM : ST_TET_BWD, stream);
         count_launch(1);   // two kernels under one scope
         int rc = det_gmax(p.dL_dcolor, 3 * p.B * HW, p.dL_ddepth, p.B * HW, const_cast<uint32_t*>(p.det_gmax), stream);
         if (rc) return rc;
-        DMR_CUDA(dmr_launch(tet_march_bwd_det_kernel, dim3(grid), dim3(MARCH_THREADS), 0, stream, p));
-        DMR_LAUNCH_CHECK("tet_march_bwd_det_kernel");
+        if (cam_rec) {
+            DMR_CUDA(dmr_launch(tet_march_bwd_cam_det_kernel, dim3(grid), dim3(MARCH_THREADS), 0, stream, p, cam_rec));
+            DMR_LAUNCH_CHECK("tet_march_bwd_cam_det_kernel");
+        } else {
+            DMR_CUDA(dmr_launch(tet_march_bwd_det_kernel, dim3(grid), dim3(MARCH_THREADS), 0, stream, p));
+            DMR_LAUNCH_CHECK("tet_march_bwd_det_kernel");
+        }
     }
     {
         ProfScope prof(ST_TET_BWD_FINISH, stream);
@@ -1011,10 +1237,14 @@ int tet_march_backward_deterministic(const TetParams& p, cudaStream_t stream)
     return 0;
 }
 
-int tet_march_backward(const TetParams& p, cudaStream_t stream)
+int tet_march_backward(const TetParams& p, cudaStream_t stream, float* cam_rec)
 {
     dim3 grid((p.W + 7) / 8, (p.H + MARCH_ROWS - 1) / MARCH_ROWS, p.B);
-    {
+    if (cam_rec) {
+        ProfScope prof(ST_TET_BWD_CAM, stream);
+        DMR_CUDA(dmr_launch(tet_march_bwd_cam_kernel, dim3(grid), dim3(MARCH_THREADS), 0, stream, p, cam_rec));
+        DMR_LAUNCH_CHECK("tet_march_bwd_cam_kernel");
+    } else {
         ProfScope prof(ST_TET_BWD, stream);
         DMR_CUDA(dmr_launch(tet_march_bwd_kernel, dim3(grid), dim3(MARCH_THREADS), 0, stream, p));
         DMR_LAUNCH_CHECK("tet_march_bwd_kernel");
@@ -1024,6 +1254,17 @@ int tet_march_backward(const TetParams& p, cudaStream_t stream)
         DMR_CUDA(dmr_launch(tet_grad_vertex_kernel, dim3((p.P + 255) / 256), dim3(256), 0, stream, p));
         DMR_LAUNCH_CHECK("tet_grad_vertex_kernel");
     }
+    return 0;
+}
+
+int tet_camera_finish(const TetParams& p, const float* cam_rec, float* dL_dmv, float* dL_dproj, cudaStream_t stream)
+{
+    if (p.B <= 0) return 0;
+    const int nrec = (int)tet_cam_records(1, p.W, p.H);
+    ProfScope prof(ST_TET_CAM_FINISH, stream);
+    DMR_CUDA(dmr_launch(tet_camera_finish_kernel, dim3(p.B), dim3(256), 0, stream, nrec, cam_rec, p.mv, p.proj, p.inv_mv,
+                        p.inv_proj, dL_dmv, dL_dproj));
+    DMR_LAUNCH_CHECK("tet_camera_finish_kernel");
     return 0;
 }
 

@@ -810,15 +810,7 @@ __global__ void __launch_bounds__(240) tri_camera_finish_kernel(int ntiles, cons
         // thread e: entry (i, j) = (e & 3, (e >> 2) & 3) of matrix e >> 4; M(r, c) = m[4c + r]
         const int m = t >> 4, e = t & 15, i = e & 3, j = e >> 2;
         const float* N = (m == 0 ? inv_mv : inv_proj) + 16 * b;
-        const float* G = s_g[m];
-        float out = 0.0f;
-#pragma unroll
-        for (int a = 0; a < 4; a++) {
-            float h = 0.0f;                                // (G N^T)(a, j) = sum_c G(a, c) N(j, c)
-#pragma unroll
-            for (int c = 0; c < 4; c++) h += G[4 * c + a] * N[4 * c + j];
-            out += N[4 * i + a] * h;                       // N^T(i, a) = N(a, i)
-        }
+        const float out = inverse_chain(N, s_g[m], i, j);
         float* dst = (m == 0 ? dL_dmv : dL_dproj) + 16 * b + e;
         *dst += -out;
     }

@@ -21,6 +21,7 @@ KINDS = {
     "first_face": (11, np.int32, 1),
     "first_tet": (12, np.int32, 1),
     "face_order": (13, np.uint32, 1),
+    "tet_jitter": (14, np.float32, 2),    # pixel coordinates of the rays; written only when ray_random_seed > 0
 }
 # The reference's 64-bit (tile | depth) keys.  The native path sorts FACES by depth and instances by tile
 # id only (csrc/common.cuh: bin_faces / bin_instances), so it never materialises them; they are recomposed

@@ -315,6 +315,37 @@ int dmr_tet_backward_deterministic(
     void* workspace, size_t workspace_bytes,
     dmr_stream_t stream);
 
+/* Camera gradients of the tet renderer (no reference counterpart: the reference returns no gradient for the      */
+/* matrices).  The same backward pass as dmr_tet_backward (deterministic == 0) or dmr_tet_backward_deterministic  */
+/* (deterministic != 0), with the same arguments and the same two gradients, plus dL/dmv_mats and dL/dproj_mats   */
+/* [B,16] (column-major, like the matrices), ADDED to the caller's zeroed buffers.  The derivative is that of the  */
+/* forward pass as implemented, with the marched path (first face and tet, faces crossed), n_contrib, termination */
+/* and the active mask held fixed, and the branch regions of the clip-w clamp and of the ray-length clamp; it     */
+/* flows through the rays (ray origin and direction formed from inv_mv_mats / inv_proj_mats, chained through the  */
+/* inverses) and through the hit-point depth (directly through mv_mats / proj_mats).  Only the steps the backward */
+/* pass walks contribute (where the reference's reverse march gives up on a ray, its earlier faces get nothing, as */
+/* for colour and opacity).  Jittered pixel coordinates (ray_random_seed > 0) are constants.  Accumulated without  */
+/* float atomics: reproducible in both modes.  `workspace`: dmr_tet_backward_camera_bytes(B, P, F, W, H,          */
+/* deterministic) bytes of device scratch.                                                                         */
+size_t dmr_tet_backward_camera_bytes(int B, int P, int F, int W, int H, int deterministic);
+int dmr_tet_backward_camera(
+    int B, int P, int F, int T, int W, int H,
+    int ray_random_seed,
+    const float* background,
+    const float* mv_mats, const float* proj_mats,
+    const float* inv_mv_mats, const float* inv_proj_mats,
+    const float* faces_intense,
+    const void* point_buffer, const void* face_buffer,
+    const void* tet_records,
+    const void* image_buffer,
+    const float* dL_dcolor, const float* dL_ddepth,
+    float* dL_dverts_color, float* dL_dfaces_opacity,
+    int deterministic,
+    float* dL_dmv,               /* [B,16] */
+    float* dL_dproj,             /* [B,16] */
+    void* workspace, size_t workspace_bytes,
+    dmr_stream_t stream);
+
 /* ------------------------------------------------------------------------ */
 /* Read-only views into the state buffers for the bit-exact parity checks    */
 /* (the reference exposes the same quantities through the fromChunk layouts, */
@@ -336,7 +367,9 @@ enum dmr_view_kind {
     DMR_VIEW_FINAL_T        = 10, /* float[B*W*H] (tet: final log T)          image buffer */
     DMR_VIEW_FIRST_FACE     = 11, /* int32[B*W*H] (tet only)                  image buffer */
     DMR_VIEW_FIRST_TET      = 12, /* int32[B*W*H] (tet only)                  image buffer */
-    DMR_VIEW_FACE_ORDER     = 13  /* uint32[B*F] faces (b*F+f) stably sorted by depth key  face buffer */
+    DMR_VIEW_FACE_ORDER     = 13, /* uint32[B*F] faces (b*F+f) stably sorted by depth key  face buffer */
+    DMR_VIEW_TET_JITTER     = 14  /* float2[B*W*H] pixel coordinates of the rays (tet only; written only when */
+                                  /* ray_random_seed > 0)                     image buffer */
 };
 int dmr_debug_view(int renderer /*0=tri,1=tet*/, int kind,
                    int B, int P, int F, int T, int W, int H, size_t R,
