@@ -381,14 +381,17 @@ def grad_sink_for(verts, verts_color, faces_opacity):
 def render_tris_backward(background, verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, inv_mv_mats,
                          inv_proj_mats, verts_depth, faces_intense, dL_dout_color, dL_dout_depth, R, pointBuffer,
                          faceBuffer, binningBuffer, imageBuffer, accumulate_into=None, deterministic=False,
-                         camera_grads=False):
+                         camera_grads=False, exact_vertex_grads=False):
     """RasterizeTrianglesBackwardCUDA (render.cu:134-208).
     Returns (dL_dverts[P,3], dL_dvcolor[P,3], dL_dfopacity[F], dL_dvdepth[B,P], dL_dfintense[B,F]).
     `accumulate_into` (beyond the reference's 18 arguments): existing contiguous fp32 (dL_dverts, dL_dvcolor,
     dL_dfopacity) tensors that the gradients are ADDED to (and that are returned) instead of fresh zero tensors.
     `deterministic`: run-to-run reproducible gradients (64-bit fixed-point accumulation, dmr_tri_backward_deterministic).
     `camera_grads`: also return dL_dmv_mats, dL_dproj_mats [B,4,4] (gradients with respect to the mv_mats / proj_mats
-    tensors passed here, through the rays; dmr_tri_backward_camera) as two more elements."""
+    tensors passed here, through the rays; dmr_tri_backward_camera) as two more elements.
+    `exact_vertex_grads`: dL_dverts is the exact derivative of the rendered image instead of the reference's formula
+    (which differentiates t in place of the second barycentric v); the other gradients are unchanged
+    (dmr_tri_backward_exact)."""
     lib = _lib.load()
     B, P, F = mv_mats.size(0), verts.size(0), faces.size(0)
     H, W = dL_dout_color.size(2), dL_dout_color.size(3)
@@ -417,7 +420,16 @@ def render_tris_backward(background, verts, faces, verts_color, faces_opacity, m
                  _ptr(binningBuffer), _ptr(imageBuffer), _ptr(gc), _ptr(gd), gp[0], gp[1], gp[2], gp[3], gp[4])
             # scratch of the call (statistics per (view, face), per-vertex accumulators): the state buffers saved for
             # backward are only read.  The caching allocator reuses the block for later work on the same stream.
-            if camera_grads:
+            if exact_vertex_grads:
+                # the workspace of the mode it modifies: the record layout is the same
+                det = int(bool(deterministic))
+                nbytes = (lib.dmr_tri_backward_camera_bytes(B, P, F, W, H, det) if camera_grads else
+                          lib.dmr_tri_backward_deterministic_bytes(B, P, F) if det else
+                          lib.dmr_tri_backward_workspace_bytes(B, P, F))
+                ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+                cam = (gp[5], gp[6]) if camera_grads else (ctypes.c_void_p(0), ctypes.c_void_p(0))
+                _lib.check(lib.dmr_tri_backward_exact(*a, det, *cam, _ptr(ws), ws.numel(), _stream()))
+            elif camera_grads:
                 ws = torch.empty(lib.dmr_tri_backward_camera_bytes(B, P, F, W, H, int(bool(deterministic))),
                                  dtype=torch.uint8, device=dev)
                 _lib.check(lib.dmr_tri_backward_camera(*a, int(bool(deterministic)), gp[5], gp[6], _ptr(ws), ws.numel(),

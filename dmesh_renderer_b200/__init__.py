@@ -42,12 +42,28 @@ def set_deterministic(flag: bool) -> bool:
     return old
 
 
+_exact_vertex_grads_default = False
+
+
+def set_exact_vertex_grads(flag: bool) -> bool:
+    """Process-wide default for the tri renderer's vertex-position gradient (extension).  False (the default): the
+    reference implementation's formula, which differentiates the ray parameter t where the forward pass uses the
+    second barycentric v.  True: the exact derivative of the rendered image, consistent with the camera gradients.
+    The other gradients are the same either way.  `TriRenderer(settings, exact_vertex_grads=...)` /
+    `render_tri(..., exact_vertex_grads=...)` override it per renderer / call.  Returns the previous value."""
+    global _exact_vertex_grads_default
+    old, _exact_vertex_grads_default = _exact_vertex_grads_default, bool(flag)
+    return old
+
+
 def render_tri(verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, verts_depth, faces_intense,
-               render_settings: TriRenderSettings, deterministic=None):
-    """reference __init__.py:18-43 (`deterministic`: see set_deterministic)"""
+               render_settings: TriRenderSettings, deterministic=None, exact_vertex_grads=None):
+    """reference __init__.py:18-43 (`deterministic`: see set_deterministic; `exact_vertex_grads`: see
+    set_exact_vertex_grads)"""
     det = _deterministic_default if deterministic is None else bool(deterministic)
+    exact = _exact_vertex_grads_default if exact_vertex_grads is None else bool(exact_vertex_grads)
     return _RenderTri.apply(verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, verts_depth, faces_intense,
-                            render_settings, det)
+                            render_settings, det, exact)
 
 
 class _RenderTri(th.autograd.Function):
@@ -55,8 +71,9 @@ class _RenderTri(th.autograd.Function):
 
     @staticmethod
     def forward(ctx, verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, verts_depth, faces_intense,
-                render_settings, deterministic=False):
+                render_settings, deterministic=False, exact_vertex_grads=False):
         ctx.deterministic = deterministic
+        ctx.exact_vertex_grads = exact_vertex_grads
         try:
             # Same computation as _C.render_tris(*13 args) (reference __init__.py:62-88), issued in two halves
             # (phase 1: preprocess + scan; phase 2 after the num_rendered read-back).
@@ -104,7 +121,7 @@ class _RenderTri(th.autograd.Function):
         grad_mv = grad_proj = None
         try:
             grads = _C.render_tris_backward(*args, accumulate_into=into, deterministic=ctx.deterministic,
-                                            camera_grads=camera)
+                                            camera_grads=camera, exact_vertex_grads=ctx.exact_vertex_grads)
         except Exception as ex:
             print("\nAn error occured in backward.\n")
             raise ex
@@ -122,16 +139,17 @@ class _RenderTri(th.autograd.Function):
         # gradient positions: reference __init__.py:156-168; positions 4 and 5 (the matrices) are an extension
         return (grad_verts, None, grad_verts_color, grad_faces_opacity,
                 grad_mv if ctx.needs_input_grad[4] else None, grad_proj if ctx.needs_input_grad[5] else None,
-                grad_verts_depth, grad_faces_intense, None, None)
+                grad_verts_depth, grad_faces_intense, None, None, None)
 
 
 class TriRenderer(th.nn.Module):
     """reference __init__.py:172-225"""
 
-    def __init__(self, render_settings: TriRenderSettings, deterministic=None):
+    def __init__(self, render_settings: TriRenderSettings, deterministic=None, exact_vertex_grads=None):
         super().__init__()
         self.render_settings = render_settings
         self.deterministic = deterministic     # None: the process-wide default (set_deterministic)
+        self.exact_vertex_grads = exact_vertex_grads   # None: the process-wide default (set_exact_vertex_grads)
 
     def forward(self, verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, verts_depth, faces_intense):
         """
@@ -144,7 +162,7 @@ class TriRenderer(th.nn.Module):
         """
         return render_tri(verts, faces.to(dtype=th.int32), verts_color, faces_opacity, mv_mats.transpose(1, 2),
                           proj_mats.transpose(1, 2), verts_depth, faces_intense, self.render_settings,
-                          self.deterministic)
+                          self.deterministic, self.exact_vertex_grads)
 
 
 # =============================================================================

@@ -35,6 +35,7 @@ SIGNATURES = {
     "dmr_tri_backward_deterministic": (c_int, [c_int] * 6 + [c_void_p] * 14 + [c_void_p, c_size_t] + [c_void_p]),
     "dmr_tri_backward_camera_bytes": (c_size_t, [c_int] * 6),
     "dmr_tri_backward_camera": (c_int, [c_int] * 6 + [c_void_p] * 14 + [c_int] + [c_void_p] * 2 + [c_void_p, c_size_t] + [c_void_p]),
+    "dmr_tri_backward_exact": (c_int, [c_int] * 6 + [c_void_p] * 14 + [c_int] + [c_void_p] * 2 + [c_void_p, c_size_t] + [c_void_p]),
     "dmr_tri_depth_chain_camera_bytes": (c_size_t, [c_int] * 2),
     "dmr_tri_depth_chain_camera": (c_int, [c_int, c_int] + [c_void_p] * 8 + [c_size_t, c_void_p]),
     "dmr_tet_records_bytes": (c_size_t, [c_int]),

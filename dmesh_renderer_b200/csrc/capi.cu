@@ -256,7 +256,8 @@ static int tri_backward_impl(int B, int P, int F, int W, int H, int R, const flo
                              const void* binning_buffer, const void* image_buffer, const float* dL_dcolor,
                              const float* dL_ddepth, float* dL_dverts, float* dL_dvcolor, float* dL_dfopacity,
                              float* dL_dvdepth, float* dL_dfintense, void* workspace, size_t workspace_bytes,
-                             bool deterministic, dmr_stream_t stream_, float* dL_dmv = nullptr, float* dL_dproj = nullptr)
+                             bool deterministic, dmr_stream_t stream_, float* dL_dmv = nullptr, float* dL_dproj = nullptr,
+                             bool exact = false)
 {
     const bool cam = dL_dmv != nullptr;
     cudaStream_t stream = (cudaStream_t)stream_;
@@ -309,7 +310,7 @@ static int tri_backward_impl(int B, int P, int F, int W, int H, int R, const flo
         p.det_vdepth = at<long long>(det_workspace, DL.vdepth);
         p.det_fopa = at<long long>(det_workspace, DL.fopa);
         DMR_CUDA(cudaMemsetAsync(det_workspace, 0, DL.total, stream));
-        int rc = tri_render_backward_deterministic(p, stream, cam_tiles);
+        int rc = tri_render_backward_deterministic(p, stream, cam_tiles, exact);
         if (rc || !cam) return rc;
         return tri_camera_finish(B, W, H, cam_tiles, inv_mv_mats, inv_proj_mats, dL_dmv, dL_dproj, stream);
     }
@@ -326,7 +327,7 @@ static int tri_backward_impl(int B, int P, int F, int W, int H, int R, const flo
     const bool use_vacc = 3 * (size_t)F >= 4 * (size_t)P;
     p.grad_vacc = use_vacc ? at<float4>(workspace, WL.grad_vacc) : nullptr;
     DMR_CUDA(cudaMemsetAsync(workspace, 0, use_vacc ? WL.total - 256 : WL.stats_end, stream));
-    int rc = tri_render_backward(p, stream, cam_tiles);
+    int rc = tri_render_backward(p, stream, cam_tiles, exact);
     if (rc || !cam) return rc;
     return tri_camera_finish(B, W, H, cam_tiles, inv_mv_mats, inv_proj_mats, dL_dmv, dL_dproj, stream);
 }
@@ -384,6 +385,20 @@ int dmr_tri_backward_camera(int B, int P, int F, int W, int H, int R, const floa
                              binning_buffer, image_buffer, dL_dcolor, dL_ddepth, dL_dverts, dL_dvcolor, dL_dfopacity,
                              dL_dvdepth, dL_dfintense, workspace, workspace_bytes, deterministic != 0, stream, dL_dmv,
                              dL_dproj);
+}
+
+int dmr_tri_backward_exact(int B, int P, int F, int W, int H, int R, const float* background, const float* inv_mv_mats,
+                           const float* inv_proj_mats, const void* point_buffer, const void* face_buffer,
+                           const void* binning_buffer, const void* image_buffer, const float* dL_dcolor,
+                           const float* dL_ddepth, float* dL_dverts, float* dL_dvcolor, float* dL_dfopacity,
+                           float* dL_dvdepth, float* dL_dfintense, int deterministic, float* dL_dmv, float* dL_dproj,
+                           void* workspace, size_t workspace_bytes, dmr_stream_t stream)
+{
+    if ((dL_dmv == nullptr) != (dL_dproj == nullptr)) { set_error("pass both dL_dmv and dL_dproj, or neither"); return DMR_EINVAL; }
+    return tri_backward_impl(B, P, F, W, H, R, background, inv_mv_mats, inv_proj_mats, point_buffer, face_buffer,
+                             binning_buffer, image_buffer, dL_dcolor, dL_ddepth, dL_dverts, dL_dvcolor, dL_dfopacity,
+                             dL_dvdepth, dL_dfintense, workspace, workspace_bytes, deterministic != 0, stream, dL_dmv,
+                             dL_dproj, true);
 }
 
 size_t dmr_tri_depth_chain_camera_bytes(int B, int P)

@@ -427,7 +427,11 @@ constexpr int DMR_TRI_BWD_MINB = 4;
 // sums them in a fixed order and stores ONE 96-byte record per (view, tile): no float atomics, so the camera
 // gradients are reproducible in both modes.  tri_camera_finish_kernel sums a view's records and applies the inverse.
 #define DMR_CAM_REC 24
-template <bool DET, bool CAM>
+// Exact vertex-position gradients (EXACT = true, opt-in; DESIGN.md 3.3).  The statistics differentiate the v the
+// forward pass uses instead of the reference's t: S24 takes dL_dv * v in place of dL_dv * t, and S3 becomes the
+// vector S3v = sum dL_dv / D * rd, whose y and z go to the pad slots 21 and 22 of the record (logical 6 keeps x).
+// Record size, reduction and stores are unchanged; tri_grad_finish_body<.., EXACT> applies the matching formula.
+template <bool DET, bool CAM, bool EXACT = false>
 __device__ __forceinline__ void tri_render_bwd_body(const TriRenderParams& p, float* __restrict__ cam_tiles)
 {
     __shared__ uint4 s_rec[RB * 9];      // staged records; two vertex-id slots (unused here: tri_grad_finish_kernel reads the
@@ -653,15 +657,19 @@ __device__ __forceinline__ void tri_render_bwd_body(const TriRenderParams& p, fl
                         const float dL_dv = dL_duc * duc_dv + dL_dvc * dvc_dv;
                         // sufficient statistics of the vertex-position gradient (see header comment)
                         const float k1 = dL_du * inv_denom;
-                        const float k24 = (dL_du * tuv.y + dL_dv * tuv.x) * inv_denom;
+                        const float k24 = (dL_du * tuv.y + dL_dv * (EXACT ? tuv.z : tuv.x)) * inv_denom;
                         v[0] = k1 * rd.x; v[1] = k1 * rd.y; v[2] = k1 * rd.z;
                         v[3] = k24 * rd.x; v[4] = k24 * rd.y; v[5] = k24 * rd.z;
                         v[6] = dL_dv * inv_denom;
+                        if constexpr (EXACT) {
+                            const float kv = v[6];
+                            v[6] = kv * rd.x; v[21] = kv * rd.y; v[22] = kv * rd.z;
+                        }
                         if constexpr (CAM) {
                             const float3 p0 = f3(a0.x, a0.y, a0.z);
                             const float3 Tv = ro - p0, E1 = f3(a1.x, a1.y, a1.z) - p0, E2 = f3(a2.x, a2.y, a2.z) - p0;
                             const float kv = dL_dv * inv_denom;
-                            const float kn = (dL_du * tuv.y + dL_dv * tuv.z) * inv_denom;
+                            const float kn = EXACT ? k24 : (dL_du * tuv.y + dL_dv * tuv.z) * inv_denom;
                             g_ro = g_ro + k1 * cross3(rd, E2) + kv * cross3(E1, rd);
                             g_rd = g_rd + k1 * cross3(E2, Tv) + kv * cross3(Tv, E1) - kn * cross3(E2, E1);
                         }
@@ -679,8 +687,10 @@ __device__ __forceinline__ void tri_render_bwd_body(const TriRenderParams& p, fl
                         long long* rec = p.det_stats + (size_t)s_rec[j * 9 + 1].w * 24 + 12 * cls;
 #pragma unroll
                         for (int k = 0; k < 12; k++) {
-                            if (cls == 1 && k >= 9) break;                       // logical 21..23: padding
-                            det_add(rec + k, v[k], (cls == 0 && k < 7) ? det_sg : det_sv);
+                            if (cls == 1 && k >= (EXACT ? 11 : 9)) break;        // logical 21..23 (EXACT: 23): padding
+                            // vertex-position statistics: logical 0..6 (EXACT: and 21, 22) take the finer scale
+                            const bool pos = cls == 0 ? k < 7 : (EXACT && k >= 9);
+                            det_add(rec + k, v[k], pos ? det_sg : det_sv);
                         }
                     }
                 } else if (have) {
@@ -776,6 +786,35 @@ __global__ void __launch_bounds__(256, DMR_TRI_BWD_CAM_MINB) tri_render_bwd_cam_
     tri_render_bwd_body<true, true>(p, cam_tiles);
 }
 
+// Exact vertex-position instantiations of the four kernels above: two more live floats per hit (kv * rd.y, kv * rd.z
+// in the reduction).  Resident CTAs per SM, measured against the default kernel: 4 (64 registers, 48 bytes of spill)
+// costs 1.006x at C4 and 1.003x at C2, 3 (80 registers, no spill) 1.07x / 1.05x (DESIGN.md 3.3).  The camera
+// instantiations keep DMR_TRI_BWD_CAM_MINB.
+constexpr int DMR_TRI_BWD_EXACT_MINB = DMR_TRI_BWD_MINB;
+__global__ void __launch_bounds__(256, DMR_TRI_BWD_EXACT_MINB) tri_render_bwd_exact_kernel(TriRenderParams p)
+{
+    griddep_wait();   // programmatic dependent launch: see dmr_launch (common.cuh)
+    tri_render_bwd_body<false, false, true>(p, nullptr);
+}
+
+__global__ void __launch_bounds__(256, DMR_TRI_BWD_EXACT_MINB) tri_render_bwd_exact_det_kernel(TriRenderParams p)
+{
+    griddep_wait();   // programmatic dependent launch: see dmr_launch (common.cuh)
+    tri_render_bwd_body<true, false, true>(p, nullptr);
+}
+
+__global__ void __launch_bounds__(256, DMR_TRI_BWD_CAM_MINB) tri_render_bwd_exact_cam_kernel(TriRenderParams p, float* cam_tiles)
+{
+    griddep_wait();   // programmatic dependent launch: see dmr_launch (common.cuh)
+    tri_render_bwd_body<false, true, true>(p, cam_tiles);
+}
+
+__global__ void __launch_bounds__(256, DMR_TRI_BWD_CAM_MINB) tri_render_bwd_exact_cam_det_kernel(TriRenderParams p, float* cam_tiles)
+{
+    griddep_wait();   // programmatic dependent launch: see dmr_launch (common.cuh)
+    tri_render_bwd_body<true, true, true>(p, cam_tiles);
+}
+
 // One CTA per view: the view's per-tile camera records (tri_render_bwd_cam_kernel) are summed in a fixed order -- a
 // thread owns one component (240 = 10 x 24 threads, coalesced reads of the flat record array), then the ten partial
 // sums of a component are added in thread order -- and chained through the inverses: with N = A^-1,
@@ -838,7 +877,8 @@ __global__ void __launch_bounds__(256) det_gmax_kernel(const float* __restrict__
 // ONCE, the world-space triangle (48 B of the record; identical in every view's record) is read once, from view 0.
 // The first version ran one thread per (view, face): at C4 (8 views per call) it re-read the triangle and
 // re-scattered to the same vertices eight times -- 2.46 GB read + 0.73 GB written, HBM-bound at 520 us.
-template <bool DET, bool MULTI>   // MULTI = false: B == 1 (no view loop, no accumulators: 54 instead of 74 registers)
+// EXACT: the statistics of tri_render_bwd_body<.., EXACT> (S3v in logical 6, 21, 22).
+template <bool DET, bool MULTI, bool EXACT = false>   // MULTI = false: B == 1 (no view loop, no accumulators: 54 instead of 74 registers)
 __device__ __forceinline__ void tri_grad_finish_body(const TriRenderParams& p)
 {
     const int nviews = MULTI ? p.B : 1;
@@ -868,12 +908,13 @@ __device__ __forceinline__ void tri_grad_finish_body(const TriRenderParams& p)
         if (DET) {
             const long long* r = p.det_stats + idx * 24;
 #pragma unroll
-            for (int i = 0; i < 21; i++) {
+            for (int i = 0; i < (EXACT ? 23 : 21); i++) {
                 const long long q = r[i];
                 any = any || q != 0;
-                st[i] = (float)((double)q * (i < 7 ? ig : iv));
+                st[i] = (float)((double)q * ((i < 7 || i >= 21) ? ig : iv));
             }
-            st[21] = st[22] = st[23] = 0.0f;
+            if constexpr (!EXACT) st[21] = st[22] = 0.0f;
+            st[23] = 0.0f;
         } else {
             const float4* st4 = reinterpret_cast<const float4*>(p.grad_stats + idx * 24);
             float sm[24];
@@ -897,10 +938,18 @@ __device__ __forceinline__ void tri_grad_finish_body(const TriRenderParams& p)
         const float* imv = p.inv_mv + 16 * b;
         const float3 T = f3(imv[12], imv[13], imv[14]) - v0;
         const float3 S1 = f3(st[0], st[1], st[2]), S24 = f3(st[3], st[4], st[5]);
-        const float S3 = st[6];
-        const float3 gE1 = S3 * cross3(E2, T) - cross3(S24, E2);
-        const float3 gE2 = cross3(T, S1) - cross3(E1, S24) + S3 * cross3(T, E1);
-        const float3 gT = cross3(S1, E2) + S3 * cross3(E1, E2);
+        float3 gE1, gE2, gT;
+        if constexpr (EXACT) {
+            const float3 S3v = f3(st[6], st[21], st[22]);
+            gE1 = cross3(S3v, T) - cross3(S24, E2);
+            gE2 = cross3(T, S1) - cross3(E1, S24);
+            gT = cross3(S1, E2) + cross3(E1, S3v);
+        } else {
+            const float S3 = st[6];
+            gE1 = S3 * cross3(E2, T) - cross3(S24, E2);
+            gE2 = cross3(T, S1) - cross3(E1, S24) + S3 * cross3(T, E1);
+            gT = cross3(S1, E2) + S3 * cross3(E1, E2);
+        }
         const float3 dp[3] = { -gE1 - gE2 - gT, gE1, gE2 };
         p.dL_dfintense[idx] = st[8];
         if constexpr (DET) {
@@ -951,6 +1000,9 @@ __device__ __forceinline__ void tri_grad_finish_body(const TriRenderParams& p)
 template <bool MULTI>
 __global__ void __launch_bounds__(256) tri_grad_finish_kernel(TriRenderParams p) { griddep_wait(); tri_grad_finish_body<false, MULTI>(p); }
 __global__ void __launch_bounds__(256) tri_grad_finish_det_kernel(TriRenderParams p) { griddep_wait(); tri_grad_finish_body<true, true>(p); }
+template <bool MULTI>
+__global__ void __launch_bounds__(256) tri_grad_finish_exact_kernel(TriRenderParams p) { griddep_wait(); tri_grad_finish_body<false, MULTI, true>(p); }
+__global__ void __launch_bounds__(256) tri_grad_finish_exact_det_kernel(TriRenderParams p) { griddep_wait(); tri_grad_finish_body<true, true, true>(p); }
 
 // Deterministic mode, last step: fixed-point accumulators -> += into the caller's fp32 gradient tensors.
 // One thread per vertex, then per (view, vertex), then per face.
@@ -1016,23 +1068,25 @@ int tri_render_forward(const TriRenderParams& p, cudaStream_t stream)
     return 0;
 }
 
-int tri_render_backward(const TriRenderParams& p, cudaStream_t stream, float* cam_tiles)
+int tri_render_backward(const TriRenderParams& p, cudaStream_t stream, float* cam_tiles, bool exact)
 {
     if (p.B <= 0 || p.W <= 0 || p.H <= 0) return 0;
     dim3 grid((p.W + DMR_TILE - 1) / DMR_TILE, (p.H + DMR_TILE - 1) / DMR_TILE, p.B);
     if (cam_tiles) {
         ProfScope prof(ST_TRI_BWD_CAM, stream);
-        DMR_CUDA(dmr_launch(tri_render_bwd_cam_kernel, dim3(grid), dim3(256), 0, stream, p, cam_tiles));
+        DMR_CUDA(dmr_launch(exact ? tri_render_bwd_exact_cam_kernel : tri_render_bwd_cam_kernel, dim3(grid), dim3(256), 0,
+                            stream, p, cam_tiles));
         DMR_LAUNCH_CHECK("tri_render_bwd_cam_kernel");
     } else {
         ProfScope prof(ST_TRI_BWD, stream);
-        DMR_CUDA(dmr_launch(tri_render_bwd_kernel, dim3(grid), dim3(256), 0, stream, p));
+        DMR_CUDA(dmr_launch(exact ? tri_render_bwd_exact_kernel : tri_render_bwd_kernel, dim3(grid), dim3(256), 0, stream, p));
         DMR_LAUNCH_CHECK("tri_render_bwd_kernel");
     }
     {
         ProfScope prof(ST_TRI_BWD_FINISH, stream);
-        if (p.B > 1) DMR_CUDA(dmr_launch(tri_grad_finish_kernel<true>, dim3((unsigned)((p.F + 255) / 256)), dim3(256), 0, stream, p));
-        else DMR_CUDA(dmr_launch(tri_grad_finish_kernel<false>, dim3((unsigned)((p.F + 255) / 256)), dim3(256), 0, stream, p));
+        const dim3 fgrid((unsigned)((p.F + 255) / 256));
+        if (p.B > 1) DMR_CUDA(dmr_launch(exact ? tri_grad_finish_exact_kernel<true> : tri_grad_finish_kernel<true>, fgrid, dim3(256), 0, stream, p));
+        else DMR_CUDA(dmr_launch(exact ? tri_grad_finish_exact_kernel<false> : tri_grad_finish_kernel<false>, fgrid, dim3(256), 0, stream, p));
         DMR_LAUNCH_CHECK("tri_grad_finish_kernel");
         if (p.grad_vacc) {
             count_launch(1);   // two kernels under one scope
@@ -1050,7 +1104,7 @@ int det_gmax(const float* a, size_t na, const float* b, size_t nb, uint32_t* gma
     return 0;
 }
 
-int tri_render_backward_deterministic(const TriRenderParams& p, cudaStream_t stream, float* cam_tiles)
+int tri_render_backward_deterministic(const TriRenderParams& p, cudaStream_t stream, float* cam_tiles, bool exact)
 {
     if (p.B <= 0 || p.W <= 0 || p.H <= 0) return 0;
     dim3 grid((p.W + DMR_TILE - 1) / DMR_TILE, (p.H + DMR_TILE - 1) / DMR_TILE, p.B);
@@ -1061,17 +1115,20 @@ int tri_render_backward_deterministic(const TriRenderParams& p, cudaStream_t str
         int rc = det_gmax(p.dL_dcolor, 3 * p.B * HW, p.dL_ddepth, p.B * HW, const_cast<uint32_t*>(p.det_gmax), stream);
         if (rc) return rc;
         if (cam_tiles) {
-            DMR_CUDA(dmr_launch(tri_render_bwd_cam_det_kernel, dim3(grid), dim3(256), 0, stream, p, cam_tiles));
+            DMR_CUDA(dmr_launch(exact ? tri_render_bwd_exact_cam_det_kernel : tri_render_bwd_cam_det_kernel, dim3(grid),
+                                dim3(256), 0, stream, p, cam_tiles));
             DMR_LAUNCH_CHECK("tri_render_bwd_cam_det_kernel");
         } else {
-            DMR_CUDA(dmr_launch(tri_render_bwd_det_kernel, dim3(grid), dim3(256), 0, stream, p));
+            DMR_CUDA(dmr_launch(exact ? tri_render_bwd_exact_det_kernel : tri_render_bwd_det_kernel, dim3(grid), dim3(256), 0,
+                                stream, p));
             DMR_LAUNCH_CHECK("tri_render_bwd_det_kernel");
         }
     }
     {
         ProfScope prof(ST_TRI_BWD_FINISH, stream);
         count_launch(1);
-        DMR_CUDA(dmr_launch(tri_grad_finish_det_kernel, dim3((unsigned)((p.F + 255) / 256)), dim3(256), 0, stream, p));
+        DMR_CUDA(dmr_launch(exact ? tri_grad_finish_exact_det_kernel : tri_grad_finish_det_kernel,
+                            dim3((unsigned)((p.F + 255) / 256)), dim3(256), 0, stream, p));
         DMR_LAUNCH_CHECK("tri_grad_finish_det_kernel");
         const size_t n = (size_t)p.P + (size_t)p.B * p.P + (size_t)p.F;
         DMR_CUDA(dmr_launch(tri_det_convert_kernel, dim3((unsigned)((n + 255) / 256)), dim3(256), 0, stream, p));

@@ -220,6 +220,30 @@ int dmr_tri_backward_camera(
     void* workspace, size_t workspace_bytes,
     dmr_stream_t stream);
 
+/* Exact vertex-position gradients (no reference counterpart).  The reference's dL_dverts                        */
+/* (ray_tri_intersection_grad, auxiliary.h:288-333) differentiates the ray parameter t where the forward pass     */
+/* uses the second barycentric v; this entry point differentiates v, so dL_dverts is the derivative of the        */
+/* rendered image (coverage, depth order, n_contrib and the clamp region held fixed) and, with camera gradients,  */
+/* consistent with dL_dmv / dL_dproj (a rigid motion of scene and camera together changes nothing).  The other    */
+/* four gradients and the camera gradients are those of dmr_tri_backward_camera.  Arguments as                    */
+/* dmr_tri_backward_camera, except that dL_dmv and dL_dproj may both be NULL (no camera gradients; passing only  */
+/* one of them is an error).  `workspace`: the byte count of the mode it modifies --                              */
+/* dmr_tri_backward_workspace_bytes, dmr_tri_backward_deterministic_bytes (deterministic != 0) or, with camera    */
+/* gradients, dmr_tri_backward_camera_bytes.  Same launches as that mode.                                         */
+int dmr_tri_backward_exact(
+    int B, int P, int F, int W, int H, int R,
+    const float* background,
+    const float* inv_mv_mats, const float* inv_proj_mats,
+    const void* point_buffer, const void* face_buffer,
+    const void* binning_buffer, const void* image_buffer,
+    const float* dL_dcolor, const float* dL_ddepth,
+    float* dL_dverts, float* dL_dvcolor, float* dL_dfopacity, float* dL_dvdepth, float* dL_dfintense,
+    int deterministic,
+    float* dL_dmv,               /* [B,16] or NULL */
+    float* dL_dproj,             /* [B,16] or NULL */
+    void* workspace, size_t workspace_bytes,
+    dmr_stream_t stream);
+
 /* dmr_tri_depth_chain plus the camera part of the fused vertex depth (no reference counterpart):                 */
 /* dL_dmv[b] / dL_dproj[b] += sum_p dL_dvdepth[b,p] * d ndc_z[b,p] / d(mv_mats[b], proj_mats[b]) (no derivative   */
 /* through a clamped clip w).  Reduced in a fixed order without float atomics.  `workspace`:                      */
