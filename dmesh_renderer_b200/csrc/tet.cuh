@@ -145,7 +145,7 @@ struct TetParams {
     float* dL_dverts_color; float* dL_dfaces_opacity;
     float4* grad_vacc;            // [P] zeroed scratch: per-vertex colour gradient (xyz), summed over views
     // deterministic mode only (tet_march_backward_deterministic): zeroed 64-bit fixed-point accumulators (det.cuh)
-    const uint32_t* det_gmax;
+    const uint32_t* det_gmax;     // [2]: bits of max |cotangent|, overflow word
     long long* det_vert;          // [P,4]: dL_dverts_color rgb, -
     long long* det_fopa;          // [F]
 };
@@ -156,16 +156,23 @@ struct TetParams {
 __host__ __device__ inline size_t tet_cam_records(size_t B, int W, int H) { return B * (size_t)((W + 7) / 8) * ((H + 7) / 8); }
 
 struct TetDetLayout {             // workspace of the deterministic backward pass
-    size_t gmax, vert, fopa, total;
-    static TetDetLayout make(size_t P, size_t F)
+    size_t gmax, vert, fopa, hi, total;   // low words vert..fopa, their high words mirrored at hi
+    __host__ __device__ static TetDetLayout make(size_t P, size_t F)
     {
         TetDetLayout L;
         size_t o = 0;
         L.gmax = o; o = align_up(o + 4, 256);
         L.vert = o; o = align_up(o + 8 * 4 * P, 256);
         L.fopa = o; o = align_up(o + 8 * F, 256);
+        L.hi = o;   o += o - L.vert;
         L.total = o;
         return L;
+    }
+    // element offset of an accumulator's high word from its low word (det.cuh)
+    __host__ __device__ static ptrdiff_t hi_offset(size_t P, size_t F)
+    {
+        const TetDetLayout L = make(P, F);
+        return (ptrdiff_t)((L.hi - L.vert) / 8);
     }
 };
 

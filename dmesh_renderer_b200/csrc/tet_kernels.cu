@@ -747,6 +747,7 @@ struct TetBwdState {
     float last_color[3], accum_rec[3];
     bool first_iter;
     float det_sv;       // deterministic mode: fixed-point scale (det.cuh)
+    ptrdiff_t det_hi;   // ... and the offset of the high words
 };
 
 // Gradient terms of one crossed face (backward.cu:252-360) and their reduction.
@@ -812,11 +813,13 @@ __device__ __forceinline__ void tet_bwd_face(const TetParams& p, TetBwdState& st
     if (DET) {
         // deterministic mode (det.cuh): 64-bit fixed-point accumulators, any arrival order gives the same bits
         const float sv = st.det_sv;
+        const ptrdiff_t hi = st.det_hi;
+        const uint32_t* gm = p.det_gmax;
         long long* a0 = p.det_vert + 4 * (size_t)vi0; long long* a1 = p.det_vert + 4 * (size_t)vi1; long long* a2 = p.det_vert + 4 * (size_t)vi2;
-        det_add(a0 + 0, g00, sv); det_add(a0 + 1, g01, sv); det_add(a0 + 2, g02, sv);
-        det_add(a1 + 0, g10, sv); det_add(a1 + 1, g11, sv); det_add(a1 + 2, g12, sv);
-        det_add(a2 + 0, g20, sv); det_add(a2 + 1, g21, sv); det_add(a2 + 2, g22, sv);
-        det_add(p.det_fopa + face, dL_dopa, sv);
+        det_add(a0 + 0, g00, sv, hi, gm); det_add(a0 + 1, g01, sv, hi, gm); det_add(a0 + 2, g02, sv, hi, gm);
+        det_add(a1 + 0, g10, sv, hi, gm); det_add(a1 + 1, g11, sv, hi, gm); det_add(a1 + 2, g12, sv, hi, gm);
+        det_add(a2 + 0, g20, sv, hi, gm); det_add(a2 + 1, g21, sv, hi, gm); det_add(a2 + 2, g22, sv, hi, gm);
+        det_add(p.det_fopa + face, dL_dopa, sv, hi, gm);
         return;
     }
     red_add_v4(reinterpret_cast<float*>(p.grad_vacc + vi0), g00, g01, g02, 0.0f);
@@ -917,7 +920,8 @@ __device__ __forceinline__ void tet_march_bwd_body(const TetParams& p, TetCamAcc
 
     TetBwdState st;
     st.det_sv = 0.0f;
-    if (DET) { float sg; det_scales(*p.det_gmax, st.det_sv, sg); }
+    st.det_hi = 0;
+    if (DET) { float sg; det_scales(*p.det_gmax, st.det_sv, sg); st.det_hi = TetDetLayout::hi_offset(p.P, p.F); }
     st.prev_log_T = fin_prev_log_T;
     st.last_alpha = 0.0f; st.last_depth = 0.0f; st.accum_recd = 0.0f;
 #pragma unroll
@@ -1178,7 +1182,7 @@ __global__ void __launch_bounds__(256) tet_det_convert_kernel(TetParams p)
     float sv, sg;
     det_scales(*p.det_gmax, sv, sg);
     size_t i = (size_t)blockIdx.x * 256 + threadIdx.x;
-    if (det_nonfinite(*p.det_gmax)) {
+    if (det_poisoned(p.det_gmax)) {
         const float nan = __int_as_float(0x7fc00000);
         if (i < (size_t)p.P) { for (int c = 0; c < 3; c++) p.dL_dverts_color[3 * i + c] = nan; }
         else if (i - (size_t)p.P < (size_t)p.F) p.dL_dfaces_opacity[i - (size_t)p.P] = nan;
@@ -1186,19 +1190,19 @@ __global__ void __launch_bounds__(256) tet_det_convert_kernel(TetParams p)
     }
     if (sv == 0.0f) return;
     const double iv = 1.0 / (double)sv;
+    const ptrdiff_t hi = TetDetLayout::hi_offset(p.P, p.F);
     if (i < (size_t)p.P) {
         const long long* a = p.det_vert + 4 * i;
 #pragma unroll
         for (int c = 0; c < 3; c++) {
-            const long long q = a[c];
-            if (q != 0) p.dL_dverts_color[3 * i + c] += (float)((double)q * iv);
+            if (det_nonzero(a + c, hi)) p.dL_dverts_color[3 * i + c] += (float)det_value(a + c, hi, iv);
         }
         return;
     }
     i -= (size_t)p.P;
     if (i < (size_t)p.F) {
-        const long long q = p.det_fopa[i];
-        if (q != 0) p.dL_dfaces_opacity[i] += (float)((double)q * iv);
+        const long long* a = p.det_fopa + i;
+        if (det_nonzero(a, hi)) p.dL_dfaces_opacity[i] += (float)det_value(a, hi, iv);
     }
 }
 

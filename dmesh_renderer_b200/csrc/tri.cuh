@@ -29,7 +29,7 @@ struct TriRenderParams {
     float* grad_stats;              // [B*F,24] zeroed scratch (face buffer)
     float4* grad_vacc;              // [2][P] zeroed scratch: per-vertex dL_dverts / dL_dvcolor accumulators
     // deterministic mode only (tri_render_backward_deterministic): zeroed 64-bit fixed-point accumulators
-    const uint32_t* det_gmax;       // bits of max |cotangent| (written by tri_det_gmax_kernel)
+    const uint32_t* det_gmax;       // [2]: bits of max |cotangent| (written by det_gmax_kernel), overflow word
     long long* det_stats;           // [B*F,24] statistics in logical order
     long long* det_vert;            // [P,8]: dL_dverts xyz, -, dL_dvcolor rgb, -
     long long* det_vdepth;          // [B*P]
@@ -37,8 +37,8 @@ struct TriRenderParams {
 };
 
 struct TriDetLayout {               // workspace of the deterministic backward pass
-    size_t gmax, stats, vert, vdepth, fopa, total;
-    static TriDetLayout make(size_t B, size_t P, size_t F)
+    size_t gmax, stats, vert, vdepth, fopa, hi, total;   // low words stats..fopa, their high words mirrored at hi
+    __host__ __device__ static TriDetLayout make(size_t B, size_t P, size_t F)
     {
         TriDetLayout L;
         size_t o = 0;
@@ -47,8 +47,15 @@ struct TriDetLayout {               // workspace of the deterministic backward p
         L.vert = o;   o = align_up(o + 8 * 8 * P, 256);
         L.vdepth = o; o = align_up(o + 8 * B * P, 256);
         L.fopa = o;   o = align_up(o + 8 * F, 256);
+        L.hi = o;     o += o - L.stats;
         L.total = o;
         return L;
+    }
+    // element offset of an accumulator's high word from its low word (det.cuh)
+    __host__ __device__ static ptrdiff_t hi_offset(size_t B, size_t P, size_t F)
+    {
+        const TriDetLayout L = make(B, P, F);
+        return (ptrdiff_t)((L.hi - L.stats) / 8);
     }
 };
 

@@ -685,12 +685,13 @@ __device__ __forceinline__ void tri_render_bwd_body(const TriRenderParams& p, fl
                         // fixed-point record in LOGICAL order: this lane holds sums 12*cls .. 12*cls+11
                         const int cls = lane & 1;
                         long long* rec = p.det_stats + (size_t)s_rec[j * 9 + 1].w * 24 + 12 * cls;
+                        const ptrdiff_t det_hi = TriDetLayout::hi_offset(p.B, p.P, p.F);
 #pragma unroll
                         for (int k = 0; k < 12; k++) {
                             if (cls == 1 && k >= (EXACT ? 11 : 9)) break;        // logical 21..23 (EXACT: 23): padding
                             // vertex-position statistics: logical 0..6 (EXACT: and 21, 22) take the finer scale
                             const bool pos = cls == 0 ? k < 7 : (EXACT && k >= 9);
-                            det_add(rec + k, v[k], pos ? det_sg : det_sv);
+                            det_add(rec + k, v[k], pos ? det_sg : det_sv, det_hi, p.det_gmax);
                         }
                     }
                 } else if (have) {
@@ -886,9 +887,11 @@ __device__ __forceinline__ void tri_grad_finish_body(const TriRenderParams& p)
     if (f >= (size_t)p.F) return;
     float det_sv = 0.0f, det_sg = 0.0f;
     double iv = 0.0, ig = 0.0;
+    ptrdiff_t hi = 0;
     if (DET) {
         det_scales(*p.det_gmax, det_sv, det_sg);
-        if (det_nonfinite(*p.det_gmax)) {
+        hi = TriDetLayout::hi_offset(p.B, p.P, p.F);
+        if (det_poisoned(p.det_gmax)) {
             for (int b = 0; b < nviews; b++) p.dL_dfintense[(size_t)b * p.F + f] = __int_as_float(0x7fc00000);
             return;
         }
@@ -909,9 +912,8 @@ __device__ __forceinline__ void tri_grad_finish_body(const TriRenderParams& p)
             const long long* r = p.det_stats + idx * 24;
 #pragma unroll
             for (int i = 0; i < (EXACT ? 23 : 21); i++) {
-                const long long q = r[i];
-                any = any || q != 0;
-                st[i] = (float)((double)q * ((i < 7 || i >= 21) ? ig : iv));
+                any = any || det_nonzero(r + i, hi);
+                st[i] = (float)det_value(r + i, hi, (i < 7 || i >= 21) ? ig : iv);
             }
             if constexpr (!EXACT) st[21] = st[22] = 0.0f;
             st[23] = 0.0f;
@@ -957,11 +959,15 @@ __device__ __forceinline__ void tri_grad_finish_body(const TriRenderParams& p)
 #pragma unroll
             for (int k = 0; k < 3; k++) {
                 long long* a = p.det_vert + 8 * (size_t)vi[k];
-                det_add(a + 0, dp[k].x, det_sg); det_add(a + 1, dp[k].y, det_sg); det_add(a + 2, dp[k].z, det_sg);
-                det_add(a + 4, st[12 + 3 * k], det_sv); det_add(a + 5, st[13 + 3 * k], det_sv); det_add(a + 6, st[14 + 3 * k], det_sv);
-                det_add(p.det_vdepth + (size_t)b * p.P + vi[k], st[9 + k], det_sv);
+                det_add(a + 0, dp[k].x, det_sg, hi, p.det_gmax);
+                det_add(a + 1, dp[k].y, det_sg, hi, p.det_gmax);
+                det_add(a + 2, dp[k].z, det_sg, hi, p.det_gmax);
+                det_add(a + 4, st[12 + 3 * k], det_sv, hi, p.det_gmax);
+                det_add(a + 5, st[13 + 3 * k], det_sv, hi, p.det_gmax);
+                det_add(a + 6, st[14 + 3 * k], det_sv, hi, p.det_gmax);
+                det_add(p.det_vdepth + (size_t)b * p.P + vi[k], st[9 + k], det_sv, hi, p.det_gmax);
             }
-            det_add(p.det_fopa + f, st[7], det_sv);
+            det_add(p.det_fopa + f, st[7], det_sv, hi, p.det_gmax);
         } else {
 #pragma unroll
             for (int k = 0; k < 3; k++) {
@@ -1013,7 +1019,7 @@ __global__ void __launch_bounds__(256) tri_det_convert_kernel(TriRenderParams p)
     det_scales(*p.det_gmax, sv, sg);
     const size_t P = (size_t)p.P, BP = (size_t)p.B * p.P, F = (size_t)p.F;
     size_t i = (size_t)blockIdx.x * 256 + threadIdx.x;
-    if (det_nonfinite(*p.det_gmax)) {
+    if (det_poisoned(p.det_gmax)) {
         const float nan = __int_as_float(0x7fc00000);
         if (i < P) { for (int c = 0; c < 3; c++) { p.dL_dverts[3 * i + c] = nan; p.dL_dvcolor[3 * i + c] = nan; } }
         else if (i - P < BP) p.dL_dvdepth[i - P] = nan;
@@ -1022,26 +1028,26 @@ __global__ void __launch_bounds__(256) tri_det_convert_kernel(TriRenderParams p)
     }
     if (sv == 0.0f) return;
     const double iv = 1.0 / (double)sv, ig = 1.0 / (double)sg;
+    const ptrdiff_t hi = TriDetLayout::hi_offset(p.B, p.P, p.F);
     if (i < P) {
         const long long* a = p.det_vert + 8 * i;
 #pragma unroll
         for (int c = 0; c < 3; c++) {
-            const long long q = a[c], r = a[4 + c];
-            if (q != 0) p.dL_dverts[3 * i + c] += (float)((double)q * ig);
-            if (r != 0) p.dL_dvcolor[3 * i + c] += (float)((double)r * iv);
+            if (det_nonzero(a + c, hi)) p.dL_dverts[3 * i + c] += (float)det_value(a + c, hi, ig);
+            if (det_nonzero(a + 4 + c, hi)) p.dL_dvcolor[3 * i + c] += (float)det_value(a + 4 + c, hi, iv);
         }
         return;
     }
     i -= P;
     if (i < BP) {
-        const long long q = p.det_vdepth[i];
-        if (q != 0) p.dL_dvdepth[i] += (float)((double)q * iv);
+        const long long* a = p.det_vdepth + i;
+        if (det_nonzero(a, hi)) p.dL_dvdepth[i] += (float)det_value(a, hi, iv);
         return;
     }
     i -= BP;
     if (i < F) {
-        const long long q = p.det_fopa[i];
-        if (q != 0) p.dL_dfopacity[i] += (float)((double)q * iv);
+        const long long* a = p.det_fopa + i;
+        if (det_nonzero(a, hi)) p.dL_dfopacity[i] += (float)det_value(a, hi, iv);
     }
 }
 
