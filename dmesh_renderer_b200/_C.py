@@ -485,11 +485,14 @@ def tri_depth_chain(verts, mv_mats, proj_mats, dL_dvdepth, dL_dverts, dL_dmv=Non
 # ---------------------------------------------------------------------------
 class _TetRecordCache:
     """The view-independent adjacency records of the tet renderer (one 128-byte TetRec per tet, csrc/tet.cuh)
-    depend only on verts / faces / tets / face_tets / tet_faces.  None of them carries a gradient in the tet
-    renderer (reference dmesh_renderer/__init__.py:407-422), so in an optimisation loop they are the same tensors in
-    every step: the records are built once and reused while the caller keeps passing the SAME tensor objects,
-    unmodified (identity + torch's in-place version counter; weak references, so a freed tensor can never match a
-    new one that happens to reuse its memory).  One entry per device."""
+    depend only on verts / faces / tets / face_tets / tet_faces.  Without vertex-position gradients none of them
+    carries a gradient (reference dmesh_renderer/__init__.py:407-422), so in an optimisation loop they are the same
+    tensors in every step: the records are built once and reused while the caller keeps passing the SAME tensor
+    objects, unmodified (identity + torch's in-place version counter; weak references, so a freed tensor can never
+    match a new one that happens to reuse its memory).  With vertex-position gradients (set_tet_vertex_grads) the
+    optimiser updates `verts` in place every step; that bumps its version counter, so the records are rebuilt.
+    Writing through `verts.data` bypasses the version counter and is not supported: the stale records would be
+    reused.  One entry per device."""
     _entries = {}
 
     @classmethod
@@ -589,7 +592,7 @@ def render_tets(background, verts, faces, verts_color, faces_opacity, mv_mats, p
 def render_tets_backward(background, verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, inv_mv_mats,
                          inv_proj_mats, verts_depth, faces_intense, tets, face_tets, tet_faces, grad_color, grad_depth,
                          pointBuffer, faceBuffer, binningBuffer, imageBuffer, ray_random_seed=None, deterministic=False,
-                         tet_records=None, camera_grads=False):
+                         tet_records=None, camera_grads=False, vertex_grads=False):
     """RenderFTetsBackwardCUDA (render.cu:338-412).
     Returns (dL_dverts_color[P,3], dL_dfaces_opacity[F]).  `ray_random_seed` is an
     optional trailing argument beyond the reference's 20: the autograd wrapper passes
@@ -598,7 +601,9 @@ def render_tets_backward(background, verts, faces, verts_color, faces_opacity, m
     gradients (dmr_tet_backward_deterministic).  `tet_records`: the adjacency records of the forward call (the
     autograd wrapper passes them; otherwise they are taken from the face buffer's attribute or rebuilt).
     `camera_grads`: also return dL_dmv_mats, dL_dproj_mats [B,4,4] (gradients with respect to the mv_mats / proj_mats
-    tensors passed here, through the rays and the hit-point depth; dmr_tet_backward_camera) as two more elements."""
+    tensors passed here, through the rays and the hit-point depth; dmr_tet_backward_camera) as two more elements.
+    `vertex_grads`: also return dL_dverts [P,3] (gradient with respect to the vertex positions, through the (t, u, v)
+    of every walked step; dmr_tet_backward_vertex) as the last element."""
     lib = _lib.load()
     B, P, F, T = mv_mats.size(0), verts.size(0), faces.size(0), tets.size(0)
     H, W = grad_color.size(2), grad_color.size(3)
@@ -611,6 +616,7 @@ def render_tets_backward(background, verts, faces, verts_color, faces_opacity, m
         dL_dfaces_opacity = torch.zeros((F,), **z)
         # [B,16] column-major = [B,4,4] gradients of the (column-major, i.e. transposed) matrix tensors given here
         cam = torch.zeros((2, B, 4, 4), **z) if camera_grads else None
+        dL_dverts = torch.zeros((P, 3), **z) if vertex_grads else None
         if B * H * W > 0 and F > 0 and T > 0:
             bg = _f32(background, "background")
             mv, pj = _f32(mv_mats, "mv_mats"), _f32(proj_mats, "proj_mats")
@@ -628,7 +634,13 @@ def render_tets_backward(background, verts, faces, verts_color, faces_opacity, m
             a = (B, P, F, T, W, H, int(ray_random_seed), _ptr(bg), _ptr(mv), _ptr(pj), _ptr(imv), _ptr(ipj), _ptr(fint),
                  _ptr(pointBuffer), _ptr(faceBuffer), _ptr(tet_rec), _ptr(imageBuffer), _ptr(gc), _ptr(gd),
                  _ptr(dL_dverts_color), _ptr(dL_dfaces_opacity))
-            if camera_grads:
+            if vertex_grads:
+                det = int(bool(deterministic))
+                ws = torch.empty(lib.dmr_tet_backward_vertex_bytes(B, P, F, W, H, det, int(bool(camera_grads))),
+                                 dtype=torch.uint8, device=dev)
+                c = (_ptr(cam[0]), _ptr(cam[1])) if camera_grads else (ctypes.c_void_p(0), ctypes.c_void_p(0))
+                _lib.check(lib.dmr_tet_backward_vertex(*a, det, *c, _ptr(dL_dverts), _ptr(ws), ws.numel(), _stream()))
+            elif camera_grads:
                 ws = torch.empty(lib.dmr_tet_backward_camera_bytes(B, P, F, W, H, int(bool(deterministic))),
                                  dtype=torch.uint8, device=dev)
                 _lib.check(lib.dmr_tet_backward_camera(*a, int(bool(deterministic)), _ptr(cam[0]), _ptr(cam[1]), _ptr(ws),
@@ -639,6 +651,9 @@ def render_tets_backward(background, verts, faces, verts_color, faces_opacity, m
             else:
                 ws = torch.empty(lib.dmr_tet_backward_workspace_bytes(P), dtype=torch.uint8, device=dev)
                 _lib.check(lib.dmr_tet_backward(*a, _ptr(ws), ws.numel(), _stream()))
+    out = (dL_dverts_color, dL_dfaces_opacity)
     if camera_grads:
-        return dL_dverts_color, dL_dfaces_opacity, cam[0], cam[1]
-    return dL_dverts_color, dL_dfaces_opacity
+        out += (cam[0], cam[1])
+    if vertex_grads:
+        out += (dL_dverts,)
+    return out

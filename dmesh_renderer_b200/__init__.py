@@ -167,7 +167,8 @@ class TriRenderer(th.nn.Module):
 
 # =============================================================================
 # TetRenderer: faces of a tetrahedral complex, exact depth order by ray marching
-# through tet adjacency; gradients to vertex colours, face opacities and (opt-in) the camera matrices.
+# through tet adjacency; gradients to vertex colours, face opacities and (opt-in) the camera matrices and the
+# vertex positions.
 # =============================================================================
 class TetRenderSettings(NamedTuple):      # reference __init__.py:237-241
     image_height: int
@@ -176,12 +177,28 @@ class TetRenderSettings(NamedTuple):      # reference __init__.py:237-241
     ray_random_seed: int
 
 
+_tet_vertex_grads_default = False
+
+
+def set_tet_vertex_grads(flag: bool) -> bool:
+    """Process-wide default for the tet renderer's vertex-position gradient (extension).  False (the default): like the
+    reference, the tet renderer returns no gradient for verts.  True: when verts requires grad, its gradient is the
+    exact derivative of the rendered colour and depth images, consistent with the camera gradients.  The other
+    gradients are the same either way.  `TetRenderer(settings, vertex_grads=...)` / `render_tet(..., vertex_grads=...)`
+    override it per renderer / call.  Returns the previous value."""
+    global _tet_vertex_grads_default
+    old, _tet_vertex_grads_default = _tet_vertex_grads_default, bool(flag)
+    return old
+
+
 def render_tet(verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, verts_depth, faces_intense, tets,
-               face_tets, tet_faces, render_settings: TetRenderSettings, deterministic=None):
-    """reference __init__.py:243-275 (`deterministic`: see set_deterministic)"""
+               face_tets, tet_faces, render_settings: TetRenderSettings, deterministic=None, vertex_grads=None):
+    """reference __init__.py:243-275 (`deterministic`: see set_deterministic; `vertex_grads`: see
+    set_tet_vertex_grads)"""
     det = _deterministic_default if deterministic is None else bool(deterministic)
+    vert = _tet_vertex_grads_default if vertex_grads is None else bool(vertex_grads)
     return _RenderTet.apply(verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, verts_depth, faces_intense,
-                            tets, face_tets, tet_faces, render_settings, det)
+                            tets, face_tets, tet_faces, render_settings, det, vert)
 
 
 class _RenderTet(th.autograd.Function):
@@ -189,8 +206,9 @@ class _RenderTet(th.autograd.Function):
 
     @staticmethod
     def forward(ctx, verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, verts_depth, faces_intense, tets,
-                face_tets, tet_faces, render_settings, deterministic=False):
+                face_tets, tet_faces, render_settings, deterministic=False, vertex_grads=False):
         ctx.deterministic = deterministic
+        ctx.vertex_grads = vertex_grads
         inv = _C._Inverses(mv_mats, proj_mats)   # th.inverse x2 (reference :298-299): one launch, no device sync
         inv_mv_mats, inv_proj_mats = inv.inv_mv, inv.inv_proj
         mv_mats, proj_mats = inv.mv, inv.proj    # contiguous copies written by the same launch
@@ -222,35 +240,42 @@ class _RenderTet(th.autograd.Function):
         # camera gradients (extension): requested by setting requires_grad on mv_mats or proj_mats; per view, through
         # autograd only
         camera = ctx.needs_input_grad[4] or ctx.needs_input_grad[5]
-        grad_mv = grad_proj = None
+        # vertex-position gradients (extension): only when switched on AND verts requires grad (DMesh passes verts
+        # that require grad, so requires_grad alone must not turn this on)
+        vertex = ctx.vertex_grads and ctx.needs_input_grad[0]
+        grad_mv = grad_proj = grad_verts = None
         try:
             grads = _C.render_tets_backward(*args, deterministic=ctx.deterministic, tet_records=ctx.tet_records,
-                                            camera_grads=camera)
+                                            camera_grads=camera, vertex_grads=vertex)
         except Exception as ex:
             print("\nAn error occured in backward.\n")
             raise ex
         grad_verts_color, grad_faces_opacity = grads[:2]
         if camera:
             grad_mv, grad_proj = grads[2], grads[3]
-        # gradient positions: reference __init__.py:407-422; positions 4 and 5 (the matrices) are an extension
-        return (None, None, grad_verts_color, grad_faces_opacity,
+        if vertex:
+            grad_verts = grads[-1]
+        # gradient positions: reference __init__.py:407-422; positions 0 (verts) and 4, 5 (the matrices) are an extension
+        return (grad_verts, None, grad_verts_color, grad_faces_opacity,
                 grad_mv if ctx.needs_input_grad[4] else None, grad_proj if ctx.needs_input_grad[5] else None,
-                None, None, None, None, None, None, None)
+                None, None, None, None, None, None, None, None)
 
 
 class TetRenderer(th.nn.Module):
     """reference __init__.py:426-488"""
 
-    def __init__(self, render_settings: TetRenderSettings, deterministic=None):
+    def __init__(self, render_settings: TetRenderSettings, deterministic=None, vertex_grads=None):
         super().__init__()
         self.render_settings = render_settings
         self.deterministic = deterministic     # None: the process-wide default (set_deterministic)
+        self.vertex_grads = vertex_grads       # None: the process-wide default (set_tet_vertex_grads)
 
     def forward(self, verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, verts_depth, faces_intense, tets,
                 face_tets, tet_faces):
         """
         Gradients for verts_color and faces_opacity, and (extension) for mv_mats / proj_mats when they require
-        grad.  verts_depth is accepted but unused (depth comes from the re-projected hit point).
+        grad and for verts when vertex_grads is on and verts requires grad.  verts_depth is accepted but unused
+        (depth comes from the re-projected hit point).
         tets [T,4], face_tets [F,2] (-1 = boundary), tet_faces [T,4]
         returns color [B,3,H,W], depth [B,1,H,W], active [B,H,W] bool
         """
@@ -259,4 +284,4 @@ class TetRenderer(th.nn.Module):
                           faces_opacity.to(dtype=f32), mv_mats.to(dtype=f32).transpose(1, 2),
                           proj_mats.to(dtype=f32).transpose(1, 2), verts_depth.to(dtype=f32),
                           faces_intense.to(dtype=f32), tets.to(dtype=i32), face_tets.to(dtype=i32),
-                          tet_faces.to(dtype=i32), self.render_settings, self.deterministic)
+                          tet_faces.to(dtype=i32), self.render_settings, self.deterministic, self.vertex_grads)

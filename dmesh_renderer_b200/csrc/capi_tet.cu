@@ -32,17 +32,28 @@ bool tet_sizes_ok(long long B, long long P, long long F, long long T, long long 
 }
 
 // scratch of the backward pass of either mode (dmr_tet_backward_workspace_bytes without its slack,
-// dmr_tet_backward_deterministic_bytes)
-size_t tet_bwd_scratch_bytes(int P, int F, bool deterministic)
+// dmr_tet_backward_deterministic_bytes); vert: with the per-vertex position accumulator (default mode: a second
+// float4[P] right behind the colour one; deterministic mode: TetDetLayout::pos)
+size_t tet_bwd_scratch_bytes(int P, int F, bool deterministic, bool vert = false)
 {
-    return deterministic ? TetDetLayout::make((size_t)P, (size_t)F).total : sizeof(float4) * (size_t)P;
+    if (deterministic) {
+        const TetDetLayout L = TetDetLayout::make((size_t)P, (size_t)F);
+        return vert ? L.total_pos : L.total;
+    }
+    return sizeof(float4) * (size_t)P * (vert ? 2 : 1);
 }
 
 // workspace of the camera-gradient backward: the mode's own scratch, then DMR_TET_CAM_REC floats per (view, march CTA)
-size_t tet_cam_bytes(int B, int P, int F, int W, int H, bool deterministic)
+size_t tet_cam_bytes(int B, int P, int F, int W, int H, bool deterministic, bool vert = false)
 {
-    return align_up(tet_bwd_scratch_bytes(P, F, deterministic), 256) +
+    return align_up(tet_bwd_scratch_bytes(P, F, deterministic, vert), 256) +
            align_up(sizeof(float) * DMR_TET_CAM_REC * tet_cam_records((size_t)B, W, H), 256) + 256;
+}
+
+// workspace of the vertex-position backward, with or without camera gradients
+size_t tet_vert_bytes(int B, int P, int F, int W, int H, bool deterministic, bool cam)
+{
+    return cam ? tet_cam_bytes(B, P, F, W, H, deterministic, true) : tet_bwd_scratch_bytes(P, F, deterministic, true) + 256;
 }
 
 }  // namespace
@@ -172,9 +183,11 @@ static int tet_backward_impl(int B, int P, int F, int T, int W, int H, int ray_r
                              const void* face_buffer, const void* tet_records, const void* image_buffer,
                              const float* dL_dcolor, const float* dL_ddepth, float* dL_dverts_color,
                              float* dL_dfaces_opacity, void* workspace, size_t workspace_bytes, bool deterministic,
-                             dmr_stream_t stream_, float* dL_dmv = nullptr, float* dL_dproj = nullptr)
+                             dmr_stream_t stream_, float* dL_dmv = nullptr, float* dL_dproj = nullptr,
+                             float* dL_dverts = nullptr)
 {
     const bool cam = dL_dmv != nullptr;
+    const bool vert = dL_dverts != nullptr;
     cudaStream_t stream = (cudaStream_t)stream_;
     if (!tet_sizes_ok(B, P, F, T, W, H)) return DMR_ETOOLARGE;
     if (B == 0 || F == 0 || T == 0) return DMR_OK;
@@ -184,17 +197,25 @@ static int tet_backward_impl(int B, int P, int F, int T, int W, int H, int ray_r
         return DMR_EINVAL;
     }
     (void)point_buffer;
+    if (vert) {
+        const size_t need = tet_vert_bytes(B, P, F, W, H, deterministic, cam);
+        if (!workspace || workspace_bytes < need) {
+            set_error("vertex-gradient backward needs a workspace of %zu bytes (dmr_tet_backward_vertex_bytes)", need);
+            return DMR_EINVAL;
+        }
+    }
     // camera gradients: one record per (view, march CTA) behind the mode's own scratch, written by every CTA, so it is
     // not cleared
     float* cam_rec = nullptr;
     if (cam) {
-        const size_t need = tet_cam_bytes(B, P, F, W, H, deterministic);
+        const size_t need = tet_cam_bytes(B, P, F, W, H, deterministic, vert);
         if (!workspace || workspace_bytes < need) {
             set_error("camera-gradient backward needs a workspace of %zu bytes (dmr_tet_backward_camera_bytes)", need);
             return DMR_EINVAL;
         }
-        cam_rec = at<float>(workspace, align_up(tet_bwd_scratch_bytes(P, F, deterministic), 256));
+        cam_rec = at<float>(workspace, align_up(tet_bwd_scratch_bytes(P, F, deterministic, vert), 256));
     }
+    TetVertGrad vg{ dL_dverts, nullptr, nullptr };
     void* det_workspace = workspace;
     const size_t det_workspace_bytes = workspace_bytes;
     TetParams p;
@@ -213,8 +234,9 @@ static int tet_backward_impl(int B, int P, int F, int T, int W, int H, int ray_r
         p.det_vert = at<long long>(det_workspace, DL.vert);
         p.det_fopa = at<long long>(det_workspace, DL.fopa);
         p.grad_vacc = nullptr;
-        DMR_CUDA(cudaMemsetAsync(det_workspace, 0, DL.total, stream));
-        int rc = tet_march_backward_deterministic(p, stream, cam_rec);
+        vg.det_pos = at<long long>(det_workspace, DL.pos);
+        DMR_CUDA(cudaMemsetAsync(det_workspace, 0, vert ? DL.total_pos : DL.total, stream));
+        int rc = tet_march_backward_deterministic(p, stream, cam_rec, vert ? &vg : nullptr);
         if (rc || !cam) return rc;
         return tet_camera_finish(p, cam_rec, dL_dmv, dL_dproj, stream);
     }
@@ -224,8 +246,9 @@ static int tet_backward_impl(int B, int P, int F, int T, int W, int H, int ray_r
         return DMR_EINVAL;
     }
     p.grad_vacc = static_cast<float4*>(workspace);
-    DMR_CUDA(cudaMemsetAsync(p.grad_vacc, 0, sizeof(float4) * (size_t)P, stream));
-    int rc = tet_march_backward(p, stream, cam_rec);
+    vg.grad_pacc = p.grad_vacc + P;
+    DMR_CUDA(cudaMemsetAsync(p.grad_vacc, 0, sizeof(float4) * (size_t)P * (vert ? 2 : 1), stream));
+    int rc = tet_march_backward(p, stream, cam_rec, vert ? &vg : nullptr);
     if (rc || !cam) return rc;
     return tet_camera_finish(p, cam_rec, dL_dmv, dL_dproj, stream);
 }
@@ -294,6 +317,31 @@ int dmr_tet_backward_camera(int B, int P, int F, int T, int W, int H, int ray_ra
                              inv_proj_mats, faces_intense, point_buffer, face_buffer, tet_records, image_buffer, dL_dcolor,
                              dL_ddepth, dL_dverts_color, dL_dfaces_opacity, workspace, workspace_bytes, deterministic != 0,
                              stream, dL_dmv, dL_dproj);
+}
+
+size_t dmr_tet_backward_vertex_bytes(int B, int P, int F, int W, int H, int deterministic, int camera)
+{
+    if (B < 0 || P < 0 || F < 0 || W < 0 || H < 0) return 0;
+    return tet_vert_bytes(B, P, F, W, H, deterministic != 0, camera != 0);
+}
+
+int dmr_tet_backward_vertex(int B, int P, int F, int T, int W, int H, int ray_random_seed, const float* background,
+                            const float* mv_mats, const float* proj_mats, const float* inv_mv_mats,
+                            const float* inv_proj_mats, const float* faces_intense, const void* point_buffer,
+                            const void* face_buffer, const void* tet_records, const void* image_buffer,
+                            const float* dL_dcolor, const float* dL_ddepth, float* dL_dverts_color,
+                            float* dL_dfaces_opacity, int deterministic, float* dL_dmv, float* dL_dproj, float* dL_dverts,
+                            void* workspace, size_t workspace_bytes, dmr_stream_t stream)
+{
+    if ((dL_dmv == nullptr) != (dL_dproj == nullptr)) {
+        set_error("dL_dmv and dL_dproj: pass both (camera gradients) or neither");
+        return DMR_EINVAL;
+    }
+    if (B > 0 && !dL_dverts) { set_error("null pointer: dL_dverts"); return DMR_EINVAL; }
+    return tet_backward_impl(B, P, F, T, W, H, ray_random_seed, background, mv_mats, proj_mats, inv_mv_mats,
+                             inv_proj_mats, faces_intense, point_buffer, face_buffer, tet_records, image_buffer, dL_dcolor,
+                             dL_ddepth, dL_dverts_color, dL_dfaces_opacity, workspace, workspace_bytes, deterministic != 0,
+                             stream, dL_dmv, dL_dproj, dL_dverts);
 }
 
 int dmr_debug_set_tet_first_split(int split)

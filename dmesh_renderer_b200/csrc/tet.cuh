@@ -55,10 +55,11 @@ struct __align__(16) TetShade {
 static_assert(sizeof(TetShade) == 64, "TetShade must be 4 x 16 bytes");
 
 // Face buffer of the tet renderer.  The view-independent adjacency records (TetRec[T]) are NOT part of it: they
-// depend only on the geometry tables, which carry no gradient and are the same in every optimisation step, so they
-// live in a separate `tet_records` buffer the caller may keep across calls (dmr_tet_records_bytes,
-// dmr_tet_forward_bin's tet_records_valid).  The backward scratch is the caller's workspace (the state buffers of
-// the forward call stay read-only).
+// depend only on the geometry tables, so they live in a separate `tet_records` buffer the caller may keep across
+// calls while the geometry stays the same (dmr_tet_records_bytes, dmr_tet_forward_bin's tet_records_valid).  With
+// vertex-position gradients (dmr_tet_backward_vertex) `verts` changes in every optimisation step, and the records
+// have to be rebuilt whenever it does.  The backward scratch is the caller's workspace (the state buffers of the
+// forward call stay read-only).
 struct TetFaceLayout {
     FaceBinLayout bin;
     size_t face_rec, shade, total;
@@ -150,6 +151,14 @@ struct TetParams {
     long long* det_fopa;          // [F]
 };
 
+// Outputs of the vertex-position backward (dmr_tet_backward_vertex), a kernel argument of its own so that TetParams, and
+// with it the parameter layout of every other kernel, stays as it is.
+struct TetVertGrad {
+    float* dL_dverts;             // [P,3], added to
+    float4* grad_pacc;            // default mode: [P] zeroed scratch, per-vertex position gradient (xyz) summed over views
+    long long* det_pos;           // deterministic mode: [P,4] zeroed fixed-point dL_dverts xyz, - (TetDetLayout::pos)
+};
+
 // Camera gradients of the backward march: one record of DMR_TET_CAM_REC floats per (view, march CTA of 8 x 8 pixels),
 // written by every CTA (layout: tet_march_bwd_cam, tet_kernels.cu).
 #define DMR_TET_CAM_REC 32
@@ -157,6 +166,9 @@ __host__ __device__ inline size_t tet_cam_records(size_t B, int W, int H) { retu
 
 struct TetDetLayout {             // workspace of the deterministic backward pass
     size_t gmax, vert, fopa, hi, total;   // low words vert..fopa, their high words mirrored at hi
+    // vertex-position gradients: a [P,4] block appended behind `total`, its high words at the same element offset
+    // (hi_offset) as every other accumulator's; total_pos is the workspace of that mode
+    size_t pos, total_pos;
     __host__ __device__ static TetDetLayout make(size_t P, size_t F)
     {
         TetDetLayout L;
@@ -166,6 +178,8 @@ struct TetDetLayout {             // workspace of the deterministic backward pas
         L.fopa = o; o = align_up(o + 8 * F, 256);
         L.hi = o;   o += o - L.vert;
         L.total = o;
+        L.pos = o;
+        L.total_pos = align_up(o + (L.hi - L.vert) + 8 * 4 * P, 256);
         return L;
     }
     // element offset of an accumulator's high word from its low word (det.cuh)
@@ -197,8 +211,10 @@ int tet_first_intersect(const TetParams& p, cudaStream_t stream);
 int tet_march_forward(const TetParams& p, cudaStream_t stream);
 // cam_rec != nullptr: the camera-gradient kernels, which also store one DMR_TET_CAM_REC-float record per (view, march
 // CTA) there
-int tet_march_backward(const TetParams& p, cudaStream_t stream, float* cam_rec = nullptr);
-int tet_march_backward_deterministic(const TetParams& p, cudaStream_t stream, float* cam_rec = nullptr);
+// vert != nullptr: the vertex-position kernels, which also add dL/dverts to vert->dL_dverts
+int tet_march_backward(const TetParams& p, cudaStream_t stream, float* cam_rec = nullptr, const TetVertGrad* vert = nullptr);
+int tet_march_backward_deterministic(const TetParams& p, cudaStream_t stream, float* cam_rec = nullptr,
+                                     const TetVertGrad* vert = nullptr);
 // records of a view -> += dL_dmv[B,16], dL_dproj[B,16]
 int tet_camera_finish(const TetParams& p, const float* cam_rec, float* dL_dmv, float* dL_dproj, cudaStream_t stream);
 

@@ -9,6 +9,7 @@
 //   tet_march_bwd_kernel        replaces TET_BACKWARD::renderCUDA (backward.cu:86-487)
 //   tet_march_bwd_cam_kernel,   the same plus gradients with respect to the camera matrices (no reference counterpart)
 //   tet_camera_finish_kernel
+//   tet_march_bwd_*vert*_kernel the same plus gradients with respect to the vertex positions (no reference counterpart)
 //
 // Forward images must match the reference to 1e-5, which requires IDENTICAL
 // branch decisions along every ray (hit tests, normal signs); all such
@@ -869,6 +870,91 @@ __device__ __forceinline__ void tet_cam_step(TetCamAcc& a, const TetBwdState& st
     a.g_rd = a.g_rd + cross3(M, Tv) - kn * N;
 }
 
+// The sensitivities of a step as tet_cam_step forms them -- k_u = dL/du / D, k_v, k_t likewise, k_n = k_u u + k_v v + k_t t
+// -- and the step's triangle, for the vertex-position instantiations (CAM: also the depth-coefficient terms into `a`).
+// tet_cam_step keeps its own copy of these lines: routed through this function, the camera kernels compile to
+// differently scheduled code.
+struct TetStepGrad {
+    float3 E1, E2, Tv, N;
+    float ku, kv, kt, kn;
+};
+
+template <bool CAM>
+__device__ __forceinline__ TetStepGrad tet_step_grad(TetCamAcc& a, const TetBwdState& st, const TetDepth& dep, float3 ro,
+                                                     float3 rd, float rt, float iu, float iv, const float4 s0,
+                                                     const float4 s1, const float4 s2, float intense, const float dLc[3],
+                                                     float gd, const float4 v0, const float4 v1, float v2z)
+{
+    const float3 c0 = f3(s0.x, s0.y, s0.z), c1 = f3(s0.w, s1.x, s1.y), c2 = f3(s1.z, s1.w, s2.x);
+    const float w = s2.y * expf(st.prev_log_T);      // T_k alpha_k of the step (does not depend on the camera)
+    const float3 dc1 = c1 - c0, dc2 = c2 - c0;
+    const float wi = w * intense;
+    const float dL_du = wi * (dLc[0] * dc1.x + dLc[1] * dc1.y + dLc[2] * dc1.z);
+    const float dL_dv = wi * (dLc[0] * dc2.x + dLc[1] * dc2.y + dLc[2] * dc2.z);
+    // depth: no derivative through a clamped w
+    const float Z = dep.az + rt * dep.bz, Wr = dep.aw + rt * dep.bw, Wc = clamp_w(Wr);
+    const float gZ = w * gd / Wc;
+    const float gW = Wc == Wr ? -gZ * (Z / Wc) : 0.0f;
+    if constexpr (CAM) { a.g_az += gZ; a.g_bz += gZ * rt; a.g_aw += gW; a.g_bw += gW * rt; }
+    const float dL_dt = gZ * dep.bz + gW * dep.bw;
+    const float3 p0 = f3(v0.x, v0.y, v0.z), p1 = f3(v0.w, v1.x, v1.y), p2 = f3(v1.z, v1.w, v2z);
+    TetStepGrad k;
+    k.E1 = p1 - p0; k.E2 = p2 - p0; k.Tv = ro - p0;
+    k.N = cross3(k.E2, k.E1);
+    const float iD = 1.0f / dot3(rd, k.N);
+    k.ku = dL_du * iD; k.kv = dL_dv * iD; k.kt = dL_dt * iD;
+    k.kn = k.kt * rt + k.ku * iu + k.kv * iv;
+    return k;
+}
+
+// Vertex-position gradients (VERT instantiations; DESIGN.md 3.4).  A vertex enters a step only through (t, u, v) of
+// the Moeller-Trumbore test against the face's triangle p0 p1 p2 (TetFaceRec, faces[] order); colours, opacities and the
+// depth coefficients do not depend on it.  With the sensitivities of tet_step_grad:
+//     g_T  = k_u (rd x E2) + k_v (E1 x rd) - k_t N           (= the camera path's dL/dro of the step)
+//     g_E1 = k_v (rd x T)  + k_t (E2 x T)  - k_n (rd x E2)
+//     g_E2 = k_u (T x rd)  + k_t (T x E1)  - k_n (E1 x rd)
+//     dL/dp0 = -g_T - g_E1 - g_E2,   dL/dp1 = g_E1,   dL/dp2 = g_E2
+// scattered to the vertex ids TetShade.i0..i2 (the same vertices in the same order): three vector reductions into
+// a.vg.grad_pacc, or nine fixed-point additions with the geometry scale a.det_sg into a.vg.det_pos.  CAM: the camera
+// terms of tet_cam_step from the same sensitivities, into the TetCamAcc part of `a`.
+struct TetVertAcc : TetCamAcc {
+    TetVertGrad vg;
+    float det_sg;   // deterministic mode: the fixed-point scale of positions (det.cuh)
+};
+
+template <bool DET, bool CAM>
+__device__ __forceinline__ void tet_vert_step(const TetParams& p, TetVertAcc& a, const TetBwdState& st, const TetDepth& dep, float3 ro, float3 rd, float rt, float iu, float iv,
+                                              const float4 s0, const float4 s1, const float4 s2, const float4 s3,
+                                              float intense, const float dLc[3], float gd, const float4 v0, const float4 v1,
+                                              float v2z)
+{
+    const TetStepGrad k = tet_step_grad<CAM>(a, st, dep, ro, rd, rt, iu, iv, s0, s1, s2, intense, dLc, gd, v0, v1, v2z);
+    const float3 M = k.ku * k.E2 - k.kv * k.E1;
+    if constexpr (CAM) {
+        a.g_ro = a.g_ro + cross3(rd, M) - k.kt * k.N;
+        a.g_rd = a.g_rd + cross3(M, k.Tv) - k.kn * k.N;
+    }
+    const float3 gT = cross3(rd, M) - k.kt * k.N;
+    const float3 gE1 = cross3(k.kv * rd + k.kt * k.E2, k.Tv) - k.kn * cross3(rd, k.E2);
+    const float3 gE2 = cross3(k.Tv, k.ku * rd + k.kt * k.E1) - k.kn * cross3(k.E1, rd);
+    const float3 g0 = -(gT + gE1 + gE2);
+    const int vi0 = __float_as_int(s2.w), vi1 = __float_as_int(s3.x), vi2 = __float_as_int(s3.y);
+    const TetVertGrad& vg = a.vg;
+    if constexpr (DET) {
+        const float sg = a.det_sg;
+        const ptrdiff_t hi = st.det_hi;
+        const uint32_t* gm = p.det_gmax;
+        long long* a0 = vg.det_pos + 4 * (size_t)vi0; long long* a1 = vg.det_pos + 4 * (size_t)vi1; long long* a2 = vg.det_pos + 4 * (size_t)vi2;
+        det_add(a0 + 0, g0.x, sg, hi, gm); det_add(a0 + 1, g0.y, sg, hi, gm); det_add(a0 + 2, g0.z, sg, hi, gm);
+        det_add(a1 + 0, gE1.x, sg, hi, gm); det_add(a1 + 1, gE1.y, sg, hi, gm); det_add(a1 + 2, gE1.z, sg, hi, gm);
+        det_add(a2 + 0, gE2.x, sg, hi, gm); det_add(a2 + 1, gE2.y, sg, hi, gm); det_add(a2 + 2, gE2.z, sg, hi, gm);
+    } else {
+        red_add_v4(reinterpret_cast<float*>(vg.grad_pacc + vi0), g0.x, g0.y, g0.z, 0.0f);
+        red_add_v4(reinterpret_cast<float*>(vg.grad_pacc + vi1), gE1.x, gE1.y, gE1.z, 0.0f);
+        red_add_v4(reinterpret_cast<float*>(vg.grad_pacc + vi2), gE2.x, gE2.y, gE2.z, 0.0f);
+    }
+}
+
 // Backward march.  Steps recorded in the face trail (all of them unless a ray composited more than
 // trail_cap faces) are replayed in reverse: face id and the forward pass's own (t,u,v) from the trail
 // (one coalesced 16-byte load), all loads independent of the previous step and issued one step ahead.  Steps beyond the cap are re-marched through the adjacency records exactly like
@@ -879,8 +965,10 @@ __device__ __forceinline__ void tet_cam_step(TetCamAcc& a, const TetBwdState& st
 // through the L1 data pipe, not by the latency of a single chain.)
 // CAM: also accumulate the camera terms of every walked step into `cam` (tet_cam_step); the face's vertices are loaded
 // with its shading record.  The early returns end the walk only: tet_march_bwd_cam reduces after it on every lane.
-template <bool DET, bool CAM>
-__device__ __forceinline__ void tet_march_bwd_body(const TetParams& p, TetCamAcc& cam)
+// VERT: also scatter the vertex-position terms of every walked step (tet_vert_step, sharing the triangle and the
+// sensitivities with CAM); `cam` is then a TetVertAcc.
+template <bool DET, bool CAM, bool VERT = false, class Acc = TetCamAcc>
+__device__ __forceinline__ void tet_march_bwd_body(const TetParams& p, Acc& cam)
 {
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int b = blockIdx.z;
@@ -921,7 +1009,12 @@ __device__ __forceinline__ void tet_march_bwd_body(const TetParams& p, TetCamAcc
     TetBwdState st;
     st.det_sv = 0.0f;
     st.det_hi = 0;
-    if (DET) { float sg; det_scales(*p.det_gmax, st.det_sv, sg); st.det_hi = TetDetLayout::hi_offset(p.P, p.F); }
+    if (DET) {
+        float sg;
+        det_scales(*p.det_gmax, st.det_sv, sg);
+        if constexpr (VERT) cam.det_sg = sg;
+        st.det_hi = TetDetLayout::hi_offset(p.P, p.F);
+    }
     st.prev_log_T = fin_prev_log_T;
     st.last_alpha = 0.0f; st.last_depth = 0.0f; st.accum_recd = 0.0f;
 #pragma unroll
@@ -954,14 +1047,17 @@ __device__ __forceinline__ void tet_march_bwd_body(const TetParams& p, TetCamAcc
             const float intense = p.faces_intense[(size_t)b * p.F + curr_face];
             float4 v0, v1;
             float v2z;
-            if constexpr (CAM) {
+            if constexpr (CAM || VERT) {
                 const float4* fr = reinterpret_cast<const float4*>(p.face_rec + (size_t)b * p.F + curr_face);
                 v0 = fr[0]; v1 = fr[1]; v2z = reinterpret_cast<const float*>(fr)[8];
             }
             tet_bwd_face<DET>(p, st, curr_face, rt, iu, iv, s0, s1, s2, s3, intense, dep, dLc, gd, bg_dot, bd_dot,
                          final_T, final_prev_T);
             // (t, u, v) of the re-march: recomputed, the same bits as the forward march's
-            if constexpr (CAM) tet_cam_step(cam, st, dep, ro, rd, rt, iu, iv, s0, s1, s2, intense, dLc, gd, v0, v1, v2z);
+            if constexpr (VERT)
+                tet_vert_step<DET, CAM>(p, cam, st, dep, ro, rd, rt, iu, iv, s0, s1, s2, s3, intense, dLc, gd, v0, v1, v2z);
+            else if constexpr (CAM)
+                tet_cam_step(cam, st, dep, ro, rd, rt, iu, iv, s0, s1, s2, intense, dLc, gd, v0, v1, v2z);
             k--;
             if (curr_face == first_face) return;         // backward.cu:363-366
             if (curr_tet == -1) return;                  // backward.cu:373-376
@@ -986,11 +1082,11 @@ __device__ __forceinline__ void tet_march_bwd_body(const TetParams& p, TetCamAcc
         s0 = sh4[0]; s1 = sh4[1]; s2 = sh4[2]; s3 = sh4[3];
         intense = fint[face];
     }
-    // CAM: the face's triangle (TetFaceRec p0 p1 p2), loaded together with the shading record
+    // CAM, VERT: the face's triangle (TetFaceRec p0 p1 p2), loaded together with the shading record
     const float4* frec = reinterpret_cast<const float4*>(p.face_rec + (size_t)b * p.F);
     float4 v0, v1;
     float v2z;
-    if constexpr (CAM) { v0 = frec[4 * face]; v1 = frec[4 * face + 1]; v2z = reinterpret_cast<const float*>(frec + 4 * face)[8]; }
+    if constexpr (CAM || VERT) { v0 = frec[4 * face]; v1 = frec[4 * face + 1]; v2z = reinterpret_cast<const float*>(frec + 4 * face)[8]; }
     for (; k >= 0; k--) {
         // issue the loads of step k-1 (face id known since the previous iteration), then work on step k
         const int nf = e_next.x & 0x7fffffff;
@@ -1000,7 +1096,7 @@ __device__ __forceinline__ void tet_march_bwd_body(const TetParams& p, TetCamAcc
         const float nint = fint[nf];
         float4 nv0, nv1;
         float nv2z;
-        if constexpr (CAM) { nv0 = frec[4 * nf]; nv1 = frec[4 * nf + 1]; nv2z = reinterpret_cast<const float*>(frec + 4 * nf)[8]; }
+        if constexpr (CAM || VERT) { nv0 = frec[4 * nf]; nv1 = frec[4 * nf + 1]; nv2z = reinterpret_cast<const float*>(frec + 4 * nf)[8]; }
         const int4 e_cur = e;
         e = e_next;
         e_next = k > 1 ? __ldcs(trail + (size_t)(k - 2) * BI) : make_int4(0, 0, 0, 0);
@@ -1008,7 +1104,10 @@ __device__ __forceinline__ void tet_march_bwd_body(const TetParams& p, TetCamAcc
         // (t, u, v) of the step: the forward march's own values
         tet_bwd_face<DET>(p, st, face, __int_as_float(e_cur.y), __int_as_float(e_cur.z), __int_as_float(e_cur.w), s0, s1, s2, s3,
                           intense, dep, dLc, gd, bg_dot, bd_dot, final_T, final_prev_T);
-        if constexpr (CAM)
+        if constexpr (VERT)
+            tet_vert_step<DET, CAM>(p, cam, st, dep, ro, rd, __int_as_float(e_cur.y), __int_as_float(e_cur.z),
+                                    __int_as_float(e_cur.w), s0, s1, s2, s3, intense, dLc, gd, v0, v1, v2z);
+        else if constexpr (CAM)
             tet_cam_step(cam, st, dep, ro, rd, __int_as_float(e_cur.y), __int_as_float(e_cur.z), __int_as_float(e_cur.w), s0, s1,
                          s2, intense, dLc, gd, v0, v1, v2z);
 
@@ -1016,7 +1115,7 @@ __device__ __forceinline__ void tet_march_bwd_body(const TetParams& p, TetCamAcc
         face = nf;
         s0 = ns0; s1 = ns1; s2 = ns2; s3 = ns3;
         intense = nint;
-        if constexpr (CAM) { v0 = nv0; v1 = nv1; v2z = nv2z; }
+        if constexpr (CAM || VERT) { v0 = nv0; v1 = nv1; v2z = nv2z; }
     }
 }
 
@@ -1033,6 +1132,22 @@ __global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_det_kernel(TetPar
     TetCamAcc unused;
     tet_march_bwd_body<true, false>(p, unused);
 }
+// Vertex-position instantiations: position gradients into vg.grad_pacc (tet_grad_position_kernel folds them into
+// vg.dL_dverts) or vg.det_pos (tet_det_convert_position_kernel).
+__global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_vert_kernel(TetParams p, TetVertGrad vg)
+{
+    griddep_wait();
+    TetVertAcc a;
+    a.vg = vg;
+    tet_march_bwd_body<false, false, true>(p, a);
+}
+__global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_vert_det_kernel(TetParams p, TetVertGrad vg)
+{
+    griddep_wait();
+    TetVertAcc a;
+    a.vg = vg;
+    tet_march_bwd_body<true, false, true>(p, a);
+}
 
 // Camera-gradient instantiations: the walk of tet_march_bwd_body<DET, true>, then per lane the chain of its pixel into
 // the matrices, and one record of DMR_TET_CAM_REC floats per (view, CTA), summed in a fixed order (no float atomics:
@@ -1044,13 +1159,13 @@ __global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_det_kernel(TetPar
 // tet_camera_finish_kernel applies the inverses and the direct depth-row terms.
 static_assert(MARCH_THREADS == 64 && MARCH_ROWS == 8, "tet_cam_records (tet.cuh) counts 8 x 8-pixel march CTAs");
 static_assert(DMR_TET_CAM_REC == 32, "one record slot per lane");
-template <bool DET>
-__device__ __forceinline__ void tet_march_bwd_cam(const TetParams& p, float* __restrict__ cam_rec)
+// VERT: Acc = TetVertAcc with its vg set by the caller.
+template <bool DET, bool VERT = false, class Acc = TetCamAcc>
+__device__ __forceinline__ void tet_march_bwd_cam(const TetParams& p, float* __restrict__ cam_rec, Acc& a)
 {
-    TetCamAcc a;
     a.g_ro = f3(0, 0, 0); a.g_rd = f3(0, 0, 0);
     a.g_az = 0.0f; a.g_bz = 0.0f; a.g_aw = 0.0f; a.g_bw = 0.0f;
-    tet_march_bwd_body<DET, true>(p, a);
+    tet_march_bwd_body<DET, true, VERT>(p, a);
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int b = blockIdx.z;
@@ -1118,12 +1233,28 @@ __device__ __forceinline__ void tet_march_bwd_cam(const TetParams& p, float* __r
 __global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_cam_kernel(TetParams p, float* cam_rec)
 {
     griddep_wait();
-    tet_march_bwd_cam<false>(p, cam_rec);
+    TetCamAcc a;
+    tet_march_bwd_cam<false>(p, cam_rec, a);
 }
 __global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_cam_det_kernel(TetParams p, float* cam_rec)
 {
     griddep_wait();
-    tet_march_bwd_cam<true>(p, cam_rec);
+    TetCamAcc a;
+    tet_march_bwd_cam<true>(p, cam_rec, a);
+}
+__global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_cam_vert_kernel(TetParams p, float* cam_rec, TetVertGrad vg)
+{
+    griddep_wait();
+    TetVertAcc a;
+    a.vg = vg;
+    tet_march_bwd_cam<false, true>(p, cam_rec, a);
+}
+__global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_cam_vert_det_kernel(TetParams p, float* cam_rec, TetVertGrad vg)
+{
+    griddep_wait();
+    TetVertAcc a;
+    a.vg = vg;
+    tet_march_bwd_cam<true, true>(p, cam_rec, a);
 }
 
 // One CTA per view: the view's records (tet_march_bwd_cam) are summed in a fixed order -- thread t owns component
@@ -1216,16 +1347,57 @@ __global__ void __launch_bounds__(256) tet_grad_vertex_kernel(TetParams p)
     o[0] += a.x; o[1] += a.y; o[2] += a.z;
 }
 
-int tet_march_backward_deterministic(const TetParams& p, cudaStream_t stream, float* cam_rec)
+// Vertex-position gradients, last step of either mode: += into dL_dverts[P,3].  The deterministic one follows the
+// poisoning rule of det.cuh, as tet_det_convert_kernel does for the other gradients of the call.
+__global__ void __launch_bounds__(256) tet_grad_position_kernel(int P, TetVertGrad vg)
+{
+    griddep_wait();   // programmatic dependent launch: see dmr_launch (common.cuh)
+    const int v = blockIdx.x * blockDim.x + threadIdx.x;
+    if (v >= P) return;
+    const float4 a = vg.grad_pacc[v];
+    float* o = vg.dL_dverts + 3 * (size_t)v;
+    o[0] += a.x; o[1] += a.y; o[2] += a.z;
+}
+
+__global__ void __launch_bounds__(256) tet_det_convert_position_kernel(int P, int F, const uint32_t* __restrict__ gmax,
+                                                                       TetVertGrad vg)
+{
+    griddep_wait();   // programmatic dependent launch: see dmr_launch (common.cuh)
+    const size_t i = (size_t)blockIdx.x * 256 + threadIdx.x;
+    if (i >= (size_t)P) return;
+    if (det_poisoned(gmax)) {
+        const float nan = __int_as_float(0x7fc00000);
+        for (int c = 0; c < 3; c++) vg.dL_dverts[3 * i + c] = nan;
+        return;
+    }
+    float sv, sg;
+    det_scales(*gmax, sv, sg);
+    if (sg == 0.0f) return;
+    const double ig = 1.0 / (double)sg;
+    const ptrdiff_t hi = TetDetLayout::hi_offset(P, F);
+    const long long* a = vg.det_pos + 4 * i;
+#pragma unroll
+    for (int c = 0; c < 3; c++) {
+        if (det_nonzero(a + c, hi)) vg.dL_dverts[3 * i + c] += (float)det_value(a + c, hi, ig);
+    }
+}
+
+int tet_march_backward_deterministic(const TetParams& p, cudaStream_t stream, float* cam_rec, const TetVertGrad* vert)
 {
     dim3 grid((p.W + 7) / 8, (p.H + MARCH_ROWS - 1) / MARCH_ROWS, p.B);
     const size_t HW = (size_t)p.W * p.H;
     {
-        ProfScope prof(cam_rec ? ST_TET_BWD_CAM : ST_TET_BWD, stream);
+        ProfScope prof(vert ? (cam_rec ? ST_TET_BWD_CAM_VERT : ST_TET_BWD_VERT) : (cam_rec ? ST_TET_BWD_CAM : ST_TET_BWD), stream);
         count_launch(1);   // two kernels under one scope
         int rc = det_gmax(p.dL_dcolor, 3 * p.B * HW, p.dL_ddepth, p.B * HW, const_cast<uint32_t*>(p.det_gmax), stream);
         if (rc) return rc;
-        if (cam_rec) {
+        if (vert && cam_rec) {
+            DMR_CUDA(dmr_launch(tet_march_bwd_cam_vert_det_kernel, dim3(grid), dim3(MARCH_THREADS), 0, stream, p, cam_rec, *vert));
+            DMR_LAUNCH_CHECK("tet_march_bwd_cam_vert_det_kernel");
+        } else if (vert) {
+            DMR_CUDA(dmr_launch(tet_march_bwd_vert_det_kernel, dim3(grid), dim3(MARCH_THREADS), 0, stream, p, *vert));
+            DMR_LAUNCH_CHECK("tet_march_bwd_vert_det_kernel");
+        } else if (cam_rec) {
             DMR_CUDA(dmr_launch(tet_march_bwd_cam_det_kernel, dim3(grid), dim3(MARCH_THREADS), 0, stream, p, cam_rec));
             DMR_LAUNCH_CHECK("tet_march_bwd_cam_det_kernel");
         } else {
@@ -1238,13 +1410,27 @@ int tet_march_backward_deterministic(const TetParams& p, cudaStream_t stream, fl
         DMR_CUDA(dmr_launch(tet_det_convert_kernel, dim3((unsigned)(((size_t)p.P + p.F + 255) / 256)), dim3(256), 0, stream, p));
         DMR_LAUNCH_CHECK("tet_det_convert_kernel");
     }
+    if (vert) {
+        ProfScope prof(ST_TET_VERT_FINISH, stream);
+        DMR_CUDA(dmr_launch(tet_det_convert_position_kernel, dim3((p.P + 255) / 256), dim3(256), 0, stream, p.P, p.F,
+                            p.det_gmax, *vert));
+        DMR_LAUNCH_CHECK("tet_det_convert_position_kernel");
+    }
     return 0;
 }
 
-int tet_march_backward(const TetParams& p, cudaStream_t stream, float* cam_rec)
+int tet_march_backward(const TetParams& p, cudaStream_t stream, float* cam_rec, const TetVertGrad* vert)
 {
     dim3 grid((p.W + 7) / 8, (p.H + MARCH_ROWS - 1) / MARCH_ROWS, p.B);
-    if (cam_rec) {
+    if (vert && cam_rec) {
+        ProfScope prof(ST_TET_BWD_CAM_VERT, stream);
+        DMR_CUDA(dmr_launch(tet_march_bwd_cam_vert_kernel, dim3(grid), dim3(MARCH_THREADS), 0, stream, p, cam_rec, *vert));
+        DMR_LAUNCH_CHECK("tet_march_bwd_cam_vert_kernel");
+    } else if (vert) {
+        ProfScope prof(ST_TET_BWD_VERT, stream);
+        DMR_CUDA(dmr_launch(tet_march_bwd_vert_kernel, dim3(grid), dim3(MARCH_THREADS), 0, stream, p, *vert));
+        DMR_LAUNCH_CHECK("tet_march_bwd_vert_kernel");
+    } else if (cam_rec) {
         ProfScope prof(ST_TET_BWD_CAM, stream);
         DMR_CUDA(dmr_launch(tet_march_bwd_cam_kernel, dim3(grid), dim3(MARCH_THREADS), 0, stream, p, cam_rec));
         DMR_LAUNCH_CHECK("tet_march_bwd_cam_kernel");
@@ -1257,6 +1443,11 @@ int tet_march_backward(const TetParams& p, cudaStream_t stream, float* cam_rec)
         ProfScope prof(ST_TET_BWD_FINISH, stream);
         DMR_CUDA(dmr_launch(tet_grad_vertex_kernel, dim3((p.P + 255) / 256), dim3(256), 0, stream, p));
         DMR_LAUNCH_CHECK("tet_grad_vertex_kernel");
+    }
+    if (vert) {
+        ProfScope prof(ST_TET_VERT_FINISH, stream);
+        DMR_CUDA(dmr_launch(tet_grad_position_kernel, dim3((p.P + 255) / 256), dim3(256), 0, stream, p.P, *vert));
+        DMR_LAUNCH_CHECK("tet_grad_position_kernel");
     }
     return 0;
 }

@@ -56,8 +56,9 @@ int    dmr_tri_state_bytes(int B, int P, int F, int W, int H, size_t out[3]);
 int    dmr_tet_state_bytes(int B, int P, int F, int T, int W, int H, size_t out[3]);
 /* The tet renderer's view-independent adjacency records (one 128-byte record per tet, replacing the per-step   */
 /* gathers of cuda_renderer/forward.cu:672-768).  They depend only on verts / faces / tets / face_tets /         */
-/* tet_faces -- none of which carries a gradient -- so a caller may build them once and reuse the buffer for      */
-/* every later call on the same geometry (dmr_tet_forward_bin: tet_records_valid).                                */
+/* tet_faces, so a caller may build them once and reuse the buffer for every later call on the same geometry     */
+/* (dmr_tet_forward_bin: tet_records_valid).  A caller that optimises verts (dmr_tet_backward_vertex) changes     */
+/* that geometry in every step and has to rebuild them after each change.                                         */
 size_t dmr_tet_records_bytes(int T);
 /* Builds them stand-alone (dmr_tet_forward_bin does the same when tet_records_valid == 0). */
 int    dmr_tet_build_records(int P, int F, int T, const float* verts, const int* faces, const int* tets,
@@ -320,9 +321,9 @@ int dmr_tet_backward(
     void* workspace, size_t workspace_bytes,
     dmr_stream_t stream);
 /* The same with run-to-run reproducible gradients (see dmr_tri_backward_deterministic: the reference's 10 scalar */
-/* atomics per crossed face, cuda_renderer/backward.cu:341-360, become 64-bit fixed-point additions with 38       */
-/* fractional bits below max |dL_dout|).  `workspace`: dmr_tet_backward_deterministic_bytes(P, F) bytes of device  */
-/* scratch (zeroed by the call).                                                                                   */
+/* atomics per crossed face, cuda_renderer/backward.cu:341-360, become two-word fixed-point additions with 48     */
+/* fractional bits below max |dL_dout|, 40 for positions).  `workspace`: dmr_tet_backward_deterministic_bytes(P,  */
+/* F) bytes of device scratch (zeroed by the call).                                                                */
 size_t dmr_tet_backward_deterministic_bytes(int P, int F);
 int dmr_tet_backward_deterministic(
     int B, int P, int F, int T, int W, int H,
@@ -367,6 +368,36 @@ int dmr_tet_backward_camera(
     int deterministic,
     float* dL_dmv,               /* [B,16] */
     float* dL_dproj,             /* [B,16] */
+    void* workspace, size_t workspace_bytes,
+    dmr_stream_t stream);
+
+/* Vertex-position gradients of the tet renderer (no reference counterpart: the reference returns no gradient for */
+/* verts).  The backward pass of dmr_tet_backward_camera, with the same arguments, except that dL_dmv and          */
+/* dL_dproj may both be NULL (no camera gradients; passing only one of them is an error), plus dL/dverts [P,3]     */
+/* ADDED to dL_dverts.  The derivative is that of the rendered colour and depth images as implemented, with the    */
+/* same things held fixed as for the camera gradients; a vertex enters through the (t, u, v) of every walked step  */
+/* whose face's triangle (faces[] order) it belongs to.  Only the steps the backward pass walks contribute.  Summed */
+/* with float atomics (deterministic == 0) or in fixed point (deterministic != 0; reproducible, NaN for non-finite */
+/* cotangents).  The other gradients are those of the mode it extends.  `workspace`:                              */
+/* dmr_tet_backward_vertex_bytes(B, P, F, W, H, deterministic, camera) bytes of device scratch, camera = whether  */
+/* dL_dmv / dL_dproj are passed: the mode's own scratch plus one per-vertex accumulator.                          */
+size_t dmr_tet_backward_vertex_bytes(int B, int P, int F, int W, int H, int deterministic, int camera);
+int dmr_tet_backward_vertex(
+    int B, int P, int F, int T, int W, int H,
+    int ray_random_seed,
+    const float* background,
+    const float* mv_mats, const float* proj_mats,
+    const float* inv_mv_mats, const float* inv_proj_mats,
+    const float* faces_intense,
+    const void* point_buffer, const void* face_buffer,
+    const void* tet_records,
+    const void* image_buffer,
+    const float* dL_dcolor, const float* dL_ddepth,
+    float* dL_dverts_color, float* dL_dfaces_opacity,
+    int deterministic,
+    float* dL_dmv,               /* [B,16] or NULL */
+    float* dL_dproj,             /* [B,16] or NULL */
+    float* dL_dverts,            /* [P,3] */
     void* workspace, size_t workspace_bytes,
     dmr_stream_t stream);
 
