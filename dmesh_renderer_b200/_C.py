@@ -592,7 +592,7 @@ def render_tets(background, verts, faces, verts_color, faces_opacity, mv_mats, p
 def render_tets_backward(background, verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, inv_mv_mats,
                          inv_proj_mats, verts_depth, faces_intense, tets, face_tets, tet_faces, grad_color, grad_depth,
                          pointBuffer, faceBuffer, binningBuffer, imageBuffer, ray_random_seed=None, deterministic=False,
-                         tet_records=None, camera_grads=False, vertex_grads=False):
+                         tet_records=None, camera_grads=False, vertex_grads=False, intensity_grads=False):
     """RenderFTetsBackwardCUDA (render.cu:338-412).
     Returns (dL_dverts_color[P,3], dL_dfaces_opacity[F]).  `ray_random_seed` is an
     optional trailing argument beyond the reference's 20: the autograd wrapper passes
@@ -603,7 +603,10 @@ def render_tets_backward(background, verts, faces, verts_color, faces_opacity, m
     `camera_grads`: also return dL_dmv_mats, dL_dproj_mats [B,4,4] (gradients with respect to the mv_mats / proj_mats
     tensors passed here, through the rays and the hit-point depth; dmr_tet_backward_camera) as two more elements.
     `vertex_grads`: also return dL_dverts [P,3] (gradient with respect to the vertex positions, through the (t, u, v)
-    of every walked step; dmr_tet_backward_vertex) as the last element."""
+    of every walked step; dmr_tet_backward_vertex) as the last element.
+    `intensity_grads`: also return dL_dfaces_intense [B,F] (gradient with respect to the face intensities, through the
+    colour of every walked step; dmr_tet_backward_intensity) as the last element, after dL_dverts when both are
+    requested."""
     lib = _lib.load()
     B, P, F, T = mv_mats.size(0), verts.size(0), faces.size(0), tets.size(0)
     H, W = grad_color.size(2), grad_color.size(3)
@@ -617,6 +620,7 @@ def render_tets_backward(background, verts, faces, verts_color, faces_opacity, m
         # [B,16] column-major = [B,4,4] gradients of the (column-major, i.e. transposed) matrix tensors given here
         cam = torch.zeros((2, B, 4, 4), **z) if camera_grads else None
         dL_dverts = torch.zeros((P, 3), **z) if vertex_grads else None
+        dL_dfint = torch.zeros((B, F), **z) if intensity_grads else None
         if B * H * W > 0 and F > 0 and T > 0:
             bg = _f32(background, "background")
             mv, pj = _f32(mv_mats, "mv_mats"), _f32(proj_mats, "proj_mats")
@@ -634,7 +638,17 @@ def render_tets_backward(background, verts, faces, verts_color, faces_opacity, m
             a = (B, P, F, T, W, H, int(ray_random_seed), _ptr(bg), _ptr(mv), _ptr(pj), _ptr(imv), _ptr(ipj), _ptr(fint),
                  _ptr(pointBuffer), _ptr(faceBuffer), _ptr(tet_rec), _ptr(imageBuffer), _ptr(gc), _ptr(gd),
                  _ptr(dL_dverts_color), _ptr(dL_dfaces_opacity))
-            if vertex_grads:
+            if intensity_grads:
+                det = int(bool(deterministic))
+                ws = torch.empty(lib.dmr_tet_backward_intensity_bytes(B, P, F, W, H, det, int(bool(camera_grads)),
+                                                                      int(bool(vertex_grads))),
+                                 dtype=torch.uint8, device=dev)
+                null = ctypes.c_void_p(0)
+                c = (_ptr(cam[0]), _ptr(cam[1])) if camera_grads else (null, null)
+                dv = _ptr(dL_dverts) if vertex_grads else null
+                _lib.check(lib.dmr_tet_backward_intensity(*a, det, *c, dv, _ptr(dL_dfint), _ptr(ws), ws.numel(),
+                                                          _stream()))
+            elif vertex_grads:
                 det = int(bool(deterministic))
                 ws = torch.empty(lib.dmr_tet_backward_vertex_bytes(B, P, F, W, H, det, int(bool(camera_grads))),
                                  dtype=torch.uint8, device=dev)
@@ -656,4 +670,6 @@ def render_tets_backward(background, verts, faces, verts_color, faces_opacity, m
         out += (cam[0], cam[1])
     if vertex_grads:
         out += (dL_dverts,)
+    if intensity_grads:
+        out += (dL_dfint,)
     return out

@@ -167,8 +167,8 @@ class TriRenderer(th.nn.Module):
 
 # =============================================================================
 # TetRenderer: faces of a tetrahedral complex, exact depth order by ray marching
-# through tet adjacency; gradients to vertex colours, face opacities and (opt-in) the camera matrices and the
-# vertex positions.
+# through tet adjacency; gradients to vertex colours, face opacities and (opt-in) the camera matrices, the
+# vertex positions and the face intensities.
 # =============================================================================
 class TetRenderSettings(NamedTuple):      # reference __init__.py:237-241
     image_height: int
@@ -191,14 +191,30 @@ def set_tet_vertex_grads(flag: bool) -> bool:
     return old
 
 
+_tet_intensity_grads_default = False
+
+
+def set_tet_intensity_grads(flag: bool) -> bool:
+    """Process-wide default for the tet renderer's face-intensity gradient (extension).  False (the default): like the
+    reference, the tet renderer returns no gradient for faces_intense.  True: when faces_intense requires grad, its
+    gradient is the exact derivative of the rendered colour image (depth does not depend on it).  The other gradients
+    are the same either way.  `TetRenderer(settings, intensity_grads=...)` / `render_tet(..., intensity_grads=...)`
+    override it per renderer / call.  Returns the previous value."""
+    global _tet_intensity_grads_default
+    old, _tet_intensity_grads_default = _tet_intensity_grads_default, bool(flag)
+    return old
+
+
 def render_tet(verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, verts_depth, faces_intense, tets,
-               face_tets, tet_faces, render_settings: TetRenderSettings, deterministic=None, vertex_grads=None):
+               face_tets, tet_faces, render_settings: TetRenderSettings, deterministic=None, vertex_grads=None,
+               intensity_grads=None):
     """reference __init__.py:243-275 (`deterministic`: see set_deterministic; `vertex_grads`: see
-    set_tet_vertex_grads)"""
+    set_tet_vertex_grads; `intensity_grads`: see set_tet_intensity_grads)"""
     det = _deterministic_default if deterministic is None else bool(deterministic)
     vert = _tet_vertex_grads_default if vertex_grads is None else bool(vertex_grads)
+    fint = _tet_intensity_grads_default if intensity_grads is None else bool(intensity_grads)
     return _RenderTet.apply(verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, verts_depth, faces_intense,
-                            tets, face_tets, tet_faces, render_settings, det, vert)
+                            tets, face_tets, tet_faces, render_settings, det, vert, fint)
 
 
 class _RenderTet(th.autograd.Function):
@@ -206,9 +222,10 @@ class _RenderTet(th.autograd.Function):
 
     @staticmethod
     def forward(ctx, verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, verts_depth, faces_intense, tets,
-                face_tets, tet_faces, render_settings, deterministic=False, vertex_grads=False):
+                face_tets, tet_faces, render_settings, deterministic=False, vertex_grads=False, intensity_grads=False):
         ctx.deterministic = deterministic
         ctx.vertex_grads = vertex_grads
+        ctx.intensity_grads = intensity_grads
         inv = _C._Inverses(mv_mats, proj_mats)   # th.inverse x2 (reference :298-299): one launch, no device sync
         inv_mv_mats, inv_proj_mats = inv.inv_mv, inv.inv_proj
         mv_mats, proj_mats = inv.mv, inv.proj    # contiguous copies written by the same launch
@@ -243,39 +260,47 @@ class _RenderTet(th.autograd.Function):
         # vertex-position gradients (extension): only when switched on AND verts requires grad (DMesh passes verts
         # that require grad, so requires_grad alone must not turn this on)
         vertex = ctx.vertex_grads and ctx.needs_input_grad[0]
-        grad_mv = grad_proj = grad_verts = None
+        # face-intensity gradients (extension): likewise only when switched on AND faces_intense requires grad (callers
+        # compute intensities from verts, e.g. a Lambertian term)
+        intensity = ctx.intensity_grads and ctx.needs_input_grad[7]
+        grad_mv = grad_proj = grad_verts = grad_fint = None
         try:
             grads = _C.render_tets_backward(*args, deterministic=ctx.deterministic, tet_records=ctx.tet_records,
-                                            camera_grads=camera, vertex_grads=vertex)
+                                            camera_grads=camera, vertex_grads=vertex, intensity_grads=intensity)
         except Exception as ex:
             print("\nAn error occured in backward.\n")
             raise ex
         grad_verts_color, grad_faces_opacity = grads[:2]
         if camera:
             grad_mv, grad_proj = grads[2], grads[3]
+        if intensity:
+            grad_fint = grads[-1]
         if vertex:
-            grad_verts = grads[-1]
-        # gradient positions: reference __init__.py:407-422; positions 0 (verts) and 4, 5 (the matrices) are an extension
+            grad_verts = grads[-2] if intensity else grads[-1]
+        # gradient positions: reference __init__.py:407-422; positions 0 (verts), 4, 5 (the matrices) and 7
+        # (faces_intense) are an extension
         return (grad_verts, None, grad_verts_color, grad_faces_opacity,
                 grad_mv if ctx.needs_input_grad[4] else None, grad_proj if ctx.needs_input_grad[5] else None,
-                None, None, None, None, None, None, None, None)
+                None, grad_fint, None, None, None, None, None, None, None)
 
 
 class TetRenderer(th.nn.Module):
     """reference __init__.py:426-488"""
 
-    def __init__(self, render_settings: TetRenderSettings, deterministic=None, vertex_grads=None):
+    def __init__(self, render_settings: TetRenderSettings, deterministic=None, vertex_grads=None, intensity_grads=None):
         super().__init__()
         self.render_settings = render_settings
         self.deterministic = deterministic     # None: the process-wide default (set_deterministic)
         self.vertex_grads = vertex_grads       # None: the process-wide default (set_tet_vertex_grads)
+        self.intensity_grads = intensity_grads   # None: the process-wide default (set_tet_intensity_grads)
 
     def forward(self, verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, verts_depth, faces_intense, tets,
                 face_tets, tet_faces):
         """
         Gradients for verts_color and faces_opacity, and (extension) for mv_mats / proj_mats when they require
-        grad and for verts when vertex_grads is on and verts requires grad.  verts_depth is accepted but unused
-        (depth comes from the re-projected hit point).
+        grad, for verts when vertex_grads is on and verts requires grad, and for faces_intense when intensity_grads
+        is on and faces_intense requires grad (returned in faces_intense's own dtype and shape, e.g. float64 or a
+        stride-0 expanded [B,F]).  verts_depth is accepted but unused (depth comes from the re-projected hit point).
         tets [T,4], face_tets [F,2] (-1 = boundary), tet_faces [T,4]
         returns color [B,3,H,W], depth [B,1,H,W], active [B,H,W] bool
         """
@@ -284,4 +309,5 @@ class TetRenderer(th.nn.Module):
                           faces_opacity.to(dtype=f32), mv_mats.to(dtype=f32).transpose(1, 2),
                           proj_mats.to(dtype=f32).transpose(1, 2), verts_depth.to(dtype=f32),
                           faces_intense.to(dtype=f32), tets.to(dtype=i32), face_tets.to(dtype=i32),
-                          tet_faces.to(dtype=i32), self.render_settings, self.deterministic, self.vertex_grads)
+                          tet_faces.to(dtype=i32), self.render_settings, self.deterministic, self.vertex_grads,
+                          self.intensity_grads)

@@ -35,7 +35,9 @@ static const char* const g_stage_names[ST_COUNT] = {
     "tile_ranges", "tri_render_forward", "tri_render_backward", "tri_grad_finish", "tet_build_records", "tet_jitter",
     "tet_first_intersect", "tet_march_forward", "tet_march_backward", "tet_grad_vertex", "tri_render_backward_camera",
     "tri_camera_finish", "depth_chain_camera", "depth_chain_camera_finish", "tet_march_backward_camera", "tet_camera_finish",
-    "tet_march_backward_vertex", "tet_march_backward_camera_vertex", "tet_vertex_finish" };
+    "tet_march_backward_vertex", "tet_march_backward_camera_vertex", "tet_vertex_finish",
+    "tet_march_backward_intensity", "tet_march_backward_camera_intensity", "tet_march_backward_vertex_intensity",
+    "tet_march_backward_camera_vertex_intensity", "tet_intensity_finish" };
 struct Prof {
     bool on = false, created = false;
     cudaEvent_t ev[ST_COUNT][2];

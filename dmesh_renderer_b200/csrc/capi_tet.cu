@@ -33,20 +33,23 @@ bool tet_sizes_ok(long long B, long long P, long long F, long long T, long long 
 
 // scratch of the backward pass of either mode (dmr_tet_backward_workspace_bytes without its slack,
 // dmr_tet_backward_deterministic_bytes); vert: with the per-vertex position accumulator (default mode: a second
-// float4[P] right behind the colour one; deterministic mode: TetDetLayout::pos)
-size_t tet_bwd_scratch_bytes(int P, int F, bool deterministic, bool vert = false)
+// float4[P] right behind the colour one; deterministic mode: TetDetLayout::pos); fint_n: number of fixed-point
+// face-intensity accumulators (deterministic mode: B*F low words, then B*F high words, behind the rest; the default
+// mode needs none)
+size_t tet_bwd_scratch_bytes(int P, int F, bool deterministic, bool vert = false, size_t fint_n = 0)
 {
     if (deterministic) {
         const TetDetLayout L = TetDetLayout::make((size_t)P, (size_t)F);
-        return vert ? L.total_pos : L.total;
+        const size_t s = vert ? L.total_pos : L.total;
+        return fint_n ? align_up(s, 256) + 2 * sizeof(long long) * fint_n : s;
     }
     return sizeof(float4) * (size_t)P * (vert ? 2 : 1);
 }
 
 // workspace of the camera-gradient backward: the mode's own scratch, then DMR_TET_CAM_REC floats per (view, march CTA)
-size_t tet_cam_bytes(int B, int P, int F, int W, int H, bool deterministic, bool vert = false)
+size_t tet_cam_bytes(int B, int P, int F, int W, int H, bool deterministic, bool vert = false, size_t fint_n = 0)
 {
-    return align_up(tet_bwd_scratch_bytes(P, F, deterministic, vert), 256) +
+    return align_up(tet_bwd_scratch_bytes(P, F, deterministic, vert, fint_n), 256) +
            align_up(sizeof(float) * DMR_TET_CAM_REC * tet_cam_records((size_t)B, W, H), 256) + 256;
 }
 
@@ -54,6 +57,13 @@ size_t tet_cam_bytes(int B, int P, int F, int W, int H, bool deterministic, bool
 size_t tet_vert_bytes(int B, int P, int F, int W, int H, bool deterministic, bool cam)
 {
     return cam ? tet_cam_bytes(B, P, F, W, H, deterministic, true) : tet_bwd_scratch_bytes(P, F, deterministic, true) + 256;
+}
+
+// workspace of the face-intensity backward, with or without camera and vertex-position gradients
+size_t tet_int_bytes(int B, int P, int F, int W, int H, bool deterministic, bool cam, bool vert)
+{
+    const size_t n = (size_t)B * F;
+    return cam ? tet_cam_bytes(B, P, F, W, H, deterministic, vert, n) : tet_bwd_scratch_bytes(P, F, deterministic, vert, n) + 256;
 }
 
 }  // namespace
@@ -184,10 +194,12 @@ static int tet_backward_impl(int B, int P, int F, int T, int W, int H, int ray_r
                              const float* dL_dcolor, const float* dL_ddepth, float* dL_dverts_color,
                              float* dL_dfaces_opacity, void* workspace, size_t workspace_bytes, bool deterministic,
                              dmr_stream_t stream_, float* dL_dmv = nullptr, float* dL_dproj = nullptr,
-                             float* dL_dverts = nullptr)
+                             float* dL_dverts = nullptr, float* dL_dfaces_intense = nullptr)
 {
     const bool cam = dL_dmv != nullptr;
     const bool vert = dL_dverts != nullptr;
+    const bool fint = dL_dfaces_intense != nullptr;
+    const size_t fint_n = fint ? (size_t)B * F : 0;
     cudaStream_t stream = (cudaStream_t)stream_;
     if (!tet_sizes_ok(B, P, F, T, W, H)) return DMR_ETOOLARGE;
     if (B == 0 || F == 0 || T == 0) return DMR_OK;
@@ -197,6 +209,13 @@ static int tet_backward_impl(int B, int P, int F, int T, int W, int H, int ray_r
         return DMR_EINVAL;
     }
     (void)point_buffer;
+    if (fint) {
+        const size_t need = tet_int_bytes(B, P, F, W, H, deterministic, cam, vert);
+        if (!workspace || workspace_bytes < need) {
+            set_error("intensity-gradient backward needs a workspace of %zu bytes (dmr_tet_backward_intensity_bytes)", need);
+            return DMR_EINVAL;
+        }
+    }
     if (vert) {
         const size_t need = tet_vert_bytes(B, P, F, W, H, deterministic, cam);
         if (!workspace || workspace_bytes < need) {
@@ -208,14 +227,15 @@ static int tet_backward_impl(int B, int P, int F, int T, int W, int H, int ray_r
     // not cleared
     float* cam_rec = nullptr;
     if (cam) {
-        const size_t need = tet_cam_bytes(B, P, F, W, H, deterministic, vert);
+        const size_t need = tet_cam_bytes(B, P, F, W, H, deterministic, vert, fint_n);
         if (!workspace || workspace_bytes < need) {
             set_error("camera-gradient backward needs a workspace of %zu bytes (dmr_tet_backward_camera_bytes)", need);
             return DMR_EINVAL;
         }
-        cam_rec = at<float>(workspace, align_up(tet_bwd_scratch_bytes(P, F, deterministic, vert), 256));
+        cam_rec = at<float>(workspace, align_up(tet_bwd_scratch_bytes(P, F, deterministic, vert, fint_n), 256));
     }
     TetVertGrad vg{ dL_dverts, nullptr, nullptr };
+    TetIntGrad ig{ dL_dfaces_intense, nullptr, (ptrdiff_t)fint_n };
     void* det_workspace = workspace;
     const size_t det_workspace_bytes = workspace_bytes;
     TetParams p;
@@ -235,8 +255,9 @@ static int tet_backward_impl(int B, int P, int F, int T, int W, int H, int ray_r
         p.det_fopa = at<long long>(det_workspace, DL.fopa);
         p.grad_vacc = nullptr;
         vg.det_pos = at<long long>(det_workspace, DL.pos);
-        DMR_CUDA(cudaMemsetAsync(det_workspace, 0, vert ? DL.total_pos : DL.total, stream));
-        int rc = tet_march_backward_deterministic(p, stream, cam_rec, vert ? &vg : nullptr);
+        ig.det_fint = at<long long>(det_workspace, align_up(vert ? DL.total_pos : DL.total, 256));
+        DMR_CUDA(cudaMemsetAsync(det_workspace, 0, tet_bwd_scratch_bytes(P, F, true, vert, fint_n), stream));
+        int rc = tet_march_backward_deterministic(p, stream, cam_rec, vert ? &vg : nullptr, fint ? &ig : nullptr);
         if (rc || !cam) return rc;
         return tet_camera_finish(p, cam_rec, dL_dmv, dL_dproj, stream);
     }
@@ -248,7 +269,7 @@ static int tet_backward_impl(int B, int P, int F, int T, int W, int H, int ray_r
     p.grad_vacc = static_cast<float4*>(workspace);
     vg.grad_pacc = p.grad_vacc + P;
     DMR_CUDA(cudaMemsetAsync(p.grad_vacc, 0, sizeof(float4) * (size_t)P * (vert ? 2 : 1), stream));
-    int rc = tet_march_backward(p, stream, cam_rec, vert ? &vg : nullptr);
+    int rc = tet_march_backward(p, stream, cam_rec, vert ? &vg : nullptr, fint ? &ig : nullptr);
     if (rc || !cam) return rc;
     return tet_camera_finish(p, cam_rec, dL_dmv, dL_dproj, stream);
 }
@@ -342,6 +363,32 @@ int dmr_tet_backward_vertex(int B, int P, int F, int T, int W, int H, int ray_ra
                              inv_proj_mats, faces_intense, point_buffer, face_buffer, tet_records, image_buffer, dL_dcolor,
                              dL_ddepth, dL_dverts_color, dL_dfaces_opacity, workspace, workspace_bytes, deterministic != 0,
                              stream, dL_dmv, dL_dproj, dL_dverts);
+}
+
+size_t dmr_tet_backward_intensity_bytes(int B, int P, int F, int W, int H, int deterministic, int camera, int vertex)
+{
+    if (B < 0 || P < 0 || F < 0 || W < 0 || H < 0) return 0;
+    return tet_int_bytes(B, P, F, W, H, deterministic != 0, camera != 0, vertex != 0);
+}
+
+int dmr_tet_backward_intensity(int B, int P, int F, int T, int W, int H, int ray_random_seed, const float* background,
+                               const float* mv_mats, const float* proj_mats, const float* inv_mv_mats,
+                               const float* inv_proj_mats, const float* faces_intense, const void* point_buffer,
+                               const void* face_buffer, const void* tet_records, const void* image_buffer,
+                               const float* dL_dcolor, const float* dL_ddepth, float* dL_dverts_color,
+                               float* dL_dfaces_opacity, int deterministic, float* dL_dmv, float* dL_dproj,
+                               float* dL_dverts, float* dL_dfaces_intense, void* workspace, size_t workspace_bytes,
+                               dmr_stream_t stream)
+{
+    if ((dL_dmv == nullptr) != (dL_dproj == nullptr)) {
+        set_error("dL_dmv and dL_dproj: pass both (camera gradients) or neither");
+        return DMR_EINVAL;
+    }
+    if (B > 0 && !dL_dfaces_intense) { set_error("null pointer: dL_dfaces_intense"); return DMR_EINVAL; }
+    return tet_backward_impl(B, P, F, T, W, H, ray_random_seed, background, mv_mats, proj_mats, inv_mv_mats,
+                             inv_proj_mats, faces_intense, point_buffer, face_buffer, tet_records, image_buffer, dL_dcolor,
+                             dL_ddepth, dL_dverts_color, dL_dfaces_opacity, workspace, workspace_bytes, deterministic != 0,
+                             stream, dL_dmv, dL_dproj, dL_dverts, dL_dfaces_intense);
 }
 
 int dmr_debug_set_tet_first_split(int split)

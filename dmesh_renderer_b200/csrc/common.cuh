@@ -42,7 +42,8 @@ enum Stage {
     ST_SORT_PASS0, ST_SORT_PASS1, ST_SORT_PASS2, ST_SORT_PASS3, ST_SORT_PASS4, ST_SORT_PASS5, ST_SORT_PASS6, ST_SORT_PASS7,
     ST_RANGES, ST_TRI_FWD, ST_TRI_BWD, ST_TRI_BWD_FINISH, ST_TET_RECORDS, ST_TET_JITTER, ST_TET_FIRST, ST_TET_FWD, ST_TET_BWD, ST_TET_BWD_FINISH,
     ST_TRI_BWD_CAM, ST_TRI_CAM_FINISH, ST_DEPTH_CAM, ST_DEPTH_CAM_FINISH, ST_TET_BWD_CAM, ST_TET_CAM_FINISH,
-    ST_TET_BWD_VERT, ST_TET_BWD_CAM_VERT, ST_TET_VERT_FINISH, ST_COUNT
+    ST_TET_BWD_VERT, ST_TET_BWD_CAM_VERT, ST_TET_VERT_FINISH,
+    ST_TET_BWD_INT, ST_TET_BWD_CAM_INT, ST_TET_BWD_VERT_INT, ST_TET_BWD_CAM_VERT_INT, ST_TET_INT_FINISH, ST_COUNT
 };
 void count_launch(int n);
 void prof_begin(int stage, cudaStream_t s, bool count = true);   // count: also counts one kernel launch

@@ -159,6 +159,14 @@ struct TetVertGrad {
     long long* det_pos;           // deterministic mode: [P,4] zeroed fixed-point dL_dverts xyz, - (TetDetLayout::pos)
 };
 
+// Outputs of the face-intensity backward (dmr_tet_backward_intensity), a kernel argument of its own like TetVertGrad.
+struct TetIntGrad {
+    float* dL_dfint;              // [B,F], added to (default mode: by the march kernels directly)
+    long long* det_fint;          // deterministic mode: [B,F] zeroed fixed-point low words, behind the mode's scratch
+    ptrdiff_t det_hi;             // ... and the element offset of their high words (B*F: a [B,F] block outgrows
+                                  // TetDetLayout::hi_offset, which is sized for P and F)
+};
+
 // Camera gradients of the backward march: one record of DMR_TET_CAM_REC floats per (view, march CTA of 8 x 8 pixels),
 // written by every CTA (layout: tet_march_bwd_cam, tet_kernels.cu).
 #define DMR_TET_CAM_REC 32
@@ -212,9 +220,11 @@ int tet_march_forward(const TetParams& p, cudaStream_t stream);
 // cam_rec != nullptr: the camera-gradient kernels, which also store one DMR_TET_CAM_REC-float record per (view, march
 // CTA) there
 // vert != nullptr: the vertex-position kernels, which also add dL/dverts to vert->dL_dverts
-int tet_march_backward(const TetParams& p, cudaStream_t stream, float* cam_rec = nullptr, const TetVertGrad* vert = nullptr);
+// fint != nullptr: the face-intensity kernels, which also add dL/dfaces_intense to fint->dL_dfint
+int tet_march_backward(const TetParams& p, cudaStream_t stream, float* cam_rec = nullptr, const TetVertGrad* vert = nullptr,
+                       const TetIntGrad* fint = nullptr);
 int tet_march_backward_deterministic(const TetParams& p, cudaStream_t stream, float* cam_rec = nullptr,
-                                     const TetVertGrad* vert = nullptr);
+                                     const TetVertGrad* vert = nullptr, const TetIntGrad* fint = nullptr);
 // records of a view -> += dL_dmv[B,16], dL_dproj[B,16]
 int tet_camera_finish(const TetParams& p, const float* cam_rec, float* dL_dmv, float* dL_dproj, cudaStream_t stream);
 

@@ -955,6 +955,34 @@ __device__ __forceinline__ void tet_vert_step(const TetParams& p, TetVertAcc& a,
     }
 }
 
+// Face-intensity gradients (INT instantiations; DESIGN.md 3.4).  The step's colour is intense * interp with
+// interp = i0 c0 + i1 c1 + i2 c2, so with tet_bwd_face's dL_dcol[ch] = dLc[ch] opacity prev_T
+//     dL/dfaces_intense[b, face] += sum_ch dL_dcol[ch] interp[ch]
+// formed from interp itself, not col / intense: a face of intensity 0 gets its (generally nonzero) gradient.  One scalar
+// reduction into ig.dL_dfint, or one fixed-point addition with the value scale into ig.det_fint.  Called after
+// tet_bwd_face for the same step, whose st.prev_log_T it reads.
+template <class Base>
+struct TetIntAcc : Base {
+    TetIntGrad ig;
+};
+
+template <bool DET>
+__device__ __forceinline__ void tet_int_step(const TetParams& p, const TetIntGrad& ig, const TetBwdState& st, int b,
+                                             int face, float iu, float iv, const float4 s0, const float4 s1,
+                                             const float4 s2, const float dLc[3])
+{
+    const float3 c0 = f3(s0.x, s0.y, s0.z), c1 = f3(s0.w, s1.x, s1.y), c2 = f3(s1.z, s1.w, s2.x);
+    const float opacity = s2.y;
+    const float i0 = 1.0f - iu - iv;
+    const float3 interp = (i0 * c0) + (iu * c1) + (iv * c2);
+    const float prev_T = expf(st.prev_log_T);
+    const float g = dLc[0] * opacity * prev_T * interp.x + dLc[1] * opacity * prev_T * interp.y +
+                    dLc[2] * opacity * prev_T * interp.z;
+    const size_t i = (size_t)b * p.F + face;
+    if constexpr (DET) det_add(ig.det_fint + i, g, st.det_sv, ig.det_hi, p.det_gmax);
+    else atomicAdd(ig.dL_dfint + i, g);
+}
+
 // Backward march.  Steps recorded in the face trail (all of them unless a ray composited more than
 // trail_cap faces) are replayed in reverse: face id and the forward pass's own (t,u,v) from the trail
 // (one coalesced 16-byte load), all loads independent of the previous step and issued one step ahead.  Steps beyond the cap are re-marched through the adjacency records exactly like
@@ -967,7 +995,8 @@ __device__ __forceinline__ void tet_vert_step(const TetParams& p, TetVertAcc& a,
 // with its shading record.  The early returns end the walk only: tet_march_bwd_cam reduces after it on every lane.
 // VERT: also scatter the vertex-position terms of every walked step (tet_vert_step, sharing the triangle and the
 // sensitivities with CAM); `cam` is then a TetVertAcc.
-template <bool DET, bool CAM, bool VERT = false, class Acc = TetCamAcc>
+// INT: also add the face-intensity term of every walked step (tet_int_step); `cam` is then a TetIntAcc<...>.
+template <bool DET, bool CAM, bool VERT = false, bool INT = false, class Acc = TetCamAcc>
 __device__ __forceinline__ void tet_march_bwd_body(const TetParams& p, Acc& cam)
 {
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -1058,6 +1087,7 @@ __device__ __forceinline__ void tet_march_bwd_body(const TetParams& p, Acc& cam)
                 tet_vert_step<DET, CAM>(p, cam, st, dep, ro, rd, rt, iu, iv, s0, s1, s2, s3, intense, dLc, gd, v0, v1, v2z);
             else if constexpr (CAM)
                 tet_cam_step(cam, st, dep, ro, rd, rt, iu, iv, s0, s1, s2, intense, dLc, gd, v0, v1, v2z);
+            if constexpr (INT) tet_int_step<DET>(p, cam.ig, st, b, curr_face, iu, iv, s0, s1, s2, dLc);
             k--;
             if (curr_face == first_face) return;         // backward.cu:363-366
             if (curr_tet == -1) return;                  // backward.cu:373-376
@@ -1110,6 +1140,8 @@ __device__ __forceinline__ void tet_march_bwd_body(const TetParams& p, Acc& cam)
         else if constexpr (CAM)
             tet_cam_step(cam, st, dep, ro, rd, __int_as_float(e_cur.y), __int_as_float(e_cur.z), __int_as_float(e_cur.w), s0, s1,
                          s2, intense, dLc, gd, v0, v1, v2z);
+        if constexpr (INT)
+            tet_int_step<DET>(p, cam.ig, st, b, face, __int_as_float(e_cur.z), __int_as_float(e_cur.w), s0, s1, s2, dLc);
 
         if (stop_here) break;
         face = nf;
@@ -1148,6 +1180,38 @@ __global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_vert_det_kernel(T
     a.vg = vg;
     tet_march_bwd_body<true, false, true>(p, a);
 }
+// Face-intensity instantiations: dL/dfaces_intense straight into ig.dL_dfint, or into ig.det_fint
+// (tet_det_convert_intensity_kernel); with or without the vertex-position terms.
+__global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_int_kernel(TetParams p, TetIntGrad ig)
+{
+    griddep_wait();
+    TetIntAcc<TetCamAcc> a;
+    a.ig = ig;
+    tet_march_bwd_body<false, false, false, true>(p, a);
+}
+__global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_int_det_kernel(TetParams p, TetIntGrad ig)
+{
+    griddep_wait();
+    TetIntAcc<TetCamAcc> a;
+    a.ig = ig;
+    tet_march_bwd_body<true, false, false, true>(p, a);
+}
+__global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_vert_int_kernel(TetParams p, TetVertGrad vg, TetIntGrad ig)
+{
+    griddep_wait();
+    TetIntAcc<TetVertAcc> a;
+    a.vg = vg;
+    a.ig = ig;
+    tet_march_bwd_body<false, false, true, true>(p, a);
+}
+__global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_vert_int_det_kernel(TetParams p, TetVertGrad vg, TetIntGrad ig)
+{
+    griddep_wait();
+    TetIntAcc<TetVertAcc> a;
+    a.vg = vg;
+    a.ig = ig;
+    tet_march_bwd_body<true, false, true, true>(p, a);
+}
 
 // Camera-gradient instantiations: the walk of tet_march_bwd_body<DET, true>, then per lane the chain of its pixel into
 // the matrices, and one record of DMR_TET_CAM_REC floats per (view, CTA), summed in a fixed order (no float atomics:
@@ -1159,13 +1223,13 @@ __global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_vert_det_kernel(T
 // tet_camera_finish_kernel applies the inverses and the direct depth-row terms.
 static_assert(MARCH_THREADS == 64 && MARCH_ROWS == 8, "tet_cam_records (tet.cuh) counts 8 x 8-pixel march CTAs");
 static_assert(DMR_TET_CAM_REC == 32, "one record slot per lane");
-// VERT: Acc = TetVertAcc with its vg set by the caller.
-template <bool DET, bool VERT = false, class Acc = TetCamAcc>
+// VERT: Acc = TetVertAcc with its vg set by the caller.  INT: Acc = TetIntAcc<...> with its ig set by the caller.
+template <bool DET, bool VERT = false, bool INT = false, class Acc = TetCamAcc>
 __device__ __forceinline__ void tet_march_bwd_cam(const TetParams& p, float* __restrict__ cam_rec, Acc& a)
 {
     a.g_ro = f3(0, 0, 0); a.g_rd = f3(0, 0, 0);
     a.g_az = 0.0f; a.g_bz = 0.0f; a.g_aw = 0.0f; a.g_bw = 0.0f;
-    tet_march_bwd_body<DET, true, VERT>(p, a);
+    tet_march_bwd_body<DET, true, VERT, INT>(p, a);
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int b = blockIdx.z;
@@ -1255,6 +1319,38 @@ __global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_cam_vert_det_kern
     TetVertAcc a;
     a.vg = vg;
     tet_march_bwd_cam<true, true>(p, cam_rec, a);
+}
+__global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_cam_int_kernel(TetParams p, float* cam_rec, TetIntGrad ig)
+{
+    griddep_wait();
+    TetIntAcc<TetCamAcc> a;
+    a.ig = ig;
+    tet_march_bwd_cam<false, false, true>(p, cam_rec, a);
+}
+__global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_cam_int_det_kernel(TetParams p, float* cam_rec, TetIntGrad ig)
+{
+    griddep_wait();
+    TetIntAcc<TetCamAcc> a;
+    a.ig = ig;
+    tet_march_bwd_cam<true, false, true>(p, cam_rec, a);
+}
+__global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_cam_vert_int_kernel(TetParams p, float* cam_rec, TetVertGrad vg,
+                                                                                   TetIntGrad ig)
+{
+    griddep_wait();
+    TetIntAcc<TetVertAcc> a;
+    a.vg = vg;
+    a.ig = ig;
+    tet_march_bwd_cam<false, true, true>(p, cam_rec, a);
+}
+__global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_cam_vert_int_det_kernel(TetParams p, float* cam_rec,
+                                                                                       TetVertGrad vg, TetIntGrad ig)
+{
+    griddep_wait();
+    TetIntAcc<TetVertAcc> a;
+    a.vg = vg;
+    a.ig = ig;
+    tet_march_bwd_cam<true, true, true>(p, cam_rec, a);
 }
 
 // One CTA per view: the view's records (tet_march_bwd_cam) are summed in a fixed order -- thread t owns component
@@ -1382,16 +1478,70 @@ __global__ void __launch_bounds__(256) tet_det_convert_position_kernel(int P, in
     }
 }
 
-int tet_march_backward_deterministic(const TetParams& p, cudaStream_t stream, float* cam_rec, const TetVertGrad* vert)
+// Face-intensity gradients, deterministic mode, last step: += into dL_dfaces_intense[B,F], poisoned like the other
+// gradients of the call (det.cuh).  An intensity term beyond the range sets the shared overflow word, so it poisons
+// those too.
+__global__ void __launch_bounds__(256) tet_det_convert_intensity_kernel(size_t n, const uint32_t* __restrict__ gmax,
+                                                                        TetIntGrad ig)
+{
+    griddep_wait();   // programmatic dependent launch: see dmr_launch (common.cuh)
+    const size_t i = (size_t)blockIdx.x * 256 + threadIdx.x;
+    if (i >= n) return;
+    if (det_poisoned(gmax)) {
+        ig.dL_dfint[i] = __int_as_float(0x7fc00000);
+        return;
+    }
+    float sv, sg;
+    det_scales(*gmax, sv, sg);
+    if (sv == 0.0f) return;
+    const long long* a = ig.det_fint + i;
+    if (det_nonzero(a, ig.det_hi)) ig.dL_dfint[i] += (float)det_value(a, ig.det_hi, 1.0 / (double)sv);
+}
+
+// The march kernel of the intensity backward for the camera / vertex-position combination, with its stage.
+static int tet_march_backward_intensity(const TetParams& p, cudaStream_t stream, dim3 grid, float* cam_rec,
+                                        const TetVertGrad* vert, const TetIntGrad& ig, bool det)
+{
+    if (vert && cam_rec) {
+        if (det) DMR_CUDA(dmr_launch(tet_march_bwd_cam_vert_int_det_kernel, grid, dim3(MARCH_THREADS), 0, stream, p, cam_rec, *vert, ig));
+        else DMR_CUDA(dmr_launch(tet_march_bwd_cam_vert_int_kernel, grid, dim3(MARCH_THREADS), 0, stream, p, cam_rec, *vert, ig));
+        DMR_LAUNCH_CHECK("tet_march_bwd_cam_vert_int_kernel");
+    } else if (vert) {
+        if (det) DMR_CUDA(dmr_launch(tet_march_bwd_vert_int_det_kernel, grid, dim3(MARCH_THREADS), 0, stream, p, *vert, ig));
+        else DMR_CUDA(dmr_launch(tet_march_bwd_vert_int_kernel, grid, dim3(MARCH_THREADS), 0, stream, p, *vert, ig));
+        DMR_LAUNCH_CHECK("tet_march_bwd_vert_int_kernel");
+    } else if (cam_rec) {
+        if (det) DMR_CUDA(dmr_launch(tet_march_bwd_cam_int_det_kernel, grid, dim3(MARCH_THREADS), 0, stream, p, cam_rec, ig));
+        else DMR_CUDA(dmr_launch(tet_march_bwd_cam_int_kernel, grid, dim3(MARCH_THREADS), 0, stream, p, cam_rec, ig));
+        DMR_LAUNCH_CHECK("tet_march_bwd_cam_int_kernel");
+    } else {
+        if (det) DMR_CUDA(dmr_launch(tet_march_bwd_int_det_kernel, grid, dim3(MARCH_THREADS), 0, stream, p, ig));
+        else DMR_CUDA(dmr_launch(tet_march_bwd_int_kernel, grid, dim3(MARCH_THREADS), 0, stream, p, ig));
+        DMR_LAUNCH_CHECK("tet_march_bwd_int_kernel");
+    }
+    return 0;
+}
+
+static int tet_int_stage(const float* cam_rec, const TetVertGrad* vert)
+{
+    return vert ? (cam_rec ? ST_TET_BWD_CAM_VERT_INT : ST_TET_BWD_VERT_INT) : (cam_rec ? ST_TET_BWD_CAM_INT : ST_TET_BWD_INT);
+}
+
+int tet_march_backward_deterministic(const TetParams& p, cudaStream_t stream, float* cam_rec, const TetVertGrad* vert,
+                                     const TetIntGrad* fint)
 {
     dim3 grid((p.W + 7) / 8, (p.H + MARCH_ROWS - 1) / MARCH_ROWS, p.B);
     const size_t HW = (size_t)p.W * p.H;
     {
-        ProfScope prof(vert ? (cam_rec ? ST_TET_BWD_CAM_VERT : ST_TET_BWD_VERT) : (cam_rec ? ST_TET_BWD_CAM : ST_TET_BWD), stream);
+        ProfScope prof(fint ? tet_int_stage(cam_rec, vert)
+                            : vert ? (cam_rec ? ST_TET_BWD_CAM_VERT : ST_TET_BWD_VERT) : (cam_rec ? ST_TET_BWD_CAM : ST_TET_BWD),
+                       stream);
         count_launch(1);   // two kernels under one scope
         int rc = det_gmax(p.dL_dcolor, 3 * p.B * HW, p.dL_ddepth, p.B * HW, const_cast<uint32_t*>(p.det_gmax), stream);
         if (rc) return rc;
-        if (vert && cam_rec) {
+        if (fint) {
+            if ((rc = tet_march_backward_intensity(p, stream, grid, cam_rec, vert, *fint, true))) return rc;
+        } else if (vert && cam_rec) {
             DMR_CUDA(dmr_launch(tet_march_bwd_cam_vert_det_kernel, dim3(grid), dim3(MARCH_THREADS), 0, stream, p, cam_rec, *vert));
             DMR_LAUNCH_CHECK("tet_march_bwd_cam_vert_det_kernel");
         } else if (vert) {
@@ -1416,13 +1566,24 @@ int tet_march_backward_deterministic(const TetParams& p, cudaStream_t stream, fl
                             p.det_gmax, *vert));
         DMR_LAUNCH_CHECK("tet_det_convert_position_kernel");
     }
+    if (fint) {
+        const size_t n = (size_t)p.B * p.F;
+        ProfScope prof(ST_TET_INT_FINISH, stream);
+        DMR_CUDA(dmr_launch(tet_det_convert_intensity_kernel, dim3((unsigned)((n + 255) / 256)), dim3(256), 0, stream, n,
+                            p.det_gmax, *fint));
+        DMR_LAUNCH_CHECK("tet_det_convert_intensity_kernel");
+    }
     return 0;
 }
 
-int tet_march_backward(const TetParams& p, cudaStream_t stream, float* cam_rec, const TetVertGrad* vert)
+int tet_march_backward(const TetParams& p, cudaStream_t stream, float* cam_rec, const TetVertGrad* vert,
+                       const TetIntGrad* fint)
 {
     dim3 grid((p.W + 7) / 8, (p.H + MARCH_ROWS - 1) / MARCH_ROWS, p.B);
-    if (vert && cam_rec) {
+    if (fint) {
+        ProfScope prof(tet_int_stage(cam_rec, vert), stream);
+        if (int rc = tet_march_backward_intensity(p, stream, grid, cam_rec, vert, *fint, false)) return rc;
+    } else if (vert && cam_rec) {
         ProfScope prof(ST_TET_BWD_CAM_VERT, stream);
         DMR_CUDA(dmr_launch(tet_march_bwd_cam_vert_kernel, dim3(grid), dim3(MARCH_THREADS), 0, stream, p, cam_rec, *vert));
         DMR_LAUNCH_CHECK("tet_march_bwd_cam_vert_kernel");

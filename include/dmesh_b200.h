@@ -401,6 +401,38 @@ int dmr_tet_backward_vertex(
     void* workspace, size_t workspace_bytes,
     dmr_stream_t stream);
 
+/* Face-intensity gradients of the tet renderer (no reference counterpart: the reference returns no gradient for   */
+/* faces_intense).  The backward pass of dmr_tet_backward_vertex, with the same arguments, except that dL_dverts   */
+/* may be NULL too (no vertex-position gradients), plus dL/dfaces_intense [B,F] ADDED to dL_dfaces_intense.  The    */
+/* derivative is that of the rendered colour image (depth does not depend on intensity), with the same things held */
+/* fixed as for the camera gradients: per walked step, sum_ch dL/dcol[ch] T alpha interp[ch], interp = the step's   */
+/* interpolated vertex colour before the multiplication by the intensity, so a face of intensity 0 gets its        */
+/* gradient too.  Only the steps the backward pass walks contribute.  Summed with float atomics (deterministic ==   */
+/* 0) or in fixed point (deterministic != 0; reproducible, NaN for non-finite cotangents).  The other gradients are */
+/* those of the mode it extends.  `workspace`: dmr_tet_backward_intensity_bytes(B, P, F, W, H, deterministic,       */
+/* camera, vertex) bytes of device scratch, camera / vertex = whether dL_dmv and dL_dproj / dL_dverts are passed:   */
+/* the mode's own scratch plus, in deterministic mode, one fixed-point accumulator per (view, face).                */
+size_t dmr_tet_backward_intensity_bytes(int B, int P, int F, int W, int H, int deterministic, int camera, int vertex);
+int dmr_tet_backward_intensity(
+    int B, int P, int F, int T, int W, int H,
+    int ray_random_seed,
+    const float* background,
+    const float* mv_mats, const float* proj_mats,
+    const float* inv_mv_mats, const float* inv_proj_mats,
+    const float* faces_intense,
+    const void* point_buffer, const void* face_buffer,
+    const void* tet_records,
+    const void* image_buffer,
+    const float* dL_dcolor, const float* dL_ddepth,
+    float* dL_dverts_color, float* dL_dfaces_opacity,
+    int deterministic,
+    float* dL_dmv,               /* [B,16] or NULL */
+    float* dL_dproj,             /* [B,16] or NULL */
+    float* dL_dverts,            /* [P,3] or NULL */
+    float* dL_dfaces_intense,    /* [B,F] */
+    void* workspace, size_t workspace_bytes,
+    dmr_stream_t stream);
+
 /* ------------------------------------------------------------------------ */
 /* Read-only views into the state buffers for the bit-exact parity checks    */
 /* (the reference exposes the same quantities through the fromChunk layouts, */
