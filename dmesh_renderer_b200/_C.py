@@ -363,10 +363,19 @@ def render_tris(background, verts, faces, verts_color, faces_opacity, mv_mats, p
 _grad_sinks = []
 
 
-def grad_sink_for(verts, verts_color, faces_opacity):
+def grad_sink_for(verts, verts_color, faces_opacity, tet=False):
+    """The innermost active sink whose leaves are exactly these tensors.  A sink without positions
+    (PackedSceneGrads(None, verts_color, faces_opacity)) holds no verts slot; only a tet call (`tet=True`) may match
+    it, on verts_color and faces_opacity alone."""
     for sink in reversed(_grad_sinks):
+        if len(sink.leaves) == 3:
+            xs = (verts, verts_color, faces_opacity)
+        elif tet:
+            xs = (verts_color, faces_opacity)
+        else:
+            continue
         ok = True
-        for x, leaf in zip((verts, verts_color, faces_opacity), sink.leaves):
+        for x, leaf in zip(xs, sink.leaves):
             g = leaf.grad
             if not (x is leaf or (x.data_ptr() == leaf.data_ptr() and x.shape == leaf.shape and x.dtype == leaf.dtype)) \
                     or g is None or g.dtype != torch.float32 or not g.is_contiguous() or g.shape != leaf.shape \
@@ -519,10 +528,13 @@ class _TetRecordCache:
 
 def render_tets(background, verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, inv_mv_mats, inv_proj_mats,
                 verts_depth, faces_intense, tets, face_tets, tet_faces, image_height, image_width, ray_random_seed,
-                inverses=None):
+                inverses=None, first_view=0):
     """RenderFTetsCUDA (render.cu:213-336).
     Returns (color[B,3,H,W], depth[B,1,H,W], active_f32[B,H,W], pointBuffer, faceBuffer, binningBuffer, imgBuffer).
     `inverses` (beyond the reference's 17 arguments): see tri_forward_finish.
+    `first_view` (beyond the reference's 17 arguments): index of this call's view 0 in a larger job.  With
+    ray_random_seed > 0 the jitter of a view then depends only on its index in the job, not on the call that renders
+    it (dmr_tet_forward_render_views); 0, the default, gives the reference's rays.
     The cached adjacency records (_TetRecordCache) travel with the returned face buffer as its attribute
     `tet_records`, for render_tets_backward."""
     if verts.dim() != 2 or verts.size(1) != 3:
@@ -581,10 +593,10 @@ def render_tets(background, verts, faces, verts_color, faces_opacity, mv_mats, p
             _Pinned.release(pinned)
         if inverses is not None:
             inverses.check()
-        _lib.check(lib.dmr_tet_forward_render(B, P, F, T, W, H, R, int(ray_random_seed), _ptr(bg), _ptr(mv), _ptr(pj),
-                                              _ptr(imv), _ptr(ipj), _ptr(fint), _ptr(point_buf), _ptr(face_buf),
-                                              _ptr(tet_rec), _ptr(bin_buf), _ptr(img_buf), _ptr(out_color),
-                                              _ptr(out_depth), _ptr(out_active), stream))
+        _lib.check(lib.dmr_tet_forward_render_views(B, P, F, T, W, H, R, int(ray_random_seed), int(first_view), _ptr(bg),
+                                                    _ptr(mv), _ptr(pj), _ptr(imv), _ptr(ipj), _ptr(fint), _ptr(point_buf),
+                                                    _ptr(face_buf), _ptr(tet_rec), _ptr(bin_buf), _ptr(img_buf),
+                                                    _ptr(out_color), _ptr(out_depth), _ptr(out_active), stream))
         face_buf.tet_records = tet_rec     # kept alive (and found by render_tets_backward) through the face buffer
     return out_color, out_depth, out_active, point_buf, face_buf, bin_buf, img_buf
 
@@ -592,7 +604,8 @@ def render_tets(background, verts, faces, verts_color, faces_opacity, mv_mats, p
 def render_tets_backward(background, verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, inv_mv_mats,
                          inv_proj_mats, verts_depth, faces_intense, tets, face_tets, tet_faces, grad_color, grad_depth,
                          pointBuffer, faceBuffer, binningBuffer, imageBuffer, ray_random_seed=None, deterministic=False,
-                         tet_records=None, camera_grads=False, vertex_grads=False, intensity_grads=False):
+                         tet_records=None, camera_grads=False, vertex_grads=False, intensity_grads=False,
+                         accumulate_into=None):
     """RenderFTetsBackwardCUDA (render.cu:338-412).
     Returns (dL_dverts_color[P,3], dL_dfaces_opacity[F]).  `ray_random_seed` is an
     optional trailing argument beyond the reference's 20: the autograd wrapper passes
@@ -606,20 +619,33 @@ def render_tets_backward(background, verts, faces, verts_color, faces_opacity, m
     of every walked step; dmr_tet_backward_vertex) as the last element.
     `intensity_grads`: also return dL_dfaces_intense [B,F] (gradient with respect to the face intensities, through the
     colour of every walked step; dmr_tet_backward_intensity) as the last element, after dL_dverts when both are
-    requested."""
+    requested.
+    `accumulate_into`: (dL_dverts_color, dL_dfaces_opacity, dL_dverts), existing contiguous fp32 tensors of shapes
+    [P,3], [F], [P,3] that the gradients are ADDED to (and that are returned) instead of fresh zero tensors, in every
+    mode.  dL_dverts may be None (a fresh tensor when vertex_grads is set); it is written only when vertex_grads is
+    set.  The camera and intensity gradients are always fresh tensors."""
     lib = _lib.load()
     B, P, F, T = mv_mats.size(0), verts.size(0), faces.size(0), tets.size(0)
     H, W = grad_color.size(2), grad_color.size(3)
     dev = verts.device
     if ray_random_seed is None:
         ray_random_seed = 0
+    into = (None, None, None)
+    if accumulate_into is not None:
+        into = tuple(accumulate_into)
+        if len(into) != 3 or into[0] is None or into[1] is None:
+            _err("accumulate_into must be (dL_dverts_color, dL_dfaces_opacity, dL_dverts or None)")
+    for t, shape, n in zip(into, ((P, 3), (F,), (P, 3)), ("dL_dverts_color", "dL_dfaces_opacity", "dL_dverts")):
+        if t is not None and (t.dtype != torch.float32 or not t.is_contiguous() or tuple(t.shape) != shape or
+                              t.device != dev):
+            _err("accumulate_into: %s must be a contiguous float32 %s tensor on %s" % (n, list(shape), dev))
     with _on_device(dev):
         z = dict(dtype=torch.float32, device=dev)
-        dL_dverts_color = torch.zeros((P, 3), **z)
-        dL_dfaces_opacity = torch.zeros((F,), **z)
+        dL_dverts_color = into[0] if into[0] is not None else torch.zeros((P, 3), **z)
+        dL_dfaces_opacity = into[1] if into[1] is not None else torch.zeros((F,), **z)
         # [B,16] column-major = [B,4,4] gradients of the (column-major, i.e. transposed) matrix tensors given here
         cam = torch.zeros((2, B, 4, 4), **z) if camera_grads else None
-        dL_dverts = torch.zeros((P, 3), **z) if vertex_grads else None
+        dL_dverts = (into[2] if into[2] is not None else torch.zeros((P, 3), **z)) if vertex_grads else None
         dL_dfint = torch.zeros((B, F), **z) if intensity_grads else None
         if B * H * W > 0 and F > 0 and T > 0:
             bg = _f32(background, "background")

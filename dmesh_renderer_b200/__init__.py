@@ -207,14 +207,14 @@ def set_tet_intensity_grads(flag: bool) -> bool:
 
 def render_tet(verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, verts_depth, faces_intense, tets,
                face_tets, tet_faces, render_settings: TetRenderSettings, deterministic=None, vertex_grads=None,
-               intensity_grads=None):
+               intensity_grads=None, first_view=0):
     """reference __init__.py:243-275 (`deterministic`: see set_deterministic; `vertex_grads`: see
-    set_tet_vertex_grads; `intensity_grads`: see set_tet_intensity_grads)"""
+    set_tet_vertex_grads; `intensity_grads`: see set_tet_intensity_grads; `first_view`: see TetRenderer.forward)"""
     det = _deterministic_default if deterministic is None else bool(deterministic)
     vert = _tet_vertex_grads_default if vertex_grads is None else bool(vertex_grads)
     fint = _tet_intensity_grads_default if intensity_grads is None else bool(intensity_grads)
     return _RenderTet.apply(verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, verts_depth, faces_intense,
-                            tets, face_tets, tet_faces, render_settings, det, vert, fint)
+                            tets, face_tets, tet_faces, render_settings, det, vert, fint, int(first_view))
 
 
 class _RenderTet(th.autograd.Function):
@@ -222,7 +222,8 @@ class _RenderTet(th.autograd.Function):
 
     @staticmethod
     def forward(ctx, verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, verts_depth, faces_intense, tets,
-                face_tets, tet_faces, render_settings, deterministic=False, vertex_grads=False, intensity_grads=False):
+                face_tets, tet_faces, render_settings, deterministic=False, vertex_grads=False, intensity_grads=False,
+                first_view=0):
         ctx.deterministic = deterministic
         ctx.vertex_grads = vertex_grads
         ctx.intensity_grads = intensity_grads
@@ -233,13 +234,15 @@ class _RenderTet(th.autograd.Function):
                 inv_proj_mats, verts_depth, faces_intense, tets, face_tets, tet_faces, render_settings.image_height,
                 render_settings.image_width, render_settings.ray_random_seed, inv)
         try:
-            color, depth, active, pointBuffer, faceBuffer, binningBuffer, imgBuffer = _C.render_tets(*args)
+            color, depth, active, pointBuffer, faceBuffer, binningBuffer, imgBuffer = _C.render_tets(
+                *args, first_view=first_view)
         except Exception as ex:
             print("\nAn error occured in forward.")
             raise ex
         active = (active > 0.5)
         ctx.render_settings = render_settings
         ctx.tet_records = getattr(faceBuffer, "tet_records", None)   # cached adjacency records (no gradient, not an input)
+        ctx.grad_sink = _C.grad_sink_for(verts, verts_color, faces_opacity, tet=True)   # PackedSceneGrads.direct()
         ctx.save_for_backward(verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, inv_mv_mats, inv_proj_mats,
                               verts_depth, faces_intense, tets, face_tets, tet_faces, pointBuffer, faceBuffer,
                               binningBuffer, imgBuffer)
@@ -264,9 +267,17 @@ class _RenderTet(th.autograd.Function):
         # compute intensities from verts, e.g. a Lambertian term)
         intensity = ctx.intensity_grads and ctx.needs_input_grad[7]
         grad_mv = grad_proj = grad_verts = grad_fint = None
+        # a gradient sink takes verts_color, faces_opacity and, when it has a verts slot and the vertex-position path
+        # runs, verts; camera and intensity gradients are per view and always go through autograd
+        sink = ctx.grad_sink
+        into = None
+        if sink is not None and sink.bind() == 0:   # (bind() != 0: see _RenderTri.backward)
+            g = [leaf.grad for leaf in sink.leaves]
+            into = (g[-2], g[-1], g[0] if len(g) == 3 and vertex else None)
         try:
             grads = _C.render_tets_backward(*args, deterministic=ctx.deterministic, tet_records=ctx.tet_records,
-                                            camera_grads=camera, vertex_grads=vertex, intensity_grads=intensity)
+                                            camera_grads=camera, vertex_grads=vertex, intensity_grads=intensity,
+                                            accumulate_into=into)
         except Exception as ex:
             print("\nAn error occured in backward.\n")
             raise ex
@@ -277,11 +288,16 @@ class _RenderTet(th.autograd.Function):
             grad_fint = grads[-1]
         if vertex:
             grad_verts = grads[-2] if intensity else grads[-1]
+        if into is not None:
+            # already added to the leaves' .grad by the kernels
+            grad_verts_color = grad_faces_opacity = None
+            if into[2] is not None:
+                grad_verts = None
         # gradient positions: reference __init__.py:407-422; positions 0 (verts), 4, 5 (the matrices) and 7
         # (faces_intense) are an extension
         return (grad_verts, None, grad_verts_color, grad_faces_opacity,
                 grad_mv if ctx.needs_input_grad[4] else None, grad_proj if ctx.needs_input_grad[5] else None,
-                None, grad_fint, None, None, None, None, None, None, None)
+                None, grad_fint, None, None, None, None, None, None, None, None)
 
 
 class TetRenderer(th.nn.Module):
@@ -295,13 +311,17 @@ class TetRenderer(th.nn.Module):
         self.intensity_grads = intensity_grads   # None: the process-wide default (set_tet_intensity_grads)
 
     def forward(self, verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, verts_depth, faces_intense, tets,
-                face_tets, tet_faces):
+                face_tets, tet_faces, first_view=0):
         """
         Gradients for verts_color and faces_opacity, and (extension) for mv_mats / proj_mats when they require
         grad, for verts when vertex_grads is on and verts requires grad, and for faces_intense when intensity_grads
         is on and faces_intense requires grad (returned in faces_intense's own dtype and shape, e.g. float64 or a
         stride-0 expanded [B,F]).  verts_depth is accepted but unused (depth comes from the re-projected hit point).
         tets [T,4], face_tets [F,2] (-1 = boundary), tet_faces [T,4]
+        first_view (extension): index of view 0 of this call in a larger job, e.g. a rank's share of the cameras
+        (multiview.shard_views(...).start).  With ray_random_seed > 0 the jittered rays of a view then depend only on
+        its index in the job, so rendering views s..e-1 with first_view=s gives exactly views s..e-1 of one call over
+        all views.  0, the default, gives the reference's rays.
         returns color [B,3,H,W], depth [B,1,H,W], active [B,H,W] bool
         """
         f32, i32 = th.float32, th.int32
@@ -310,4 +330,4 @@ class TetRenderer(th.nn.Module):
                           proj_mats.to(dtype=f32).transpose(1, 2), verts_depth.to(dtype=f32),
                           faces_intense.to(dtype=f32), tets.to(dtype=i32), face_tets.to(dtype=i32),
                           tet_faces.to(dtype=i32), self.render_settings, self.deterministic, self.vertex_grads,
-                          self.intensity_grads)
+                          self.intensity_grads, first_view)

@@ -42,6 +42,7 @@ SIGNATURES = {
     "dmr_tet_build_records": (c_int, [c_int] * 3 + [c_void_p] * 6 + [c_void_p]),
     "dmr_tet_forward_bin": (c_int, [c_int] * 6 + [c_void_p] * 12 + [c_int] + [c_void_p] * 2),
     "dmr_tet_forward_render": (c_int, [c_int] * 8 + [c_void_p] * 14 + [c_void_p]),
+    "dmr_tet_forward_render_views": (c_int, [c_int] * 9 + [c_void_p] * 14 + [c_void_p]),
     "dmr_tet_backward_workspace_bytes": (c_size_t, [c_int]),
     "dmr_tet_backward": (c_int, [c_int] * 7 + [c_void_p] * 14 + [c_void_p, c_size_t] + [c_void_p]),
     "dmr_tet_backward_deterministic_bytes": (c_size_t, [c_int] * 2),

@@ -158,9 +158,22 @@ int dmr_tet_forward_render(int B, int P, int F, int T, int W, int H, int R, int 
                            const float* background, const float* mv_mats, const float* proj_mats,
                            const float* inv_mv_mats, const float* inv_proj_mats, const float* faces_intense,
                            const void* point_buffer, void* face_buffer, const void* tet_records, void* binning_buffer,
-                           void* image_buffer, float* out_color, float* out_depth, float* out_active, dmr_stream_t stream_)
+                           void* image_buffer, float* out_color, float* out_depth, float* out_active, dmr_stream_t stream)
+{
+    return dmr_tet_forward_render_views(B, P, F, T, W, H, R, ray_random_seed, 0, background, mv_mats, proj_mats,
+                                        inv_mv_mats, inv_proj_mats, faces_intense, point_buffer, face_buffer, tet_records,
+                                        binning_buffer, image_buffer, out_color, out_depth, out_active, stream);
+}
+
+int dmr_tet_forward_render_views(int B, int P, int F, int T, int W, int H, int R, int ray_random_seed, int first_view,
+                                 const float* background, const float* mv_mats, const float* proj_mats,
+                                 const float* inv_mv_mats, const float* inv_proj_mats, const float* faces_intense,
+                                 const void* point_buffer, void* face_buffer, const void* tet_records,
+                                 void* binning_buffer, void* image_buffer, float* out_color, float* out_depth,
+                                 float* out_active, dmr_stream_t stream_)
 {
     cudaStream_t stream = (cudaStream_t)stream_;
+    if (first_view < 0) { set_error("first_view must not be negative (got %d)", first_view); return DMR_EINVAL; }
     if (!tet_sizes_ok(B, P, F, T, W, H) || R < 0) return DMR_ETOOLARGE;
     if (B == 0) return DMR_OK;
     if (!background || !mv_mats || !proj_mats || !inv_mv_mats || !inv_proj_mats || !face_buffer || !image_buffer ||
@@ -178,7 +191,7 @@ int dmr_tet_forward_render(int B, int P, int F, int T, int W, int H, int R, int 
     fill_params(p, B, P, F, T, W, H, ray_random_seed, background, mv_mats, proj_mats, inv_mv_mats, inv_proj_mats,
                 faces_intense, face_buffer, tet_records, image_buffer);
     if (ray_random_seed > 0)
-        if ((rc = tet_jitter(B, W, H, ray_random_seed, at<float2>(image_buffer, IL.jitter), stream))) return rc;
+        if ((rc = tet_jitter(B, W, H, ray_random_seed, first_view, at<float2>(image_buffer, IL.jitter), stream))) return rc;
     if ((rc = bin_instances(B, F, W, H, (size_t)R, face_buffer, FL.bin, binning_buffer, ranges, stream))) return rc;
     if (R > 0) p.face_list = at<uint32_t>(binning_buffer, BinningLayout::make((size_t)R).vals_sorted);
     p.out_color = out_color; p.out_depth = out_depth; p.out_active = out_active;

@@ -214,7 +214,8 @@ int tet_preprocess_faces(int B, int P, int F, int W, int H, const int* faces, co
 int tet_build_records(int P, int F, int T, const float* verts, const int* faces, const float* verts_color,
                       const float* faces_opacity, const int* tets, const int* face_tets, const int* tet_faces,
                       TetRec* tet_rec, TetShade* shade, cudaStream_t stream);
-int tet_jitter(int B, int W, int H, int seed, float2* jitter, cudaStream_t stream);
+// first_view: index, in the whole job, of the call's view 0; it offsets the cuRAND subsequence of every pixel
+int tet_jitter(int B, int W, int H, int seed, int first_view, float2* jitter, cudaStream_t stream);
 int tet_first_intersect(const TetParams& p, cudaStream_t stream);
 int tet_march_forward(const TetParams& p, cudaStream_t stream);
 // cam_rec != nullptr: the camera-gradient kernels, which also store one DMR_TET_CAM_REC-float record per (view, march

@@ -210,14 +210,17 @@ int tet_build_records(int P, int F, int T, const float* verts, const int* faces,
 // jittered pixel coordinates (ray_random_seed > 0): XORWOW, sequence = pixel index
 // forward.cu:82-88, 120-123.  Stored (8 B/px) so that first-intersect, march and
 // backward see the same ray without re-running curand_init three times.
+// The sequence counts pixels from view `first_view` of the whole job, (first_view + b)*H*W + y*W + x, so a view
+// gets the same rays whichever call (or rank) renders it; first_view = 0 is the reference's pixel index.
 // ---------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) tet_jitter_kernel(int BI, int W, int H, int seed, float2* __restrict__ jitter)
+__global__ void __launch_bounds__(256) tet_jitter_kernel(int BI, int W, int H, int seed, int first_view,
+                                                         float2* __restrict__ jitter)
 {
     griddep_wait();   // programmatic dependent launch: see dmr_launch (common.cuh)
     int idx = blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= BI) return;
     curandState st;
-    curand_init(seed, idx, 0, &st);
+    curand_init(seed, (unsigned long long)first_view * W * H + (unsigned long long)idx, 0, &st);
     int pixel_id = idx % (W * H);
     int pixel_x = pixel_id % W, pixel_y = pixel_id / W;
     float2 o;
@@ -226,12 +229,13 @@ __global__ void __launch_bounds__(256) tet_jitter_kernel(int BI, int W, int H, i
     jitter[idx] = o;
 }
 
-int tet_jitter(int B, int W, int H, int seed, float2* jitter, cudaStream_t stream)
+int tet_jitter(int B, int W, int H, int seed, int first_view, float2* jitter, cudaStream_t stream)
 {
     int BI = B * W * H;
     if (BI <= 0) return 0;
     ProfScope prof(ST_TET_JITTER, stream);
-    DMR_CUDA(dmr_launch(tet_jitter_kernel, dim3((BI + 255) / 256), dim3(256), 0, stream, BI, W, H, seed, jitter));
+    DMR_CUDA(dmr_launch(tet_jitter_kernel, dim3((BI + 255) / 256), dim3(256), 0, stream, BI, W, H, seed, first_view,
+                        jitter));
     DMR_LAUNCH_CHECK("tet_jitter_kernel");
     return 0;
 }

@@ -9,6 +9,12 @@ cameras, and ONE all-reduce(SUM) over a single packed fp32 buffer
 that has to be exchanged.  Per-view gradients (verts_depth, faces_intense rows)
 stay rank-local.  One process per GPU, torch.distributed (NCCL over NVLink 5 /
 NVSwitch on the B200 box, gloo in the CPU tests); nothing else communicates.
+
+The tet renderer takes part through tet_multiview_step.  Without vertex-position
+gradients it has no dL_dverts, so PackedSceneGrads(None, verts_color,
+faces_opacity) packs just [dL_dvcolor | dL_dfopacity] = (3P + F) floats.  Each
+call passes the job index of its first view (first_view), so jittered rays
+(ray_random_seed > 0) do not depend on how the views are sharded or split.
 """
 import contextlib
 from typing import Callable, Optional, Sequence, Tuple
@@ -56,6 +62,10 @@ def shard_views(num_views: int, rank: int, world_size: int) -> range:
 class PackedSceneGrads:
     """Scene leaves (verts, verts_color, faces_opacity) whose .grad tensors are
     views into ONE contiguous fp32 buffer, so the step needs a single collective.
+    Layout [verts | verts_color | faces_opacity], 6P + F floats.  verts=None gives
+    the tet renderer's layout without positions, [verts_color | faces_opacity],
+    3P + F floats; `leaves` then holds the two tensors, and only TetRenderer calls
+    can use it as a sink (see direct()).
 
     On a CUDA job with world_size > 1 the buffer is allocated in SYMMETRIC memory
     (torch.distributed._symmetric_memory: peer-mapped on every rank + an NVLS multicast
@@ -66,17 +76,20 @@ class PackedSceneGrads:
 
     def __init__(self, verts: torch.Tensor, verts_color: torch.Tensor, faces_opacity: torch.Tensor, group=None,
                  use_nvls: Optional[bool] = None):
-        self.leaves = [verts, verts_color, faces_opacity]
+        self.leaves = [t for t in (verts, verts_color, faces_opacity) if t is not None]
+        if len(self.leaves) < 2 or verts_color is None or faces_opacity is None:
+            raise ValueError("PackedSceneGrads needs verts_color and faces_opacity")
         self.group = group
+        device = verts_color.device
         n = sum(t.numel() for t in self.leaves)
         self._nvls = None
         # which collective all_reduce() runs and, for the fallback, why: "nvls" | "nccl: <reason>" | "none: <reason>"
         self.collective = "nccl: use_nvls=False" if use_nvls is False else "none: single process"
         full = None
         if use_nvls is not False:
-            full = self._try_symmetric(n, verts.device, group)
+            full = self._try_symmetric(n, device, group)
         if full is None:
-            full = torch.zeros(n, dtype=torch.float32, device=verts.device)
+            full = torch.zeros(n, dtype=torch.float32, device=device)
         self._full = full              # padded to a multiple of 4 * world_size floats in the NVLS case
         self.flat = full[:n]
         for t in self.leaves:
@@ -153,10 +166,13 @@ class PackedSceneGrads:
 
     @contextlib.contextmanager
     def direct(self):
-        """While active, TriRenderer calls on these leaves accumulate their scene gradients straight into the packed
-        buffer from the backward kernels (no intermediate gradient tensors, no autograd accumulation kernels).
-        The leaves must be passed to the renderer themselves (not views or functions of them); gradient hooks on
-        them do not see this contribution.  The choice is made at forward time, so backward may run later."""
+        """While active, TriRenderer and TetRenderer calls on these leaves accumulate their scene gradients straight
+        into the packed buffer from the backward kernels (no intermediate gradient tensors, no autograd accumulation
+        kernels).  The leaves must be passed to the renderer themselves (not views or functions of them); gradient
+        hooks on them do not see this contribution.  The choice is made at forward time, so backward may run later.
+        A tet call adds into the verts slot only when its vertex-position gradients run; a buffer without that slot
+        (verts=None) serves tet calls only.  Camera, intensity and other per-view gradients always go through
+        autograd."""
         from . import _C
         self.bind()
         _C._grad_sinks.append(self)
@@ -214,5 +230,48 @@ def multiview_step(render: Callable, scene_grads: PackedSceneGrads, faces: torch
             gc, gd = cotangent_fn(color, depth)
             torch.autograd.backward([color, depth], [gc, gd])
             outs.append((color.detach(), depth.detach()))
+    scene_grads.all_reduce(group)
+    return outs
+
+
+def tet_multiview_step(render: Callable, scene_grads: PackedSceneGrads, verts: torch.Tensor, faces: torch.Tensor,
+                       tets: torch.Tensor, face_tets: torch.Tensor, tet_faces: torch.Tensor, mv_mats: torch.Tensor,
+                       proj_mats: torch.Tensor, verts_depth: torch.Tensor, faces_intense: torch.Tensor,
+                       cotangent_fn: Callable[[torch.Tensor, torch.Tensor], Tuple[torch.Tensor, torch.Tensor]],
+                       group=None, views_per_call: Optional[int] = None,
+                       first_view: int = 0) -> Sequence[Tuple[torch.Tensor, torch.Tensor, torch.Tensor]]:
+    """One optimisation step of the tet renderer on this rank's cameras (multiview_step for TetRenderer).
+
+    render            a TetRenderer-like callable (verts, faces, verts_color, faces_opacity, mv, proj, verts_depth,
+                      faces_intense, tets, face_tets, tet_faces, first_view=...) -> (color, depth, active)
+    scene_grads       PackedSceneGrads(verts, verts_color, faces_opacity) (6P + F floats; verts gets gradients when the
+                      renderer's vertex_grads is on) or PackedSceneGrads(None, verts_color, faces_opacity) (3P + F)
+    verts             the scene's vertex positions; when scene_grads has a verts slot, its own verts leaf
+    mv_mats ...       THIS RANK's slice: [B_local,4,4], [B_local,P], [B_local,F]
+    cotangent_fn      (color, depth) -> (dL_dcolor, dL_ddepth)
+    views_per_call    split the local views into calls of this many views (None = one call)
+    first_view        index of mv_mats[0] among all the job's cameras: shard_views(B, rank, world_size).start.  Call s
+                      renders with first_view + s, so jittered rays match one call over all views.
+
+    After the call every rank holds the view-summed gradients of the whole job in the leaves' .grad.  Returns the
+    list of (color, depth, active) outputs.
+    """
+    if len(scene_grads.leaves) == 3 and verts is not scene_grads.leaves[0]:
+        raise ValueError("tet_multiview_step: scene_grads holds vertex positions, so verts must be its verts leaf "
+                         "(scene_grads.leaves[0])")
+    verts_color, faces_opacity = scene_grads.leaves[-2:]
+    scene_grads.zero_()
+    B = mv_mats.shape[0]
+    step = views_per_call or max(B, 1)
+    outs = []
+    with scene_grads.direct():
+        for s in range(0, B, step):
+            e = min(B, s + step)
+            color, depth, active = render(verts, faces, verts_color, faces_opacity, mv_mats[s:e], proj_mats[s:e],
+                                          verts_depth[s:e], faces_intense[s:e], tets, face_tets, tet_faces,
+                                          first_view=first_view + s)
+            gc, gd = cotangent_fn(color, depth)
+            torch.autograd.backward([color, depth], [gc, gd])
+            outs.append((color.detach(), depth.detach(), active))
     scene_grads.all_reduce(group)
     return outs

@@ -297,6 +297,26 @@ int dmr_tet_forward_render(
     float* out_color, float* out_depth, float* out_active,
     dmr_stream_t stream);
 
+/* dmr_tet_forward_render for views first_view .. first_view + B - 1 of a    */
+/* larger job (a camera-sharded multi-view step): the jitter of pixel (x, y) */
+/* of call view b uses cuRAND subsequence (first_view + b)*H*W + y*W + x, so */
+/* a view gets the same rays whichever call renders it.  first_view = 0 is   */
+/* dmr_tet_forward_render; a negative first_view returns DMR_EINVAL before   */
+/* any CUDA call.  The backward entry points re-read the stored rays and     */
+/* take no first_view.                                                       */
+int dmr_tet_forward_render_views(
+    int B, int P, int F, int T, int W, int H, int R,
+    int ray_random_seed, int first_view,
+    const float* background,
+    const float* mv_mats, const float* proj_mats,
+    const float* inv_mv_mats, const float* inv_proj_mats,
+    const float* faces_intense,
+    const void* point_buffer, void* face_buffer,
+    const void* tet_records,
+    void* binning_buffer, void* image_buffer,
+    float* out_color, float* out_depth, float* out_active,
+    dmr_stream_t stream);
+
 /* ------------------------------------------------------------------------ */
 /* Tet renderer, backward.  Replaces CudaRenderer::Renderer::backward        */
 /* (renderer_impl.cu:413-498) -> TET_BACKWARD::renderCUDA                    */
