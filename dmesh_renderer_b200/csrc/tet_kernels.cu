@@ -535,6 +535,34 @@ __device__ __forceinline__ float tet_depth_at(const TetDepth& d, float t)
     const float pw = 1.0f / clamp_w(d.aw + t * d.bw);
     return (d.az + t * d.bz) * pw;
 }
+// The ~1e-7 above is relative to the clip coordinates' magnitude at the camera, not to w: both chains cancel the
+// camera's own offset (w = 0 at the eye), each leaving a different rounding error of about eps * |rw . ro| in w and
+// likewise in z, so they part by roughly eps * (m_z + |depth| m_w) / |w|.  Hit points close to the camera plane --
+// a camera inside the mesh -- make that visible in the depth image (measured 1.1e-5 on a Delaunay mesh seen from
+// inside, tests/test_gpu_tet_general_meshes.py).  The forward march takes the reference's chain for such steps:
+// tet_depth_scale gives max(m_z, m_w) of a view (uniform: ro is the eye), and a step whose |w| is below
+// (1 + |depth|) * scale / 16 -- where the two chains may part by more than ~16 * 4 eps ~ 4e-6 -- is evaluated again
+// by tet_depth_exact.  Cameras outside the mesh never need it (C3: |w| >= 2.2 against at most 2 * 8 / 16 = 1).
+__device__ __forceinline__ float tet_depth_scale(const float* __restrict__ mv, const float* __restrict__ pj,
+                                                 const float* __restrict__ inv_mv)
+{
+    float rz[4], rw[4];
+    tet_depth_rows(mv, pj, rz, rw);
+    float mz = fabsf(rz[3]), mw = fabsf(rw[3]);
+#pragma unroll
+    for (int k = 0; k < 3; k++) { mz += fabsf(rz[k] * inv_mv[12 + k]); mw += fabsf(rw[k] * inv_mv[12 + k]); }
+    return fmaxf(mz, mw) * (1.0f / 16.0f);
+}
+// forward.cu:628-631 as the reference evaluates it (second pass of the forward march only: the first pass hands such
+// rays over, as it does rays through irregular tets -- a call in its loop costs it spills, the march is register-bound)
+__device__ __forceinline__ float tet_depth_exact(const float* __restrict__ mv, const float* __restrict__ pj, float3 ro,
+                                              float3 rd, float t)
+{
+    const float3 pt = ro + (rd * t);
+    const float4 pn = xform44(xform43(pt, mv), pj);
+    const float pw = 1.0f / clamp_w(pn.w);
+    return pn.z * pw;
+}
 
 // Hit test of one side of an IRREGULAR tet (TetRec code 0xF: the side is not made of the tet's own four vertices --
 // inconsistent input tables, or two vertices of the tet coincide -- so the compact record cannot present its
@@ -640,6 +668,7 @@ __global__ void __launch_bounds__(MARCH_THREADS, MARCH_MIN_BLOCKS) tet_march_fwd
     float3 ro, rd;
     tet_pixel_ray(p, b, px, py, bpix, ro, rd);
     const TetDepth dep = tet_depth_setup(p.mv + 16 * b, p.proj + 16 * b, ro, rd);
+    const float dep_scale = tet_depth_scale(p.mv + 16 * b, p.proj + 16 * b, p.inv_mv + 16 * b);
 
     const int first_face = p.first_face[bpix], first_tet = p.first_tet[bpix];
     bool done = false;
@@ -686,7 +715,12 @@ __global__ void __launch_bounds__(MARCH_THREADS, MARCH_MIN_BLOCKS) tet_march_fwd
         col = col * intense;
         const float tmp_T = T_cur;
         C = C + tmp_T * opacity * col;
-        const float pd = tet_depth_at(dep, rt);
+        const float pw = dep.aw + rt * dep.bw;
+        float pd = (dep.az + rt * dep.bz) * (1.0f / clamp_w(pw));   // tet_depth_at
+        if (fabsf(pw) < (1.0f + fabsf(pd)) * dep_scale) {            // close to the camera plane
+            if (!IRR) { redo = true; break; }                         // the second pass re-marches the ray
+            pd = tet_depth_exact(p.mv + 16 * b, p.proj + 16 * b, ro, rd, rt);
+        }
         D += tmp_T * opacity * pd;
 
         prev_log_T = log_T;
