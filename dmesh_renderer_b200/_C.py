@@ -390,7 +390,7 @@ def grad_sink_for(verts, verts_color, faces_opacity, tet=False):
 def render_tris_backward(background, verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, inv_mv_mats,
                          inv_proj_mats, verts_depth, faces_intense, dL_dout_color, dL_dout_depth, R, pointBuffer,
                          faceBuffer, binningBuffer, imageBuffer, accumulate_into=None, deterministic=False,
-                         camera_grads=False, exact_vertex_grads=False):
+                         camera_grads=False, exact_vertex_grads=False, dL_dout_alpha=None, background_grad=False):
     """RasterizeTrianglesBackwardCUDA (render.cu:134-208).
     Returns (dL_dverts[P,3], dL_dvcolor[P,3], dL_dfopacity[F], dL_dvdepth[B,P], dL_dfintense[B,F]).
     `accumulate_into` (beyond the reference's 18 arguments): existing contiguous fp32 (dL_dverts, dL_dvcolor,
@@ -400,7 +400,11 @@ def render_tris_backward(background, verts, faces, verts_color, faces_opacity, m
     tensors passed here, through the rays; dmr_tri_backward_camera) as two more elements.
     `exact_vertex_grads`: dL_dverts is the exact derivative of the rendered image instead of the reference's formula
     (which differentiates t in place of the second barycentric v); the other gradients are unchanged
-    (dmr_tri_backward_exact)."""
+    (dmr_tri_backward_exact).
+    `dL_dout_alpha`: cotangent [B,1,H,W] of the alpha image (tri_alpha); it changes dL_dfopacity only
+    (dmr_tri_backward_alpha, in every mode above).
+    `background_grad`: also return dL_dbackground, float32 [3], as the last element (dmr_tri_background_grad; zero
+    when P == 0, where the images do not depend on the background)."""
     lib = _lib.load()
     B, P, F = mv_mats.size(0), verts.size(0), faces.size(0)
     H, W = dL_dout_color.size(2), dL_dout_color.size(3)
@@ -429,7 +433,20 @@ def render_tris_backward(background, verts, faces, verts_color, faces_opacity, m
                  _ptr(binningBuffer), _ptr(imageBuffer), _ptr(gc), _ptr(gd), gp[0], gp[1], gp[2], gp[3], gp[4])
             # scratch of the call (statistics per (view, face), per-vertex accumulators): the state buffers saved for
             # backward are only read.  The caching allocator reuses the block for later work on the same stream.
-            if exact_vertex_grads:
+            if dL_dout_alpha is not None:
+                # the workspace of the mode it modifies
+                det = int(bool(deterministic))
+                ga = _f32(dL_dout_alpha, "dL_dout_alpha")
+                if ga.numel() != B * H * W:
+                    _err("dL_dout_alpha must have dimensions (B, 1, H, W)")
+                nbytes = (lib.dmr_tri_backward_camera_bytes(B, P, F, W, H, det) if camera_grads else
+                          lib.dmr_tri_backward_deterministic_bytes(B, P, F) if det else
+                          lib.dmr_tri_backward_workspace_bytes(B, P, F))
+                ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+                cam = (gp[5], gp[6]) if camera_grads else (ctypes.c_void_p(0), ctypes.c_void_p(0))
+                _lib.check(lib.dmr_tri_backward_alpha(*a, det, int(bool(exact_vertex_grads)), *cam, _ptr(ga), _ptr(ws),
+                                                      ws.numel(), _stream()))
+            elif exact_vertex_grads:
                 # the workspace of the mode it modifies: the record layout is the same
                 det = int(bool(deterministic))
                 nbytes = (lib.dmr_tri_backward_camera_bytes(B, P, F, W, H, det) if camera_grads else
@@ -457,11 +474,48 @@ def render_tris_backward(background, verts, faces, verts_color, faces_opacity, m
             dL_dfopacity = flat[offs[2]:offs[2] + sizes[2]]
         dL_dvdepth = flat[offs[3]:offs[3] + sizes[3]].view(B, P)
         dL_dfintense = flat[offs[4]:offs[4] + sizes[4]].view(B, F)
+        out = (dL_dverts, dL_dvcolor, dL_dfopacity, dL_dvdepth, dL_dfintense)
         if camera_grads:
             # [B,16] column-major = [B,4,4] gradients of the (column-major, i.e. transposed) matrix tensors given here
-            return (dL_dverts, dL_dvcolor, dL_dfopacity, dL_dvdepth, dL_dfintense,
-                    flat[offs[5]:offs[5] + sizes[5]].view(B, 4, 4), flat[offs[6]:offs[6] + sizes[6]].view(B, 4, 4))
-    return dL_dverts, dL_dvcolor, dL_dfopacity, dL_dvdepth, dL_dfintense
+            out += (flat[offs[5]:offs[5] + sizes[5]].view(B, 4, 4), flat[offs[6]:offs[6] + sizes[6]].view(B, 4, 4))
+        if background_grad:
+            out += (_background_grad(lib.dmr_tri_background_grad_bytes, lib.dmr_tri_background_grad, B, W, H,
+                                     imageBuffer, dL_dout_color, dev),)
+    return out
+
+
+def _background_grad(nbytes_fn, grad_fn, B, W, H, imageBuffer, dL_dout_color, dev):
+    """dL/dbackground [3] fp32 of one renderer call (dmr_tri_background_grad / dmr_tet_background_grad); zero when
+    the call kept no image state (tri with P == 0: zero images that do not depend on the background)."""
+    out = torch.zeros(3, dtype=torch.float32, device=dev)
+    if imageBuffer is None or imageBuffer.numel() == 0 or B * W * H == 0:
+        return out
+    _require_cuda(dL_dout_color)
+    gc = _f32(dL_dout_color, "dL_dout_color")
+    ws = torch.empty(nbytes_fn(B), dtype=torch.uint8, device=dev)
+    _lib.check(grad_fn(B, W, H, _ptr(imageBuffer), _ptr(gc), _ptr(out), _ptr(ws), ws.numel(), _stream()))
+    return out
+
+
+def _alpha(fn, B, W, H, imageBuffer, dev):
+    out = torch.zeros((B, 1, H, W), dtype=torch.float32, device=dev)
+    if imageBuffer is not None and imageBuffer.numel() > 0 and out.numel() > 0:
+        _lib.check(fn(B, W, H, _ptr(imageBuffer), _ptr(out), _stream()))
+    return out
+
+
+def tri_alpha(imageBuffer, B, H, W, device):
+    """Alpha image [B,1,H,W] fp32 of a tri forward call: 1 - final_T (dmr_tri_alpha); zeros when P == 0 (the call's
+    image buffer is empty).  Enqueue after the forward call's last phase 2."""
+    with _on_device(device):
+        return _alpha(_lib.load().dmr_tri_alpha, B, W, H, imageBuffer, device)
+
+
+def tet_alpha(imageBuffer, B, H, W, device):
+    """Alpha image [B,1,H,W] fp32 of a tet forward call: 1 - expf(final_log_T) on active pixels, 0 on inactive ones
+    (dmr_tet_alpha)."""
+    with _on_device(device):
+        return _alpha(_lib.load().dmr_tet_alpha, B, W, H, imageBuffer, device)
 
 
 def tri_depth_chain(verts, mv_mats, proj_mats, dL_dvdepth, dL_dverts, dL_dmv=None, dL_dproj=None):
@@ -605,7 +659,7 @@ def render_tets_backward(background, verts, faces, verts_color, faces_opacity, m
                          inv_proj_mats, verts_depth, faces_intense, tets, face_tets, tet_faces, grad_color, grad_depth,
                          pointBuffer, faceBuffer, binningBuffer, imageBuffer, ray_random_seed=None, deterministic=False,
                          tet_records=None, camera_grads=False, vertex_grads=False, intensity_grads=False,
-                         accumulate_into=None):
+                         accumulate_into=None, dL_dout_alpha=None, background_grad=False):
     """RenderFTetsBackwardCUDA (render.cu:338-412).
     Returns (dL_dverts_color[P,3], dL_dfaces_opacity[F]).  `ray_random_seed` is an
     optional trailing argument beyond the reference's 20: the autograd wrapper passes
@@ -623,7 +677,10 @@ def render_tets_backward(background, verts, faces, verts_color, faces_opacity, m
     `accumulate_into`: (dL_dverts_color, dL_dfaces_opacity, dL_dverts), existing contiguous fp32 tensors of shapes
     [P,3], [F], [P,3] that the gradients are ADDED to (and that are returned) instead of fresh zero tensors, in every
     mode.  dL_dverts may be None (a fresh tensor when vertex_grads is set); it is written only when vertex_grads is
-    set.  The camera and intensity gradients are always fresh tensors."""
+    set.  The camera and intensity gradients are always fresh tensors.
+    `dL_dout_alpha`: cotangent [B,1,H,W] of the alpha image (tet_alpha); it changes dL_dfaces_opacity only
+    (dmr_tet_backward_alpha, in every mode above).
+    `background_grad`: also return dL_dbackground, float32 [3], as the last element (dmr_tet_background_grad)."""
     lib = _lib.load()
     B, P, F, T = mv_mats.size(0), verts.size(0), faces.size(0), tets.size(0)
     H, W = grad_color.size(2), grad_color.size(3)
@@ -664,7 +721,25 @@ def render_tets_backward(background, verts, faces, verts_color, faces_opacity, m
             a = (B, P, F, T, W, H, int(ray_random_seed), _ptr(bg), _ptr(mv), _ptr(pj), _ptr(imv), _ptr(ipj), _ptr(fint),
                  _ptr(pointBuffer), _ptr(faceBuffer), _ptr(tet_rec), _ptr(imageBuffer), _ptr(gc), _ptr(gd),
                  _ptr(dL_dverts_color), _ptr(dL_dfaces_opacity))
-            if intensity_grads:
+            if dL_dout_alpha is not None:
+                det = int(bool(deterministic))
+                ga = _f32(dL_dout_alpha, "dL_dout_alpha")
+                if ga.numel() != B * H * W:
+                    _err("dL_dout_alpha must have dimensions (batch_size, 1, H, W)")
+                cm, vx = int(bool(camera_grads)), int(bool(vertex_grads))
+                # the workspace of the mode it modifies
+                nbytes = (lib.dmr_tet_backward_intensity_bytes(B, P, F, W, H, det, cm, vx) if intensity_grads else
+                          lib.dmr_tet_backward_vertex_bytes(B, P, F, W, H, det, cm) if vertex_grads else
+                          lib.dmr_tet_backward_camera_bytes(B, P, F, W, H, det) if camera_grads else
+                          lib.dmr_tet_backward_deterministic_bytes(P, F) if det else
+                          lib.dmr_tet_backward_workspace_bytes(P))
+                ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+                null = ctypes.c_void_p(0)
+                c = (_ptr(cam[0]), _ptr(cam[1])) if camera_grads else (null, null)
+                dv = _ptr(dL_dverts) if vertex_grads else null
+                fi = _ptr(dL_dfint) if intensity_grads else null
+                _lib.check(lib.dmr_tet_backward_alpha(*a, det, *c, dv, fi, _ptr(ga), _ptr(ws), ws.numel(), _stream()))
+            elif intensity_grads:
                 det = int(bool(deterministic))
                 ws = torch.empty(lib.dmr_tet_backward_intensity_bytes(B, P, F, W, H, det, int(bool(camera_grads)),
                                                                       int(bool(vertex_grads))),
@@ -698,4 +773,8 @@ def render_tets_backward(background, verts, faces, verts_color, faces_opacity, m
         out += (dL_dverts,)
     if intensity_grads:
         out += (dL_dfint,)
+    if background_grad:
+        with _on_device(dev):
+            out += (_background_grad(lib.dmr_tet_background_grad_bytes, lib.dmr_tet_background_grad, B, W, H, imageBuffer,
+                                     grad_color, dev),)
     return out

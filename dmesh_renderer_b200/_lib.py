@@ -36,6 +36,10 @@ SIGNATURES = {
     "dmr_tri_backward_camera_bytes": (c_size_t, [c_int] * 6),
     "dmr_tri_backward_camera": (c_int, [c_int] * 6 + [c_void_p] * 14 + [c_int] + [c_void_p] * 2 + [c_void_p, c_size_t] + [c_void_p]),
     "dmr_tri_backward_exact": (c_int, [c_int] * 6 + [c_void_p] * 14 + [c_int] + [c_void_p] * 2 + [c_void_p, c_size_t] + [c_void_p]),
+    "dmr_tri_backward_alpha": (c_int, [c_int] * 6 + [c_void_p] * 14 + [c_int] * 2 + [c_void_p] * 3 + [c_void_p, c_size_t] + [c_void_p]),
+    "dmr_tri_alpha": (c_int, [c_int] * 3 + [c_void_p] * 2 + [c_void_p]),
+    "dmr_tri_background_grad_bytes": (c_size_t, [c_int]),
+    "dmr_tri_background_grad": (c_int, [c_int] * 3 + [c_void_p] * 4 + [c_size_t] + [c_void_p]),
     "dmr_tri_depth_chain_camera_bytes": (c_size_t, [c_int] * 2),
     "dmr_tri_depth_chain_camera": (c_int, [c_int, c_int] + [c_void_p] * 8 + [c_size_t, c_void_p]),
     "dmr_tet_records_bytes": (c_size_t, [c_int]),
@@ -53,6 +57,10 @@ SIGNATURES = {
     "dmr_tet_backward_vertex": (c_int, [c_int] * 7 + [c_void_p] * 14 + [c_int] + [c_void_p] * 3 + [c_void_p, c_size_t] + [c_void_p]),
     "dmr_tet_backward_intensity_bytes": (c_size_t, [c_int] * 8),
     "dmr_tet_backward_intensity": (c_int, [c_int] * 7 + [c_void_p] * 14 + [c_int] + [c_void_p] * 4 + [c_void_p, c_size_t] + [c_void_p]),
+    "dmr_tet_backward_alpha": (c_int, [c_int] * 7 + [c_void_p] * 14 + [c_int] + [c_void_p] * 5 + [c_void_p, c_size_t] + [c_void_p]),
+    "dmr_tet_alpha": (c_int, [c_int] * 3 + [c_void_p] * 2 + [c_void_p]),
+    "dmr_tet_background_grad_bytes": (c_size_t, [c_int]),
+    "dmr_tet_background_grad": (c_int, [c_int] * 3 + [c_void_p] * 4 + [c_size_t] + [c_void_p]),
     "dmr_debug_view": (c_int, [c_int] * 8 + [c_size_t, c_void_p, ctypes.POINTER(c_void_p), ctypes.POINTER(c_size_t)]),
     "dmr_nvls_allreduce_sum_f32_fused": (c_int, [c_void_p, c_size_t, c_int, c_int, c_void_p, c_void_p, ctypes.c_uint, c_void_p]),
     "dmr_camera_inverses": (c_int, [c_int, c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_int64, c_void_p, ctypes.c_int64,

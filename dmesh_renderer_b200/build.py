@@ -16,7 +16,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libdmesh_b200.so")
 OBJ = os.path.join(HERE, "csrc", "_obj")
 
-SOURCES = ["capi.cu", "capi_tet.cu", "preprocess.cu", "binning.cu", "radix_sort.cu", "tri_render.cu", "tet_kernels.cu", "collective.cu", "inverse.cu"]
+SOURCES = ["capi.cu", "capi_tet.cu", "preprocess.cu", "binning.cu", "radix_sort.cu", "tri_render.cu", "tet_kernels.cu", "collective.cu", "inverse.cu", "image.cu"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

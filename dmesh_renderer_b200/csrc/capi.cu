@@ -37,7 +37,8 @@ static const char* const g_stage_names[ST_COUNT] = {
     "tri_camera_finish", "depth_chain_camera", "depth_chain_camera_finish", "tet_march_backward_camera", "tet_camera_finish",
     "tet_march_backward_vertex", "tet_march_backward_camera_vertex", "tet_vertex_finish",
     "tet_march_backward_intensity", "tet_march_backward_camera_intensity", "tet_march_backward_vertex_intensity",
-    "tet_march_backward_camera_vertex_intensity", "tet_intensity_finish" };
+    "tet_march_backward_camera_vertex_intensity", "tet_intensity_finish", "tri_alpha", "tri_render_backward_alpha",
+    "tri_background_grad", "tet_alpha", "tet_march_backward_alpha", "tet_background_grad" };
 struct Prof {
     bool on = false, created = false;
     cudaEvent_t ev[ST_COUNT][2];
@@ -260,7 +261,7 @@ static int tri_backward_impl(int B, int P, int F, int W, int H, int R, const flo
                              const float* dL_ddepth, float* dL_dverts, float* dL_dvcolor, float* dL_dfopacity,
                              float* dL_dvdepth, float* dL_dfintense, void* workspace, size_t workspace_bytes,
                              bool deterministic, dmr_stream_t stream_, float* dL_dmv = nullptr, float* dL_dproj = nullptr,
-                             bool exact = false)
+                             bool exact = false, const float* dL_dalpha = nullptr)
 {
     const bool cam = dL_dmv != nullptr;
     cudaStream_t stream = (cudaStream_t)stream_;
@@ -313,7 +314,7 @@ static int tri_backward_impl(int B, int P, int F, int W, int H, int R, const flo
         p.det_vdepth = at<long long>(det_workspace, DL.vdepth);
         p.det_fopa = at<long long>(det_workspace, DL.fopa);
         DMR_CUDA(cudaMemsetAsync(det_workspace, 0, DL.total, stream));
-        int rc = tri_render_backward_deterministic(p, stream, cam_tiles, exact);
+        int rc = tri_render_backward_deterministic(p, stream, cam_tiles, exact, dL_dalpha);
         if (rc || !cam) return rc;
         return tri_camera_finish(B, W, H, cam_tiles, inv_mv_mats, inv_proj_mats, dL_dmv, dL_dproj, stream);
     }
@@ -330,7 +331,7 @@ static int tri_backward_impl(int B, int P, int F, int W, int H, int R, const flo
     const bool use_vacc = 3 * (size_t)F >= 4 * (size_t)P;
     p.grad_vacc = use_vacc ? at<float4>(workspace, WL.grad_vacc) : nullptr;
     DMR_CUDA(cudaMemsetAsync(workspace, 0, use_vacc ? WL.total - 256 : WL.stats_end, stream));
-    int rc = tri_render_backward(p, stream, cam_tiles, exact);
+    int rc = tri_render_backward(p, stream, cam_tiles, exact, dL_dalpha);
     if (rc || !cam) return rc;
     return tri_camera_finish(B, W, H, cam_tiles, inv_mv_mats, inv_proj_mats, dL_dmv, dL_dproj, stream);
 }
@@ -402,6 +403,50 @@ int dmr_tri_backward_exact(int B, int P, int F, int W, int H, int R, const float
                              binning_buffer, image_buffer, dL_dcolor, dL_ddepth, dL_dverts, dL_dvcolor, dL_dfopacity,
                              dL_dvdepth, dL_dfintense, workspace, workspace_bytes, deterministic != 0, stream, dL_dmv,
                              dL_dproj, true);
+}
+
+int dmr_tri_backward_alpha(int B, int P, int F, int W, int H, int R, const float* background, const float* inv_mv_mats,
+                           const float* inv_proj_mats, const void* point_buffer, const void* face_buffer,
+                           const void* binning_buffer, const void* image_buffer, const float* dL_dcolor,
+                           const float* dL_ddepth, float* dL_dverts, float* dL_dvcolor, float* dL_dfopacity,
+                           float* dL_dvdepth, float* dL_dfintense, int deterministic, int exact, float* dL_dmv,
+                           float* dL_dproj, const float* dL_dalpha, void* workspace, size_t workspace_bytes,
+                           dmr_stream_t stream)
+{
+    if ((dL_dmv == nullptr) != (dL_dproj == nullptr)) { set_error("pass both dL_dmv and dL_dproj, or neither"); return DMR_EINVAL; }
+    if (B > 0 && !dL_dalpha) { set_error("null pointer: dL_dalpha"); return DMR_EINVAL; }
+    return tri_backward_impl(B, P, F, W, H, R, background, inv_mv_mats, inv_proj_mats, point_buffer, face_buffer,
+                             binning_buffer, image_buffer, dL_dcolor, dL_ddepth, dL_dverts, dL_dvcolor, dL_dfopacity,
+                             dL_dvdepth, dL_dfintense, workspace, workspace_bytes, deterministic != 0, stream, dL_dmv,
+                             dL_dproj, exact != 0, dL_dalpha);
+}
+
+int dmr_tri_alpha(int B, int W, int H, const void* image_buffer, float* out_alpha, dmr_stream_t stream)
+{
+    if (!sizes_ok(B, 0, 0, W, H)) return DMR_ETOOLARGE;
+    if (B == 0) return DMR_OK;
+    if (!image_buffer || !out_alpha) { set_error("null pointer"); return DMR_EINVAL; }
+    const TriImageLayout IL = TriImageLayout::make(B, W, H);
+    return image_alpha(false, B, W, H, at<float>(image_buffer, IL.final_T), nullptr, out_alpha, (cudaStream_t)stream);
+}
+
+size_t dmr_tri_background_grad_bytes(int B) { return B < 0 ? 0 : image_bg_grad_bytes(B); }
+
+int dmr_tri_background_grad(int B, int W, int H, const void* image_buffer, const float* dL_dcolor, float* dL_dbg,
+                            void* workspace, size_t workspace_bytes, dmr_stream_t stream)
+{
+    if (!sizes_ok(B, 0, 0, W, H)) return DMR_ETOOLARGE;
+    if (!dL_dbg) { set_error("null pointer: dL_dbg"); return DMR_EINVAL; }
+    if (B > 0 && (!image_buffer || !dL_dcolor)) { set_error("null pointer"); return DMR_EINVAL; }
+    const size_t need = image_bg_grad_bytes(B);
+    if (!workspace || workspace_bytes < need) {
+        set_error("background gradient needs a workspace of %zu bytes (dmr_tri_background_grad_bytes)", need);
+        return DMR_EINVAL;
+    }
+    if (B == 0) { DMR_CUDA(cudaMemsetAsync(dL_dbg, 0, 3 * sizeof(float), (cudaStream_t)stream)); return DMR_OK; }
+    const TriImageLayout IL = TriImageLayout::make(B, W, H);
+    return image_bg_grad(false, B, W, H, at<float>(image_buffer, IL.final_T), nullptr, dL_dcolor, dL_dbg, workspace,
+                         (cudaStream_t)stream);
 }
 
 size_t dmr_tri_depth_chain_camera_bytes(int B, int P)

@@ -207,7 +207,8 @@ static int tet_backward_impl(int B, int P, int F, int T, int W, int H, int ray_r
                              const float* dL_dcolor, const float* dL_ddepth, float* dL_dverts_color,
                              float* dL_dfaces_opacity, void* workspace, size_t workspace_bytes, bool deterministic,
                              dmr_stream_t stream_, float* dL_dmv = nullptr, float* dL_dproj = nullptr,
-                             float* dL_dverts = nullptr, float* dL_dfaces_intense = nullptr)
+                             float* dL_dverts = nullptr, float* dL_dfaces_intense = nullptr,
+                             const float* dL_dalpha = nullptr)
 {
     const bool cam = dL_dmv != nullptr;
     const bool vert = dL_dverts != nullptr;
@@ -270,7 +271,7 @@ static int tet_backward_impl(int B, int P, int F, int T, int W, int H, int ray_r
         vg.det_pos = at<long long>(det_workspace, DL.pos);
         ig.det_fint = at<long long>(det_workspace, align_up(vert ? DL.total_pos : DL.total, 256));
         DMR_CUDA(cudaMemsetAsync(det_workspace, 0, tet_bwd_scratch_bytes(P, F, true, vert, fint_n), stream));
-        int rc = tet_march_backward_deterministic(p, stream, cam_rec, vert ? &vg : nullptr, fint ? &ig : nullptr);
+        int rc = tet_march_backward_deterministic(p, stream, cam_rec, vert ? &vg : nullptr, fint ? &ig : nullptr, dL_dalpha);
         if (rc || !cam) return rc;
         return tet_camera_finish(p, cam_rec, dL_dmv, dL_dproj, stream);
     }
@@ -282,7 +283,7 @@ static int tet_backward_impl(int B, int P, int F, int T, int W, int H, int ray_r
     p.grad_vacc = static_cast<float4*>(workspace);
     vg.grad_pacc = p.grad_vacc + P;
     DMR_CUDA(cudaMemsetAsync(p.grad_vacc, 0, sizeof(float4) * (size_t)P * (vert ? 2 : 1), stream));
-    int rc = tet_march_backward(p, stream, cam_rec, vert ? &vg : nullptr, fint ? &ig : nullptr);
+    int rc = tet_march_backward(p, stream, cam_rec, vert ? &vg : nullptr, fint ? &ig : nullptr, dL_dalpha);
     if (rc || !cam) return rc;
     return tet_camera_finish(p, cam_rec, dL_dmv, dL_dproj, stream);
 }
@@ -402,6 +403,55 @@ int dmr_tet_backward_intensity(int B, int P, int F, int T, int W, int H, int ray
                              inv_proj_mats, faces_intense, point_buffer, face_buffer, tet_records, image_buffer, dL_dcolor,
                              dL_ddepth, dL_dverts_color, dL_dfaces_opacity, workspace, workspace_bytes, deterministic != 0,
                              stream, dL_dmv, dL_dproj, dL_dverts, dL_dfaces_intense);
+}
+
+int dmr_tet_backward_alpha(int B, int P, int F, int T, int W, int H, int ray_random_seed, const float* background,
+                           const float* mv_mats, const float* proj_mats, const float* inv_mv_mats,
+                           const float* inv_proj_mats, const float* faces_intense, const void* point_buffer,
+                           const void* face_buffer, const void* tet_records, const void* image_buffer,
+                           const float* dL_dcolor, const float* dL_ddepth, float* dL_dverts_color,
+                           float* dL_dfaces_opacity, int deterministic, float* dL_dmv, float* dL_dproj,
+                           float* dL_dverts, float* dL_dfaces_intense, const float* dL_dalpha, void* workspace,
+                           size_t workspace_bytes, dmr_stream_t stream)
+{
+    if ((dL_dmv == nullptr) != (dL_dproj == nullptr)) {
+        set_error("dL_dmv and dL_dproj: pass both (camera gradients) or neither");
+        return DMR_EINVAL;
+    }
+    if (B > 0 && !dL_dalpha) { set_error("null pointer: dL_dalpha"); return DMR_EINVAL; }
+    return tet_backward_impl(B, P, F, T, W, H, ray_random_seed, background, mv_mats, proj_mats, inv_mv_mats,
+                             inv_proj_mats, faces_intense, point_buffer, face_buffer, tet_records, image_buffer, dL_dcolor,
+                             dL_ddepth, dL_dverts_color, dL_dfaces_opacity, workspace, workspace_bytes, deterministic != 0,
+                             stream, dL_dmv, dL_dproj, dL_dverts, dL_dfaces_intense, dL_dalpha);
+}
+
+int dmr_tet_alpha(int B, int W, int H, const void* image_buffer, float* out_alpha, dmr_stream_t stream)
+{
+    if (!tet_sizes_ok(B, 0, 0, 0, W, H)) return DMR_ETOOLARGE;
+    if (B == 0) return DMR_OK;
+    if (!image_buffer || !out_alpha) { set_error("null pointer"); return DMR_EINVAL; }
+    const TetImageLayout IL = TetImageLayout::make(B, W, H);
+    return image_alpha(true, B, W, H, at<float>(image_buffer, IL.final_log_T), at<uint8_t>(image_buffer, IL.active),
+                       out_alpha, (cudaStream_t)stream);
+}
+
+size_t dmr_tet_background_grad_bytes(int B) { return B < 0 ? 0 : image_bg_grad_bytes(B); }
+
+int dmr_tet_background_grad(int B, int W, int H, const void* image_buffer, const float* dL_dcolor, float* dL_dbg,
+                            void* workspace, size_t workspace_bytes, dmr_stream_t stream)
+{
+    if (!tet_sizes_ok(B, 0, 0, 0, W, H)) return DMR_ETOOLARGE;
+    if (!dL_dbg) { set_error("null pointer: dL_dbg"); return DMR_EINVAL; }
+    if (B > 0 && (!image_buffer || !dL_dcolor)) { set_error("null pointer"); return DMR_EINVAL; }
+    const size_t need = image_bg_grad_bytes(B);
+    if (!workspace || workspace_bytes < need) {
+        set_error("background gradient needs a workspace of %zu bytes (dmr_tet_background_grad_bytes)", need);
+        return DMR_EINVAL;
+    }
+    if (B == 0) { DMR_CUDA(cudaMemsetAsync(dL_dbg, 0, 3 * sizeof(float), (cudaStream_t)stream)); return DMR_OK; }
+    const TetImageLayout IL = TetImageLayout::make(B, W, H);
+    return image_bg_grad(true, B, W, H, at<float>(image_buffer, IL.final_log_T), at<uint8_t>(image_buffer, IL.active),
+                         dL_dcolor, dL_dbg, workspace, (cudaStream_t)stream);
 }
 
 int dmr_debug_set_tet_first_split(int split)

@@ -43,7 +43,8 @@ enum Stage {
     ST_RANGES, ST_TRI_FWD, ST_TRI_BWD, ST_TRI_BWD_FINISH, ST_TET_RECORDS, ST_TET_JITTER, ST_TET_FIRST, ST_TET_FWD, ST_TET_BWD, ST_TET_BWD_FINISH,
     ST_TRI_BWD_CAM, ST_TRI_CAM_FINISH, ST_DEPTH_CAM, ST_DEPTH_CAM_FINISH, ST_TET_BWD_CAM, ST_TET_CAM_FINISH,
     ST_TET_BWD_VERT, ST_TET_BWD_CAM_VERT, ST_TET_VERT_FINISH,
-    ST_TET_BWD_INT, ST_TET_BWD_CAM_INT, ST_TET_BWD_VERT_INT, ST_TET_BWD_CAM_VERT_INT, ST_TET_INT_FINISH, ST_COUNT
+    ST_TET_BWD_INT, ST_TET_BWD_CAM_INT, ST_TET_BWD_VERT_INT, ST_TET_BWD_CAM_VERT_INT, ST_TET_INT_FINISH,
+    ST_TRI_ALPHA, ST_TRI_BWD_ALPHA, ST_TRI_BG_GRAD, ST_TET_ALPHA, ST_TET_BWD_ALPHA, ST_TET_BG_GRAD, ST_COUNT
 };
 void count_launch(int n);
 void prof_begin(int stage, cudaStream_t s, bool count = true);   // count: also counts one kernel launch
@@ -373,5 +374,13 @@ int bin_instances(int B, int F, int W, int H, size_t R, const void* face_buffer,
                   void* binning_buffer, uint2* ranges /* [B*tiles] */, cudaStream_t stream);
 
 uint32_t higher_msb(uint32_t n);
+
+// image.cu: alpha image and background gradient of either renderer from its image state.  t: tri final_T, tet
+// final_log_T (both [B,H,W]); active: tet only ([B,H,W] bytes), nullptr for tri.  image_bg_grad writes dL_dbg[3] and
+// needs image_bg_grad_bytes(B) bytes of workspace.
+int image_alpha(bool tet, int B, int W, int H, const float* t, const uint8_t* active, float* alpha, cudaStream_t stream);
+size_t image_bg_grad_bytes(int B);
+int image_bg_grad(bool tet, int B, int W, int H, const float* t, const uint8_t* active, const float* dL_dcolor, float* dL_dbg,
+                  void* workspace, cudaStream_t stream);
 
 }  // namespace dmr

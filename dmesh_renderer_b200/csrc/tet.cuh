@@ -222,10 +222,12 @@ int tet_march_forward(const TetParams& p, cudaStream_t stream);
 // CTA) there
 // vert != nullptr: the vertex-position kernels, which also add dL/dverts to vert->dL_dverts
 // fint != nullptr: the face-intensity kernels, which also add dL/dfaces_intense to fint->dL_dfint
+// dL_dalpha != nullptr: the alpha-cotangent instantiations of the same mode ([B,H,W] cotangent of the alpha image)
 int tet_march_backward(const TetParams& p, cudaStream_t stream, float* cam_rec = nullptr, const TetVertGrad* vert = nullptr,
-                       const TetIntGrad* fint = nullptr);
+                       const TetIntGrad* fint = nullptr, const float* dL_dalpha = nullptr);
 int tet_march_backward_deterministic(const TetParams& p, cudaStream_t stream, float* cam_rec = nullptr,
-                                     const TetVertGrad* vert = nullptr, const TetIntGrad* fint = nullptr);
+                                     const TetVertGrad* vert = nullptr, const TetIntGrad* fint = nullptr,
+                                     const float* dL_dalpha = nullptr);
 // records of a view -> += dL_dmv[B,16], dL_dproj[B,16]
 int tet_camera_finish(const TetParams& p, const float* cam_rec, float* dL_dmv, float* dL_dproj, cudaStream_t stream);
 

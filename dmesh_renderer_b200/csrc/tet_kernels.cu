@@ -17,6 +17,7 @@
 #include "tet.cuh"
 #include "det.cuh"
 #include <curand_kernel.h>
+#include <type_traits>
 
 namespace dmr {
 
@@ -1034,8 +1035,11 @@ __device__ __forceinline__ void tet_int_step(const TetParams& p, const TetIntGra
 // VERT: also scatter the vertex-position terms of every walked step (tet_vert_step, sharing the triangle and the
 // sensitivities with CAM); `cam` is then a TetVertAcc.
 // INT: also add the face-intensity term of every walked step (tet_int_step); `cam` is then a TetIntAcc<...>.
-template <bool DET, bool CAM, bool VERT = false, bool INT = false, class Acc = TetCamAcc>
-__device__ __forceinline__ void tet_march_bwd_body(const TetParams& p, Acc& cam)
+// ALPHA: the image also has an alpha cotangent dL_dalpha [B,H,W] (alpha = 1 - expf(final_log_T) on active pixels, the
+// factor the forward pass multiplies the background by; DESIGN.md 3.4): it enters where the background term does, as
+// bd_dot - dL_dalpha, so tet_bwd_face is unchanged.
+template <bool DET, bool CAM, bool VERT = false, bool INT = false, class Acc = TetCamAcc, bool ALPHA = false>
+__device__ __forceinline__ void tet_march_bwd_body(const TetParams& p, Acc& cam, const float* __restrict__ dL_dalpha = nullptr)
 {
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int b = blockIdx.z;
@@ -1072,6 +1076,7 @@ __device__ __forceinline__ void tet_march_bwd_body(const TetParams& p, Acc& cam)
     // backward.cu:324-329
     float bg_dot = 0; bg_dot += p.bg[0] * g0; bg_dot += p.bg[1] * g1; bg_dot += p.bg[2] * g2;
     float bd_dot = 0; bd_dot += 1.0 * gd;
+    if constexpr (ALPHA) bd_dot -= dL_dalpha[bpix];
 
     TetBwdState st;
     st.det_sv = 0.0f;
@@ -1262,12 +1267,13 @@ __global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_vert_int_det_kern
 static_assert(MARCH_THREADS == 64 && MARCH_ROWS == 8, "tet_cam_records (tet.cuh) counts 8 x 8-pixel march CTAs");
 static_assert(DMR_TET_CAM_REC == 32, "one record slot per lane");
 // VERT: Acc = TetVertAcc with its vg set by the caller.  INT: Acc = TetIntAcc<...> with its ig set by the caller.
-template <bool DET, bool VERT = false, bool INT = false, class Acc = TetCamAcc>
-__device__ __forceinline__ void tet_march_bwd_cam(const TetParams& p, float* __restrict__ cam_rec, Acc& a)
+template <bool DET, bool VERT = false, bool INT = false, class Acc = TetCamAcc, bool ALPHA = false>
+__device__ __forceinline__ void tet_march_bwd_cam(const TetParams& p, float* __restrict__ cam_rec, Acc& a,
+                                                  const float* __restrict__ dL_dalpha = nullptr)
 {
     a.g_ro = f3(0, 0, 0); a.g_rd = f3(0, 0, 0);
     a.g_az = 0.0f; a.g_bz = 0.0f; a.g_aw = 0.0f; a.g_bw = 0.0f;
-    tet_march_bwd_body<DET, true, VERT, INT>(p, a);
+    tet_march_bwd_body<DET, true, VERT, INT, Acc, ALPHA>(p, a, dL_dalpha);
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int b = blockIdx.z;
@@ -1389,6 +1395,44 @@ __global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_cam_vert_int_det_
     a.vg = vg;
     a.ig = ig;
     tet_march_bwd_cam<true, true, true>(p, cam_rec, a);
+}
+
+// Alpha-cotangent instantiations: the sixteen kernels above (default / deterministic x camera x vertex x intensity)
+// plus dL/dalpha, which travels as an argument of its own so that TetParams stays as it is.  The accumulator type is
+// the one the kernel each stands in for uses; -Xptxas -v of all of them in DESIGN.md 3.4.
+template <bool VERT, bool INT>
+using TetAlphaAcc = std::conditional_t<INT, TetIntAcc<std::conditional_t<VERT, TetVertAcc, TetCamAcc>>,
+                                       std::conditional_t<VERT, TetVertAcc, TetCamAcc>>;
+template <bool DET, bool CAM, bool VERT, bool INT>
+__global__ void __launch_bounds__(MARCH_THREADS) tet_march_bwd_alpha_kernel(TetParams p, float* cam_rec, TetVertGrad vg,
+                                                                            TetIntGrad ig, const float* __restrict__ dL_dalpha)
+{
+    griddep_wait();
+    TetAlphaAcc<VERT, INT> a;
+    if constexpr (VERT) a.vg = vg;
+    if constexpr (INT) a.ig = ig;
+    if constexpr (CAM) tet_march_bwd_cam<DET, VERT, INT, TetAlphaAcc<VERT, INT>, true>(p, cam_rec, a, dL_dalpha);
+    else tet_march_bwd_body<DET, false, VERT, INT, TetAlphaAcc<VERT, INT>, true>(p, a, dL_dalpha);
+}
+
+template <bool DET>
+static cudaError_t launch_tet_bwd_alpha(const TetParams& p, cudaStream_t stream, dim3 grid, float* cam_rec,
+                                        const TetVertGrad* vert, const TetIntGrad* fint, const float* dL_dalpha)
+{
+    const TetVertGrad vg = vert ? *vert : TetVertGrad{};
+    const TetIntGrad ig = fint ? *fint : TetIntGrad{};
+    void (*k)(TetParams, float*, TetVertGrad, TetIntGrad, const float*);
+    switch ((cam_rec ? 1 : 0) | (vert ? 2 : 0) | (fint ? 4 : 0)) {
+        case 0: k = tet_march_bwd_alpha_kernel<DET, false, false, false>; break;
+        case 1: k = tet_march_bwd_alpha_kernel<DET, true, false, false>; break;
+        case 2: k = tet_march_bwd_alpha_kernel<DET, false, true, false>; break;
+        case 3: k = tet_march_bwd_alpha_kernel<DET, true, true, false>; break;
+        case 4: k = tet_march_bwd_alpha_kernel<DET, false, false, true>; break;
+        case 5: k = tet_march_bwd_alpha_kernel<DET, true, false, true>; break;
+        case 6: k = tet_march_bwd_alpha_kernel<DET, false, true, true>; break;
+        default: k = tet_march_bwd_alpha_kernel<DET, true, true, true>; break;
+    }
+    return dmr_launch(k, grid, dim3(MARCH_THREADS), 0, stream, p, cam_rec, vg, ig, dL_dalpha);
 }
 
 // One CTA per view: the view's records (tet_march_bwd_cam) are summed in a fixed order -- thread t owns component
@@ -1566,18 +1610,25 @@ static int tet_int_stage(const float* cam_rec, const TetVertGrad* vert)
 }
 
 int tet_march_backward_deterministic(const TetParams& p, cudaStream_t stream, float* cam_rec, const TetVertGrad* vert,
-                                     const TetIntGrad* fint)
+                                     const TetIntGrad* fint, const float* dL_dalpha)
 {
     dim3 grid((p.W + 7) / 8, (p.H + MARCH_ROWS - 1) / MARCH_ROWS, p.B);
     const size_t HW = (size_t)p.W * p.H;
     {
-        ProfScope prof(fint ? tet_int_stage(cam_rec, vert)
-                            : vert ? (cam_rec ? ST_TET_BWD_CAM_VERT : ST_TET_BWD_VERT) : (cam_rec ? ST_TET_BWD_CAM : ST_TET_BWD),
+        ProfScope prof(dL_dalpha ? ST_TET_BWD_ALPHA
+                       : fint    ? tet_int_stage(cam_rec, vert)
+                       : vert    ? (cam_rec ? ST_TET_BWD_CAM_VERT : ST_TET_BWD_VERT) : (cam_rec ? ST_TET_BWD_CAM : ST_TET_BWD),
                        stream);
         count_launch(1);   // two kernels under one scope
         int rc = det_gmax(p.dL_dcolor, 3 * p.B * HW, p.dL_ddepth, p.B * HW, const_cast<uint32_t*>(p.det_gmax), stream);
         if (rc) return rc;
-        if (fint) {
+        if (dL_dalpha) {
+            // the fixed-point scale covers max |dL_dalpha| too: a second maximum into the same word (order-independent)
+            count_launch(1);
+            if ((rc = det_gmax(dL_dalpha, p.B * HW, nullptr, 0, const_cast<uint32_t*>(p.det_gmax), stream))) return rc;
+            DMR_CUDA(launch_tet_bwd_alpha<true>(p, stream, grid, cam_rec, vert, fint, dL_dalpha));
+            DMR_LAUNCH_CHECK("tet_march_bwd_alpha_det_kernel");
+        } else if (fint) {
             if ((rc = tet_march_backward_intensity(p, stream, grid, cam_rec, vert, *fint, true))) return rc;
         } else if (vert && cam_rec) {
             DMR_CUDA(dmr_launch(tet_march_bwd_cam_vert_det_kernel, dim3(grid), dim3(MARCH_THREADS), 0, stream, p, cam_rec, *vert));
@@ -1615,10 +1666,14 @@ int tet_march_backward_deterministic(const TetParams& p, cudaStream_t stream, fl
 }
 
 int tet_march_backward(const TetParams& p, cudaStream_t stream, float* cam_rec, const TetVertGrad* vert,
-                       const TetIntGrad* fint)
+                       const TetIntGrad* fint, const float* dL_dalpha)
 {
     dim3 grid((p.W + 7) / 8, (p.H + MARCH_ROWS - 1) / MARCH_ROWS, p.B);
-    if (fint) {
+    if (dL_dalpha) {
+        ProfScope prof(ST_TET_BWD_ALPHA, stream);
+        DMR_CUDA(launch_tet_bwd_alpha<false>(p, stream, grid, cam_rec, vert, fint, dL_dalpha));
+        DMR_LAUNCH_CHECK("tet_march_bwd_alpha_kernel");
+    } else if (fint) {
         ProfScope prof(tet_int_stage(cam_rec, vert), stream);
         if (int rc = tet_march_backward_intensity(p, stream, grid, cam_rec, vert, *fint, false)) return rc;
     } else if (vert && cam_rec) {

@@ -66,9 +66,11 @@ int tri_preprocess_faces(int B, int P, int F, int W, int H, const int* faces, co
 int tri_render_forward(const TriRenderParams& p, cudaStream_t stream);
 // cam_tiles != nullptr: the camera-gradient kernels, which also store one 24-float record per (view, tile) there.
 // exact: the exact vertex-position instantiations (same launches, same workspace).
-int tri_render_backward(const TriRenderParams& p, cudaStream_t stream, float* cam_tiles = nullptr, bool exact = false);
+// dL_dalpha != nullptr: the alpha-cotangent instantiations ([B,H,W] cotangent of alpha = 1 - final_T)
+int tri_render_backward(const TriRenderParams& p, cudaStream_t stream, float* cam_tiles = nullptr, bool exact = false,
+                        const float* dL_dalpha = nullptr);
 int tri_render_backward_deterministic(const TriRenderParams& p, cudaStream_t stream, float* cam_tiles = nullptr,
-                                      bool exact = false);
+                                      bool exact = false, const float* dL_dalpha = nullptr);
 // per-tile camera records of a view -> += dL_dmv[B,16], dL_dproj[B,16]
 int tri_camera_finish(int B, int W, int H, const float* cam_tiles, const float* inv_mv, const float* inv_proj, float* dL_dmv,
                       float* dL_dproj, cudaStream_t stream);

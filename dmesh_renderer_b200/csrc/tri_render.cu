@@ -431,8 +431,14 @@ constexpr int DMR_TRI_BWD_MINB = 4;
 // forward pass uses instead of the reference's t: S24 takes dL_dv * v in place of dL_dv * t, and S3 becomes the
 // vector S3v = sum dL_dv / D * rd, whose y and z go to the pad slots 21 and 22 of the record (logical 6 keeps x).
 // Record size, reduction and stores are unchanged; tri_grad_finish_body<.., EXACT> applies the matching formula.
-template <bool DET, bool CAM, bool EXACT = false>
-__device__ __forceinline__ void tri_render_bwd_body(const TriRenderParams& p, float* __restrict__ cam_tiles)
+// Alpha cotangent (ALPHA = true, opt-in; DESIGN.md 3.3).  alpha = 1 - T_final, and T_final is the factor the forward
+// pass multiplies the background by, so dL/dalpha enters exactly where the background term does: the per-pixel
+// constant bg . dL_dC + dL_dD becomes bg . dL_dC + dL_dD - dL_dalpha.  One more load per pixel, before the walk.
+// The cotangent arrives as a parameter pack, empty for every other instantiation: those keep exactly their two
+// parameters (an unused defaulted pointer changed ptxas's register assignment in the camera kernels).
+template <bool DET, bool CAM, bool EXACT = false, bool ALPHA = false, class... AlphaPtr>
+__device__ __forceinline__ void tri_render_bwd_body(const TriRenderParams& p, float* __restrict__ cam_tiles,
+                                                    AlphaPtr... dL_dalpha)
 {
     __shared__ uint4 s_rec[RB * 9];      // staged records; two vertex-id slots (unused here: tri_grad_finish_kernel reads the
                                          // global record) carry the face id and 1 / (1 - opacity) of the instance
@@ -476,6 +482,11 @@ __device__ __forceinline__ void tri_render_bwd_body(const TriRenderParams& p, fl
     // backward.cu:293-298
     float bg_dot = 0; bg_dot += bg0 * dLc0; bg_dot += bg1 * dLc1; bg_dot += bg2 * dLc2;
     float bd_dot = 0; bd_dot += 1.0 * dLd;
+    if constexpr (ALPHA) {
+        static_assert(sizeof...(AlphaPtr) == 1, "ALPHA takes the cotangent pointer");
+        const float* const dla = (dL_dalpha, ...);
+        if (inside) bd_dot -= dla[bpix];
+    }
     const float bgk = -T_final * (bg_dot + bd_dot), bgk1 = -prev_T_final * (bg_dot + bd_dot);
 
     float acc0 = 0, acc1 = 0, acc2 = 0, accd = 0;
@@ -816,6 +827,29 @@ __global__ void __launch_bounds__(256, DMR_TRI_BWD_CAM_MINB) tri_render_bwd_exac
     tri_render_bwd_body<true, true, true>(p, cam_tiles);
 }
 
+// Alpha-cotangent instantiations: the eight kernels above (default / deterministic x camera x exact) plus dL/dalpha,
+// which travels as an argument of its own so that TriRenderParams stays as it is.  Resident CTAs per SM as the kernel
+// each one stands in for; -Xptxas -v of all of them in DESIGN.md 3.3.
+template <bool DET, bool CAM, bool EXACT>
+__global__ void __launch_bounds__(256, CAM ? DMR_TRI_BWD_CAM_MINB : EXACT ? DMR_TRI_BWD_EXACT_MINB : DMR_TRI_BWD_MINB)
+tri_render_bwd_alpha_kernel(TriRenderParams p, float* cam_tiles, const float* __restrict__ dL_dalpha)
+{
+    griddep_wait();   // programmatic dependent launch: see dmr_launch (common.cuh)
+    tri_render_bwd_body<DET, CAM, EXACT, true>(p, cam_tiles, dL_dalpha);
+}
+
+template <bool DET>
+static cudaError_t launch_tri_bwd_alpha(dim3 grid, cudaStream_t stream, const TriRenderParams& p, float* cam_tiles, bool exact,
+                                        const float* dL_dalpha)
+{
+    if (cam_tiles)
+        return exact ? dmr_launch(tri_render_bwd_alpha_kernel<DET, true, true>, grid, dim3(256), 0, stream, p, cam_tiles, dL_dalpha)
+                     : dmr_launch(tri_render_bwd_alpha_kernel<DET, true, false>, grid, dim3(256), 0, stream, p, cam_tiles, dL_dalpha);
+    float* const none = nullptr;
+    return exact ? dmr_launch(tri_render_bwd_alpha_kernel<DET, false, true>, grid, dim3(256), 0, stream, p, none, dL_dalpha)
+                 : dmr_launch(tri_render_bwd_alpha_kernel<DET, false, false>, grid, dim3(256), 0, stream, p, none, dL_dalpha);
+}
+
 // One CTA per view: the view's per-tile camera records (tri_render_bwd_cam_kernel) are summed in a fixed order -- a
 // thread owns one component (240 = 10 x 24 threads, coalesced reads of the flat record array), then the ten partial
 // sums of a component are added in thread order -- and chained through the inverses: with N = A^-1,
@@ -1074,11 +1108,15 @@ int tri_render_forward(const TriRenderParams& p, cudaStream_t stream)
     return 0;
 }
 
-int tri_render_backward(const TriRenderParams& p, cudaStream_t stream, float* cam_tiles, bool exact)
+int tri_render_backward(const TriRenderParams& p, cudaStream_t stream, float* cam_tiles, bool exact, const float* dL_dalpha)
 {
     if (p.B <= 0 || p.W <= 0 || p.H <= 0) return 0;
     dim3 grid((p.W + DMR_TILE - 1) / DMR_TILE, (p.H + DMR_TILE - 1) / DMR_TILE, p.B);
-    if (cam_tiles) {
+    if (dL_dalpha) {
+        ProfScope prof(ST_TRI_BWD_ALPHA, stream);
+        DMR_CUDA(launch_tri_bwd_alpha<false>(grid, stream, p, cam_tiles, exact, dL_dalpha));
+        DMR_LAUNCH_CHECK("tri_render_bwd_alpha_kernel");
+    } else if (cam_tiles) {
         ProfScope prof(ST_TRI_BWD_CAM, stream);
         DMR_CUDA(dmr_launch(exact ? tri_render_bwd_exact_cam_kernel : tri_render_bwd_cam_kernel, dim3(grid), dim3(256), 0,
                             stream, p, cam_tiles));
@@ -1110,17 +1148,24 @@ int det_gmax(const float* a, size_t na, const float* b, size_t nb, uint32_t* gma
     return 0;
 }
 
-int tri_render_backward_deterministic(const TriRenderParams& p, cudaStream_t stream, float* cam_tiles, bool exact)
+int tri_render_backward_deterministic(const TriRenderParams& p, cudaStream_t stream, float* cam_tiles, bool exact,
+                                      const float* dL_dalpha)
 {
     if (p.B <= 0 || p.W <= 0 || p.H <= 0) return 0;
     dim3 grid((p.W + DMR_TILE - 1) / DMR_TILE, (p.H + DMR_TILE - 1) / DMR_TILE, p.B);
     const size_t HW = (size_t)p.W * p.H;
     {
-        ProfScope prof(cam_tiles ? ST_TRI_BWD_CAM : ST_TRI_BWD, stream);
+        ProfScope prof(dL_dalpha ? ST_TRI_BWD_ALPHA : cam_tiles ? ST_TRI_BWD_CAM : ST_TRI_BWD, stream);
         count_launch(1);   // two kernels under one scope
         int rc = det_gmax(p.dL_dcolor, 3 * p.B * HW, p.dL_ddepth, p.B * HW, const_cast<uint32_t*>(p.det_gmax), stream);
         if (rc) return rc;
-        if (cam_tiles) {
+        if (dL_dalpha) {
+            // the fixed-point scale covers max |dL_dalpha| too: a second maximum into the same word (order-independent)
+            count_launch(1);
+            if ((rc = det_gmax(dL_dalpha, p.B * HW, nullptr, 0, const_cast<uint32_t*>(p.det_gmax), stream))) return rc;
+            DMR_CUDA(launch_tri_bwd_alpha<true>(grid, stream, p, cam_tiles, exact, dL_dalpha));
+            DMR_LAUNCH_CHECK("tri_render_bwd_alpha_det_kernel");
+        } else if (cam_tiles) {
             DMR_CUDA(dmr_launch(exact ? tri_render_bwd_exact_cam_det_kernel : tri_render_bwd_cam_det_kernel, dim3(grid),
                                 dim3(256), 0, stream, p, cam_tiles));
             DMR_LAUNCH_CHECK("tri_render_bwd_cam_det_kernel");

@@ -67,6 +67,13 @@ class PackedSceneGrads:
     3P + F floats; `leaves` then holds the two tensors, and only TetRenderer calls
     can use it as a sink (see direct()).
 
+    bg (optional): the background colour, a float32 tensor of 3 elements that the
+    renderers' settings carry.  Its gradient slot is appended after faces_opacity
+    (and before any padding), so the one all-reduce sums it too and the ranks'
+    backgrounds stay equal; the renderers' backward passes reach it through
+    ordinary autograd accumulation into the bound .grad view.  `leaves` does not
+    include it.
+
     On a CUDA job with world_size > 1 the buffer is allocated in SYMMETRIC memory
     (torch.distributed._symmetric_memory: peer-mapped on every rank + an NVLS multicast
     address) and the all-reduce is the hand-written in-switch reduction kernel of
@@ -75,13 +82,16 @@ class PackedSceneGrads:
     every rank of `group` must create its PackedSceneGrads at the same point."""
 
     def __init__(self, verts: torch.Tensor, verts_color: torch.Tensor, faces_opacity: torch.Tensor, group=None,
-                 use_nvls: Optional[bool] = None):
+                 use_nvls: Optional[bool] = None, bg: Optional[torch.Tensor] = None):
         self.leaves = [t for t in (verts, verts_color, faces_opacity) if t is not None]
         if len(self.leaves) < 2 or verts_color is None or faces_opacity is None:
             raise ValueError("PackedSceneGrads needs verts_color and faces_opacity")
+        if bg is not None and (bg.dtype != torch.float32 or bg.numel() != 3 or not bg.is_leaf):
+            raise ValueError("PackedSceneGrads: bg must be a float32 leaf tensor of 3 elements")
+        self.bg = bg
         self.group = group
         device = verts_color.device
-        n = sum(t.numel() for t in self.leaves)
+        n = sum(t.numel() for t in self._slots())
         self._nvls = None
         # which collective all_reduce() runs and, for the fallback, why: "nvls" | "nccl: <reason>" | "none: <reason>"
         self.collective = "nccl: use_nvls=False" if use_nvls is False else "none: single process"
@@ -92,19 +102,22 @@ class PackedSceneGrads:
             full = torch.zeros(n, dtype=torch.float32, device=device)
         self._full = full              # padded to a multiple of 4 * world_size floats in the NVLS case
         self.flat = full[:n]
-        for t in self.leaves:
+        for t in self._slots():
             if not t.requires_grad:
                 t.requires_grad_(True)
         self.bind()
+
+    def _slots(self):
+        return self.leaves + ([self.bg] if self.bg is not None else [])
 
     def bind(self):
         """(Re-)attach the leaves' .grad tensors to the packed buffer.  Anything that REPLACES .grad --
         optimizer.zero_grad() with its default set_to_none=True, `leaf.grad = None` -- silently disconnects a leaf:
         autograd would then accumulate into a fresh tensor and all_reduce() would exchange a stale buffer.  zero_(),
         direct() and all_reduce() therefore call this first; a gradient found in a foreign tensor is moved into the
-        packed buffer so that nothing is lost.  Returns the number of leaves that had to be re-attached."""
+        packed buffer so that nothing is lost.  Returns the number of leaves (bg included) that had to be re-attached."""
         o, fixed = 0, 0
-        for t in self.leaves:
+        for t in self._slots():
             view = self.flat[o:o + t.numel()].view_as(t)
             g = t.grad
             if g is None or g.data_ptr() != view.data_ptr() or g.shape != view.shape or g.dtype != view.dtype:
@@ -211,11 +224,13 @@ def multiview_step(render: Callable, scene_grads: PackedSceneGrads, faces: torch
     render            a TriRenderer-like callable (verts, faces, verts_color, faces_opacity,
                       mv, proj, verts_depth, faces_intense) -> (color, depth)
     mv_mats ...       THIS RANK's slice: [B_local,4,4], [B_local,P], [B_local,F]
-    cotangent_fn      (color, depth) -> (dL_dcolor, dL_ddepth)   (e.g. gradient of an image loss)
+    cotangent_fn      (color, depth) -> (dL_dcolor, dL_ddepth)   (e.g. gradient of an image loss); when the
+                      renderer also returns an alpha image (TriRenderer(..., return_alpha=True)):
+                      (color, depth, alpha) -> (dL_dcolor, dL_ddepth, dL_dalpha)
     views_per_call    split the local views into calls of this many views (None = one call)
 
     After the call every rank holds the view-summed gradients of the whole job in
-    scene_grads.leaves[i].grad.  Returns the list of (color, depth) outputs.
+    scene_grads.leaves[i].grad (and scene_grads.bg.grad).  Returns the list of (color, depth[, alpha]) outputs.
     """
     verts, verts_color, faces_opacity = scene_grads.leaves
     scene_grads.zero_()
@@ -225,11 +240,10 @@ def multiview_step(render: Callable, scene_grads: PackedSceneGrads, faces: torch
     with scene_grads.direct():
         for s in range(0, B, step):
             e = min(B, s + step)
-            color, depth = render(verts, faces, verts_color, faces_opacity, mv_mats[s:e], proj_mats[s:e],
-                                  verts_depth[s:e], faces_intense[s:e])
-            gc, gd = cotangent_fn(color, depth)
-            torch.autograd.backward([color, depth], [gc, gd])
-            outs.append((color.detach(), depth.detach()))
+            images = render(verts, faces, verts_color, faces_opacity, mv_mats[s:e], proj_mats[s:e],
+                            verts_depth[s:e], faces_intense[s:e])        # (color, depth) or (color, depth, alpha)
+            torch.autograd.backward(list(images), list(cotangent_fn(*images)))
+            outs.append(tuple(x.detach() for x in images))
     scene_grads.all_reduce(group)
     return outs
 
@@ -248,13 +262,14 @@ def tet_multiview_step(render: Callable, scene_grads: PackedSceneGrads, verts: t
                       renderer's vertex_grads is on) or PackedSceneGrads(None, verts_color, faces_opacity) (3P + F)
     verts             the scene's vertex positions; when scene_grads has a verts slot, its own verts leaf
     mv_mats ...       THIS RANK's slice: [B_local,4,4], [B_local,P], [B_local,F]
-    cotangent_fn      (color, depth) -> (dL_dcolor, dL_ddepth)
+    cotangent_fn      (color, depth) -> (dL_dcolor, dL_ddepth); when the renderer also returns an alpha image
+                      (TetRenderer(..., return_alpha=True)): (color, depth, alpha) -> (dL_dcolor, dL_ddepth, dL_dalpha)
     views_per_call    split the local views into calls of this many views (None = one call)
     first_view        index of mv_mats[0] among all the job's cameras: shard_views(B, rank, world_size).start.  Call s
                       renders with first_view + s, so jittered rays match one call over all views.
 
-    After the call every rank holds the view-summed gradients of the whole job in the leaves' .grad.  Returns the
-    list of (color, depth, active) outputs.
+    After the call every rank holds the view-summed gradients of the whole job in the leaves' .grad (and
+    scene_grads.bg.grad).  Returns the list of (color, depth, active[, alpha]) outputs.
     """
     if len(scene_grads.leaves) == 3 and verts is not scene_grads.leaves[0]:
         raise ValueError("tet_multiview_step: scene_grads holds vertex positions, so verts must be its verts leaf "
@@ -267,11 +282,10 @@ def tet_multiview_step(render: Callable, scene_grads: PackedSceneGrads, verts: t
     with scene_grads.direct():
         for s in range(0, B, step):
             e = min(B, s + step)
-            color, depth, active = render(verts, faces, verts_color, faces_opacity, mv_mats[s:e], proj_mats[s:e],
-                                          verts_depth[s:e], faces_intense[s:e], tets, face_tets, tet_faces,
-                                          first_view=first_view + s)
-            gc, gd = cotangent_fn(color, depth)
-            torch.autograd.backward([color, depth], [gc, gd])
-            outs.append((color.detach(), depth.detach(), active))
+            out = render(verts, faces, verts_color, faces_opacity, mv_mats[s:e], proj_mats[s:e], verts_depth[s:e],
+                         faces_intense[s:e], tets, face_tets, tet_faces, first_view=first_view + s)
+            images = out[:2] + out[3:]                           # (color, depth) or (color, depth, alpha)
+            torch.autograd.backward(list(images), list(cotangent_fn(*images)))
+            outs.append((out[0].detach(), out[1].detach(), out[2]) + tuple(x.detach() for x in out[3:]))
     scene_grads.all_reduce(group)
     return outs

@@ -245,6 +245,42 @@ int dmr_tri_backward_exact(
     void* workspace, size_t workspace_bytes,
     dmr_stream_t stream);
 
+/* Alpha (coverage) cotangent of the tri renderer (no reference counterpart).  The backward pass of               */
+/* dmr_tri_backward_exact (exact != 0) or of the reference formula (exact == 0), with the same arguments, plus      */
+/* dL_dalpha [B,H,W], the cotangent of alpha = 1 - final_T (dmr_tri_alpha).  alpha depends on the opacities only, so */
+/* only dL_dfopacity changes: dL_dalpha enters where the background term does (the per-pixel constant              */
+/* bg . dL_dC + dL_dD becomes bg . dL_dC + dL_dD - dL_dalpha).  In deterministic mode the fixed-point scale covers   */
+/* max |dL_dalpha| as well.  `workspace`: the byte count of the mode it modifies, as for dmr_tri_backward_exact.     */
+/* dL_dalpha must not be NULL for B > 0.                                                                            */
+int dmr_tri_backward_alpha(
+    int B, int P, int F, int W, int H, int R,
+    const float* background,
+    const float* inv_mv_mats, const float* inv_proj_mats,
+    const void* point_buffer, const void* face_buffer,
+    const void* binning_buffer, const void* image_buffer,
+    const float* dL_dcolor, const float* dL_ddepth,
+    float* dL_dverts, float* dL_dvcolor, float* dL_dfopacity, float* dL_dvdepth, float* dL_dfintense,
+    int deterministic, int exact,
+    float* dL_dmv,               /* [B,16] or NULL */
+    float* dL_dproj,             /* [B,16] or NULL */
+    const float* dL_dalpha,      /* [B,H,W] */
+    void* workspace, size_t workspace_bytes,
+    dmr_stream_t stream);
+
+/* Alpha image of a tri forward call (no reference counterpart): out_alpha[B,H,W] = 1 - final_T, the transmittance */
+/* the forward pass multiplied the background by (the T < 1e-4 termination included, so a fully covered pixel gets  */
+/* alpha just below 1).  Reads the image buffer of dmr_tri_forward_render; call it after the last phase 2.  With    */
+/* R == 0 the image buffer holds final_T = 1 and alpha is 0.                                                         */
+int dmr_tri_alpha(int B, int W, int H, const void* image_buffer, float* out_alpha, dmr_stream_t stream);
+
+/* Gradient with respect to the background colour (no reference counterpart): dL_dbg[c] = sum over views and pixels */
+/* of final_T * dL_dcolor[b,c,:,:], WRITTEN (not added) to dL_dbg[3].  A fixed-order reduction without float        */
+/* atomics (reproducible).  Reads only the image buffer and dL_dcolor, so it applies when R == 0 too.  `workspace`:  */
+/* dmr_tri_background_grad_bytes(B) bytes of device scratch.                                                         */
+size_t dmr_tri_background_grad_bytes(int B);
+int dmr_tri_background_grad(int B, int W, int H, const void* image_buffer, const float* dL_dcolor, float* dL_dbg,
+                            void* workspace, size_t workspace_bytes, dmr_stream_t stream);
+
 /* dmr_tri_depth_chain plus the camera part of the fused vertex depth (no reference counterpart):                 */
 /* dL_dmv[b] / dL_dproj[b] += sum_p dL_dvdepth[b,p] * d ndc_z[b,p] / d(mv_mats[b], proj_mats[b]) (no derivative   */
 /* through a clamped clip w).  Reduced in a fixed order without float atomics.  `workspace`:                      */
@@ -452,6 +488,46 @@ int dmr_tet_backward_intensity(
     float* dL_dfaces_intense,    /* [B,F] */
     void* workspace, size_t workspace_bytes,
     dmr_stream_t stream);
+
+/* Alpha (coverage) cotangent of the tet renderer (no reference counterpart).  The backward pass of                 */
+/* dmr_tet_backward_intensity, with the same arguments, except that dL_dfaces_intense may be NULL too (no intensity  */
+/* gradients), plus dL_dalpha [B,H,W], the cotangent of alpha (dmr_tet_alpha).  Only dL_dfaces_opacity changes: the */
+/* cotangent enters where the background term does, summed over the same walked steps as every other gradient.      */
+/* In deterministic mode the fixed-point scale covers max |dL_dalpha| as well.  `workspace`: the byte count of the   */
+/* mode it modifies (dmr_tet_backward_workspace_bytes, _deterministic_bytes, _camera_bytes, _vertex_bytes or         */
+/* _intensity_bytes).  dL_dalpha must not be NULL for B > 0.                                                         */
+int dmr_tet_backward_alpha(
+    int B, int P, int F, int T, int W, int H,
+    int ray_random_seed,
+    const float* background,
+    const float* mv_mats, const float* proj_mats,
+    const float* inv_mv_mats, const float* inv_proj_mats,
+    const float* faces_intense,
+    const void* point_buffer, const void* face_buffer,
+    const void* tet_records,
+    const void* image_buffer,
+    const float* dL_dcolor, const float* dL_ddepth,
+    float* dL_dverts_color, float* dL_dfaces_opacity,
+    int deterministic,
+    float* dL_dmv,               /* [B,16] or NULL */
+    float* dL_dproj,             /* [B,16] or NULL */
+    float* dL_dverts,            /* [P,3] or NULL */
+    float* dL_dfaces_intense,    /* [B,F] or NULL */
+    const float* dL_dalpha,      /* [B,H,W] */
+    void* workspace, size_t workspace_bytes,
+    dmr_stream_t stream);
+
+/* Alpha image of a tet forward call (no reference counterpart): out_alpha[B,H,W] = 1 - expf(final_log_T) on active */
+/* pixels (bit-identical to 1 - the transmittance the forward pass multiplied the background by) and 0 on inactive  */
+/* ones (numerical failure, shown as the background).  Reads the image buffer of dmr_tet_forward_render(_views).    */
+int dmr_tet_alpha(int B, int W, int H, const void* image_buffer, float* out_alpha, dmr_stream_t stream);
+
+/* Gradient with respect to the background colour (no reference counterpart): dL_dbg[c] = sum over views and pixels */
+/* of w * dL_dcolor[b,c,:,:], w = expf(final_log_T) on active pixels and 1 on inactive ones, WRITTEN to dL_dbg[3].   */
+/* Fixed-order reduction without float atomics.  `workspace`: dmr_tet_background_grad_bytes(B) bytes.               */
+size_t dmr_tet_background_grad_bytes(int B);
+int dmr_tet_background_grad(int B, int W, int H, const void* image_buffer, const float* dL_dcolor, float* dL_dbg,
+                            void* workspace, size_t workspace_bytes, dmr_stream_t stream);
 
 /* ------------------------------------------------------------------------ */
 /* Read-only views into the state buffers for the bit-exact parity checks    */
