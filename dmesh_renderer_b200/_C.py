@@ -282,7 +282,7 @@ def tri_forward_begin(background, verts, faces, verts_color, faces_opacity, mv_m
     return st
 
 
-def tri_forward_finish(st, inv_mv_mats, inv_proj_mats, inverses=None, speculative=False):
+def tri_forward_finish(st, inv_mv_mats, inv_proj_mats, inverses=None, speculative=False, face_weights=False):
     """Phase 2 of a forward call started by tri_forward_begin: the one host sync (R), binning buffer, sort, render.
     `inverses`: the _Inverses object the matrices came from, whose deferred singularity check runs after the sync.
     `speculative`: launch phase 2 BEFORE num_rendered has reached the host, on a binning buffer sized from the
@@ -290,7 +290,10 @@ def tri_forward_finish(st, inv_mv_mats, inv_proj_mats, inverses=None, speculativ
     goes straight from the scan into the binning kernels while the host is still waiting for the 4-byte read-back
     (the reference drains the pipeline there, rasterizer_impl.cu:287-299).  If the scene grew past the buffer, the
     kernels emit nothing and phase 2 is simply run again with an exact buffer.  In this mode element 0 of the result is
-    the CAPACITY the binning buffer was laid out for (>= num_rendered); pass it to render_tris_backward as `R`."""
+    the CAPACITY the binning buffer was laid out for (>= num_rendered); pass it to render_tris_backward as `R`.
+    `face_weights`: phase 2 also computes the per-(view, face) visibility statistics
+    (dmr_tri_forward_render_face_weights), appended to the result as face_weights [B,F] fp32 and face_hits [B,F]
+    int32; zeros when P == 0.  Every phase 2 zeroes its accumulators, so a re-run phase 2 counts once."""
     for t, n in ((inv_mv_mats, "inv_mv_mats"), (inv_proj_mats, "inv_proj_mats")):
         if t.dim() != 3 or t.size(1) != 4 or t.size(2) != 4:
             _err("%s must have dimensions (B, 4, 4)" % n)
@@ -305,9 +308,12 @@ def tri_forward_finish(st, inv_mv_mats, inv_proj_mats, inverses=None, speculativ
             if inverses is not None:
                 torch.cuda.current_stream().synchronize()
                 inverses.check()
-            return (0, z((B, NUM_CHANNELS, H, W), dtype=torch.float32, device=dev),
-                    z((B, 1, H, W), dtype=torch.float32, device=dev),
-                    torch.empty(0, **u8), torch.empty(0, **u8), torch.empty(0, **u8), torch.empty(0, **u8))
+            out = (0, z((B, NUM_CHANNELS, H, W), dtype=torch.float32, device=dev),
+                   z((B, 1, H, W), dtype=torch.float32, device=dev),
+                   torch.empty(0, **u8), torch.empty(0, **u8), torch.empty(0, **u8), torch.empty(0, **u8))
+            if face_weights:
+                out += (z((B, F), dtype=torch.float32, device=dev), z((B, F), dtype=torch.int32, device=dev))
+            return out
         _require_cuda(inv_mv_mats, inv_proj_mats)
         imv, ipj = _f32(inv_mv_mats, "inv_mv_mats"), _f32(inv_proj_mats, "inv_proj_mats")
         key = ("tri", B, P, F, 0, W, H)
@@ -316,29 +322,39 @@ def tri_forward_finish(st, inv_mv_mats, inv_proj_mats, inverses=None, speculativ
         out_color, out_depth = st.outs
         # everything that does not depend on R is prepared before the wait
         a = (_ptr(st.bg), _ptr(imv), _ptr(ipj), _ptr(point_buf), _ptr(face_buf))
-        b2 = (_ptr(img_buf), _ptr(out_color), _ptr(out_depth), _stream())
+        b2 = (_ptr(img_buf), _ptr(out_color), _ptr(out_depth))
+        render = lib.dmr_tri_forward_render
+        if face_weights:
+            fw = torch.empty((B, F), dtype=torch.float32, device=dev)
+            fh = torch.empty((B, F), dtype=torch.int32, device=dev)
+            fws = torch.empty(lib.dmr_tri_face_weights_bytes(B, F), **u8)
+            b2 += (_ptr(fw), _ptr(fh), _ptr(fws), fws.numel())
+            render = lib.dmr_tri_forward_render_face_weights
+        b2 += (_stream(),)
         try:
             if speculative and spec is not None:
                 # phase 2 goes out first; the wait below overlaps with it
-                _lib.check(lib.dmr_tri_forward_render(B, P, F, W, H, cap, *a, _ptr(spec), *b2))
+                _lib.check(render(B, P, F, W, H, cap, *a, _ptr(spec), *b2))
                 R = _read_R(lib, st.pinned, key)
                 bin_buf = spec
                 if R > cap:     # the scene outgrew the speculative buffer: nothing was emitted, run phase 2 again
                     cap = R
                     bin_buf = torch.empty(lib.dmr_binning_bytes(cap), **u8)
-                    _lib.check(lib.dmr_tri_forward_render(B, P, F, W, H, cap, *a, _ptr(bin_buf), *b2))
+                    _lib.check(render(B, P, F, W, H, cap, *a, _ptr(bin_buf), *b2))
                 R = cap         # the layout count of the binning buffer (see the docstring)
             else:
                 # (Measured and rejected: one native call that waits for R and launches phase 2 without returning to
                 # Python in between -- 1163 vs 1159 views/s at C2: the bubble is the D2H + launch latency, not the
                 # interpreter.)
                 R, bin_buf = _wait_R(lib, st.pinned, key, spec, u8)   # the one sync: R sizes the binning buffer
-                _lib.check(lib.dmr_tri_forward_render(B, P, F, W, H, R, *a, _ptr(bin_buf), *b2))
+                _lib.check(render(B, P, F, W, H, R, *a, _ptr(bin_buf), *b2))
         finally:
             _Pinned.release(st.pinned)
             st.pinned = None
         if inverses is not None:
             inverses.check()
+    if face_weights:
+        return R, out_color, out_depth, point_buf, face_buf, bin_buf, img_buf, fw, fh
     return R, out_color, out_depth, point_buf, face_buf, bin_buf, img_buf
 
 
@@ -516,6 +532,27 @@ def tet_alpha(imageBuffer, B, H, W, device):
     (dmr_tet_alpha)."""
     with _on_device(device):
         return _alpha(_lib.load().dmr_tet_alpha, B, W, H, imageBuffer, device)
+
+
+def tet_face_weights(B, P, F, T, H, W, ray_random_seed, inv_mv_mats, inv_proj_mats, pointBuffer, faceBuffer, imageBuffer,
+                     tet_records=None):
+    """Per-(view, face) visibility statistics of a tet forward call (dmr_tet_face_weights): face_weights [B,F] fp32
+    (sum of the blending weights expf(log_T) * opacity of the face's composited steps on active pixels) and face_hits
+    [B,F] int32 (their number).  Pass the forward call's sizes, seed, inverse matrices and state buffers; the
+    adjacency records default to the face buffer's attribute (render_tets)."""
+    dev = faceBuffer.device
+    with _on_device(dev):
+        fw = torch.zeros((B, F), dtype=torch.float32, device=dev)
+        fh = torch.zeros((B, F), dtype=torch.int32, device=dev)
+        if B * F > 0 and T > 0:
+            lib = _lib.load()
+            tet_rec = tet_records if tet_records is not None else faceBuffer.tet_records
+            imv, ipj = _f32(inv_mv_mats, "inv_mv_mats"), _f32(inv_proj_mats, "inv_proj_mats")
+            ws = torch.empty(lib.dmr_tet_face_weights_bytes(B, F), dtype=torch.uint8, device=dev)
+            _lib.check(lib.dmr_tet_face_weights(B, P, F, T, int(W), int(H), int(ray_random_seed), _ptr(imv), _ptr(ipj),
+                                                _ptr(pointBuffer), _ptr(faceBuffer), _ptr(tet_rec), _ptr(imageBuffer),
+                                                _ptr(fw), _ptr(fh), _ptr(ws), ws.numel(), _stream()))
+    return fw, fh
 
 
 def tri_depth_chain(verts, mv_mats, proj_mats, dL_dvdepth, dL_dverts, dL_dmv=None, dL_dproj=None):

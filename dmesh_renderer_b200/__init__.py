@@ -57,14 +57,16 @@ def set_exact_vertex_grads(flag: bool) -> bool:
 
 
 def render_tri(verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, verts_depth, faces_intense,
-               render_settings: TriRenderSettings, deterministic=None, exact_vertex_grads=None, return_alpha=False):
+               render_settings: TriRenderSettings, deterministic=None, exact_vertex_grads=None, return_alpha=False,
+               return_face_weights=False):
     """reference __init__.py:18-43 (`deterministic`: see set_deterministic; `exact_vertex_grads`: see
-    set_exact_vertex_grads; `return_alpha`: see TriRenderer.forward).  render_settings.bg is passed to autograd as
-    an input of its own: with bg.requires_grad set it gets its gradient."""
+    set_exact_vertex_grads; `return_alpha`, `return_face_weights`: see TriRenderer.forward).  render_settings.bg is
+    passed to autograd as an input of its own: with bg.requires_grad set it gets its gradient."""
     det = _deterministic_default if deterministic is None else bool(deterministic)
     exact = _exact_vertex_grads_default if exact_vertex_grads is None else bool(exact_vertex_grads)
     return _RenderTri.apply(verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, verts_depth, faces_intense,
-                            render_settings, det, exact, bool(return_alpha), render_settings.bg)
+                            render_settings, det, exact, bool(return_alpha), render_settings.bg,
+                            bool(return_face_weights))
 
 
 def _bg_for_render(bg):
@@ -78,7 +80,8 @@ class _RenderTri(th.autograd.Function):
 
     @staticmethod
     def forward(ctx, verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, verts_depth, faces_intense,
-                render_settings, deterministic=False, exact_vertex_grads=False, return_alpha=False, bg=None):
+                render_settings, deterministic=False, exact_vertex_grads=False, return_alpha=False, bg=None,
+                return_face_weights=False):
         ctx.deterministic = deterministic
         ctx.exact_vertex_grads = exact_vertex_grads
         ctx.return_alpha = return_alpha
@@ -97,8 +100,9 @@ class _RenderTri(th.autograd.Function):
                                            render_settings.image_width)
             # speculative: phase 2 is enqueued before num_rendered reaches the host; `num_rendered` is then the count
             # the binning buffer was laid out for (>= the real one), which is what backward needs
-            num_rendered, color, depth, pointBuffer, faceBuffer, binningBuffer, imgBuffer = \
-                _C.tri_forward_finish(pending, inv_mv_mats, inv_proj_mats, inv, speculative=True)
+            out = _C.tri_forward_finish(pending, inv_mv_mats, inv_proj_mats, inv, speculative=True,
+                                        face_weights=return_face_weights)
+            num_rendered, color, depth, pointBuffer, faceBuffer, binningBuffer, imgBuffer = out[:7]
         except Exception as ex:
             print("\nAn error occured in forward.")
             print(ex)
@@ -110,14 +114,20 @@ class _RenderTri(th.autograd.Function):
         ctx.grad_sink = _C.grad_sink_for(verts, verts_color, faces_opacity)   # multiview.PackedSceneGrads.direct()
         ctx.save_for_backward(verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, inv_mv_mats, inv_proj_mats,
                               verts_depth, faces_intense, pointBuffer, faceBuffer, binningBuffer, imgBuffer)
+        res = (color, depth)
         if return_alpha:
             # alpha = 1 - final_T, read from the image state after phase 2 (zeros when P == 0)
-            alpha = _C.tri_alpha(imgBuffer, color.size(0), color.size(2), color.size(3), color.device)
-            return color, depth, alpha
-        return color, depth
+            res += (_C.tri_alpha(imgBuffer, color.size(0), color.size(2), color.size(3), color.device),)
+        if return_face_weights:
+            # face_weights, face_hits: statistics of phase 2, no gradient
+            ctx.mark_non_differentiable(*out[7:])
+            res += tuple(out[7:])
+        return res
 
     @staticmethod
-    def backward(ctx, grad_out_color, grad_out_depth, grad_out_alpha=None):
+    def backward(ctx, grad_out_color, grad_out_depth, *grad_rest):
+        # grad_rest: the alpha cotangent (return_alpha), then those of the face statistics (ignored)
+        grad_out_alpha = grad_rest[0] if ctx.return_alpha else None
         num_rendered = ctx.num_rendered
         (verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, inv_mv_mats, inv_proj_mats, verts_depth,
          faces_intense, pointBuffer, faceBuffer, binningBuffer, imgBuffer) = ctx.saved_tensors
@@ -161,19 +171,20 @@ class _RenderTri(th.autograd.Function):
         # extension
         return (grad_verts, None, grad_verts_color, grad_faces_opacity,
                 grad_mv if ctx.needs_input_grad[4] else None, grad_proj if ctx.needs_input_grad[5] else None,
-                grad_verts_depth, grad_faces_intense, None, None, None, None, grad_bg)
+                grad_verts_depth, grad_faces_intense, None, None, None, None, grad_bg, None)
 
 
 class TriRenderer(th.nn.Module):
     """reference __init__.py:172-225"""
 
     def __init__(self, render_settings: TriRenderSettings, deterministic=None, exact_vertex_grads=None,
-                 return_alpha=False):
+                 return_alpha=False, return_face_weights=False):
         super().__init__()
         self.render_settings = render_settings
         self.deterministic = deterministic     # None: the process-wide default (set_deterministic)
         self.exact_vertex_grads = exact_vertex_grads   # None: the process-wide default (set_exact_vertex_grads)
         self.return_alpha = bool(return_alpha)
+        self.return_face_weights = bool(return_face_weights)
 
     def forward(self, verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, verts_depth, faces_intense):
         """
@@ -186,10 +197,16 @@ class TriRenderer(th.nn.Module):
         return_alpha (extension): also return alpha [B,1,H,W] fp32, differentiable: 1 - the transmittance the
         background was multiplied by (zeros when there are no vertices), for mask / silhouette losses.  Its gradient
         reaches faces_opacity only.  render_settings.bg gets a gradient when it requires grad.
+        return_face_weights (extension): also return face_weights [B,F] fp32 and face_hits [B,F] int32, last, without
+        gradient: per view, the sum over the pixels where a face was composited of T * alpha -- the factor its colour
+        was multiplied by -- and the number of those pixels (for pruning, finding unseen faces, refinement).  Summed
+        over faces, face_weights[b] equals alpha[b].sum() up to fp32 rounding.  Weights are accumulated in 64-bit fixed
+        point with 32 fractional bits, so the statistics are bit-identical from run to run in both modes, and a weight
+        below 2^-33 adds 0 (face_hits > 0 with face_weights == 0 is possible).  Images and gradients are unchanged.
         """
         return render_tri(verts, faces.to(dtype=th.int32), verts_color, faces_opacity, mv_mats.transpose(1, 2),
                           proj_mats.transpose(1, 2), verts_depth, faces_intense, self.render_settings,
-                          self.deterministic, self.exact_vertex_grads, self.return_alpha)
+                          self.deterministic, self.exact_vertex_grads, self.return_alpha, self.return_face_weights)
 
 
 # =============================================================================
@@ -234,17 +251,17 @@ def set_tet_intensity_grads(flag: bool) -> bool:
 
 def render_tet(verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, verts_depth, faces_intense, tets,
                face_tets, tet_faces, render_settings: TetRenderSettings, deterministic=None, vertex_grads=None,
-               intensity_grads=None, first_view=0, return_alpha=False):
+               intensity_grads=None, first_view=0, return_alpha=False, return_face_weights=False):
     """reference __init__.py:243-275 (`deterministic`: see set_deterministic; `vertex_grads`: see
-    set_tet_vertex_grads; `intensity_grads`: see set_tet_intensity_grads; `first_view`, `return_alpha`: see
-    TetRenderer.forward).  render_settings.bg is passed to autograd as an input of its own: with bg.requires_grad set
+    set_tet_vertex_grads; `intensity_grads`: see set_tet_intensity_grads; `first_view`, `return_alpha`,
+    `return_face_weights`: see TetRenderer.forward).  render_settings.bg is passed to autograd as an input of its own: with bg.requires_grad set
     it gets its gradient."""
     det = _deterministic_default if deterministic is None else bool(deterministic)
     vert = _tet_vertex_grads_default if vertex_grads is None else bool(vertex_grads)
     fint = _tet_intensity_grads_default if intensity_grads is None else bool(intensity_grads)
     return _RenderTet.apply(verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, verts_depth, faces_intense,
                             tets, face_tets, tet_faces, render_settings, det, vert, fint, int(first_view),
-                            bool(return_alpha), render_settings.bg)
+                            bool(return_alpha), render_settings.bg, bool(return_face_weights))
 
 
 class _RenderTet(th.autograd.Function):
@@ -253,7 +270,7 @@ class _RenderTet(th.autograd.Function):
     @staticmethod
     def forward(ctx, verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, verts_depth, faces_intense, tets,
                 face_tets, tet_faces, render_settings, deterministic=False, vertex_grads=False, intensity_grads=False,
-                first_view=0, return_alpha=False, bg=None):
+                first_view=0, return_alpha=False, bg=None, return_face_weights=False):
         ctx.deterministic = deterministic
         ctx.vertex_grads = vertex_grads
         ctx.intensity_grads = intensity_grads
@@ -281,13 +298,22 @@ class _RenderTet(th.autograd.Function):
                               verts_depth, faces_intense, tets, face_tets, tet_faces, pointBuffer, faceBuffer,
                               binningBuffer, imgBuffer)
         ctx.mark_non_differentiable(active)
+        res = (color, depth, active)
         if return_alpha:
-            alpha = _C.tet_alpha(imgBuffer, color.size(0), color.size(2), color.size(3), color.device)
-            return color, depth, active, alpha
-        return color, depth, active
+            res += (_C.tet_alpha(imgBuffer, color.size(0), color.size(2), color.size(3), color.device),)
+        if return_face_weights:
+            # face_weights, face_hits: a post-pass over the forward state, no gradient
+            stats = _C.tet_face_weights(color.size(0), verts.size(0), faces.size(0), tets.size(0), color.size(2),
+                                        color.size(3), render_settings.ray_random_seed, inv_mv_mats, inv_proj_mats,
+                                        pointBuffer, faceBuffer, imgBuffer, ctx.tet_records)
+            ctx.mark_non_differentiable(*stats)
+            res += stats
+        return res
 
     @staticmethod
-    def backward(ctx, grad_out_color, grad_out_depth, grad_out_active, grad_out_alpha=None):
+    def backward(ctx, grad_out_color, grad_out_depth, grad_out_active, *grad_rest):
+        # grad_rest: the alpha cotangent (return_alpha), then those of the face statistics (ignored)
+        grad_out_alpha = grad_rest[0] if ctx.return_alpha else None
         render_settings = ctx.render_settings
         (verts, faces, verts_color, faces_opacity, mv_mats, proj_mats, inv_mv_mats, inv_proj_mats, verts_depth,
          faces_intense, tets, face_tets, tet_faces, pointBuffer, faceBuffer, binningBuffer, imgBuffer) = ctx.saved_tensors
@@ -341,17 +367,18 @@ class _RenderTet(th.autograd.Function):
         # (faces_intense) and 17 (bg) are an extension
         return (grad_verts, None, grad_verts_color, grad_faces_opacity,
                 grad_mv if ctx.needs_input_grad[4] else None, grad_proj if ctx.needs_input_grad[5] else None,
-                None, grad_fint, None, None, None, None, None, None, None, None, None, grad_bg)
+                None, grad_fint, None, None, None, None, None, None, None, None, None, grad_bg, None)
 
 
 class TetRenderer(th.nn.Module):
     """reference __init__.py:426-488"""
 
     def __init__(self, render_settings: TetRenderSettings, deterministic=None, vertex_grads=None, intensity_grads=None,
-                 return_alpha=False):
+                 return_alpha=False, return_face_weights=False):
         super().__init__()
         self.render_settings = render_settings
         self.return_alpha = bool(return_alpha)
+        self.return_face_weights = bool(return_face_weights)
         self.deterministic = deterministic     # None: the process-wide default (set_deterministic)
         self.vertex_grads = vertex_grads       # None: the process-wide default (set_tet_vertex_grads)
         self.intensity_grads = intensity_grads   # None: the process-wide default (set_tet_intensity_grads)
@@ -372,6 +399,12 @@ class TetRenderer(th.nn.Module):
         return_alpha (extension): also return alpha [B,1,H,W] fp32, differentiable: 1 - the transmittance the
         background was multiplied by on active pixels, 0 on inactive ones.  Its gradient reaches faces_opacity only.
         render_settings.bg gets a gradient when it requires grad.
+        return_face_weights (extension): also return face_weights [B,F] fp32 and face_hits [B,F] int32, last, without
+        gradient: per view, the sum over the active pixels where a face was composited of expf(log_T) * opacity -- the
+        factor its colour was multiplied by -- and the number of those pixels.  Inactive pixels count for nothing.
+        Summed over faces, face_weights[b] equals alpha[b].sum() up to fp32 rounding (not where a face of opacity 1
+        ends a ray).  Same fixed-point format and reproducibility as TriRenderer's.  Computed by one post-pass over
+        the forward state; images and gradients are unchanged.
         """
         f32, i32 = th.float32, th.int32
         return render_tet(verts.to(dtype=f32), faces.to(dtype=i32), verts_color.to(dtype=f32),
@@ -379,4 +412,4 @@ class TetRenderer(th.nn.Module):
                           proj_mats.to(dtype=f32).transpose(1, 2), verts_depth.to(dtype=f32),
                           faces_intense.to(dtype=f32), tets.to(dtype=i32), face_tets.to(dtype=i32),
                           tet_faces.to(dtype=i32), self.render_settings, self.deterministic, self.vertex_grads,
-                          self.intensity_grads, first_view, self.return_alpha)
+                          self.intensity_grads, first_view, self.return_alpha, self.return_face_weights)

@@ -29,6 +29,8 @@ SIGNATURES = {
     "dmr_tri_forward_bin": (c_int, [c_int] * 5 + [c_void_p] * 11 + [c_void_p]),
     "dmr_tri_depth_chain": (c_int, [c_int, c_int] + [c_void_p] * 5 + [c_void_p]),
     "dmr_tri_forward_render": (c_int, [c_int] * 6 + [c_void_p] * 9 + [c_void_p]),
+    "dmr_tri_face_weights_bytes": (c_size_t, [c_int] * 2),
+    "dmr_tri_forward_render_face_weights": (c_int, [c_int] * 6 + [c_void_p] * 11 + [c_void_p, c_size_t] + [c_void_p]),
     "dmr_tri_backward_workspace_bytes": (c_size_t, [c_int] * 3),
     "dmr_tri_backward": (c_int, [c_int] * 6 + [c_void_p] * 14 + [c_void_p, c_size_t] + [c_void_p]),
     "dmr_tri_backward_deterministic_bytes": (c_size_t, [c_int] * 3),
@@ -61,6 +63,8 @@ SIGNATURES = {
     "dmr_tet_alpha": (c_int, [c_int] * 3 + [c_void_p] * 2 + [c_void_p]),
     "dmr_tet_background_grad_bytes": (c_size_t, [c_int]),
     "dmr_tet_background_grad": (c_int, [c_int] * 3 + [c_void_p] * 4 + [c_size_t] + [c_void_p]),
+    "dmr_tet_face_weights_bytes": (c_size_t, [c_int] * 2),
+    "dmr_tet_face_weights": (c_int, [c_int] * 7 + [c_void_p] * 8 + [c_void_p, c_size_t] + [c_void_p]),
     "dmr_debug_view": (c_int, [c_int] * 8 + [c_size_t, c_void_p, ctypes.POINTER(c_void_p), ctypes.POINTER(c_size_t)]),
     "dmr_nvls_allreduce_sum_f32_fused": (c_int, [c_void_p, c_size_t, c_int, c_int, c_void_p, c_void_p, ctypes.c_uint, c_void_p]),
     "dmr_camera_inverses": (c_int, [c_int, c_void_p, ctypes.c_int64, ctypes.c_int64, ctypes.c_int64, c_void_p, ctypes.c_int64,

@@ -38,7 +38,8 @@ static const char* const g_stage_names[ST_COUNT] = {
     "tet_march_backward_vertex", "tet_march_backward_camera_vertex", "tet_vertex_finish",
     "tet_march_backward_intensity", "tet_march_backward_camera_intensity", "tet_march_backward_vertex_intensity",
     "tet_march_backward_camera_vertex_intensity", "tet_intensity_finish", "tri_alpha", "tri_render_backward_alpha",
-    "tri_background_grad", "tet_alpha", "tet_march_backward_alpha", "tet_background_grad" };
+    "tri_background_grad", "tet_alpha", "tet_march_backward_alpha", "tet_background_grad", "tri_face_weights",
+    "tet_face_weights" };
 struct Prof {
     bool on = false, created = false;
     cudaEvent_t ev[ST_COUNT][2];
@@ -223,10 +224,12 @@ int dmr_tri_depth_chain(int B, int P, const float* verts, const float* mv_mats, 
     return depth_chain(B, P, verts, mv_mats, proj_mats, dL_dvdepth, dL_dverts, (cudaStream_t)stream);
 }
 
-int dmr_tri_forward_render(int B, int P, int F, int W, int H, int R, const float* background,
-                           const float* inv_mv_mats, const float* inv_proj_mats, const void* point_buffer,
-                           void* face_buffer, void* binning_buffer, void* image_buffer, float* out_color,
-                           float* out_depth, dmr_stream_t stream_)
+// phase 2; face_weights != nullptr: also the face statistics (face_weights, face_hits, workspace checked by the caller)
+static int tri_forward_render_impl(int B, int P, int F, int W, int H, int R, const float* background,
+                                   const float* inv_mv_mats, const float* inv_proj_mats, const void* point_buffer,
+                                   void* face_buffer, void* binning_buffer, void* image_buffer, float* out_color,
+                                   float* out_depth, dmr_stream_t stream_, float* face_weights = nullptr,
+                                   int* face_hits = nullptr, void* workspace = nullptr)
 {
     cudaStream_t stream = (cudaStream_t)stream_;
     if (!sizes_ok(B, P, F, W, H) || R < 0) return DMR_ETOOLARGE;
@@ -234,6 +237,12 @@ int dmr_tri_forward_render(int B, int P, int F, int W, int H, int R, const float
     if (!background || !inv_mv_mats || !inv_proj_mats || !image_buffer || !out_color || !out_depth ||
         (R > 0 && (!binning_buffer || !face_buffer))) { set_error("null pointer"); return DMR_EINVAL; }
     (void)point_buffer;
+    FaceWeightAcc fw{};
+    if (face_weights) {
+        // zeroed before every phase 2: a call repeated after a too-small speculative binning buffer starts afresh
+        fw = face_weights_acc(workspace, B, F);
+        DMR_CUDA(cudaMemsetAsync(workspace, 0, face_weights_bytes(B, F), stream));
+    }
     TriFaceLayout FL = TriFaceLayout::make((size_t)B * F);
     TriImageLayout IL = TriImageLayout::make(B, W, H);
     uint2* ranges = at<uint2>(image_buffer, IL.ranges);
@@ -252,7 +261,43 @@ int dmr_tri_forward_render(int B, int P, int F, int W, int H, int R, const float
     p.prev_T = at<float>(image_buffer, IL.prev_T);
     p.n_contrib = at<uint32_t>(image_buffer, IL.n_contrib);
     p.out_color = out_color; p.out_depth = out_depth;
-    return tri_render_forward(p, stream);
+    if (!face_weights) return tri_render_forward(p, stream);
+    if ((rc = tri_render_forward(p, stream, &fw))) return rc;
+    ProfScope prof(ST_TRI_FACE_WEIGHTS, stream);
+    return face_weights_convert(B, F, fw, face_weights, face_hits, stream);
+}
+
+int dmr_tri_forward_render(int B, int P, int F, int W, int H, int R, const float* background,
+                           const float* inv_mv_mats, const float* inv_proj_mats, const void* point_buffer,
+                           void* face_buffer, void* binning_buffer, void* image_buffer, float* out_color,
+                           float* out_depth, dmr_stream_t stream)
+{
+    return tri_forward_render_impl(B, P, F, W, H, R, background, inv_mv_mats, inv_proj_mats, point_buffer, face_buffer,
+                                   binning_buffer, image_buffer, out_color, out_depth, stream);
+}
+
+size_t dmr_tri_face_weights_bytes(int B, int F) { return (B < 0 || F < 0) ? 0 : face_weights_bytes(B, F); }
+
+int dmr_tri_forward_render_face_weights(int B, int P, int F, int W, int H, int R, const float* background,
+                                        const float* inv_mv_mats, const float* inv_proj_mats, const void* point_buffer,
+                                        void* face_buffer, void* binning_buffer, void* image_buffer, float* out_color,
+                                        float* out_depth, float* face_weights, int* face_hits, void* workspace,
+                                        size_t workspace_bytes, dmr_stream_t stream)
+{
+    if (!sizes_ok(B, P, F, W, H) || R < 0) return DMR_ETOOLARGE;
+    if ((long long)W * H >= (1LL << 31)) { set_error("face statistics need fewer than 2^31 pixels per view"); return DMR_ETOOLARGE; }
+    if ((size_t)B * F == 0)   // [B,0] statistics: nothing to count, but the images and the image state as without them
+        return tri_forward_render_impl(B, P, F, W, H, R, background, inv_mv_mats, inv_proj_mats, point_buffer, face_buffer,
+                                       binning_buffer, image_buffer, out_color, out_depth, stream);
+    if (!face_weights || !face_hits) { set_error("null pointer: face_weights / face_hits"); return DMR_EINVAL; }
+    const size_t need = face_weights_bytes(B, F);
+    if (!workspace || workspace_bytes < need) {
+        set_error("face statistics need a workspace of %zu bytes (dmr_tri_face_weights_bytes)", need);
+        return DMR_EINVAL;
+    }
+    return tri_forward_render_impl(B, P, F, W, H, R, background, inv_mv_mats, inv_proj_mats, point_buffer, face_buffer,
+                                   binning_buffer, image_buffer, out_color, out_depth, stream, face_weights, face_hits,
+                                   workspace);
 }
 
 static int tri_backward_impl(int B, int P, int F, int W, int H, int R, const float* background, const float* inv_mv_mats,

@@ -454,6 +454,37 @@ int dmr_tet_background_grad(int B, int W, int H, const void* image_buffer, const
                          dL_dcolor, dL_dbg, workspace, (cudaStream_t)stream);
 }
 
+size_t dmr_tet_face_weights_bytes(int B, int F) { return (B < 0 || F < 0) ? 0 : face_weights_bytes(B, F); }
+
+int dmr_tet_face_weights(int B, int P, int F, int T, int W, int H, int ray_random_seed, const float* inv_mv_mats,
+                         const float* inv_proj_mats, const void* point_buffer, const void* face_buffer,
+                         const void* tet_records, const void* image_buffer, float* face_weights, int* face_hits,
+                         void* workspace, size_t workspace_bytes, dmr_stream_t stream_)
+{
+    cudaStream_t stream = (cudaStream_t)stream_;
+    if (!tet_sizes_ok(B, P, F, T, W, H)) return DMR_ETOOLARGE;
+    if ((long long)W * H >= (1LL << 31)) { set_error("face statistics need fewer than 2^31 pixels per view"); return DMR_ETOOLARGE; }
+    if (B == 0 || F == 0) return DMR_OK;
+    if (!face_weights || !face_hits || !face_buffer || !image_buffer || !inv_mv_mats || !inv_proj_mats ||
+        (T > 0 && !tet_records)) {
+        set_error("null pointer");
+        return DMR_EINVAL;
+    }
+    const size_t need = face_weights_bytes(B, F);
+    if (!workspace || workspace_bytes < need) {
+        set_error("face statistics need a workspace of %zu bytes (dmr_tet_face_weights_bytes)", need);
+        return DMR_EINVAL;
+    }
+    (void)point_buffer;
+    const FaceWeightAcc fw = face_weights_acc(workspace, B, F);
+    DMR_CUDA(cudaMemsetAsync(workspace, 0, need, stream));
+    TetParams p;
+    // the post-pass reads the rays (inverses, stored jitter), the records and the per-pixel state only
+    fill_params(p, B, P, F, T, W, H, ray_random_seed, nullptr, nullptr, nullptr, inv_mv_mats, inv_proj_mats, nullptr,
+                face_buffer, tet_records, image_buffer);
+    return tet_face_weights(p, fw, face_weights, face_hits, stream);
+}
+
 int dmr_debug_set_tet_first_split(int split)
 {
     g_tet_first_split_override = (split > 0 && split <= 16) ? split : 0;

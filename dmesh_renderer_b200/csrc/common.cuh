@@ -44,7 +44,8 @@ enum Stage {
     ST_TRI_BWD_CAM, ST_TRI_CAM_FINISH, ST_DEPTH_CAM, ST_DEPTH_CAM_FINISH, ST_TET_BWD_CAM, ST_TET_CAM_FINISH,
     ST_TET_BWD_VERT, ST_TET_BWD_CAM_VERT, ST_TET_VERT_FINISH,
     ST_TET_BWD_INT, ST_TET_BWD_CAM_INT, ST_TET_BWD_VERT_INT, ST_TET_BWD_CAM_VERT_INT, ST_TET_INT_FINISH,
-    ST_TRI_ALPHA, ST_TRI_BWD_ALPHA, ST_TRI_BG_GRAD, ST_TET_ALPHA, ST_TET_BWD_ALPHA, ST_TET_BG_GRAD, ST_COUNT
+    ST_TRI_ALPHA, ST_TRI_BWD_ALPHA, ST_TRI_BG_GRAD, ST_TET_ALPHA, ST_TET_BWD_ALPHA, ST_TET_BG_GRAD,
+    ST_TRI_FACE_WEIGHTS, ST_TET_FACE_WEIGHTS, ST_COUNT
 };
 void count_launch(int n);
 void prof_begin(int stage, cudaStream_t s, bool count = true);   // count: also counts one kernel launch
@@ -112,6 +113,22 @@ __device__ __forceinline__ void red_add_v4(float* a, float x, float y, float z, 
 __device__ __forceinline__ void red_add_v2(float* a, float x, float y)
 {
     asm volatile("red.global.add.v2.f32 [%0], {%1, %2};" ::"l"(a), "f"(x), "f"(y));
+}
+
+// Per-(view, face) visibility statistics of a forward call (dmr_tri_forward_render_face_weights, dmr_tet_face_weights):
+// the sum of the blending weights T * alpha of the face's composited hits as 64-bit fixed point with 32 fractional
+// bits (each weight rounded to nearest, so one below 2^-33 adds 0), and the number of those hits.  Integer sums do not
+// depend on the order of the reductions: the same bits in every run, without a separate deterministic path.  A weight
+// is at most 1 (2^32 in fixed point), so a sum cannot wrap while a view has fewer than 2^31 pixels.
+struct FaceWeightAcc {
+    unsigned long long* weight;   // [B*F], zeroed
+    uint32_t* hits;               // [B*F], zeroed
+};
+__device__ __forceinline__ void face_weight_add(const FaceWeightAcc& a, size_t i, float w)
+{
+    const unsigned long long q = __float2ull_rn(w * 4294967296.0f);
+    asm volatile("red.global.add.u64 [%0], %1;" ::"l"(a.weight + i), "l"(q));
+    asm volatile("red.global.add.u32 [%0], %1;" ::"l"(a.hits + i), "r"(1u));
 }
 
 // column-major 4x4 * (p,1): auxiliary.h:71-90
@@ -382,5 +399,12 @@ int image_alpha(bool tet, int B, int W, int H, const float* t, const uint8_t* ac
 size_t image_bg_grad_bytes(int B);
 int image_bg_grad(bool tet, int B, int W, int H, const float* t, const uint8_t* active, const float* dL_dcolor, float* dL_dbg,
                   void* workspace, cudaStream_t stream);
+
+// image.cu: the face statistics' workspace (12 * B * F bytes: the fixed-point weights, then the hit counts) and the
+// conversion of its accumulators into face_weights [B*F] fp32 and face_hits [B*F] int32 (one launch; the caller
+// opens the profile stage)
+size_t face_weights_bytes(int B, int F);
+FaceWeightAcc face_weights_acc(void* workspace, int B, int F);
+int face_weights_convert(int B, int F, const FaceWeightAcc& acc, float* face_weights, int* face_hits, cudaStream_t stream);
 
 }  // namespace dmr

@@ -1,5 +1,6 @@
 // image.cu -- per-pixel outputs of the image state that both renderers share in form: the alpha (coverage) image
-// and the gradient with respect to the background colour.
+// and the gradient with respect to the background colour; and the conversion of the per-(view, face) visibility
+// statistics (FaceWeightAcc, common.cuh) into their output format.
 //
 // The forward passes composite colour = C + w * bg with a per-pixel background weight w:
 //   tri: w = final_T (the transmittance after the last composited face, T < 1e-4 termination included);
@@ -108,6 +109,37 @@ int image_bg_grad(bool tet, int B, int W, int H, const float* t, const uint8_t* 
     DMR_LAUNCH_CHECK("bg_grad_partial_kernel");
     DMR_CUDA(dmr_launch(bg_grad_finish_kernel, dim3(1), dim3(96), 0, stream, (int)(nbx * B), (const float*)partial, dL_dbg));
     DMR_LAUNCH_CHECK("bg_grad_finish_kernel");
+    return 0;
+}
+
+size_t face_weights_bytes(int B, int F) { return 12 * (size_t)B * F; }
+
+FaceWeightAcc face_weights_acc(void* workspace, int B, int F)
+{
+    FaceWeightAcc a;
+    a.weight = static_cast<unsigned long long*>(workspace);
+    a.hits = reinterpret_cast<uint32_t*>(a.weight + (size_t)B * F);
+    return a;
+}
+
+// fixed point (2^-32) -> fp32: one rounding (the scale is a power of two)
+__global__ void __launch_bounds__(256) face_weights_convert_kernel(size_t n, FaceWeightAcc acc, float* __restrict__ face_weights,
+                                                                   int* __restrict__ face_hits)
+{
+    griddep_wait();   // programmatic dependent launch: see dmr_launch (common.cuh)
+    for (size_t i = (size_t)blockIdx.x * 256 + threadIdx.x; i < n; i += (size_t)gridDim.x * 256) {
+        face_weights[i] = __ull2float_rn(acc.weight[i]) * 0x1p-32f;
+        face_hits[i] = (int)acc.hits[i];
+    }
+}
+
+int face_weights_convert(int B, int F, const FaceWeightAcc& acc, float* face_weights, int* face_hits, cudaStream_t stream)
+{
+    const size_t n = (size_t)B * F;
+    if (n == 0) return 0;
+    const unsigned nblk = (unsigned)std::min<size_t>((n + 255) / 256, 148 * 8);
+    DMR_CUDA(dmr_launch(face_weights_convert_kernel, dim3(nblk), dim3(256), 0, stream, n, acc, face_weights, face_hits));
+    DMR_LAUNCH_CHECK("face_weights_convert_kernel");
     return 0;
 }
 

@@ -228,6 +228,10 @@ int tet_march_backward(const TetParams& p, cudaStream_t stream, float* cam_rec =
 int tet_march_backward_deterministic(const TetParams& p, cudaStream_t stream, float* cam_rec = nullptr,
                                      const TetVertGrad* vert = nullptr, const TetIntGrad* fint = nullptr,
                                      const float* dL_dalpha = nullptr);
+// face statistics of the forward call whose state p points at (after tet_march_forward): adds every composited step's
+// blending weight and 1 to fw's (view, face) accumulators (zeroed by the caller) and converts them into face_weights
+// [B*F] fp32 and face_hits [B*F] int32
+int tet_face_weights(const TetParams& p, const FaceWeightAcc& fw, float* face_weights, int* face_hits, cudaStream_t stream);
 // records of a view -> += dL_dmv[B,16], dL_dproj[B,16]
 int tet_camera_finish(const TetParams& p, const float* cam_rec, float* dL_dmv, float* dL_dproj, cudaStream_t stream);
 

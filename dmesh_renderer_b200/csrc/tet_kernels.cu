@@ -1435,6 +1435,75 @@ static cudaError_t launch_tet_bwd_alpha(const TetParams& p, cudaStream_t stream,
     return dmr_launch(k, grid, dim3(MARCH_THREADS), 0, stream, p, cam_rec, vg, ig, dL_dalpha);
 }
 
+// Face visibility statistics of a forward call (dmr_tet_face_weights; DESIGN.md 3.4), after the forward march: one
+// thread per pixel, active pixels only (an inactive pixel shows the background and has alpha 0).  Every composited
+// step adds its blending weight expf(log_T) * opacity -- the factor the forward march multiplies the step's colour by
+// -- and 1 to the (view, face) accumulators.  Not in the march itself: its first pass hands rays through irregular
+// tets to a second launch that re-marches them from the first face, and it does not know yet whether a pixel ends
+// inactive.  The steps of the trail are walked forward with the march's own recurrence for log_T, and the steps of a
+// ray longer than the trail are marched again from its last recorded step with the march's own exit search
+// (tet_step<EXIT>), so every weight is the forward's bits.
+__global__ void __launch_bounds__(MARCH_THREADS) tet_face_weights_kernel(TetParams p, FaceWeightAcc fw)
+{
+    griddep_wait();
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int b = blockIdx.z;
+    const uint32_t px = blockIdx.x * 8 + (lane & 7);
+    const uint32_t py = blockIdx.y * MARCH_ROWS + warp * 4 + (lane >> 3);
+    if (!(px < (uint32_t)p.W && py < (uint32_t)p.H)) return;
+    const size_t HW = (size_t)p.W * p.H;
+    const size_t BI = (size_t)p.B * HW;
+    const size_t bpix = (size_t)b * HW + (size_t)py * p.W + px;
+    if (!p.active[bpix]) return;
+    const int n = (int)p.n_contrib[bpix];
+    const size_t fbase = (size_t)b * p.F;
+
+    // steps 0 .. min(n, cap) - 1 from the trail, tet_march_fwd_kernel's arithmetic; curr_tet follows the march (the tet
+    // behind face k is the first entry of face_tets[face k] that is neither the previous tet nor -1, as TetRec.next)
+    const int nt = min(n, p.trail_cap);
+    const int4* trail = p.trail + bpix;
+    float log_T = 0.0f;
+    int curr_face = -1, curr_tet = p.first_tet[bpix];
+    for (int k = 0; k < nt; k++) {
+        curr_face = trail[(size_t)k * BI].x & 0x7fffffff;
+        const float4* sh4 = reinterpret_cast<const float4*>(p.shade + curr_face);
+        const float4 s2 = sh4[2];   // (c2.z, opacity, log1m, i0)
+        if (k > 0 && n > nt) {
+            const int4 s3 = reinterpret_cast<const int4*>(sh4)[3];   // (i1, i2, t0, t1)
+            curr_tet = (s3.z != curr_tet && s3.z != -1) ? s3.z : (s3.w != curr_tet && s3.w != -1) ? s3.w : -1;
+        }
+        const float opacity = s2.y;
+        face_weight_add(fw, fbase + curr_face, expf(log_T) * opacity);
+        if (opacity < 1.0f) log_T += s2.z;
+        else log_T = logf(DMR_T_EPS * 0.1f);
+    }
+    // steps beyond the trail: marched again from the last recorded one with the march's own exit search (irregular
+    // tets included, as its second pass), same recurrence
+    if (n > nt) {
+        float3 ro, rd;
+        tet_pixel_ray(p, b, px, py, bpix, ro, rd);
+        for (int k = nt; k < n && curr_tet >= 0; k++) {
+            const TetStep s = tet_step<true, true>(p, b, p.tet_rec + curr_tet, curr_face, ro, rd);
+            curr_face = s.face; curr_tet = s.tet;
+            const float4 s2 = reinterpret_cast<const float4*>(p.shade + curr_face)[2];
+            const float opacity = s2.y;
+            face_weight_add(fw, fbase + curr_face, expf(log_T) * opacity);
+            if (opacity < 1.0f) log_T += s2.z;
+            else log_T = logf(DMR_T_EPS * 0.1f);
+        }
+    }
+}
+
+int tet_face_weights(const TetParams& p, const FaceWeightAcc& fw, float* face_weights, int* face_hits, cudaStream_t stream)
+{
+    dim3 grid((p.W + 7) / 8, (p.H + MARCH_ROWS - 1) / MARCH_ROWS, p.B);
+    ProfScope prof(ST_TET_FACE_WEIGHTS, stream);
+    count_launch(1);   // two kernels under one scope
+    DMR_CUDA(dmr_launch(tet_face_weights_kernel, grid, dim3(MARCH_THREADS), 0, stream, p, fw));
+    DMR_LAUNCH_CHECK("tet_face_weights_kernel");
+    return face_weights_convert(p.B, p.F, fw, face_weights, face_hits, stream);
+}
+
 // One CTA per view: the view's records (tet_march_bwd_cam) are summed in a fixed order -- thread t owns component
 // t % 32 of every eighth record (coalesced reads of the flat record array), then the eight partial sums of a component
 // are added in thread order -- and chained into the matrices: through the inverses, dL/dA = -A^-T (dL/dA^-1) A^-T,

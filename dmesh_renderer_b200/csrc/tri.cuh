@@ -63,7 +63,9 @@ int tri_preprocess_faces(int B, int P, int F, int W, int H, const int* faces, co
                          const float* verts_color, const float* faces_opacity, const float* faces_intense,
                          uint32_t* tiles_touched, uint32_t* depth_key, uint2* rect, TriRecord* records,
                          const SortPre& face_sort, cudaStream_t stream);
-int tri_render_forward(const TriRenderParams& p, cudaStream_t stream);
+// fw != nullptr: the face-statistics instantiation, which also adds every hit's blending weight and 1 to fw's
+// (view, face) accumulators (zeroed by the caller)
+int tri_render_forward(const TriRenderParams& p, cudaStream_t stream, const FaceWeightAcc* fw = nullptr);
 // cam_tiles != nullptr: the camera-gradient kernels, which also store one 24-float record per (view, tile) there.
 // exact: the exact vertex-position instantiations (same launches, same workspace).
 // dL_dalpha != nullptr: the alpha-cotangent instantiations ([B,H,W] cotangent of alpha = 1 - final_T)

@@ -208,15 +208,22 @@ constexpr int HS = HB / 32;      // 32-entry slices of the compacted list of suc
 //       whole pass are known up front, so a lane with few hits in one 32-instance slice moves straight on to the
 //       next one: the number of SIMD passes is the largest per-pixel hit count over HB instances, not the sum of
 //       the per-slice maxima (the shading path ran at 15 of 32 lanes before).
+//
+// Face visibility statistics (FW = true, opt-in; DESIGN.md 3.3): every hit also adds its blending weight alpha * T --
+// the factor its colour is multiplied by -- and 1 to the (view, face) accumulators of `fw` (FaceWeightAcc, common.cuh),
+// the hit that triggers the T < 1e-4 termination included.  The face id of a hit is read again from the tile's face
+// list (a line the staging has just read).  `tid` is threadIdx.x read by the kernel itself: there the compiler knows it
+// is below the launch bound of 256 (read in here, only below 1024), and the index arithmetic of the plain kernel stays
+// the SASS it was before the body moved out of it.
 constexpr int DMR_TRI_FWD_MINB = 4;
-__global__ void __launch_bounds__(256, DMR_TRI_FWD_MINB) tri_render_fwd_kernel(TriRenderParams p)
+template <bool FW>
+__device__ __forceinline__ void tri_render_fwd_body(const TriRenderParams& p, const int tid, const FaceWeightAcc fw)
 {
-    griddep_wait();   // programmatic dependent launch: see dmr_launch (common.cuh)
     __shared__ uint4 s_rec[RB * 9];
     __shared__ unsigned char s_bmask[RB];         // [staged instance]: warp blocks of the tile it can touch (tile_block_mask)
     __shared__ unsigned char s_cidx[8 * HB];      // [warp][compacted position] -> position in the staged round
     __shared__ uint32_t s_pmask[8 * HS * 32];     // [warp][slice][lane]: covered compacted instances of the lane's pixel
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int lane = tid & 31, warp = tid >> 5;
     const int b = blockIdx.z;
     const int tiles_x = gridDim.x, tiles_y = gridDim.y;
     const int bx0 = blockIdx.x * DMR_TILE + (warp & 1) * 8, by0 = blockIdx.y * DMR_TILE + (warp >> 1) * 4;
@@ -310,6 +317,9 @@ __global__ void __launch_bounds__(256, DMR_TRI_FWD_MINB) tri_render_fwd_kernel(T
                         C1 += c1_ * alpha * T;
                         C2 += c2_ * alpha * T;
                         D += iD * alpha * T;
+                        if constexpr (FW) {
+                            face_weight_add(fw, (size_t)b * p.F + p.face_list[range.x + (uint32_t)(r * RB + j)], alpha * T);
+                        }
                         pT = T;
                         T = test_T;
                         last_contributor = (uint32_t)(r * RB + j + 1);
@@ -333,6 +343,18 @@ __global__ void __launch_bounds__(256, DMR_TRI_FWD_MINB) tri_render_fwd_kernel(T
         p.out_color[(size_t)b * 3 * HW + 2 * HW + pix] = C2 + T * p.bg[2];
         p.out_depth[bpix] = D + T * 1.0f;
     }
+}
+
+__global__ void __launch_bounds__(256, DMR_TRI_FWD_MINB) tri_render_fwd_kernel(TriRenderParams p)
+{
+    griddep_wait();   // programmatic dependent launch: see dmr_launch (common.cuh)
+    tri_render_fwd_body<false>(p, threadIdx.x, FaceWeightAcc{});
+}
+
+__global__ void __launch_bounds__(256, DMR_TRI_FWD_MINB) tri_render_fwd_face_weights_kernel(TriRenderParams p, FaceWeightAcc fw)
+{
+    griddep_wait();
+    tri_render_fwd_body<true>(p, threadIdx.x, fw);
 }
 
 // ---------------------------------------------------------------------------
@@ -1098,11 +1120,16 @@ __global__ void __launch_bounds__(256) tri_grad_vertex_kernel(TriRenderParams p)
     if (c.x != 0.0f || c.y != 0.0f || c.z != 0.0f) { dc[0] += c.x; dc[1] += c.y; dc[2] += c.z; }
 }
 
-int tri_render_forward(const TriRenderParams& p, cudaStream_t stream)
+int tri_render_forward(const TriRenderParams& p, cudaStream_t stream, const FaceWeightAcc* fw)
 {
     if (p.B <= 0 || p.W <= 0 || p.H <= 0) return 0;
     dim3 grid((p.W + DMR_TILE - 1) / DMR_TILE, (p.H + DMR_TILE - 1) / DMR_TILE, p.B);
     ProfScope prof(ST_TRI_FWD, stream);
+    if (fw) {
+        DMR_CUDA(dmr_launch(tri_render_fwd_face_weights_kernel, dim3(grid), dim3(256), 0, stream, p, *fw));
+        DMR_LAUNCH_CHECK("tri_render_fwd_face_weights_kernel");
+        return 0;
+    }
     DMR_CUDA(dmr_launch(tri_render_fwd_kernel, dim3(grid), dim3(256), 0, stream, p));
     DMR_LAUNCH_CHECK("tri_render_fwd_kernel");
     return 0;

@@ -147,6 +147,34 @@ int dmr_tri_forward_render(
     float* out_color, float* out_depth,
     dmr_stream_t stream);
 
+/* Face visibility statistics of the tri renderer (no reference counterpart).  dmr_tri_forward_render, with the    */
+/* same arguments and the same images, plus, per view b and face f:                                                 */
+/*   face_weights[b,f] (fp32) = sum, over the pixels of view b at which f was composited, of T * alpha -- the factor */
+/*                              the forward pass multiplies the face's colour by (every hit within n_contrib, the    */
+/*                              one that triggers the T < 1e-4 termination included);                                */
+/*   face_hits[b,f] (int32)   = the number of those pixels.                                                          */
+/* Summed over f, face_weights[b] is the sum of view b's alpha image (dmr_tri_alpha) up to fp32 rounding.  Each      */
+/* weight is accumulated as 64-bit fixed point with 32 fractional bits, rounded to nearest: the statistics are       */
+/* bit-identical from run to run (integer sums), and a weight below 2^-33 adds 0, so face_hits > 0 with              */
+/* face_weights == 0 is possible.  Both outputs [B,F] are written (zeros for faces never composited).  `workspace`:  */
+/* dmr_tri_face_weights_bytes(B, F) = 12*B*F bytes of device scratch, zeroed by every call, so a call repeated with  */
+/* a larger binning buffer (R too small) gives the statistics of that call alone.  W*H must stay below 2^31.  With   */
+/* B*F == 0 there is nothing to count: the call is dmr_tri_forward_render (the statistics pointers and the workspace */
+/* are not used).                                                                                                    */
+size_t dmr_tri_face_weights_bytes(int B, int F);
+int dmr_tri_forward_render_face_weights(
+    int B, int P, int F, int W, int H, int R,
+    const float* background,     /* [3] device */
+    const float* inv_mv_mats,    /* [B,16] */
+    const float* inv_proj_mats,  /* [B,16] */
+    const void* point_buffer, void* face_buffer,
+    void* binning_buffer, void* image_buffer,
+    float* out_color, float* out_depth,
+    float* face_weights,         /* [B,F] */
+    int* face_hits,              /* [B,F] */
+    void* workspace, size_t workspace_bytes,
+    dmr_stream_t stream);
+
 /* ------------------------------------------------------------------------ */
 /* Tri renderer, backward.                                                   */
 /* Replaces CudaRasterizer::Rasterizer::backward                              */
@@ -528,6 +556,30 @@ int dmr_tet_alpha(int B, int W, int H, const void* image_buffer, float* out_alph
 size_t dmr_tet_background_grad_bytes(int B);
 int dmr_tet_background_grad(int B, int W, int H, const void* image_buffer, const float* dL_dcolor, float* dL_dbg,
                             void* workspace, size_t workspace_bytes, dmr_stream_t stream);
+
+/* Face visibility statistics of the tet renderer (no reference counterpart), from the state of a forward call     */
+/* (dmr_tet_forward_render(_views); call it after that call, with the same sizes, seed and inverses).  Per view b    */
+/* and face f: face_weights[b,f] (fp32) = sum, over the active pixels of view b at which f was composited, of       */
+/* expf(log_T) * opacity -- the factor the forward march multiplies the step's colour by -- and face_hits[b,f]      */
+/* (int32) = the number of those steps.  Inactive pixels (numerical failure, shown as the background) contribute    */
+/* nothing.  Summed over f, face_weights[b] is the sum of view b's alpha image (dmr_tet_alpha) up to fp32 rounding,  */
+/* except where a face of opacity >= 1 ends a ray (the march then sets T = 1e-5).  Every weight is the forward      */
+/* march's own bits: the face trail is walked forward, and the steps of a ray longer than the trail are marched     */
+/* again from its last recorded step.  Fixed-point format, outputs and workspace as                                 */
+/* dmr_tri_forward_render_face_weights (dmr_tet_face_weights_bytes(B, F) bytes, zeroed by the call); the state      */
+/* buffers are only read.                                                                                            */
+size_t dmr_tet_face_weights_bytes(int B, int F);
+int dmr_tet_face_weights(
+    int B, int P, int F, int T, int W, int H,
+    int ray_random_seed,
+    const float* inv_mv_mats, const float* inv_proj_mats,
+    const void* point_buffer, const void* face_buffer,
+    const void* tet_records,
+    const void* image_buffer,
+    float* face_weights,         /* [B,F] */
+    int* face_hits,              /* [B,F] */
+    void* workspace, size_t workspace_bytes,
+    dmr_stream_t stream);
 
 /* ------------------------------------------------------------------------ */
 /* Read-only views into the state buffers for the bit-exact parity checks    */
